@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N ...            # reference CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/<name>.npy
 
 Workload (default ``c3``, BASELINE.json configs[2], the configuration the metric's "fit ... at
 1/2/4/8 B200" is quoted on): RealNVP fit on synthetic N(0,1) rows, D=32, Cd=8, 16 coupling
@@ -204,7 +205,14 @@ def main():
     ap.add_argument("--no-c1-reference", action="store_true", help="skip the ~45 s reference-CPU-path run of configs[0]")
     ap.add_argument("--e2e-rows-per-gpu", type=int, default=0, help="rows per GPU of the end-to-end fit (default 10 M at N=1)")
     ap.add_argument("--c4-rows-per-gpu", type=int, default=125_000_000, help="configs[3]: 1 B rows over 8 GPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, weights, Adam moments) as DIR/<name>.npy (float32); "
+                         "the inputs depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         return run_reference(args, wl)
@@ -340,6 +348,18 @@ def main():
         dist.all_reduce(kern_ms, op=dist.ReduceOp.MAX)
     clocks = sampler.stop() if rank == 0 else None
     total_ms = float(ms)
+
+    # what a caller of the timed step holds after the last timed step: its loss, the updated weights (nf.parameters() order,
+    # reference layout) and the Adam moments; written now, before the measurements below run more steps on this engine.
+    # Replicas are identical under data parallelism, so rank 0 writes them.  c5, the largest workload, comes to 28 MB.
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        outputs = {"loss": losses[W + K - 1], "params": eng.flat, "adam_exp_avg": eng.exp_avg, "adam_exp_avg_sq": eng.exp_avg_sq}
+        outputs = {k: v.detach().cpu().numpy().astype(np.float32) for k, v in outputs.items()}
+        assert sum(v.nbytes for v in outputs.values()) <= 64 << 20
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in outputs.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
 
     # ---- the same step under SUSTAINED load: after ~0.3 s of back-to-back steps a B200 runs this kernel mix at its power
     # cap (sw_power_cap, ~1.78 GHz instead of 1.965): long fits (and the end-to-end figure below) see this rate, the K-step

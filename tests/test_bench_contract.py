@@ -1,8 +1,12 @@
-"""bench.py contract checks that need no GPU: the reference arm prints ONE JSON line with the agreed keys."""
+"""bench.py contract checks: the reference arm prints ONE JSON line with the agreed keys (no GPU needed); on a GPU, --steps sets
+the timed window and --dump-outputs writes what its last step computed."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -28,3 +32,27 @@ def test_flops_per_row_matches_the_survey_table():
     for name, (fwd, fit) in want.items():
         D, Cd, L, hidden, _, _ = WORKLOADS[name]
         assert flops_per_row(D, Cd, L, hidden[0]) == (fwd, fit), name
+
+
+@pytest.mark.gpu
+def test_steps_and_dump_outputs(tmp_path):
+    runs = {}
+    for k in (2, 3):
+        out = tmp_path / f"steps{k}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(k), "--warmup", "3", "--no-e2e",
+                            "--no-sustained", "--no-others", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines = [l for l in r.stdout.splitlines() if l.strip()]
+        assert len(lines) == 1, lines
+        d = json.loads(lines[0])
+        assert d["steps"] == k
+        arrays = {f.stem: np.load(f) for f in out.iterdir()}
+        assert set(arrays) == {"loss", "params", "adam_exp_avg", "adam_exp_avg_sq"}
+        assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in arrays.values())
+        assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+        assert float(arrays["loss"]) == d["config"]["final_loss"]
+        runs[k] = d, arrays
+    # the timed window holds exactly --steps steps, and the dumped weights are those after the last of them
+    assert runs[3][0]["gpu_launches"] * 2 == runs[2][0]["gpu_launches"] * 3
+    assert not np.array_equal(runs[2][1]["params"], runs[3][1]["params"])
