@@ -191,6 +191,25 @@ int rnvp_debug_set_trace(void* d_buf);
  * D[128,N] = A[128,K] * B[N,K]^T on device buffers; passes = 1 (plain TF32) or 3 (split, fp32-grade). */
 int rnvp_mma_selftest(const float* d_A, const float* d_B, float* d_D, int N, int K, int passes, void* stream);
 
+/* Bootstrap metrics (rnvp_metrics.cu).  A bootstrap draw is given as per-row counts (bincount of the resampled row
+ * indices), uint16, one row of counts per draw.  Precondition: within every draw, the counts of any 128 consecutive rows
+ * of X (or of Y, tiles starting at row 0 of each) sum to at most 46340; otherwise d_median and d_mmd are NaN.
+ *
+ * rnvp_mmd_draws replaces mmd_calc over resample(X), resample(Y) (probaforms/metrics/mmd.py:8-21, :55-61) for n_draws
+ * draws at once: d_median[b] = np.median of the pairwise distances of the drawn rows, d_mmd[b] = the RBF-kernel MMD with
+ * gamma = 1 / (2 median^2).  d_X [n][D], d_Y [m][D] fp32; d_counts [n_draws][n+m] (X's counts first).  No n^2 buffer:
+ * the workspace (rnvp_mmd_workspace_bytes) grows with n_draws only. */
+int64_t rnvp_mmd_workspace_bytes(int64_t n, int64_t m, int D, int n_draws);
+int rnvp_mmd_draws(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D,
+                   const uint16_t* d_counts /* [n_draws][n+m] */, int n_draws,
+                   double* d_median /* [n_draws] */, double* d_mmd /* [n_draws] */,
+                   void* d_workspace, int64_t workspace_bytes, void* stream);
+/* The moments behind X_boot.mean(axis=0) and np.cov(X_boot, rowvar=False) of frechet_distance
+ * (probaforms/metrics/fd.py:40-47): d_sum[b] = sum_i c_bi x_i, d_outer[b] = sum_i c_bi x_i x_i^T in fp64
+ * (fp32 products, fp64 combination; centre the rows first for an accurate covariance).  d_counts [n_draws][n]. */
+int rnvp_boot_moments(const float* d_X, int64_t n, int D, const uint16_t* d_counts /* [n_draws][n] */, int n_draws,
+                      double* d_sum /* [n_draws][D] */, double* d_outer /* [n_draws][D][D] */, void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

@@ -59,6 +59,11 @@ SIGNATURES = {
                                          C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]),
     "rnvp_host_copy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),
     "rnvp_mma_selftest": (C.c_int, [c_f32_p, c_f32_p, c_f32_p, C.c_int, C.c_int, C.c_int, c_stream]),
+    "rnvp_mmd_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int, C.c_int]),
+    "rnvp_mmd_draws": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_boot_moments": (C.c_int, [c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                    c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

@@ -334,6 +334,12 @@ extern "C" {
 
 int rnvp_version(void) { return 100; }
 const char* rnvp_last_error(void) { return g_err.c_str(); }
+}  // extern "C"
+
+// rnvp_last_error() for the entry points of other translation units (rnvp_metrics.cu)
+int rnvp_fail(int code, const char* msg) { return fail(code, msg); }
+
+extern "C" {
 
 int rnvp_desc_create(int D, int Cd, int L, int n_hidden, const int* hidden, int act, rnvp_desc** out) {
   if (!out) return fail(RNVP_EINVAL, "out is null");
