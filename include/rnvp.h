@@ -210,6 +210,28 @@ int rnvp_mmd_draws(const float* d_X, int64_t n, const float* d_Y, int64_t m, int
 int rnvp_boot_moments(const float* d_X, int64_t n, int D, const uint16_t* d_counts /* [n_draws][n] */, int n_draws,
                       double* d_sum /* [n_draws][D] */, double* d_outer /* [n_draws][D][D] */, void* stream);
 
+/* Per-feature bootstrap metrics (rnvp_metrics1d.cu).  d_sorted [D][n+m] fp64 is each feature's pooled column [x; y]
+ * sorted ascending, d_src [D][n+m] the row of each sorted position (rows < n are x's); d_counts [n_draws][n+m] uint16 as
+ * above (x's counts first).  Requires n + m < 2^31.
+ *
+ * rnvp_rank_draws replaces, for every draw b and feature d, _ks1d, _cvm1d, _roc1d, _anderson1d
+ * (probaforms/metrics/ks1d.py:11-30) and the histogram _kl1d, _js1d (div1d.py:6-44) over the drawn column:
+ * d_stats[b][d][] = { ks_2samp statistic, cramervonmises_2samp statistic (NaN when n or m is 1), ROC AUC folded as
+ * |auc - 0.5| + 0.5, anderson_ksamp's midrank A2kN (before the (A2kN - 1) / sigma standardisation), histogram KL,
+ * histogram JS (bins, eps = 1e-5 / bins), the number of distinct drawn values }.  Workspace: rnvp_rank_workspace_bytes. */
+#define RNVP_RANK_NSTAT 7
+int64_t rnvp_rank_workspace_bytes(int D, int n_draws, int bins);
+int rnvp_rank_draws(const double* d_sorted, const int32_t* d_src, int64_t n, int64_t m, int D,
+                    const uint16_t* d_counts /* [n_draws][n+m] */, int n_draws, int bins, double eps,
+                    double* d_stats /* [n_draws][D][RNVP_RANK_NSTAT] */, void* d_workspace, int64_t workspace_bytes,
+                    void* stream);
+/* The kernel sums behind compute_probs1d_kde (div1d.py:47-63): on the grid g = linspace(min, max, bins) of the drawn
+ * pooled column, d_sums[b][d][0][k] = sum_{x rows} c_i exp(-(g_k - x_i)^2 / (2 h_x^2)) and d_sums[b][d][1][k] the same
+ * over the y rows with h_y, in fp64.  Normalised to sum 1 they are the reference's p and q. */
+int rnvp_kde_draws(const double* d_sorted, const int32_t* d_src, int64_t n, int64_t m, int D,
+                   const uint16_t* d_counts /* [n_draws][n+m] */, int n_draws, int bins, double h_x, double h_y,
+                   double* d_sums /* [n_draws][D][2][bins] */, void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

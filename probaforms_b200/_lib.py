@@ -64,6 +64,11 @@ SIGNATURES = {
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_boot_moments": (C.c_int, [c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                     c_stream]),
+    "rnvp_rank_workspace_bytes": (C.c_int64, [C.c_int, C.c_int, C.c_int]),
+    "rnvp_rank_draws": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                  C.c_double, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_kde_draws": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                 C.c_double, C.c_double, C.c_void_p, c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

@@ -1,4 +1,4 @@
-"""Bootstrap two-sample metrics on the GPU, drop-in for ``probaforms.metrics``' multivariate pair.
+"""Bootstrap two-sample metrics on the GPU, drop-in for ``probaforms.metrics``.
 
     from probaforms_b200.metrics import maximum_mean_discrepancy, frechet_distance
     mu, sd = maximum_mean_discrepancy(X, Y, n_iters=100, standardize=False)
@@ -11,6 +11,9 @@ the reference's order (per iteration ``resample(X)`` then ``resample(Y)``, which
 vector; the kernels of ``rnvp_metrics.cu`` evaluate all draws from the counts without materialising the resampled
 rows or any (n+m)^2 distance matrix.  Inputs are 2-D numpy arrays or torch tensors; a CUDA tensor is used on its device.
 There is no CPU path.
+
+The eight per-feature metrics (kolmogorov_smirnov_1d, cramer_von_mises_1d, ...) live in ``onedim.py`` and share the draws
+and input handling above; ``__all__`` holds the ten names of ``probaforms.metrics``.
 """
 import ctypes as C
 
@@ -19,7 +22,18 @@ import torch
 
 from .. import _lib
 
-__all__ = ["maximum_mean_discrepancy", "frechet_distance"]
+__all__ = [
+    "frechet_distance",
+    "maximum_mean_discrepancy",
+    "kolmogorov_smirnov_1d",
+    "kullback_leibler_1d",
+    "jensen_shannon_1d",
+    "kullback_leibler_1d_kde",
+    "jensen_shannon_1d_kde",
+    "cramer_von_mises_1d",
+    "roc_auc_score_1d",
+    "anderson_darling_1d",
+]
 
 TILE = 128                # row tile of rnvp_mmd_draws: the counts of one tile must sum to at most MAX_TILE_COUNT
 MAX_TILE_COUNT = 46340
@@ -70,22 +84,34 @@ def _prepare(A, B, standardize):
     return A64, B64
 
 
-def _bootstrap_counts(n, m, n_iters):
+def _draw_counts(n, m, n_iters, check=None):
     """Per-draw row counts [n_iters][n+m] uint16 (X's rows first), drawn from the global np.random state exactly as
-    n_iters rounds of sklearn.utils.resample(X), resample(Y) consume it."""
+    n_iters rounds of sklearn.utils.resample(X), resample(Y) consume it.  check(c, size) may refuse a draw."""
     counts = np.empty((n_iters, n + m), dtype=np.uint16)
     for b in range(n_iters):
         cx = np.bincount(np.random.randint(0, n, size=n), minlength=n)
         cy = np.bincount(np.random.randint(0, m, size=m), minlength=m)
         for c, size in ((cx, n), (cy, m)):
-            pad = -size % TILE
-            tile_max = int(np.pad(c, (0, pad)).reshape(-1, TILE).sum(axis=1).max())
-            if tile_max > MAX_TILE_COUNT:
-                raise ValueError(f"a bootstrap draw puts {tile_max} rows into one {TILE}-row tile "
-                                 f"(at most {MAX_TILE_COUNT} are supported)")
+            if size > 65535 and int(c.max()) > 65535:
+                raise ValueError(f"a bootstrap draw takes one row {int(c.max())} times (at most 65535 are supported)")
+            if check is not None:
+                check(c, size)
         counts[b, :n] = cx
         counts[b, n:] = cy
     return counts
+
+
+def _check_tile_limit(c, size):
+    pad = -size % TILE
+    tile_max = int(np.pad(c, (0, pad)).reshape(-1, TILE).sum(axis=1).max())
+    if tile_max > MAX_TILE_COUNT:
+        raise ValueError(f"a bootstrap draw puts {tile_max} rows into one {TILE}-row tile "
+                         f"(at most {MAX_TILE_COUNT} are supported)")
+
+
+def _bootstrap_counts(n, m, n_iters):
+    """_draw_counts with the row-tile limit of rnvp_mmd_draws, which the MMD and FD paths share."""
+    return _draw_counts(n, m, n_iters, _check_tile_limit)
 
 
 def _stream(dev):
@@ -181,3 +207,8 @@ def frechet_distance(X_real, X_fake, n_iters=100, standardize=False):
     counts = _counts_to(_bootstrap_counts(n, F64.shape[0], n_iters), R64.device)
     frd = _fd_draws(R64, F64, counts[:, :n].contiguous(), counts[:, n:].contiguous()).cpu().numpy()
     return frd.mean(axis=0), frd.std(axis=0)
+
+
+# the per-feature metrics use the helpers above
+from .onedim import (anderson_darling_1d, cramer_von_mises_1d, jensen_shannon_1d, jensen_shannon_1d_kde,  # noqa: E402
+                     kolmogorov_smirnov_1d, kullback_leibler_1d, kullback_leibler_1d_kde, roc_auc_score_1d)
