@@ -67,9 +67,9 @@ int64_t rnvp_workspace_bytes(const rnvp_desc* d, int64_t N);
 /* offsets[2*k], offsets[2*k+1] = (float offset, numel) of the k-th tensor of nf.parameters();
  * n = 4*(n_hidden+1)*L entries pairs.  Returns the number of tensors. */
 int rnvp_param_tensors(const rnvp_desc* d, int64_t* offsets, int max_tensors);
-/* plan introspection: mode 0 forward, 1 inverse, 2 fused forward+backward, 3 backward-only sweep (used after the
- * tcgen05 forward), 4 = "is the whole fit step on the tensor cores" (kernel_family 2 iff yes); rows per CTA tile, shared
- * memory, ops per tile of the FP32 program, kernel family (0 tile, 1 small-flow, 2 tcgen05) */
+/* plan introspection: mode 0 forward, 1 inverse, 2 fused forward+backward, 4 = "is the whole fit step on the tensor
+ * cores" (kernel_family 2 iff yes; mode 3 is not used and gives RNVP_EINVAL); rows per CTA tile, shared memory, ops per
+ * tile of the FP32 program, kernel family (0 tile, 1 small-flow, 2 tcgen05) */
 int rnvp_plan_info(const rnvp_desc* d, int mode, int* tile_rows, int* smem_bytes, int* n_ops, int* kernel_family);
 
 /* flat (reference layout) -> packed; run after every parameter update */
@@ -104,8 +104,8 @@ int rnvp_sample(const rnvp_desc* d, const float* d_packed, const float* d_C, int
  * loss = -nf.log_prob(X, C), realnvp.py:246-250, is scale = -1/N).  Weight gradients are ACCUMULATED into
  * d_gpacked (caller zeroes it), sum_rows logp is accumulated into d_logp_sum (1 float, may be NULL), per-row
  * logp optionally written.  Kernel families: small flows and the generic FP32 tile kernel recompute the
- * hidden activations in the backward sweep (nothing but x_T per layer is kept); the tensor-core fit paths
- * (D = 32 flows with H <= 128; D = 64 / 128 flows with H a multiple of 128) hand h, u and delta2 of every
+ * hidden activations in the backward sweep (nothing but x_T per layer is kept); the tensor-core fit path
+ * (tcgen05-eligible flows with D <= 64, or with H a multiple of 128) hands h, u and delta2 of every
  * (layer, row) to the weight-gradient sweep through activation records in d_workspace (see
  * rnvp_wgrad_sweep), which is why rnvp_workspace_bytes grows with N there. */
 int rnvp_backward(const rnvp_desc* d, const float* d_packed, const float* d_X, const float* d_C,
@@ -147,15 +147,17 @@ int rnvp_fit_epoch(const rnvp_desc* d, float* d_flat, float* d_packed, float* d_
  * h [2][H] (nn_t | nn_s) | u = [x_K, c, 0..] (ceil8(D/2+Cd)) | delta2 [2][D/2],
  * stored in blocks of 32 rows as d_records[L][Npad/32][rec/4][32][4]: float4 column group q of row r of a block sits
  * in slot (r ^ (q & 7)).  Npad is a multiple of 32; padding rows must hold zeros in delta1 / delta2.
- * Flows whose fit step runs on the tensor cores: D = 32 with H <= 128 (multiple of 16), D = 64 / 128 with H a
+ * Flows whose fit step runs on the tensor cores: tcgen05-eligible flows (see rnvp_set_path) with D <= 64, or with H a
  * multiple of 128 (one 128-lane block of hidden units per CTA, rnvp_wgrad_tc.cu). */
 int rnvp_wgrad_record_floats(const rnvp_desc* d);
 int rnvp_wgrad_sweep(const rnvp_desc* d, const float* d_packed, int64_t Npad, const float* d_records, float* d_gpacked,
                      void* stream);
 
 /* Kernel-family selection for rnvp_forward / rnvp_inverse: 0 = auto (tcgen05 TF32x3 kernels where the shape is
- * eligible -- one hidden layer, D/2 in {16,32} --, else the small-flow or FP32 tile kernels), 1 = FP32-FMA kernels
- * only, 2 = same as auto.  rnvp_plan_info reports the family chosen (0 tile, 1 small-flow, 2 tcgen05). */
+ * eligible -- one hidden layer, 8 < D <= 128, Cd <= 16 (D <= 64) or 32, H a multiple of 32, and for D <= 32 the
+ * whole-layer weight images within the shared memory of one CTA --, else the small-flow or FP32 tile kernels),
+ * 1 = FP32-FMA kernels only, 2 = same as auto.  rnvp_plan_info reports the family chosen (0 tile, 1 small-flow,
+ * 2 tcgen05). */
 int rnvp_set_path(rnvp_desc* d, int path);
 
 /* Host-side row order of one epoch, produced incrementally (replaces the per-epoch DataLoader(shuffle=True) of
@@ -183,8 +185,9 @@ int rnvp_host_gather_xc(const void* src_x, int x_is_f64, int64_t width_x, const 
                            const int64_t* idx, int64_t row0, int64_t n, float* dst_x, float* dst_c, int threads);
 int rnvp_host_copy(void* dst, const void* src, int64_t bytes, int threads);
 
-/* Development aid: when d_buf (device, 4*2048*2 int64) is non-null, CTA 0 of the tcgen05 fit kernel logs (tag, clock64)
- * pairs of its backward sweep (tile-0 epilogue, tile-1 epilogue, and their two MMA issuers); tools/trace_mma.py prints the timeline. */
+/* Development aid: when d_buf (device, >= 40 int64) is non-null and the library was built with -DRNVP_WG_TRACE, every
+ * role of CTA 0 of the tcgen05 weight-gradient sweep writes the cycles it spent in each of its mbarrier waits
+ * (d_buf[role * 8 + wait site], see rnvp_wgrad_tc.cu; tools/trace_wgrad.py prints them).  Other builds ignore it. */
 int rnvp_debug_set_trace(void* d_buf);
 
 /* Tensor-core primitive self-test (tcgen05.mma kind::tf32, A in TMEM, B in shared memory):

@@ -18,7 +18,7 @@
 #include <cstdlib>
 #include "rnvp_planner.h"
 #include "rnvp_small.h"
-#include "rnvp_mma.h"
+#include "rnvp_wide.h"
 #include "rnvp_wgrad.h"
 
 cudaError_t rnvp_launch_tile(int mode, int TR, const RnvpKArgs& a, int grid, size_t smem_bytes, cudaStream_t stream);
@@ -28,10 +28,8 @@ cudaError_t rnvp_launch_small(int NE, int NC, int act, int mode, const RnvpSmall
 int rnvp_small_rows_per_block();
 int rnvp_small_fit_rows_per_block();
 int rnvp_small_fit_max_layers();
-cudaError_t rnvp_launch_mma(int DH, int act, int mode, const RnvpMmaArgs& a, int grid, size_t smem, cudaStream_t st);
-size_t rnvp_mma_smem_bytes(int w1_floats, int w2_floats, int w1t_floats);
 cudaError_t rnvp_launch_wgrad_tc(int NU, int TP, const RnvpWgradTcArgs& a, int grid, cudaStream_t st);
-cudaError_t rnvp_launch_wide(int DH, int act, int mode, const RnvpMmaArgs& a, int grid, cudaStream_t st);
+cudaError_t rnvp_launch_wide(int DH, int act, int mode, const RnvpWideArgs& a, int grid, cudaStream_t st);
 int rnvp_wide_ctas_per_sm(int DH);
 cudaError_t rnvp_launch_mma_selftest(const float* A, const float* B, float* D, int N, int K, int passes, cudaStream_t st);
 
@@ -268,15 +266,13 @@ int run_small(rnvp_desc* d, int mode, int l0, int l1, const float* packed, const
   return 0;
 }
 
-long long* g_mma_trace = nullptr;   // development aid, see rnvp_debug_set_trace
+long long* g_wg_trace = nullptr;    // development aid: wait accounting of -DRNVP_WG_TRACE builds, see rnvp_debug_set_trace
 bool use_mma(const rnvp_desc* d) { return d->mma_ok && d->path != 1; }
-// fit step entirely on the tensor-core path (tcgen05 forward + backward sweeps, mma.sync weight-gradient sweep)
+// fit step entirely on the tensor-core path (tcgen05 forward + backward sweeps, tcgen05 weight-gradient sweep)
 bool use_mma_bwd(const rnvp_desc* d) { return use_mma(d) && d->m_wt_floats > 0; }
-// forward sweep of a fit step on the tensor cores (stash for the FP32 backward sweep): resident-image kernels only
-bool use_mma_fwd_stash(const rnvp_desc* d) { return use_mma(d) && !d->m_stream; }
-// rows covered by the record / stash arrays of a tensor-core fit step: whole row tiles of the sweep kernel (pairs of 128-row
-// tiles in rnvp_mma.cu, single tiles in rnvp_wide.cu), so that the weight-gradient sweep never reads an unwritten record
-int64_t fit_npad(const rnvp_desc* d, int64_t N) { return d->m_netseq ? (N + 127) / 128 * 128 : (N + 255) / 256 * 256; }
+// rows covered by the record / stash arrays of a tensor-core fit step: whole 128-row tiles of the sweep kernel, so that
+// the weight-gradient sweep never reads an unwritten record
+int64_t fit_npad(int64_t N) { return (N + 127) / 128 * 128; }
 // record stride of the activation records exchanged between the backward sweep and the weight-gradient sweep
 int wgrad_rec_floats(const rnvp_desc* d) {
   const int K1P = (d->mDH + d->Cd + 7) & ~7;
@@ -289,7 +285,7 @@ int run_mma(rnvp_desc* d, int mode, int l0, int l1, const float* packed, const f
             unsigned long long seed = 0, long long row_offset = 0) {
   if (l0 < 0 || l1 > d->L || l0 >= l1) return fail(RNVP_EINVAL, "bad layer range");
   if (N <= 0) return 0;
-  RnvpMmaArgs a;
+  RnvpWideArgs a;
   a.wimg = packed + d->mma_off;
   a.X = X; a.C = C; a.idx = idx; a.N = N;
   a.out_x = out_x; a.out_logdet = out_logdet; a.out_logp = out_logp;
@@ -297,33 +293,17 @@ int run_mma(rnvp_desc* d, int mode, int l0, int l1, const float* packed, const f
   a.layer_floats = d->m_layer_floats; a.w1_floats = d->m_w1_floats; a.w2_floats = d->m_w2_floats;
   a.stash = stash; a.loss_sum = loss_sum; a.L_total = d->L;
   a.do_bwd = records != nullptr; a.scale = scale; a.records = records; a.rec = 0; a.Npad = 0;
-  a.rec_swz = 7;
   a.wt_floats = records ? d->m_wt_floats : 0;
-  a.trace = g_mma_trace;
   a.seed = seed; a.row_offset = row_offset; a.Dreal = d->D;
-  // wide kernels (one tile per CTA, two threads per row, chunk images streamed): every D >= 64 flow -- measured on c4 they are
-  // 22 % faster than the resident-image kernel (129 vs 106 M rows/s log-prob) although the images would fit; RNVP_RESIDENT=1
-  // (development knob) keeps the resident kernel.  Only the hybrid fit (tensor-core forward + FP32 backward sweep, H not a
-  // multiple of 128) still needs the resident kernel's row-major stash.
-  static const bool keep_resident = [] { const char* e = getenv("RNVP_RESIDENT"); return e && atoi(e) != 0; }();
-  if (d->m_stream || (d->m_netseq && !(mode == 2 && !records) && !(keep_resident && mode != 2))) {
-    if (mode == 2 && !records) return fail(RNVP_ESHAPE, "streamed tcgen05 kernels run the fit step with their own backward sweep only");
-    const long long tiles = (N + 127) / 128;
-    if (tiles > 0x7fffffffLL) return fail(RNVP_EINVAL, "too many rows for one launch");
-    a.n_pairs = (int)tiles;                      // rnvp_wide.cu walks single 128-row tiles
-    if (records) { a.rec = wgrad_rec_floats(d); a.Npad = fit_npad(d, N); }
-    const long long ctas = (long long)d->num_sms * rnvp_wide_ctas_per_sm(d->mDH);   // DH <= 32: two CTAs per SM
-    cudaError_t e = rnvp_launch_wide(d->mDH, d->act, mode, a, (int)std::min<long long>(tiles, ctas), stream);
-    if (e != cudaSuccess) return cuda_fail(e, "tcgen05 streamed kernel launch");
-    return 0;
-  }
-  const long long pairs = (N + 255) / 256;
-  if (pairs > 0x7fffffffLL) return fail(RNVP_EINVAL, "too many rows for one launch");
-  a.n_pairs = (int)pairs;
-  if (records) { a.rec = wgrad_rec_floats(d); a.Npad = pairs * 256; }
-  const int grid = (int)std::min<long long>(pairs, d->num_sms);
-  cudaError_t e = rnvp_launch_mma(d->mDH, d->act, mode, a, grid, rnvp_mma_smem_bytes(d->m_w1_floats, d->m_w2_floats, a.wt_floats), stream);
-  if (e != cudaSuccess) return cuda_fail(e, "tcgen05 kernel launch");
+  // one 128-row tile per CTA, two threads per row, weight images streamed per chunk step (rnvp_wide.cu)
+  if (mode == 2 && !records) return fail(RNVP_ESHAPE, "tcgen05 kernels run the fit step with their own backward sweep only");
+  const long long tiles = (N + 127) / 128;
+  if (tiles > 0x7fffffffLL) return fail(RNVP_EINVAL, "too many rows for one launch");
+  a.n_tiles = (int)tiles;
+  if (records) { a.rec = wgrad_rec_floats(d); a.Npad = fit_npad(N); }
+  const long long ctas = (long long)d->num_sms * rnvp_wide_ctas_per_sm(d->mDH);   // DH <= 32: two CTAs per SM
+  cudaError_t e = rnvp_launch_wide(d->mDH, d->act, mode, a, (int)std::min<long long>(tiles, ctas), stream);
+  if (e != cudaSuccess) return cuda_fail(e, "tcgen05 streamed kernel launch");
   return 0;
 }
 
@@ -366,9 +346,6 @@ int rnvp_desc_create(int D, int Cd, int L, int n_hidden, const int* hidden, int 
   d->device = dev;
   d->num_sms = prop.multiProcessorCount;
   d->max_smem = (int)prop.sharedMemPerBlockOptin;
-  // D = 32 flows run on the wide kernels by default (two CTAs per SM: measured +7.6 % on the c3 fit step, +6 % sample, -5 % log-prob
-  // against the resident-image kernel of rnvp_mma.cu, which RNVP_WIDE16=0 selects for comparison)
-  { const char* w = getenv("RNVP_WIDE16"); d->m_wide16 = !(w && atoi(w) == 0); }
   build_layout(d);
   if (d->P >= 0x7fffffffLL) { delete d; return fail(RNVP_ESHAPE, "flow too large (>= 2^31 parameters)"); }
   std::vector<int> p2f, f2p, f2p2;
@@ -426,7 +403,7 @@ int rnvp_desc_create(int D, int Cd, int L, int n_hidden, const int* hidden, int 
   // (shapes the tile planner cannot fit are reported when such a program is actually needed)
   {
     Program* p = nullptr;
-    for (int mode = 0; mode <= 3; ++mode) get_program(d, mode, 0, d->L, &p);
+    for (int mode = 0; mode <= 2; ++mode) get_program(d, mode, 0, d->L, &p);
     g_err.clear();
   }
   *out = d;
@@ -458,10 +435,9 @@ int64_t rnvp_workspace_bytes(const rnvp_desc* dc, int64_t N) {
   if (!d) return -1;
   if (use_small_fit(d)) return 16;                      // the row-per-thread fit kernel keeps its stash in local memory
   if (use_mma_bwd(d)) {
-    const int64_t n = std::max<int64_t>(N, 1), npad = fit_npad(d, n);
+    const int64_t npad = fit_npad(std::max<int64_t>(N, 1));
     return (npad * d->L * 2 * d->mDH + (int64_t)d->L * npad * wgrad_rec_floats(d)) * 4;
   }
-  if (use_mma_fwd_stash(d)) return std::max<int64_t>(N, 1) * (d->D + (int64_t)d->L * 2 * d->mDH) * 4;
   Program* p = nullptr;
   if (get_program(d, 2, 0, d->L, &p)) return -1;
   return (int64_t)p->stash_per_cta * 4 * d->num_sms * p->occupancy;
@@ -486,7 +462,7 @@ int rnvp_param_tensors(const rnvp_desc* d, int64_t* offsets, int max_tensors) {
 int rnvp_plan_info(const rnvp_desc* dc, int mode, int* tile_rows, int* smem_bytes, int* n_ops, int* kernel_family) {
   rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
-  if (mode < 0 || mode > 4) return fail(RNVP_EINVAL, "mode must be 0..4");
+  if (mode < 0 || mode == 3 || mode > 4) return fail(RNVP_EINVAL, "mode must be 0, 1, 2 or 4");
   Program* p = nullptr;
   int rc = get_program(d, mode == 4 ? 2 : mode, 0, d->L, &p);
   if (rc) return rc;
@@ -497,7 +473,7 @@ int rnvp_plan_info(const rnvp_desc* dc, int mode, int* tile_rows, int* smem_byte
     if (kernel_family) *kernel_family = use_mma_bwd(d) ? 2 : 0;
     return 0;
   }
-  if (kernel_family) *kernel_family = (mode >= 2 ? (use_mma_fwd_stash(d) || use_mma_bwd(d)) : use_mma(d)) ? 2 : (((mode < 2 && d->small_ok) || (mode == 2 && use_small_fit(d))) ? 1 : 0);
+  if (kernel_family) *kernel_family = (mode == 2 ? use_mma_bwd(d) : use_mma(d)) ? 2 : (((mode < 2 && d->small_ok) || (mode == 2 && use_small_fit(d))) ? 1 : 0);
   return 0;
 }
 
@@ -595,7 +571,7 @@ int rnvp_backward(const rnvp_desc* dc, const float* d_packed, const float* d_X, 
                      (cudaStream_t)stream, d_gpacked, d_logp_sum, scale);
   if (use_mma_bwd(d) && N > 0) {
     // forward + backward sweeps in one tcgen05 launch (per-layer records to the workspace), then the weight-gradient sweep
-    const int64_t npad = fit_npad(d, N);
+    const int64_t npad = fit_npad(N);
     const int64_t stash_f = npad * d->L * 2 * d->mDH, rec_f = (int64_t)d->L * npad * wgrad_rec_floats(d);   // both blocked by 32 rows
     if (!d_workspace || workspace_bytes < (stash_f + rec_f) * 4)
       return fail(RNVP_EINVAL, "rnvp_backward: workspace too small (see rnvp_workspace_bytes)");
@@ -605,20 +581,6 @@ int rnvp_backward(const rnvp_desc* dc, const float* d_packed, const float* d_X, 
                      (cudaStream_t)stream, stash, d_logp_sum, records, scale);
     if (rc) return rc;
     return rnvp_wgrad_sweep(d, d_packed, npad, records, d_gpacked, stream);
-  }
-  if (use_mma_fwd_stash(d) && N > 0) {
-    // forward sweep on the tensor cores (z, per-layer x_T and s to the workspace), backward sweep on the FP32 tile kernel
-    const int64_t need = (int64_t)N * (d->D + (int64_t)d->L * 2 * d->mDH) * 4;
-    if (!d_workspace || workspace_bytes < need)
-      return fail(RNVP_EINVAL, "rnvp_backward: workspace too small (see rnvp_workspace_bytes)");
-    float* z = (float*)d_workspace;
-    float* stash = z + (size_t)N * d->D;
-    int rc = run_mma(d, 2, 0, d->L, d_packed, d_X, d_C, (const long long*)d_idx, N, z, nullptr, d_logp,
-                     (cudaStream_t)stream, stash, d_logp_sum);
-    if (rc) return rc;
-    a.X = z;
-    a.gstash = stash; a.gstash_row = d->L * 2 * d->mDH; a.gstash_half = d->mDH;
-    return run_tile(d, 3, 0, d->L, a, nullptr, 0, (cudaStream_t)stream);
   }
   a.X = d_X;
   a.out_logp = d_logp; a.loss_sum = d_logp_sum;
@@ -696,8 +658,8 @@ int rnvp_wgrad_sweep(const rnvp_desc* dc, const float* d_packed, int64_t Npad, c
   rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
   if (!d->mma_ok || d->m_wt_floats == 0)
-    return fail(RNVP_ESHAPE, "rnvp_wgrad_sweep: needs a flow whose fit step runs on the tensor cores (D = 32 with H <= 128, or a "
-                             "wide flow with H a multiple of 128)");
+    return fail(RNVP_ESHAPE, "rnvp_wgrad_sweep: needs a flow whose fit step runs on the tensor cores (a tcgen05 flow with D <= 64, "
+                             "or with H a multiple of 128)");
   if (!d_records || !d_gpacked || !d_packed) return fail(RNVP_EINVAL, "rnvp_wgrad_sweep: null buffer");
   if (Npad <= 0 || Npad % 32) return fail(RNVP_EINVAL, "rnvp_wgrad_sweep: Npad must be a positive multiple of 32");
   const int K1P = (d->mDH + d->Cd + 7) & ~7, TP = d->mDH;
@@ -721,7 +683,7 @@ int rnvp_wgrad_sweep(const rnvp_desc* dc, const float* d_packed, int64_t Npad, c
       }
       a.n_slices = best_s;
     }
-    a.gpacked = d_gpacked; a.packed = d_packed; a.act = d->act; a.layers = d->d_wg; a.trace = g_mma_trace;
+    a.gpacked = d_gpacked; a.packed = d_packed; a.act = d->act; a.layers = d->d_wg; a.trace = g_wg_trace;
     { const char* o = getenv("RNVP_WG_ONE_ISSUER"); a.one_issuer = (o && atoi(o)) ? 1 : 0; }
     { const char* o = getenv("RNVP_WG_SLICES"); if (o && atoi(o) > 0) a.n_slices = (int)std::min<long long>(Npad / 32, atoi(o)); }
     const int NU = TP == 16 ? 32 : (TP == 32 ? 48 : 96);           // dW1 tile columns of the three kernel variants (>= K1P8)
@@ -730,7 +692,7 @@ int rnvp_wgrad_sweep(const rnvp_desc* dc, const float* d_packed, int64_t Npad, c
   }
 }
 
-int rnvp_debug_set_trace(void* d_buf) { g_mma_trace = (long long*)d_buf; return 0; }
+int rnvp_debug_set_trace(void* d_buf) { g_wg_trace = (long long*)d_buf; return 0; }
 
 int rnvp_set_path(rnvp_desc* d, int path) {
   if (check_desc(d)) return RNVP_EINVAL;

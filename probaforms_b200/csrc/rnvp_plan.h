@@ -22,7 +22,6 @@ enum RnvpOpKind {
   OP_COUPLE_G = 4,    // x_T = (y_T-t)*exp(-s)                 (realnvp.py:128)
   OP_STORE_F = 5,     // z, logdet, logp = logdet + N(0,I).log_prob(z)  (nflow.py:115)
   OP_STORE_G = 6,     // x
-  OP_SEED_B = 7,      // loss partial + g_z, g_logdet seeds for the backward sweep
   OP_COUPLE_B = 8,    // d(coupling): delta2_t, delta2_s, g_x_T
   OP_WGRAD = 9,       // dW, db of one Linear (both nets) -> red.global.add into packed grads
   OP_DGRAD = 10,      // delta_{q-1} = (delta_q W_q) * act'(h_{q-1})  /  du for q = 0
@@ -36,9 +35,7 @@ enum RnvpOpFlags {
   F_FIRST = 8,        // DGRAD: first chunk of the reduction
   F_LAST = 16,        // DGRAD: last chunk of the reduction
   F_TO_GU = 32,       // DGRAD: q = 0, result is du (input gradient), no act'
-  F_NET_S_ONLY = 64,  // LINEAR: only nn_s needs this output (t is unused in the backward sweep)
-  F_GSTASH = 128      // backward-only program: x_T and s come from the row-major global stash written by the
-                      // tcgen05 forward kernel ([row][layer][x_T(|T|max) | s(|T|max)]); LOAD: X rows are not gathered
+  F_NET_S_ONLY = 64   // LINEAR: only nn_s needs this output (t is unused in the backward sweep)
 };
 
 struct RnvpOp {
@@ -95,9 +92,9 @@ struct RnvpKArgs {
   float* loss_sum;                    // sum over rows of logp (backward), atomically accumulated
   float* stash;                       // per-CTA x_T stash, gridDim.x * stash_per_cta floats
   int stash_per_cta;
-  const float* gstash;                // backward-only program: global stash of the forward kernel
-  int gstash_row, gstash_half;        // floats per row (L*2*half) and per half (|T|max)
-  float scale;                        // backward: d(out)/d(logp_row); g_logdet = scale, g_z = -z*scale
+  // 16-byte aligned: the tile kernels' register allocation depends on where the fields from here on sit (ptxas -v:
+  // rnvp_tile_kernel<2, 0> needs 128 registers with this alignment and 164 without)
+  alignas(16) float scale;            // backward: d(out)/d(logp_row); g_logdet = scale, g_z = -z*scale
   int D, Cd;
   // inverse program with X == nullptr: latent rows drawn in-kernel (rnvp_philox.cuh), keyed on row_offset + row
   unsigned long long seed;

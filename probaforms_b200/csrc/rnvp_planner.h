@@ -48,14 +48,10 @@ struct FlowGeom {
   int sNE = 0, sNC = 0, srec = 0, snet = 0, small_floats = 0;
   int64_t small_off = 0;
   int64_t packed_gather = 0;     // floats covered by the plain gather map p2f (tile + small layouts)
-  // tcgen05 layout (rnvp_mma.cu): one hidden layer, even D with D/2 in {16,32}; TF32 hi/lo images of the
-  // weights in the no-swizzle K-major core-matrix layout, per layer [W1 chunks | W2 chunks | b2]
+  // tcgen05 layout (rnvp_wide.cu): one hidden layer, 8 < D <= 128; TF32 hi/lo images of the weights in the no-swizzle
+  // K-major core-matrix layout, per layer [W1 chunks | W2 chunks | b2 | W2T chunks | W1T chunks]
   bool mma_ok = false;
   int mDH = 0, mCDMAX = 0, mCU = 0, mK1P = 0, mNTP = 0;
-  bool m_netseq = false;
-  bool m_wide16 = false;   // D = 32 flows on the wide kernels too (two CTAs per SM); set by rnvp_desc_create (RNVP_WIDE16=0 turns it off)
-  bool m_padded = false;   // D != 2 * mDH: padded feature slots (wide kernels only)
-  bool m_stream = false;   // weight images streamed per chunk step (rnvp_wide.cu) instead of resident per layer
   int m_w1_floats = 0, m_w2_floats = 0, m_b2_floats = 0, m_layer_floats = 0;
   int m_wt_floats = 0;   // transposed images for the backward sweep (W2T then W1T, m_wt_floats each), 0 if not built
   int64_t mma_off = 0, mma_floats = 0;
@@ -117,34 +113,24 @@ inline void build_layout(FlowGeom* d) {
   d->packed_gather = d->packed;
   // tcgen05 layout
   d->mma_ok = false;
-  d->m_stream = false;
-  d->m_padded = false;
   if (nh == 1 && D > 8 && D <= 128) {
     // the kernels are built for DH = D/2 in {16, 32, 64}; any other D (odd ones included) runs as the next larger shape
     // with zero-weight padding features: |K|, |T| <= DH, the images hold zeros beyond them, the row loads are guarded
     const int DH = D <= 32 ? 16 : (D <= 64 ? 32 : 64), H = d->hidden[0];
-    d->m_padded = D != 2 * DH;
     const int CDMAX = DH == 16 ? 16 : (DH == 32 ? 16 : 32), CU = 32;
-    const bool netseq = DH >= 32 || d->m_wide16 || d->m_padded || Cd > 8;   // (the resident D = 32 kernel: exact shape, Cd <= 8 only)               // nn_t chunks before nn_s chunks (rnvp_mma.cu / rnvp_wide.cu)
     const int K1P = (DH + Cd + 1 + 7) & ~7, NTP = (DH + 15) & ~15;
-    const int tile_cols = netseq ? 2 * K1P + 2 * CU + 2 * NTP : 2 * K1P + 4 * CU + 4 * NTP;
     const int64_t w1 = (int64_t)4 * H * K1P, w2 = (int64_t)4 * NTP * H;
-    // whole-layer images resident in shared memory (rnvp_mma.cu), or streamed per chunk step (rnvp_wide.cu: D = 64 / 128
-    // flows whose images are too large, e.g. BASELINE configs[4] with 1.36 MB per layer)
-    const bool resident = DH <= 32 && tile_cols <= 256 && (w1 + w2 + 32 * NTP) * 4 + 2048 <= d->max_smem;
-    const bool streamed = !resident && DH >= 32;
-    if (Cd <= CDMAX && H % CU == 0 && H >= CU && (resident || streamed)) {
+    // The weight images are streamed per chunk step, so no shape needs them to fit shared memory.  DH = 16 flows still run
+    // on the tensor cores only where the whole-layer images would fit: that rule decides which flows take the tcgen05 path.
+    const bool fits = DH >= 32 || (w1 + w2 + 32 * NTP) * 4 + 2048 <= d->max_smem;
+    if (Cd <= CDMAX && H % CU == 0 && H >= CU && fits) {
       d->mma_ok = true;
-      d->m_stream = streamed;
-      d->mDH = DH; d->mCDMAX = CDMAX; d->mCU = CU; d->mK1P = K1P; d->mNTP = NTP; d->m_netseq = netseq;
+      d->mDH = DH; d->mCDMAX = CDMAX; d->mCU = CU; d->mK1P = K1P; d->mNTP = NTP;
       d->m_b2_floats = 32 * NTP;                               // 2 nets x [hi | lo] x [NTP x 8]
       d->m_w1_floats = (int)w1; d->m_w2_floats = (int)w2 + d->m_b2_floats;  // b2 images ride with the W2 copy
-      // backward sweep (concurrent-net kernels only): K-major images of the transposed operands, per half-chunk of 16
-      // units and net a [16 x 16] block [hi | lo]: W2T (units x transformed features) and W1T (x_K columns x units)
-      // (resident kernels).  Streamed kernels: per chunk step (net, chunk of CU units) a W2T block [hi | lo] of [CU x DH] and
-      // a W1T block [hi | lo] of [NTP x CU]; the tcgen05 weight-gradient sweep needs whole 128-unit lane blocks per net
-      // (D = 64 flows with resident images, e.g. c4, run their FIT step on the streamed kernels too: same chunk images)
-      d->m_wt_floats = (!netseq && H % 16 == 0 && H <= 128) ? 4 * H * 16 : ((netseq && (DH < 64 || H % 128 == 0)) ? 4 * H * NTP : 0);
+      // backward sweep: per chunk step (net, chunk of CU units) a W2T block [hi | lo] of [CU x DH] and a W1T block [hi | lo]
+      // of [NTP x CU]; for DH = 64 the tcgen05 weight-gradient sweep needs whole 128-unit lane blocks per net
+      d->m_wt_floats = (DH < 64 || H % 128 == 0) ? 4 * H * NTP : 0;
       d->m_layer_floats = d->m_w1_floats + d->m_w2_floats + 2 * d->m_wt_floats;
       d->mma_off = (d->packed + 31) & ~(int64_t)31;            // 128-byte aligned for the bulk copies
       d->mma_floats = (int64_t)d->L * d->m_layer_floats;
@@ -173,15 +159,13 @@ inline void build_mma_map(const FlowGeom* d, std::vector<int>& m2f) {
     const LinearGeom& g0 = lg.lin[0];
     const LinearGeom& g1 = lg.lin[1];
     const int64_t base = (int64_t)i * d->m_layer_floats;
-    // W1 image: one block [hi | lo] per chunk step.  Concurrent nets: block c has rows 0..CU-1 = t units and
-    // CU..2CU-1 = s units of chunk c.  NETSEQ: blocks 0..NC-1 are the t chunks, NC..2NC-1 the s chunks (CU rows each).
-    const int rows1 = d->m_netseq ? CU : 2 * CU, nblk1 = d->m_netseq ? 2 * NC : NC;
-    for (int cc = 0; cc < nblk1; ++cc)
+    // W1 image: one block [hi | lo] of CU rows per chunk step; blocks 0..NC-1 are the nn_t chunks, NC..2NC-1 the nn_s chunks
+    for (int cc = 0; cc < 2 * NC; ++cc)
       for (int part = 0; part < 2; ++part) {
-        const int64_t blk = base + ((int64_t)cc * 2 + part) * (rows1 * K1P);
-        for (int n = 0; n < rows1; ++n) {
-          const int net = d->m_netseq ? cc / NC : n / CU;
-          const int unit = (d->m_netseq ? cc % NC : cc) * CU + n % CU;
+        const int64_t blk = base + ((int64_t)cc * 2 + part) * (CU * K1P);
+        for (int n = 0; n < CU; ++n) {
+          const int net = cc / NC;
+          const int unit = (cc % NC) * CU + n;
           for (int k = 0; k < K1P; ++k) {
             int64_t f = -1;
             if (k < DH) { const int xk = lg.par == 0 ? 2 * k + 1 : 2 * k; if (xk < D) f = g0.flat_w[net] + (int64_t)unit * (D + Cd) + xk; }
@@ -214,8 +198,8 @@ inline void build_mma_map(const FlowGeom* d, std::vector<int>& m2f) {
           if (ft >= D) continue;
           m2f[base3 + (net * 2 + part) * (NTP * 8) + mma_tiled_off(r, (DH + Cd) & 7, 8)] = (int)(4 * (g1.flat_b[net] + ft) + part);
         }
-    if (d->m_wt_floats && d->m_netseq) {
-      // streamed backward images, indexed by chunk step cc = net * NC + c
+    if (d->m_wt_floats) {
+      // backward images, indexed by chunk step cc = net * NC + c
       const int64_t base4 = base2 + d->m_w2_floats, base5 = base4 + d->m_wt_floats;
       for (int net = 0; net < 2; ++net)
         for (int c = 0; c < NC; ++c)
@@ -230,21 +214,6 @@ inline void build_mma_map(const FlowGeom* d, std::vector<int>& m2f) {
                 const int xk = lg.par == 0 ? 2 * e + 1 : 2 * e;            // conditioning feature e
                 if (ft < D) m2f[o2 + mma_tiled_off(un, e, NTP)] = (int)(4 * (g1.flat_w[net] + (int64_t)ft * H + unit) + part);
                 if (xk < D) m2f[o1 + mma_tiled_off(e, un, CU)] = (int)(4 * (g0.flat_w[net] + (int64_t)unit * (D + Cd) + xk) + part);
-              }
-          }
-    } else if (d->m_wt_floats) {
-      const int64_t base4 = base2 + d->m_w2_floats, base5 = base4 + d->m_wt_floats;
-      for (int hc = 0; hc < H / 16; ++hc)
-        for (int net = 0; net < 2; ++net)
-          for (int part = 0; part < 2; ++part) {
-            const int64_t off = (((int64_t)hc * 2 + net) * 2 + part) * 256;
-            for (int un = 0; un < 16; ++un)
-              for (int e = 0; e < DH; ++e) {
-                const int unit = hc * 16 + un;
-                const int ft = lg.par == 0 ? 2 * e : 2 * e + 1;            // transformed feature e
-                const int xk = lg.par == 0 ? 2 * e + 1 : 2 * e;            // conditioning feature e
-                m2f[base4 + off + mma_tiled_off(un, e, 16)] = (int)(4 * (g1.flat_w[net] + (int64_t)ft * H + unit) + part);
-                m2f[base5 + off + mma_tiled_off(e, un, 16)] = (int)(4 * (g0.flat_w[net] + (int64_t)unit * (D + Cd) + xk) + part);
               }
           }
     }
@@ -581,12 +550,7 @@ struct Builder {
     for (int i = l0; i < l1; ++i) { stash_off[i] = stash_per_cta; stash_per_cta += R * d->layers[i].nT; }
     stash_per_cta = ceil4(std::max(stash_per_cta, 4));
 
-    {
-      RnvpOp ld = base_op(OP_LOAD, -1);
-      if (mode == 3) ld.flags = F_GSTASH;
-      ops.push_back(ld);
-    }
-    if (mode == 3) ops.push_back(base_op(OP_SEED_B, -1));
+    ops.push_back(base_op(OP_LOAD, -1));
     if (mode == 0 || mode == 2) {
       for (int i = l0; i < l1; ++i)
         if (d->layers[i].nT > 0) emit_forward_layer(i, mode == 2);
@@ -603,25 +567,19 @@ struct Builder {
       }
       ops.push_back(base_op(OP_STORE_G, -1));
     }
-    if (mode >= 2) {
-      // mode 3 = backward sweep only: z, x_T and s of every layer were left in global memory by the tcgen05
-      // forward kernel, so the forward sweep and the recomputation of s are skipped
+    if (mode == 2) {
       int prev_with_gu = -1;
       for (int i = l1 - 1; i >= l0; --i) {
         const LayerGeom& lg = d->layers[i];
         if (lg.nT == 0) continue;
         RnvpOp b = base_op(OP_BUILD_U, i);
-        b.flags = F_RESTORE | (mode == 3 ? F_GSTASH : 0);
+        b.flags = F_RESTORE;
         b.stash_off = stash_off[i];
         if (prev_with_gu == i + 1) b.flags |= F_ADDGU;
         ops.push_back(b);
         for (int q = 0; q < nh; ++q) emit_linear(i, q, 0);
-        if (mode == 2) emit_linear(i, nh, F_NET_S_ONLY);
-        {
-          RnvpOp cb = base_op(OP_COUPLE_B, i);
-          if (mode == 3) cb.flags = F_GSTASH;
-          ops.push_back(cb);
-        }
+        emit_linear(i, nh, F_NET_S_ONLY);
+        ops.push_back(base_op(OP_COUPLE_B, i));
         for (int q = nh; q >= 0; --q) {
           emit_wgrad(i, q);
           if (q > 0) emit_dgrad(i, q, false);

@@ -1,6 +1,6 @@
 // Weight-gradient sweep of the fit step on the 5th-generation tensor cores (tcgen05 / TMEM).
 //
-// The backward sweep (rnvp_mma.cu) runs with one thread per ROW, so what it leaves behind per (layer, row) is row-major:
+// The backward sweep (rnvp_wide.cu) owns ROWS (two threads per row), so what it leaves behind per (layer, row) is row-major:
 //     record = [ h (2H: nn_t | nn_s) | u = [x_K, c] (K1P8) | delta2 (2*TP: t | s) ]
 // while the weight gradients are contractions OVER ROWS:
 //     dW1[j][k] = sum_r delta1[r][j] u[r][k]     db1[j] = sum_r delta1[r][j]     delta1 = (delta2 W2) * act'(h)

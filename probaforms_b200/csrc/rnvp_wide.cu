@@ -1,8 +1,8 @@
 // tcgen05 path for WIDE flows (BASELINE configs[4]: D = 128, Cd = 32, H = 512; also D = 64 flows whose weight images do
 // not fit shared memory): fused forward (log-density) and inverse (sampling) passes with the conditioner weights STREAMED.
 //
-// rnvp_mma.cu keeps the TF32 hi/lo images of a whole coupling layer in shared memory and walks two 128-row tiles per
-// CTA.  Here a layer's images are 1.36 MB (c5), a row is 128 + 32 floats and the hidden layer has 2 x 512 units, so:
+// The weight images of a whole coupling layer do not stay resident in shared memory: a layer's images are 1.36 MB (c5),
+// a row is 128 + 32 floats and the hidden layer has 2 x 512 units, so:
 //   * one persistent CTA per SM owns ONE 128-row tile at a time; TMEM holds u = [x_K, c, 1] (hi/lo, 2 x K1PMAX columns), a
 //     double-buffered GEMM1 accumulator chunk (D1 / A_hi in place, A_lo; 2 x 2 x CU columns) and the GEMM2 accumulators
 //     [D2 | C2] (2 x NTP columns) -- 464 of 512 columns for c5;
@@ -12,7 +12,8 @@
 //     (43 KB per stage for c5: every SM reads the same 1.36 MB per tile-layer -- 29 B/cycle/SM, under the L2 cap);
 //   * the MMA issuer (warp 1, one elected lane) runs GEMM1 of chunk step cc+1 BEFORE it waits for the activations of chunk
 //     step cc, so the tensor core works on the next chunk while the epilogue warps turn the current one into tanh(.);
-//     error-compensated TF32 split as in rnvp_mma.cu (corrections first in GEMM1, merged A_hi x [B_hi ; B_lo] in GEMM2);
+//     error-compensated TF32 split A_hi*B_hi + A_lo*B_hi + A_hi*B_lo (corrections first in GEMM1, merged A_hi x [B_hi ; B_lo]
+//     in GEMM2);
 //   * warps 2-9 are the epilogue: TWO THREADS PER ROW (a thread cannot hold a 128-D row): thread (row, half) owns half of
 //     the transformed and half of the conditioning features, writes its half of u, converts its 16 columns of every D1
 //     chunk and applies the coupling to its 32 features; the two partial log-dets / squared norms meet in shared memory.
@@ -26,7 +27,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "tc05.cuh"
-#include "rnvp_mma.h"
+#include "rnvp_wide.h"
 #include "rnvp_philox.cuh"
 
 namespace {
@@ -50,7 +51,8 @@ __device__ __forceinline__ float act_wide(float v) {
   }
   return fmaxf(v, 0.0f);
 }
-// exp(x) on the MUFU with the argument's rounding error compensated (see rnvp_mma.cu exp_mma)
+// exp(x) = 2^(x*log2e) on the MUFU with the argument's rounding error compensated: t = rn(x*log2e), r = x*log2e - t
+// (exact residual through FMA + the low part of log2e), exp = ex2(t)*(1 + r*ln2).  ~2 ulp in 6 instructions, against ~25 for expf()
 __device__ __forceinline__ float exp_wide(float x) {
   const float t = x * 1.4426950216293335f;
   const float r = fmaf(x, 1.9259629911266175e-8f, fmaf(x, 1.4426950216293335f, -t));
@@ -76,7 +78,7 @@ enum { WB_WF = 0, WB_WE = WD_STAGES, WB_UF = 2 * WD_STAGES, WB_D1F0, WB_D1F1, WB
 #define RNVP_WIDE32_CTAS 2
 #endif
 template <int DH, int CDMAX, int CU, int ACT, int MODE>
-__global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WIDE32_CTAS : 1)) rnvp_wide_kernel(const __grid_constant__ RnvpMmaArgs a) {
+__global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WIDE32_CTAS : 1)) rnvp_wide_kernel(const __grid_constant__ RnvpWideArgs a) {
   constexpr int K1PMAX = (DH + CDMAX + 1 + 7) & ~7;
   constexpr int NTP = (DH + 15) & ~15;
   constexpr int NB1 = (DH == 32 && RNVP_WIDE32_CTAS == 2) ? 1 : 2;      // buffers of the D1 (forward) / dh (backward) chunk ring
@@ -123,7 +125,7 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
   __syncthreads();
   fence_after_sync();
   const uint32_t tbase = *tmem_slot;
-  const int my_tiles = (a.n_pairs - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;     // n_pairs = number of 128-row tiles here
+  const int my_tiles = (a.n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer: one ring stage per chunk step
@@ -623,7 +625,7 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
 }
 
 template <int DH, int CDMAX>
-cudaError_t launch_wide_shape(int act, int mode, const RnvpMmaArgs& a, int grid, size_t smem, cudaStream_t st) {
+cudaError_t launch_wide_shape(int act, int mode, const RnvpWideArgs& a, int grid, size_t smem, cudaStream_t st) {
 #define RNVP_WIDE_LAUNCH(ACT_, MODE_)                                                                       \
   {                                                                                                          \
     auto k = rnvp_wide_kernel<DH, CDMAX, 32, ACT_, MODE_>;                                                   \
@@ -652,7 +654,7 @@ size_t rnvp_wide_smem_bytes(int DH, int CDMAX) {
 
 int rnvp_wide_ctas_per_sm(int DH) { return DH == 16 ? 2 : (DH == 32 ? RNVP_WIDE32_CTAS : 1); }
 
-cudaError_t rnvp_launch_wide(int DH, int act, int mode, const RnvpMmaArgs& a, int grid, cudaStream_t st) {
+cudaError_t rnvp_launch_wide(int DH, int act, int mode, const RnvpWideArgs& a, int grid, cudaStream_t st) {
   if (DH == 64) return launch_wide_shape<64, 32>(act, mode, a, grid, rnvp_wide_smem_bytes(64, 32), st);
   if (DH == 32) return launch_wide_shape<32, 16>(act, mode, a, grid, rnvp_wide_smem_bytes(32, 16), st);
   if (DH == 16) return launch_wide_shape<16, 16>(act, mode, a, grid, rnvp_wide_smem_bytes(16, 16), st);

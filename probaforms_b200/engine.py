@@ -83,9 +83,10 @@ class FlowEngine:
 
     @property
     def fit_on_tensor_cores(self):
-        """True when rnvp_backward runs entirely on the tensor cores: tcgen05 forward + backward sweeps (rnvp_mma_kernel<..,2> for
-        D = 32 flows with H <= 128, rnvp_wide_kernel<..,2> for wide flows with H a multiple of 128) followed by
-        rnvp_wgrad_tc_kernel (plan_info pseudo-mode 4)."""
+        """True when rnvp_backward runs entirely on the tensor cores: tcgen05 forward + backward sweeps
+        (rnvp_wide_kernel<..,2>, for tcgen05-eligible flows with D <= 64 or with H a multiple of 128) followed by
+        rnvp_wgrad_tc_kernel (plan_info pseudo-mode 4).  Equal to ``_bwd_two_kernels``, which counts that fit step's
+        two launches."""
         return self.plan_info(4)["kernel_family"] == 2
 
     def __del__(self):

@@ -215,6 +215,43 @@ extern "C" int rnvp_emulate(int mode, int D, int Cd, int L, int nh, const int* h
   return 0;
 }
 
+namespace {
+// FNV-1a over raw bytes: a stable fingerprint of a layout map or an op program
+uint64_t fnv1a(const void* p, size_t n, uint64_t h = 1469598103934665603ull) {
+  const unsigned char* b = (const unsigned char*)p;
+  for (size_t i = 0; i < n; ++i) { h ^= b[i]; h *= 1099511628211ull; }
+  return h;
+}
+}  // namespace
+
+// Tensor-core layout and FP32 programs of a one-hidden-layer flow as rnvp_desc_create builds them
+// (default max_smem).  out[26]: mma_ok, mDH, mK1P, mNTP, m_w1_floats, m_w2_floats, m_wt_floats, m_layer_floats,
+// mma_off, mma_floats, packed, packed_tile, small_ok, digest of build_mma_map's m2f, then per FP32 mode 0, 1, 2:
+// planned (0/1), TR, shared-memory bytes, digest of the smem carve-up, ops and chunks.
+extern "C" int rnvp_emul_tc_layout(int D, int Cd, int L, int H, int act, long long* out) {
+  FlowGeom g;
+  g.D = D; g.Cd = Cd; g.L = L; g.nh = 1; g.act = act; g.hidden[0] = H;
+  build_layout(&g);
+  std::vector<int> m2f;
+  build_mma_map(&g, m2f);
+  const long long head[14] = {g.mma_ok, g.mDH, g.mK1P, g.mNTP, g.m_w1_floats, g.m_w2_floats, g.m_wt_floats, g.m_layer_floats,
+                              g.mma_off, g.mma_floats, g.packed, g.packed_tile, g.small_ok,
+                              (long long)fnv1a(m2f.data(), m2f.size() * sizeof(int))};
+  for (int k = 0; k < 14; ++k) out[k] = head[k];
+  for (int mode = 0; mode < 3; ++mode) {
+    long long* o = out + 14 + 4 * mode;
+    Builder b;
+    b.d = &g; b.mode = mode; b.l0 = 0; b.l1 = L;
+    if (!b.plan_best(0)) { o[0] = 0; o[1] = o[2] = o[3] = -1; continue; }
+    b.build();
+    o[0] = 1; o[1] = b.TR; o[2] = (long long)b.sm.total_floats * 4;
+    uint64_t h = fnv1a(&b.sm, sizeof(b.sm));
+    h = fnv1a(b.ops.data(), b.ops.size() * sizeof(RnvpOp), h);
+    o[3] = (long long)fnv1a(b.chunks.data(), b.chunks.size() * sizeof(RnvpChunk), h);
+  }
+  return 0;
+}
+
 extern "C" long long rnvp_emul_param_count(int D, int Cd, int L, int nh, const int* hidden) {
   FlowGeom g;
   g.D = D; g.Cd = Cd; g.L = L; g.nh = nh; g.act = 1;

@@ -100,25 +100,30 @@ def test_perm_abi_edge_cases():
 
 
 def test_record_block_layout_contract():
-    """The activation-record layout shared by rnvp_mma.cu (writer: one row per lane, float4 per column group) and
-    rnvp_wgrad.cu (reader: blk_off): [column group of 4][32 slots][4 floats], slot = row ^ (group & 1).  Checks that the
-    map is a bijection of a block and that the fragment loads of the weight-gradient sweep are bank-conflict free."""
+    """The activation-record layout shared by rnvp_wide.cu (writer: one row per lane, float4 per column group) and
+    rnvp_wgrad_tc.cu (reader): [column group of 4][32 slots][4 floats], slot = row ^ (group & 7) (include/rnvp.h).
+    Checks that the map is a bijection of a block, that the writer's warp-wide float4 stores cover 512 contiguous bytes,
+    and that both read patterns of the weight-gradient sweep are bank-conflict free."""
     rec = 312                                                   # c3: 2*128 + 24 + 32 floats per record
     def blk_off(c, r):
-        return (c >> 2) * 128 + ((r ^ ((c >> 2) & 1)) << 2) + (c & 3)
+        return (c >> 2) * 128 + ((r ^ ((c >> 2) & 7)) << 2) + (c & 3)
     seen = {blk_off(c, r) for c in range(rec) for r in range(32)}
     assert seen == set(range(32 * rec))
-    # writer side: lane = row stores the float4 of column group cg at base + cg*128 + ((lane ^ (cg & 1)) << 2)
+    # writer side: lane = row stores the float4 of column group cg at base + cg*128 + ((lane ^ (cg & 7)) << 2)
     for cg in range(rec // 4):
+        offs = []
         for lane in range(32):
-            assert cg * 128 + ((lane ^ (cg & 1)) << 2) == blk_off(4 * cg, lane)
-    # reader side: lane = 4*g + t loads (column base + g, rows r0 + 2t and r0 + 2t + 1) for any column base % 8 == 0
-    for base in (0, 16, 256, 280):
-        for r0 in (0, 8, 24):
-            for odd in (0, 1):
-                banks = {blk_off(base + g, r0 + 2 * t + odd) % 32 for g in range(8) for t in range(4)}
-                assert len(banks) == 32
-    # B operand of the dh product: lane loads (column base + t [+4], row r0 + g)
-    for plus in (0, 4):
-        banks = {blk_off(280 + plus + t, 8 + g) % 32 for g in range(8) for t in range(4)}
-        assert len(banks) == 32
+            off = cg * 128 + ((lane ^ (cg & 7)) << 2)
+            assert off == blk_off(4 * cg, lane)
+            offs.append(off)
+        assert sorted(offs) == list(range(cg * 128, cg * 128 + 128, 4))   # one 512-byte segment per warp instruction
+    # per-row 16-byte reads (u and delta2 columns), lanes = rows: each quarter-warp phase of 8 float4s hits 32 banks
+    for cg in range(rec // 4):
+        for phase in range(4):
+            banks = {(blk_off(4 * cg, r) + k) % 32 for r in range(8 * phase, 8 * phase + 8) for k in range(4)}
+            assert len(banks) == 32
+    # per-unit 4-byte reads (h columns), lanes = 32 consecutive hidden units, one row at a time
+    for u0 in range(0, 2 * 128, 32):
+        for r in range(32):
+            banks = {blk_off(u0 + lane, r) % 32 for lane in range(32)}
+            assert len(banks) == 32

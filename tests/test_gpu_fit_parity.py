@@ -1,8 +1,8 @@
 """Oracle parity of the FIT path at the configurations bench.py times (run on the B200 box with ``-m gpu``).
 
-The tensor-core fit kernels (rnvp_mma_kernel<..,2> + the weight-gradient sweep) are compared here with
+The tensor-core fit kernels (rnvp_wide_kernel<..,2> + the weight-gradient sweep) are compared here with
 ``oracle.loss_and_grads`` / ``oracle.fit`` directly -- not with the library's own FP32 kernels -- on full-size batches:
-148 persistent CTAs x 2 row-tile pairs, ring-phase wrap-around, the int64 row gather, ragged tails.
+persistent CTAs walking several 128-row tiles each, ring-phase wrap-around, the int64 row gather, ragged tails.
 
 Tolerances (DESIGN.md section 2): loss rel 1e-5 (north_star's fp32 bound); gradients 2e-5 * max|grad| because the
 packed accumulator is filled with red.global.add in a run-dependent order over up to 75,776 rows (the reference's own

@@ -22,7 +22,7 @@ except Exception as e:
 PY
 timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 120 --csv --log-file $out/${tag}_launches.csv \
     python bench.py --steps 3 --warmup 3 --no-e2e --no-cpu-baseline --no-others > /dev/null 2>&1
-timeout 300 ncu --set full --clock-control none --import-source on -k regex:"rnvp_mma_kernel|rnvp_wide_kernel|rnvp_wgrad_tc" -s 2 -c 2 \
+timeout 300 ncu --set full --clock-control none --import-source on -k regex:"rnvp_wide_kernel|rnvp_wgrad_tc" -s 2 -c 2 \
     -o $out/${tag}_c3fit -f python tools/quick_bench.py --workloads c3 --rows 75776 --passes bwd --reps 2 > /dev/null 2>&1
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:"rnvp_wide_kernel|rnvp_wgrad_tc" -s 2 -c 2 \
     -o $out/${tag}_c5fit -f python tools/quick_bench.py --workloads c5 --rows 16384 --passes bwd --reps 2 > /dev/null 2>&1

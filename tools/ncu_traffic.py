@@ -18,7 +18,7 @@ for r in rows[2:]:
     if len(r) < len(hdr):
         continue
     name = r[ix["Kernel Name"]]
-    key = "rnvp_wgrad_tc_kernel" if "wgrad_tc" in name else ("fit_sweep_kernel" if ("rnvp_mma_kernel" in name or "rnvp_wide_kernel" in name) else name.split("(")[0][:48])
+    key = "rnvp_wgrad_tc_kernel" if "wgrad_tc" in name else ("fit_sweep_kernel" if "rnvp_wide_kernel" in name else name.split("(")[0][:48])
 
     def val(metric):
         v, u = float(r[ix[metric]].replace(",", "")), rows[1][ix[metric]]
@@ -27,7 +27,7 @@ for r in rows[2:]:
                 "dram_bytes_read": val("dram__bytes_read.sum"), "dram_bytes_write": val("dram__bytes_write.sum"),
                 "duration_us_under_ncu": val("gpu__time_duration.sum"), "kernel": name[:120]}
 json.dump({"source": os.path.relpath(tracked), "commit": commit,
-           "command": "ncu --set full --clock-control none -k regex:rnvp_mma_kernel|rnvp_wide_kernel|rnvp_wgrad_tc python tools/quick_bench.py "
+           "command": "ncu --set full --clock-control none -k regex:rnvp_wide_kernel|rnvp_wgrad_tc python tools/quick_bench.py "
                       "--workloads c3 --rows 75776 --passes bwd --reps 2", "kernels": out},
           open("profiles/traffic.json", "w"), indent=1)
 print(json.dumps(out, indent=1))
