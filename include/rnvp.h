@@ -235,6 +235,47 @@ int rnvp_kde_draws(const double* d_sorted, const int32_t* d_src, int64_t n, int6
                    const uint16_t* d_counts /* [n_draws][n+m] */, int n_draws, int bins, double h_x, double h_y,
                    double* d_sums /* [n_draws][D][2][bins] */, void* stream);
 
+/* ConditionalNormal (rnvp_cnormal.cu; probaforms/models/cnormal.py).  Net: model = Linear(Cd, h0), act, ..., act
+ * (no final Linear), heads mu, log_sigma = Linear(h_last, D), out = Linear(D, D).  Parameters cross the boundary as one
+ * flat fp32 buffer in Net.parameters() order: model.{2k}.weight [h_k, h_{k-1}], model.{2k}.bias, mu.weight, mu.bias,
+ * log_sigma.weight, log_sigma.bias, out.weight [D, D], out.bias.  act: RNVP_ACT_TANH, _RELU or _SIGMOID (any other
+ * activation string is ReLU upstream, cnormal.py:39-46).  Shapes: D <= 128, Cd <= 256, 1 to 4 hidden layers of width
+ * <= 512 (RNVP_ESHAPE otherwise).  M is the caller-owned D x D inverse (W_out^T)^-1, row-major. */
+enum { RNVP_ACT_SIGMOID = 3 };
+typedef struct rnvp_cn_desc rnvp_cn_desc;
+int rnvp_cn_desc_create(int D, int Cd, int n_hidden, const int* hidden, int act, int independent, rnvp_cn_desc** out);
+void rnvp_cn_desc_destroy(rnvp_cn_desc* d);
+int64_t rnvp_cn_param_count(const rnvp_cn_desc* d);
+/* scratch bytes of rnvp_cn_grad / rnvp_cn_fit_epoch for batches of up to N rows (per-CTA gradient partials) */
+int64_t rnvp_cn_workspace_bytes(const rnvp_cn_desc* d, int64_t N);
+/* d_M = (W_out^T)^-1 by Gauss-Jordan with partial pivoting in fp32 (one CTA); *d_status = 1 on an exact-zero pivot,
+ * untouched otherwise (the caller zeroes it) */
+int rnvp_cn_inverse(const rnvp_cn_desc* d, const float* d_params, float* d_M, int* d_status, void* stream);
+/* Net.forward for inference (cnormal.py:77-91): d_mu, d_sigma = exp(log_sigma), d_xtilde = mu + eps * sigma (then out()
+ * in full-covariance mode), d_inv = (X - out.bias) M.  Every output may be NULL; d_inv needs d_X and d_M.  eps is d_eps
+ * [N][D] when given (parity mode), else Philox keyed on (seed, row_offset + row, j) as in rnvp_sample. */
+int rnvp_cn_forward(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,
+                    int64_t N, uint64_t seed, int64_t row_offset, const float* d_eps, float* d_mu, float* d_sigma,
+                    float* d_xtilde, float* d_inv, void* stream);
+/* loss (cnormal.py:140-151) and its gradient on the N rows X[idx[r]], C[idx[r]] (d_idx may be NULL): d_gflat [P] in
+ * the flat layout (zeros for out.* in independent mode, where the loss does not depend on them), *d_loss */
+int rnvp_cn_grad(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,
+                 const int64_t* d_idx, int64_t N, float* d_gflat, float* d_loss, void* d_workspace,
+                 int64_t workspace_bytes, void* stream);
+/* One epoch of ConditionalNormal.fit (cnormal.py:193-209) as one call: for every consecutive batch_size slice of d_perm
+ * (last partial batch kept), loss + gradient + torch.optim.Adam step (step count step0 + 1, ...; out.* skipped in
+ * independent mode), loss to d_losses[s], and in full mode d_M refreshed for the next step.  A batch of at most the
+ * kernel's tile (64 rows for small nets) is one launch.  If a refreshed W_out has an exact-zero pivot, *d_status =
+ * (fit step index of the next step) + 1 and every later step of this and later calls with the same d_status is a
+ * no-op.  Workspace: rnvp_cn_workspace_bytes(d, batch_size). */
+int rnvp_cn_fit_epoch(const rnvp_cn_desc* d, float* d_params, float* d_exp_avg, float* d_exp_avg_sq, float* d_M,
+                      const float* d_X, const float* d_C, const int64_t* d_perm, int64_t n, int64_t batch_size,
+                      double lr, double beta1, double beta2, double eps, double weight_decay, int64_t step0,
+                      float* d_losses, int* d_status, void* d_workspace, int64_t workspace_bytes, void* stream);
+/* Host only: advance a torch CPU generator state (Generator.get_state() bytes, 5056) exactly as torch.randn(numel) in
+ * float32 does, for numel >= 16 (numel 32-bit draws, plus 16 when numel % 16 != 0); smaller numel: RNVP_EINVAL. */
+int rnvp_cn_rng_advance(uint8_t* state, int64_t state_bytes, int64_t numel);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

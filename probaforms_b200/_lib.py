@@ -69,6 +69,20 @@ SIGNATURES = {
                                   C.c_double, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_kde_draws": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                  C.c_double, C.c_double, C.c_void_p, c_stream]),
+    "rnvp_cn_desc_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int, C.c_int,
+                                      C.POINTER(c_desc_p)]),
+    "rnvp_cn_desc_destroy": (None, [c_desc_p]),
+    "rnvp_cn_param_count": (C.c_int64, [c_desc_p]),
+    "rnvp_cn_workspace_bytes": (C.c_int64, [c_desc_p, C.c_int64]),
+    "rnvp_cn_inverse": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, C.c_void_p, c_stream]),
+    "rnvp_cn_forward": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, C.c_int64, C.c_uint64, C.c_int64,
+                                  c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_stream]),
+    "rnvp_cn_grad": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64, c_f32_p, c_f32_p,
+                               C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_cn_fit_epoch": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64,
+                                    C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, C.c_int64,
+                                    c_f32_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_cn_rng_advance": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

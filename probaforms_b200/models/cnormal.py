@@ -1,0 +1,435 @@
+"""Conditional Normal model with the reference's API (probaforms/models/cnormal.py:18-240).
+
+Same constructor, defaults, public attributes (``model``, ``opt``, ``loss_history``, ...), ``fit(X, C)`` /
+``sample(C)`` and ``state_dict`` keys (``model.{2k}.*``, ``mu.*``, ``log_sigma.*``, ``out.*`` under ``model``) as
+``probaforms.models.ConditionalNormal``; the arithmetic runs in the FP32 kernels of ``rnvp_cnormal.cu``.
+
+``fit`` reproduces the reference's training run: ``Net`` is built on the CPU under the global generator (same
+initial parameters), every epoch's batches are the reference's ``DataLoader(shuffle=True)`` batches, Adam is the
+reference's (the ``out`` tensors get no gradient and no update with independent covariance), and the global torch RNG
+is left exactly where the reference leaves it -- including the ``torch.randn(nb, D)`` that the reference's
+``Net.forward`` draws (and discards) at every step, which is replayed on the host without generating the values.
+A whole epoch is one library call; a batch of up to 64 rows (the default ``batch_size`` is 32) is one kernel launch.
+
+``sample`` differs from the reference in its noise: one int64 is drawn from the global generator per call and the
+normals come from Philox keyed on (seed, row, feature) inside the kernel, as in ``RealNVP.sample``; the noise values
+and the global RNG state after ``sample`` are therefore not the reference's.  ``Net.forward`` is inference-only (no
+autograd).  CUDA only; there is no CPU fallback.
+"""
+import ctypes as ct
+import threading
+
+import numpy as np
+import torch
+import torch.nn as nn
+
+from .interfaces import GenModel
+from .realnvp import _LossLog, _default_device
+from .. import _lib
+from ..batching import StreamingPermutation, batch_bounds
+
+ACT = {"tanh": 1, "relu": 2, "sigmoid": 3}         # include/rnvp.h RNVP_ACT_*; every other string is ReLU upstream
+
+
+class _Desc:
+    """Owns one ``rnvp_cn_desc`` (shape, activation, covariance mode) on the current CUDA device."""
+
+    def __init__(self, D, Cd, hidden, activation, independent):
+        self.lib = _lib.load()
+        hid = (ct.c_int * len(hidden))(*hidden)
+        h = ct.c_void_p()
+        rc = self.lib.rnvp_cn_desc_create(D, Cd, len(hidden), hid, ACT.get(activation, 2), int(bool(independent)),
+                                          ct.byref(h))
+        if rc != 0:
+            msg = self.lib.rnvp_last_error().decode()
+            if rc == -2:                                   # RNVP_ESHAPE
+                raise ValueError(msg)
+            raise _lib.RnvpError(f"rnvp_cn_desc_create failed (code {rc}): {msg}")
+        self.h, self.D, self.Cd, self.independent = h, D, Cd, bool(independent)
+        self.P = int(self.lib.rnvp_cn_param_count(h))
+
+    def workspace(self, n, dev):
+        nbytes = int(self.lib.rnvp_cn_workspace_bytes(self.h, max(int(n), 1)))
+        return torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=dev), nbytes
+
+    def __del__(self):
+        if getattr(self, "h", None):
+            self.lib.rnvp_cn_desc_destroy(self.h)
+            self.h = None
+
+
+def _stream(dev):
+    return ct.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+
+
+class Net(nn.Module):
+    """The reference's Net (cnormal.py:18-91): ``model`` = Linear, act, ..., ``mu``, ``log_sigma``, ``out``.
+
+    'tanh' gives Tanh, 'relu' ReLU, 'sigmoid' Sigmoid and every other string ReLU, as upstream.  The modules hold the
+    parameters (built on the CPU, so names, shapes, default init and RNG order are the reference's); ``to_device``
+    makes them views of one flat device buffer, the layout the kernels read.
+    """
+
+    def __init__(self, var_size, cond_size, hidden=(10,), activation='tanh', independent_covariance=False):
+        super().__init__()
+        self.independent_covariance = independent_covariance
+        self.var_size, self.cond_size = var_size, cond_size
+        self.hidden, self.activation = tuple(hidden), activation
+        layers = []
+        for i in range(len(hidden)):
+            layers.append(nn.Linear(cond_size if i == 0 else hidden[i - 1], hidden[i]))
+            layers.append({"tanh": nn.Tanh, "relu": nn.ReLU, "sigmoid": nn.Sigmoid}.get(activation, nn.ReLU)())
+        self.model = nn.Sequential(*layers)
+        self.mu = nn.Linear(hidden[-1], var_size)
+        self.log_sigma = nn.Linear(hidden[-1], var_size)
+        self.out = nn.Linear(var_size, var_size)
+        self._desc, self._flat = None, None
+
+    def __getstate__(self):
+        state = self.__dict__.copy()
+        state["_desc"], state["_flat"] = None, None
+        return state
+
+    def to_device(self, dev):
+        """Move the parameters into one flat fp32 buffer on ``dev`` (parameter tensors become views of it)."""
+        if self._desc is None:
+            with torch.cuda.device(dev):
+                self._desc = _Desc(self.var_size, self.cond_size, self.hidden, self.activation,
+                                   self.independent_covariance)
+        params = list(self.parameters())
+        flat = torch.cat([p.detach().reshape(-1).to(torch.float32) for p in params]).to(dev)
+        off = 0
+        for p in params:
+            n = p.numel()
+            p.data = flat[off:off + n].view(p.shape)
+            off += n
+        self._flat = flat
+        return self
+
+    def _ready(self):
+        p = self.mu.weight
+        if self._flat is None or p.data_ptr() != self._flat.data_ptr() + 4 * self.mu_offset() or p.device.type != "cuda":
+            self.to_device(p.device if p.device.type == "cuda" else _default_device())
+        return self._desc, self._flat
+
+    def mu_offset(self):
+        return sum(p.numel() for p in self.model.parameters())
+
+    def inverse_out(self):
+        """M = (out.weight^T)^-1 on the device; raises torch.linalg.LinAlgError if a pivot is exactly zero."""
+        desc, flat = self._ready()
+        dev = flat.device
+        M = torch.empty(self.var_size, self.var_size, dtype=torch.float32, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        _lib.check(desc.lib.rnvp_cn_inverse(desc.h, flat.data_ptr(), M.data_ptr(), ct.c_void_p(status.data_ptr()),
+                                            _stream(dev)), "rnvp_cn_inverse")
+        if int(status.item()) != 0:
+            raise torch.linalg.LinAlgError("linalg.inv: The diagonal element 1 is zero, the inversion could not be "
+                                           "completed because the input matrix is singular.")
+        return M
+
+    @torch.no_grad()
+    def forward(self, X, C, eps=None, seed=None):
+        """(x_tilde, inv, mu, sigma) as in the reference (cnormal.py:77-91), computed by one inference kernel.
+
+        ``eps`` [n, var_size] supplies the noise (parity mode); otherwise it is Philox keyed on (seed, row, feature),
+        with ``seed`` drawn as one int64 from the global generator when not given.  ``inv`` is None without ``X``."""
+        desc, flat = self._ready()
+        dev = flat.device
+        Cd = torch.as_tensor(C, dtype=torch.float32).to(dev).contiguous()
+        if Cd.dim() != 2 or Cd.shape[1] != self.cond_size:
+            raise ValueError(f"C must be [n, {self.cond_size}], got shape {tuple(Cd.shape)}")
+        n, D = Cd.shape[0], self.var_size
+        Xd = M = None
+        if X is not None:
+            Xd = torch.as_tensor(X, dtype=torch.float32).to(dev).contiguous()
+            if tuple(Xd.shape) != (n, D):
+                raise ValueError(f"X must be [{n}, {D}], got shape {tuple(Xd.shape)}")
+            M = self.inverse_out()
+        if eps is not None:
+            eps = torch.as_tensor(eps, dtype=torch.float32).to(dev).contiguous()
+            if tuple(eps.shape) != (n, D):
+                raise ValueError(f"eps must be [{n}, {D}], got shape {tuple(eps.shape)}")
+            seed = 0
+        elif seed is None:
+            seed = int(torch.empty((), dtype=torch.int64).random_().item())
+        mu, sigma, xt = (torch.empty(n, D, dtype=torch.float32, device=dev) for _ in range(3))
+        inv = torch.empty(n, D, dtype=torch.float32, device=dev) if Xd is not None else None
+        ptr = lambda t: None if t is None else t.data_ptr()   # noqa: E731
+        _lib.check(desc.lib.rnvp_cn_forward(desc.h, flat.data_ptr(), ptr(M), ptr(Xd), Cd.data_ptr(), n,
+                                            ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), 0, ptr(eps), mu.data_ptr(),
+                                            sigma.data_ptr(), xt.data_ptr(), ptr(inv), _stream(dev)),
+                   "rnvp_cn_forward")
+        return xt, inv, mu, sigma
+
+
+class _RngReplay:
+    """The reference's use of the global torch generator during ``fit``, replayed on a helper thread.
+
+    Per epoch the reference's fresh ``DataLoader(shuffle=True)`` draws two int64 (the second seeds the row order) and
+    every step's ``Net.forward`` draws ``torch.randn(nb, D)``.  The replay runs on a private generator cloned from the
+    global state after ``Net`` init: the int64 draws go through torch, the normals are skipped with
+    ``rnvp_cn_rng_advance`` (the words ``torch.randn`` would consume, without computing the values); below 16 elements
+    torch takes a cached double path, so those few draws are made with ``torch.randn`` on the private generator."""
+
+    def __init__(self, lib, n, bs, D, n_epochs):
+        self.lib = lib
+        self.gen = torch.Generator()
+        self.gen.set_state(torch.get_rng_state())
+        self.numels = [nb * D for _, nb in batch_bounds(n, bs)]
+        self.seeds = []
+        self._cv = threading.Condition()
+        self._err = None
+        self._thread = threading.Thread(target=self._run, args=(n_epochs,), daemon=True)
+        self._thread.start()
+
+    def _run(self, n_epochs):
+        try:
+            for _ in range(n_epochs):
+                torch.empty((), dtype=torch.int64).random_(generator=self.gen)
+                seed = int(torch.empty((), dtype=torch.int64).random_(generator=self.gen).item())
+                with self._cv:
+                    self.seeds.append(seed)
+                    self._cv.notify_all()
+                advance(self.lib, self.gen, self.numels)
+        except Exception as e:                                              # pragma: no cover
+            with self._cv:
+                self._err = e
+                self._cv.notify_all()
+
+    def seed(self, epoch):
+        with self._cv:
+            while len(self.seeds) <= epoch and self._err is None:
+                self._cv.wait()
+            if self._err is not None:
+                raise self._err
+            return self.seeds[epoch]
+
+    def final_state(self):
+        self._thread.join()
+        if self._err is not None:
+            raise self._err
+        return self.gen.get_state()
+
+
+def advance(lib, gen, numels):
+    """Advance ``gen`` as ``torch.randn(k)`` (float32) would, for every k in ``numels``, in order."""
+    state = gen.get_state()
+    for k in numels:
+        if k >= 16:
+            _lib.check(lib.rnvp_cn_rng_advance(ct.c_void_p(state.data_ptr()), state.numel(), int(k)),
+                       "rnvp_cn_rng_advance")
+        elif k > 0:
+            gen.set_state(state)
+            torch.randn(int(k), generator=gen)
+            state = gen.get_state()
+    gen.set_state(state)
+
+
+def state_at_step(lib, state, n, bs, D, step):
+    """The global generator state the reference leaves when fit step ``step`` (0-based over the whole fit) raises in
+    its forward pass: from ``state`` (right after Net init), every epoch's two DataLoader draws and every step's
+    ``torch.randn(nb, D)`` up to and including that step's."""
+    gen = torch.Generator()
+    gen.set_state(state)
+    numels = [nb * D for _, nb in batch_bounds(n, bs)]
+    s = 0
+    while True:
+        torch.empty((), dtype=torch.int64).random_(generator=gen)
+        torch.empty((), dtype=torch.int64).random_(generator=gen)
+        for k in numels:
+            advance(lib, gen, [k])
+            if s == step:
+                return gen.get_state()
+            s += 1
+
+
+def epoch_plan(lib, n, bs, D, n_epochs):
+    """Host-only replay of ``fit``'s RNG use from the current global state (a test and inspection aid): returns the
+    per-epoch sampler seeds and the generator state the reference leaves behind.  The global state is not changed."""
+    rp = _RngReplay(lib, n, bs, D, n_epochs)
+    state = rp.final_state()
+    return list(rp.seeds), state
+
+
+class ConditionalNormal(GenModel):
+    """Conditional Normal model (reference cnormal.py:94-240); parameters as upstream:
+
+    use_independent_covariance, hidden, activation ('tanh' | 'relu' | 'sigmoid', anything else is ReLU), batch_size,
+    n_epochs, lr, weight_decay, verbose (>0: progress bar over epochs).
+    """
+
+    def __init__(self, use_independent_covariance=False, hidden=(10,), activation='tanh', batch_size=32, n_epochs=10,
+                 lr=0.0001, weight_decay=0, verbose=0):
+        super().__init__()
+        self.independent_covariance = use_independent_covariance
+        self.hidden = hidden
+        self.activation = activation
+        self.batch_size = batch_size
+        self.n_epochs = n_epochs
+        self.lr = lr
+        self.weight_decay = weight_decay
+        self.verbose = verbose
+        self.opt = None
+        self._device = None
+        self._perm_host = [None, None]
+
+    def custom_loss(self, mu, sigma, x):
+        loss = (x - mu)**2 / (2 * sigma**2) + torch.log(sigma)
+        loss = torch.mean(loss)
+        return loss
+
+    def compute_loss(self, x_batch, cond_batch):
+        """The reference's loss on one batch (cnormal.py:145-151), computed by the fit kernels (no autograd graph)."""
+        net = self.model
+        desc, flat = net._ready()
+        dev = flat.device
+        Xd = torch.as_tensor(x_batch, dtype=torch.float32).to(dev).contiguous()
+        Cd = torch.as_tensor(cond_batch, dtype=torch.float32).to(dev).contiguous()
+        if Xd.dim() != 2 or Xd.shape[1] != net.var_size or Cd.dim() != 2 or Cd.shape != (Xd.shape[0], net.cond_size):
+            raise ValueError(f"x_batch must be [n, {net.var_size}] and cond_batch [n, {net.cond_size}]")
+        return self._grad(Xd, Cd)[0]
+
+    def _grad(self, Xd, Cd, idx=None):
+        """(loss, flat gradient) of one batch through rnvp_cn_grad."""
+        desc, flat = self.model._ready()
+        dev = flat.device
+        n = idx.numel() if idx is not None else Xd.shape[0]
+        M = None if desc.independent else self.model.inverse_out()
+        ws, nbytes = desc.workspace(n, dev)
+        g = torch.empty(desc.P, dtype=torch.float32, device=dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        _lib.check(desc.lib.rnvp_cn_grad(desc.h, flat.data_ptr(), None if M is None else M.data_ptr(), Xd.data_ptr(),
+                                         Cd.data_ptr(), None if idx is None else idx.data_ptr(), n, g.data_ptr(),
+                                         loss.data_ptr(), ws.data_ptr(), nbytes, _stream(dev)), "rnvp_cn_grad")
+        return loss, g
+
+    def _model_init(self, X, C):
+        var_size = X.shape[1]
+        cond_size = C.shape[1]
+        if self._device is None:
+            self._device = _default_device()
+        self.model = Net(var_size=var_size, cond_size=cond_size, hidden=self.hidden, activation=self.activation,
+                         independent_covariance=self.independent_covariance)
+        self.opt = torch.optim.Adam(list(self.model.parameters()), lr=self.lr, weight_decay=self.weight_decay)
+        self.model.to_device(self._device)
+
+    def fit(self, X, C=None):
+        """Fit on X [n, var_size], conditions C [n, cond_size] or None (cnormal.py:166-217).  Rebuilds ``Net`` and
+        ``Adam`` on every call, as upstream.  ``loss_history`` gets one 0-d CPU tensor per step.  Raises
+        torch.linalg.LinAlgError when ``out.weight`` becomes singular; ``model`` and ``loss_history`` then hold the
+        state before the step that could not run."""
+        from ..ingest import upload_resident
+        if not hasattr(X, "shape"):
+            X = np.asarray(X)
+        if len(tuple(X.shape)) != 2:
+            raise ValueError(f"X must be 2-D [n, var_size], got shape {tuple(X.shape)}")
+        n = X.shape[0]
+        if C is None:
+            C = torch.zeros(n, 1)
+        elif not hasattr(C, "shape"):
+            C = np.asarray(C)
+        if len(tuple(C.shape)) != 2 or C.shape[0] != n:
+            raise ValueError(f"C must be 2-D with {n} rows, got shape {tuple(C.shape)}")
+        if self._device is None:
+            self._device = _default_device()
+        self._model_init(X, C)
+        dev, net = self._device, self.model
+        desc, flat = net._ready()
+        lib, D, bs = desc.lib, net.var_size, int(self.batch_size)
+        if bs < 1:
+            raise ValueError("batch_size must be >= 1")
+        self.model.train(True)
+        self.loss_history = []
+        init_state = torch.get_rng_state()
+        try:
+            M = net.inverse_out()                # the reference inverts out.weight at the first step in both modes
+        except torch.linalg.LinAlgError:
+            if self.n_epochs > 0 and n > 0:      # the reference raises inside step 0, after that step's draws
+                torch.set_rng_state(state_at_step(lib, init_state, n, bs, D, 0))
+            raise
+        replay = _RngReplay(lib, n, bs, D, self.n_epochs)
+        Xd = upload_resident(lib, X, dev)
+        Cd = upload_resident(lib, C, dev)
+        P = desc.P
+        exp_avg = torch.zeros(P, dtype=torch.float32, device=dev)
+        exp_avg_sq = torch.zeros(P, dtype=torch.float32, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        ws, nbytes = desc.workspace(min(bs, max(n, 1)), dev)
+        perm_dev = [torch.empty(max(n, 1), dtype=torch.int64, device=dev) for _ in range(2)]
+        copied = [None, None]
+        bounds = batch_bounds(n, bs)
+        log = _LossLog(self.loss_history)
+        epochs = range(self.n_epochs)
+        bar = None
+        if self.verbose >= 1:
+            from tqdm.auto import tqdm
+            bar = tqdm(epochs, unit='epoch')
+            epochs = bar
+        stream = _stream(dev)
+        nxt = StreamingPermutation(lib, replay.seed(0), n, host=self._perm_host[0]) if self.n_epochs > 0 else None
+        for ep in epochs:
+            sp = nxt
+            self._perm_host[ep & 1] = sp.host
+            k = ep & 1
+            perm_dev[k][:n].copy_(sp.full(), non_blocking=True)
+            ev = torch.cuda.Event()
+            ev.record(torch.cuda.current_stream(dev))
+            copied[k] = ev
+            losses = torch.empty(len(bounds), dtype=torch.float32, device=dev)
+            _lib.check(lib.rnvp_cn_fit_epoch(desc.h, flat.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
+                                             M.data_ptr(), Xd.data_ptr(), Cd.data_ptr(), perm_dev[k].data_ptr(), n, bs,
+                                             self.lr, 0.9, 0.999, 1e-8, self.weight_decay, ep * len(bounds),
+                                             losses.data_ptr(), ct.c_void_p(status.data_ptr()), ws.data_ptr(), nbytes,
+                                             stream), "rnvp_cn_fit_epoch")
+            if ep + 1 < self.n_epochs:
+                # the next order is shuffled into the other host buffer while this epoch runs; that buffer's last copy
+                # (two epochs ago) must have left it
+                if copied[k ^ 1] is not None:
+                    copied[k ^ 1].synchronize()
+                nxt = StreamingPermutation(lib, replay.seed(ep + 1), n, host=self._perm_host[(ep + 1) & 1])
+            host = log.push(losses)
+            if bar is not None and host is not None:
+                bar.set_description(f"loss: {float(host[-1]):.4f}")
+        log.flush()
+        final_state = replay.final_state()
+        self._publish_state(exp_avg, exp_avg_sq, self.n_epochs * len(bounds))
+        failed = int(status.item())
+        torch.set_rng_state(final_state if not failed else state_at_step(lib, init_state, n, bs, D, failed - 1))
+        if failed:
+            del self.loss_history[failed - 1:]
+            self._publish_state(exp_avg, exp_avg_sq, failed - 1)
+            raise torch.linalg.LinAlgError(
+                f"ConditionalNormal.fit: out.weight became singular after step {failed - 1} (linalg.inv: the input "
+                "matrix is singular); model and loss_history hold the state before the step that could not run")
+
+    def _publish_state(self, exp_avg, exp_avg_sq, steps):
+        """``opt.state`` as torch.optim.Adam leaves it: step, exp_avg, exp_avg_sq (views of the device moments) for
+        every tensor that had a gradient."""
+        self.opt.state.clear()
+        if steps <= 0:
+            return
+        off = 0
+        params = list(self.model.parameters())
+        n_grad = len(params) - (2 if self.independent_covariance else 0)
+        for i, p in enumerate(params):
+            numel = p.numel()
+            if i < n_grad:
+                self.opt.state[p] = {"step": torch.tensor(float(steps)),
+                                     "exp_avg": exp_avg[off:off + numel].view(p.shape),
+                                     "exp_avg_sq": exp_avg_sq[off:off + numel].view(p.shape)}
+            off += numel
+
+    def sample(self, C=100, seed=None, eps=None):
+        """Rows drawn for the conditions C [n, cond_size], or ``C`` rows with zero conditions if it is an int
+        (cnormal.py:219-240); float32 numpy [n, var_size].  Noise: ``eps`` [n, var_size] if given, else Philox keyed
+        on (seed, row, feature), ``seed`` drawn as one int64 from the global generator when not given (so the values
+        and the RNG state after the call are not the reference's; ``torch.manual_seed`` still makes it reproducible)."""
+        if getattr(self, "model", None) is None or not isinstance(self.model, Net):
+            raise RuntimeError("ConditionalNormal.sample: call fit() first")
+        if type(C) != type(1):
+            Cs = C
+        else:
+            Cs = torch.zeros(C, 1)
+        x_tilde, _, _, _ = self.model(None, Cs, eps=eps, seed=seed)
+        return x_tilde.cpu().numpy()
