@@ -252,6 +252,25 @@ extern "C" int rnvp_emul_tc_layout(int D, int Cd, int L, int H, int act, long lo
   return 0;
 }
 
+// Which tcgen05 image entries carry RNVP_IMG_SCALED.  out[4]: mapped entries of the forward W1 images, of them the
+// scaled ones, mapped entries of every other image, of them the scaled ones.
+extern "C" int rnvp_emul_img_scaled(int D, int Cd, int L, int H, int act, long long* out) {
+  FlowGeom g;
+  g.D = D; g.Cd = Cd; g.L = L; g.nh = 1; g.act = act; g.hidden[0] = H;
+  build_layout(&g);
+  if (!g.mma_ok) return -1;
+  std::vector<int> m2f;
+  build_mma_map(&g, m2f);
+  for (int k = 0; k < 4; ++k) out[k] = 0;
+  for (size_t m = 0; m < m2f.size(); ++m) {
+    if (m2f[m] < 0) continue;
+    const int q = (int)(m % g.m_layer_floats) < g.m_w1_floats ? 0 : 2;
+    out[q] += 1;
+    out[q + 1] += (m2f[m] & RNVP_IMG_SCALED) ? 1 : 0;
+  }
+  return 0;
+}
+
 extern "C" long long rnvp_emul_param_count(int D, int Cd, int L, int nh, const int* hidden) {
   FlowGeom g;
   g.D = D; g.Cd = Cd; g.L = L; g.nh = nh; g.act = 1;

@@ -120,3 +120,58 @@ def test_row_gather_and_ragged_tail(emul):
     idx = np.random.RandomState(0).permutation(X.shape[0])[:37].astype(np.int64)
     z, ld, lp, *_ = run(emul, 0, D, Cd, L, hidden, act, flat, X, Cn, 37, idx=idx)
     assert rel_err(lp, g["logp"][idx]) < TOL and rel_err(z, g["z"][idx]) < TOL
+
+
+RELU_TC_CASES = ["relu_odd_d9", "relu_dh16", "relu_dh32", "relu_dh64", "relu_d100_h96", "sigmoid_string_tc"]
+
+
+@pytest.mark.parametrize("name", RELU_TC_CASES)
+def test_programs_relu_tensor_core_shapes(emul, name):
+    """The FP32 tile programs (act = 2) of the ReLU flows whose tcgen05 kernels tests/test_gpu_relu.py compares with them."""
+    g = load_golden(name)
+    D, Cd, L, hidden, act = cfg(g)
+    assert act != "tanh"
+    nh = len(hidden)
+    if "N" in g:
+        seed, N = int(g["seed"]), int(g["N"])
+        p = O.init_params(D, Cd, L, hidden, seed=seed)
+        gen = torch.Generator().manual_seed(seed + 1000)
+        X, Cn, eps = (torch.randn(N, w, generator=gen).numpy() for w in (D, Cd, D))
+        idx, gvals, gmax = g["grad_idx"], g["grad_vals"], float(g["grad_absmax"])
+    else:
+        p = golden_params(g)
+        X, Cn, eps = (np.ascontiguousarray(g[k]) for k in ("X", "C", "eps"))
+        N = X.shape[0]
+        gvals = np.concatenate([g["g/" + k].reshape(-1) for k in O.param_order(L, nh)])
+        idx, gmax = np.arange(gvals.size), float(np.abs(gvals).max())
+    flat = flat_of(p, L, nh)
+    z, ld, lp, *_ = run(emul, 0, D, Cd, L, hidden, act, flat, X, Cn, N)
+    assert rel_err(z, g["z"]) < TOL and rel_err(ld, g["logdet"]) < TOL and rel_err(lp, g["logp"]) < TOL
+    x, *_ = run(emul, 1, D, Cd, L, hidden, act, flat, eps, Cn, N)
+    assert rel_err(x, g["sample"]) < TOL
+    _, _, lp2, gflat, loss_sum, _ = run(emul, 2, D, Cd, L, hidden, act, flat, X, Cn, N, scale=-1.0 / N)
+    assert rel_err(lp2, g["logp"]) < TOL
+    assert abs(-loss_sum / N - float(g["loss"])) < TOL * abs(float(g["loss"]))
+    assert np.max(np.abs(gflat[idx] - gvals)) < 2e-5 * gmax
+    for i in range(L):                                   # masked entries are exact zeros
+        mask = O.layer_mask(D, i).numpy()
+        gt = dict(zip(O.param_order(L, nh), np.split(gflat, np.cumsum([p[k].numel() for k in O.param_order(L, nh)])[:-1])))
+        for net in "ts":
+            w1 = gt[f"layers.{i}.nn_{net}.0.weight"].reshape(hidden[0], D + Cd)
+            assert np.all(w1[:, :D][:, mask == 0] == 0)
+            w2 = gt[f"layers.{i}.nn_{net}.{2 * nh}.weight"].reshape(D, hidden[-1])
+            assert np.all(w2[mask == 1] == 0) and np.all(gt[f"layers.{i}.nn_{net}.{2 * nh}.bias"][mask == 1] == 0)
+
+
+@pytest.mark.parametrize("D,Cd,L,H", [(9, 2, 3, 32), (32, 8, 4, 64), (64, 16, 3, 128), (128, 32, 2, 512), (100, 30, 2, 96)])
+def test_only_tanh_flows_prescale_the_forward_w1_image(emul, D, Cd, L, H):
+    """RNVP_IMG_SCALED marks every forward W1 image entry of a tanh flow (the tanh epilogue expects 2 log2(e) * a) and no
+    entry of a ReLU flow, whose epilogue applies max(a, 0) to the plain pre-activation."""
+    fn = emul.rnvp_emul_img_scaled
+    fn.argtypes = [C.c_int] * 5 + [C.POINTER(C.c_longlong)]
+    for act, scaled in ((1, True), (2, False)):
+        out = (C.c_longlong * 4)()
+        assert fn(D, Cd, L, H, act, out) == 0
+        w1, w1_scaled, other, other_scaled = list(out)
+        assert w1 > 0 and other > 0 and other_scaled == 0
+        assert w1_scaled == (w1 if scaled else 0), (act, list(out))
