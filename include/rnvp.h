@@ -185,9 +185,10 @@ int rnvp_host_gather_xc(const void* src_x, int x_is_f64, int64_t width_x, const 
                            const int64_t* idx, int64_t row0, int64_t n, float* dst_x, float* dst_c, int threads);
 int rnvp_host_copy(void* dst, const void* src, int64_t bytes, int threads);
 
-/* Development aid: when d_buf (device, >= 40 int64) is non-null and the library was built with -DRNVP_WG_TRACE, every
+/* Development aid: when d_buf (device, >= 43 int64) is non-null and the library was built with -DRNVP_WG_TRACE, every
  * role of CTA 0 of the tcgen05 weight-gradient sweep writes the cycles it spent in each of its mbarrier waits
- * (d_buf[role * 8 + wait site], see rnvp_wgrad_tc.cu; tools/trace_wgrad.py prints them).  Other builds ignore it. */
+ * (d_buf[role * 8 + wait site]; d_buf[40..42]: CTA 0's rows, rows per stage, cycles from entry to the end of its flush;
+ * see rnvp_wgrad_tc.cu; tools/trace_wgrad.py prints them).  Other builds ignore it. */
 int rnvp_debug_set_trace(void* d_buf);
 
 /* Tensor-core primitive self-test (tcgen05.mma kind::tf32, A in TMEM, B in shared memory):

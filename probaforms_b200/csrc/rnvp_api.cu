@@ -669,24 +669,28 @@ int rnvp_wgrad_sweep(const rnvp_desc* dc, const float* d_packed, int64_t Npad, c
     a.gR = d_records; a.rec = wgrad_rec_floats(d); a.Npad = Npad; a.H = d->hidden[0];
     a.K1P8 = K1P; a.K1 = d->mDH + d->Cd; a.TP = TP; a.Cd = d->Cd;
     a.n_mblocks = (2 * d->hidden[0] + 127) / 128;
+    const int NU = TP == 16 ? 32 : (TP == 32 ? 48 : 96);           // dW1 tile columns of the three kernel variants (>= K1P8)
+    const int rows = rnvp_wgrad_tc_rows(NU, TP);                   // rows per stage of that variant (the last stage may be short)
+    const long long stages = (Npad + rows - 1) / rows;
     {
-      // Row slices per (layer, unit block).  One wave of CTAs leaves num_sms % (L * n_mblocks) SMs idle (c3: 128 CTAs on
-      // 148 SMs); cutting finer fills whole waves but every CTA pays a fixed prologue (W2^T image, pipeline fill) and
-      // flush worth about 10 stages.  Pick the slice count with the best modelled efficiency.
-      const long long stages = Npad / 32, pairs = (long long)d->L * a.n_mblocks;
+      // Row slices per (layer, unit block), cut on stage boundaries.  One wave of CTAs leaves num_sms % (L * n_mblocks) SMs
+      // idle (c3: 128 CTAs on 148 SMs); cutting finer fills whole waves but every CTA pays a fixed prologue (W2^T image,
+      // pipeline fill) and flush worth about `fixed` stages (wait accounting of CTA 0, tools/trace_wgrad.py: 2.7-3.9 stages
+      // of 64 rows on c3; about 10 of 32 rows).  Pick the slice count with the best modelled efficiency.
+      const double fixed = rows == 64 ? 4.0 : 10.0;
+      const long long pairs = (long long)d->L * a.n_mblocks;
       double best = 0.0;
       int best_s = 1;
       for (long long s = 1; s <= std::min<long long>(stages, 64); ++s) {
         const long long ctas = pairs * s, waves = (ctas + d->num_sms - 1) / d->num_sms, per = (stages + s - 1) / s;
-        const double eff = (double)ctas / (double)(waves * d->num_sms) * (double)per / (double)(per + 10);
+        const double eff = (double)ctas / (double)(waves * d->num_sms) * (double)per / ((double)per + fixed);
         if (eff > best * 1.005) { best = eff; best_s = (int)s; }
       }
       a.n_slices = best_s;
     }
     a.gpacked = d_gpacked; a.packed = d_packed; a.act = d->act; a.layers = d->d_wg; a.trace = g_wg_trace;
     { const char* o = getenv("RNVP_WG_ONE_ISSUER"); a.one_issuer = (o && atoi(o)) ? 1 : 0; }
-    { const char* o = getenv("RNVP_WG_SLICES"); if (o && atoi(o) > 0) a.n_slices = (int)std::min<long long>(Npad / 32, atoi(o)); }
-    const int NU = TP == 16 ? 32 : (TP == 32 ? 48 : 96);           // dW1 tile columns of the three kernel variants (>= K1P8)
+    { const char* o = getenv("RNVP_WG_SLICES"); if (o && atoi(o) > 0) a.n_slices = (int)std::min<long long>(stages, atoi(o)); }
     cudaError_t e = rnvp_launch_wgrad_tc(NU, TP, a, d->L * a.n_mblocks * a.n_slices, (cudaStream_t)stream);
     return e == cudaSuccess ? 0 : cuda_fail(e, "rnvp_wgrad_tc_kernel");
   }

@@ -24,4 +24,5 @@ struct RnvpWgradTcArgs {
   long long* trace;                // development aid (rnvp_debug_set_trace): wait accounting of CTA 0
   int one_issuer;                  // development knob: issuer A also issues the dW2 products (issuer B idles)
 };
-size_t rnvp_wgrad_tc_smem_bytes(int NU, int TP, int NBUF, int NOP, int NSLOT, int K1P8, int NN);
+size_t rnvp_wgrad_tc_smem_bytes(int NU, int TP, int ROWS, int NBUF, int NOP, int NSLOT, int K1P8, int NN);
+int rnvp_wgrad_tc_rows(int NU, int TP);   // rows per stage of the kernel variant (NU, TP): slices are cut in such stages

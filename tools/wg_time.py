@@ -1,6 +1,6 @@
 """Time the weight-gradient sweep alone on the records of one c3 step (development aid)."""
-import sys, ctypes as C, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, ctypes as C, torch
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..'))
 from probaforms_b200.models import RealNVPLayer, NormalizingFlow
 dev = torch.device('cuda:0')
 D, Cd, L, H, N = 32, 8, 16, 128, 75776
