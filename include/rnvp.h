@@ -277,6 +277,51 @@ int rnvp_cn_fit_epoch(const rnvp_cn_desc* d, float* d_params, float* d_exp_avg, 
  * float32 does, for numel >= 16 (numel 32-bit draws, plus 16 when numel % 16 != 0); smaller numel: RNVP_EINVAL. */
 int rnvp_cn_rng_advance(uint8_t* state, int64_t state_bytes, int64_t numel);
 
+/* CVAE (rnvp_cvae.cu; probaforms/models/cvae.py).  Encoder: model = Linear(D + Cd, h0), act, ..., act, heads mu,
+ * log_sigma = Linear(h_last, latent); Decoder: model = Linear(latent + Cd, h0), act, ..., act, Linear(h_last, D)
+ * (cvae.py:14-110).  Parameters cross the boundary as one flat fp32 buffer in the order of the reference's Adam
+ * (cvae.py:173): encoder.model.{2k}.weight [h_k, h_{k-1}], encoder.model.{2k}.bias, encoder.mu.weight, .bias,
+ * encoder.log_sigma.weight, .bias, then decoder.model.{2k}.weight, .bias and decoder.model.{2 nh}.weight [D, h_last],
+ * .bias.  act: RNVP_ACT_TANH or _RELU (every other activation string is ReLU upstream, cvae.py:27-32).  Cd may be 0 (the
+ * reference's C=None, cvae.py:158-161); d_C may then be NULL.  Shapes: D <= 128, Cd <= 256, latent <= 128, 1 to 4
+ * hidden layers of width <= 512 (RNVP_ESHAPE otherwise).  eps buffers are [N][latent], indexed by batch position. */
+typedef struct rnvp_cv_desc rnvp_cv_desc;
+int rnvp_cv_desc_create(int D, int Cd, int latent, int n_hidden, const int* hidden, int act, rnvp_cv_desc** out);
+void rnvp_cv_desc_destroy(rnvp_cv_desc* d);
+int64_t rnvp_cv_param_count(const rnvp_cv_desc* d);
+/* scratch bytes for gradient batches of up to batch_rows rows (per-CTA gradient partials) and loss passes of up to
+ * loss_rows rows (per-CTA loss partials) */
+int64_t rnvp_cv_workspace_bytes(const rnvp_cv_desc* d, int64_t batch_rows, int64_t loss_rows);
+/* Encoder.forward for inference (cvae.py:38-62): d_mu, d_log_sigma [N][latent] of the rows [X | C] */
+int rnvp_cv_encode(const rnvp_cv_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
+                   float* d_mu, float* d_log_sigma, void* stream);
+/* Decoder.forward for inference (cvae.py:89-110): d_x [N][D] of the rows [Z | C]; Z is d_Z [N][latent] when given
+ * (parity mode), else Philox normals keyed on (seed, row_offset + row, j) as in rnvp_sample (replaces the CPU
+ * torch.normal of sample, cvae.py:283-290) */
+int rnvp_cv_decode(const rnvp_cv_desc* d, const float* d_params, const float* d_Z, const float* d_C, int64_t N,
+                   uint64_t seed, int64_t row_offset, float* d_x, void* stream);
+/* compute_loss (cvae.py:190-199) and its gradient on the N rows X[idx[r]], C[idx[r]] (d_idx may be NULL) with the
+ * caller's eps (sample_z, cvae.py:181-183): d_gflat [P] in the flat layout, *d_loss (may be NULL).
+ * Workspace: rnvp_cv_workspace_bytes(d, N, 0). */
+int rnvp_cv_grad(const rnvp_cv_desc* d, const float* d_params, const float* d_X, const float* d_C,
+                 const int64_t* d_idx, const float* d_eps, int64_t N, double kl_weight, float* d_gflat, float* d_loss,
+                 void* d_workspace, int64_t workspace_bytes, void* stream);
+/* compute_loss alone (forward only) into *d_loss.  Workspace: rnvp_cv_workspace_bytes(d, 0, N). */
+int rnvp_cv_loss(const rnvp_cv_desc* d, const float* d_params, const float* d_X, const float* d_C,
+                 const int64_t* d_idx, const float* d_eps, int64_t N, double kl_weight, float* d_loss,
+                 void* d_workspace, int64_t workspace_bytes, void* stream);
+/* One epoch of CVAE.fit (cvae.py:232-255) as one call: for every consecutive batch_size slice of d_perm (last partial
+ * batch kept), loss + gradient + torch.optim.Adam step (step count step0 + 1, ...), then compute_loss over all n rows
+ * in dataset order into *d_loss.  Noise: d_noise holds every step's [nb][latent] eps in step order followed by the
+ * [n][latent] eps of the epoch loss; when NULL, Philox keyed on (seed, position in the epoch order, j) for the steps and
+ * (seed, n + row, j) for the epoch loss.  A batch of at most the kernel's tile (64 rows for small nets) is one launch.
+ * Workspace: rnvp_cv_workspace_bytes(d, min(batch_size, n), n). */
+int rnvp_cv_fit_epoch(const rnvp_cv_desc* d, float* d_params, float* d_exp_avg, float* d_exp_avg_sq, const float* d_X,
+                      const float* d_C, const int64_t* d_perm, int64_t n, int64_t batch_size, double lr, double beta1,
+                      double beta2, double eps, double weight_decay, double kl_weight, int64_t step0,
+                      const float* d_noise, uint64_t seed, float* d_loss, void* d_workspace, int64_t workspace_bytes,
+                      void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

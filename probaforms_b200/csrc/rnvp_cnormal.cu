@@ -20,6 +20,7 @@
 
 #include "../../include/rnvp.h"
 #include "rnvp_adam.cuh"
+#include "rnvp_mlp.cuh"
 #include "rnvp_philox.cuh"
 
 int rnvp_fail(int code, const char* msg);   // rnvp_api.cu: sets rnvp_last_error()
@@ -71,73 +72,6 @@ __device__ __forceinline__ CnTile carve(const CnShape& s, float* sm) {
   t.z = sm; sm += R * t.ldd;
   t.xb = sm;
   return t;
-}
-
-__device__ __forceinline__ float act_f(int act, float x) {
-  if (act == RNVP_ACT_TANH) return tanhf(x);
-  if (act == RNVP_ACT_SIGMOID) return 1.0f / (1.0f + expf(-x));
-  return fmaxf(x, 0.0f);
-}
-// derivative from the activation's OUTPUT y
-__device__ __forceinline__ float act_d(int act, float y) {
-  if (act == RNVP_ACT_TANH) return fmaf(-y, y, 1.0f);
-  if (act == RNVP_ACT_SIGMOID) return y * (1.0f - y);
-  return y > 0.0f ? 1.0f : 0.0f;
-}
-
-// out[r][i] = act?(b[i] + sum_j in[r][j] W[i][j]) for r < nr, i < no; consecutive threads walk rows (W is warp-uniform)
-__device__ __forceinline__ void dense_rows(const float* __restrict__ in, int ldi, int ni, const float* __restrict__ W,
-                                  const float* __restrict__ bias, float* out, int ldo, int no, int nr, int act) {
-  for (int t = threadIdx.x; t < nr * no; t += blockDim.x) {
-    const int i = t / nr, r = t - i * nr;
-    const float* x = in + r * ldi;
-    const float* w = W + (size_t)i * ni;
-    float acc = bias[i];
-    for (int j = 0; j < ni; ++j) acc = fmaf(x[j], __ldg(w + j), acc);
-    out[r * ldo + i] = act ? act_f(act, acc) : acc;
-  }
-}
-
-// gW[i][j] = sum_r dA[r][i] in[r][j], gb[i] = sum_r dA[r][i] (rows in order: the sums are deterministic)
-__device__ __forceinline__ void wgrad(const float* dA, int lda, int no, const float* in, int ldi, int ni, int nr,
-                             float* __restrict__ gW, float* __restrict__ gb) {
-  for (int t = threadIdx.x; t < no * ni; t += blockDim.x) {
-    const int i = t / ni, j = t - i * ni;
-    float acc = 0.0f;
-    for (int r = 0; r < nr; ++r) acc = fmaf(dA[r * lda + i], in[r * ldi + j], acc);
-    gW[t] = acc;
-  }
-  if (gb)
-    for (int i = threadIdx.x; i < no; i += blockDim.x) {
-      float acc = 0.0f;
-      for (int r = 0; r < nr; ++r) acc += dA[r * lda + i];
-      gb[i] = acc;
-    }
-}
-
-// dIn[r][j] = (sum_i dA[r][i] W[i][j]) * act'(In[r][j]), written over In (each element reads only itself)
-__device__ __forceinline__ void back_rows(const float* dA, int lda, int no, const float* __restrict__ W, float* io, int ldi,
-                                 int ni, int nr, int act) {
-  for (int t = threadIdx.x; t < nr * ni; t += blockDim.x) {
-    const int j = t / nr, r = t - j * nr;
-    const float* g = dA + r * lda;
-    float acc = 0.0f;
-    for (int i = 0; i < no; ++i) acc = fmaf(g[i], __ldg(W + (size_t)i * ni + j), acc);
-    io[r * ldi + j] = acc * act_d(act, io[r * ldi + j]);
-  }
-}
-
-// deterministic block sum of one value per thread (fixed tree); result valid in every thread
-__device__ __forceinline__ float block_sum(float v, float* scratch) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const int w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  __syncthreads();
-  if ((threadIdx.x & 31) == 0) scratch[w] = v;
-  __syncthreads();
-  float s = 0.0f;
-  for (int k = 0; k < nw; ++k) s += scratch[k];
-  __syncthreads();
-  return s;
 }
 
 __device__ __forceinline__ void load_tile(const CnShape& s, const CnTile& t, const float* __restrict__ params,
@@ -454,12 +388,6 @@ struct rnvp_cn_desc {
 namespace {
 
 int check_cn(const rnvp_cn_desc* d) { return d ? 0 : rnvp_fail(RNVP_EINVAL, "null ConditionalNormal descriptor"); }
-
-RnvpAdamCoef adam_coef(double lr, double b1, double b2, double eps, double wd, int64_t step) {
-  const double bc1 = 1.0 - pow(b1, (double)step), bc2 = 1.0 - pow(b2, (double)step);
-  return RnvpAdamCoef{(float)wd, (float)(1.0 - b1), (float)b2, (float)(1.0 - b2), (float)(lr / bc1), (float)sqrt(bc2),
-                      (float)eps};
-}
 
 cudaError_t launch_step(const rnvp_cn_desc* d, float* params, float* m, float* v, float* M, const float* X,
                         const float* C, const int64_t* idx, int64_t nb, float* gflat, float* loss_dst, int* status,

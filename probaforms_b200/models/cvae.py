@@ -1,0 +1,553 @@
+"""Conditional VAE with the reference's API (probaforms/models/cvae.py:14-292).
+
+Same constructor, defaults, public attributes (``encoder``, ``decoder``, ``opt``, ``criterion``, ``loss_history``,
+``lat_size``, ...), ``fit(X, C)`` / ``sample(C)``, ``sample_z`` / ``custom_loss`` / ``compute_loss`` and
+``state_dict`` keys (``encoder.model.{2k}.*``, ``encoder.mu.*``, ``encoder.log_sigma.*``, ``decoder.model.{2k}.*``)
+as ``probaforms.models.CVAE``; the arithmetic runs in the FP32 kernels of ``rnvp_cvae.cu``.
+
+``fit`` reproduces the reference's training run: the encoder and decoder are built on the CPU under the global
+generator (same initial parameters), every epoch's batches are the reference's ``DataLoader(shuffle=True)`` batches,
+Adam is the reference's, and the global torch RNG is left exactly where the reference leaves it.  The latent noise
+drives training, so by default (``noise='torch'``) a helper thread draws the reference's own values -- every step's
+``torch.randn(nb, latent)``, then the end-of-epoch ``torch.randn(n, latent)`` -- on a private generator cloned after
+init, one epoch ahead of the GPU.  A whole epoch, its end-of-epoch loss included, is one library call; a batch of up to
+64 rows (the default ``batch_size`` is 32) is one kernel launch.
+
+``noise='device'`` draws the latent noise from Philox inside the kernels instead, keyed on the epoch's sampler seed
+(which the reference draws anyway) and the row's position in the epoch; the helper thread then only skips the
+reference's normals in the generator state.  The global RNG state after ``fit`` is still the reference's, but the
+training trajectory is a different (equally distributed) one.  The default mode is bound by the host's ``torch.randn``
+for large batches; the device mode is not.
+
+``sample`` differs from the reference in its noise: one int64 is drawn from the global generator per call and the
+latent normals come from Philox keyed on (seed, row, latent index) inside the kernel, as in ``RealNVP.sample``; ``z=``
+supplies the reference's noise for parity.  ``Encoder.forward`` and ``Decoder.forward`` are inference-only (no
+autograd).  CUDA only; there is no CPU fallback.
+"""
+import ctypes as ct
+import threading
+
+import numpy as np
+import torch
+import torch.nn as nn
+
+from .interfaces import GenModel
+from .realnvp import _LossLog, _default_device
+from .cnormal import _stream, advance
+from .. import _lib
+from ..batching import StreamingPermutation, batch_bounds
+
+
+def _act_code(activation):
+    return 1 if activation == 'tanh' else 2          # include/rnvp.h RNVP_ACT_*: every other string is ReLU upstream
+
+
+def _layers(n_inputs, hidden, activation):
+    layers = []
+    for i in range(len(hidden)):
+        layers.append(nn.Linear(n_inputs if i == 0 else hidden[i - 1], hidden[i]))
+        layers.append(nn.Tanh() if activation == 'tanh' else nn.ReLU())
+    return layers
+
+
+class _Desc:
+    """Owns one ``rnvp_cv_desc`` (shape and activation of an encoder-decoder pair) on the current CUDA device."""
+
+    def __init__(self, D, Cd, latent, hidden, activation):
+        self.lib = _lib.load()
+        hid = (ct.c_int * len(hidden))(*hidden)
+        h = ct.c_void_p()
+        rc = self.lib.rnvp_cv_desc_create(D, Cd, latent, len(hidden), hid, _act_code(activation), ct.byref(h))
+        if rc != 0:
+            msg = self.lib.rnvp_last_error().decode()
+            if rc in (-1, -2):                             # RNVP_EINVAL, RNVP_ESHAPE
+                raise ValueError(msg)
+            raise _lib.RnvpError(f"rnvp_cv_desc_create failed (code {rc}): {msg}")
+        self.h, self.D, self.Cd, self.L = h, D, Cd, latent
+        self.P = int(self.lib.rnvp_cv_param_count(h))
+
+    def workspace(self, batch_rows, loss_rows, dev):
+        nbytes = int(self.lib.rnvp_cv_workspace_bytes(self.h, int(batch_rows), int(loss_rows)))
+        return torch.empty(max(nbytes, 4) // 4, dtype=torch.float32, device=dev), nbytes
+
+    def __del__(self):
+        if getattr(self, "h", None):
+            self.lib.rnvp_cv_desc_destroy(self.h)
+            self.h = None
+
+
+class _Pair:
+    """The device side of one encoder-decoder pair: the descriptor and one flat fp32 buffer of which every parameter
+    of both modules is a view (``encoder.parameters()`` then ``decoder.parameters()``, the layout the kernels read)."""
+
+    def __init__(self, encoder, decoder, D, Cd, dev):
+        self.encoder, self.decoder, self.D, self.Cd = encoder, decoder, D, Cd
+        with torch.cuda.device(dev):
+            self.desc = _Desc(D, Cd, encoder.lat_size, encoder.hidden, encoder.activation)
+        self.flat = None
+        self.pack(dev)
+
+    def params(self):
+        return list(self.encoder.parameters()) + list(self.decoder.parameters())
+
+    def pack(self, dev):
+        params = self.params()
+        flat = torch.cat([p.detach().reshape(-1).to(torch.float32) for p in params]).to(dev)
+        off = 0
+        for p in params:
+            n = p.numel()
+            p.data = flat[off:off + n].view(p.shape)
+            off += n
+        self.flat = flat
+
+    def ready(self):
+        """(desc, flat); re-packs when a parameter is no longer a view of ``flat`` (e.g. after ``Module.to``)."""
+        params = self.params()
+        off, ok = 0, True
+        for p in params:
+            if p.device.type != "cuda" or p.data_ptr() != self.flat.data_ptr() + 4 * off:
+                ok = False
+                break
+            off += p.numel()
+        if not ok:
+            p = params[0]
+            self.pack(p.device if p.device.type == "cuda" else _default_device())
+        return self.desc, self.flat
+
+
+def _rows(A, dev, width, what):
+    """A [n, width] float32 contiguous device tensor; RuntimeError on a width mismatch, as the reference's Linear."""
+    t = torch.as_tensor(A, dtype=torch.float32).to(dev).contiguous()
+    if t.dim() != 2 or t.shape[1] != width:
+        raise RuntimeError(f"{what} must be [n, {width}], got shape {tuple(t.shape)}")
+    return t
+
+
+class Encoder(nn.Module):
+    """The reference's Encoder (cvae.py:14-62): ``model`` = Linear, act, ..., act; heads ``mu`` and ``log_sigma``.
+
+    'tanh' gives Tanh and every other string ReLU, as upstream.  The modules hold the parameters (built on the CPU, so
+    names, shapes, default init and RNG order are the reference's).  ``forward`` runs in the kernels of the ``CVAE``
+    that owns the module (after ``fit``)."""
+
+    def __init__(self, n_inputs, lat_size, hidden=(10,), activation='tanh'):
+        super().__init__()
+        self.n_inputs, self.lat_size = n_inputs, lat_size
+        self.hidden, self.activation = tuple(hidden), activation
+        self.model = nn.Sequential(*_layers(n_inputs, hidden, activation))
+        self.mu = nn.Linear(hidden[-1], lat_size)
+        self.log_sigma = nn.Linear(hidden[-1], lat_size)
+        self._pair = None
+
+    def __getstate__(self):
+        state = self.__dict__.copy()
+        state["_pair"] = None
+        return state
+
+    @torch.no_grad()
+    def forward(self, X, C=None):
+        """(mu, log_sigma) [n, lat_size] of the rows [X | C] (cvae.py:38-62), computed by one inference kernel."""
+        if self._pair is None:
+            raise RuntimeError("Encoder.forward runs on the kernels of a fitted CVAE; call CVAE.fit first")
+        desc, flat = self._pair.ready()
+        dev = flat.device
+        Xd = _rows(X, dev, desc.D, "X")
+        n = Xd.shape[0]
+        Cd = None
+        if C is not None:
+            Cd = _rows(C, dev, desc.Cd, "C")
+            if Cd.shape[0] != n:
+                raise RuntimeError(f"C must have {n} rows, got {Cd.shape[0]}")
+        if (Cd is None) != (desc.Cd == 0):
+            raise RuntimeError(f"the encoder takes {desc.D + desc.Cd} input columns")
+        mu = torch.empty(n, desc.L, dtype=torch.float32, device=dev)
+        ls = torch.empty(n, desc.L, dtype=torch.float32, device=dev)
+        _lib.check(desc.lib.rnvp_cv_encode(desc.h, flat.data_ptr(), Xd.data_ptr(), None if Cd is None else Cd.data_ptr(),
+                                           n, mu.data_ptr(), ls.data_ptr(), _stream(dev)), "rnvp_cv_encode")
+        return mu, ls
+
+
+class Decoder(nn.Module):
+    """The reference's Decoder (cvae.py:66-110): ``model`` = Linear, act, ..., act, Linear.  ``forward`` runs in the
+    kernels of the ``CVAE`` that owns the module (after ``fit``)."""
+
+    def __init__(self, n_inputs, n_outputs, hidden=(10,), activation='tanh'):
+        super().__init__()
+        self.n_inputs, self.n_outputs = n_inputs, n_outputs
+        self.hidden, self.activation = tuple(hidden), activation
+        self.model = nn.Sequential(*_layers(n_inputs, hidden, activation), nn.Linear(hidden[-1], n_outputs))
+        self._pair = None
+
+    def __getstate__(self):
+        state = self.__dict__.copy()
+        state["_pair"] = None
+        return state
+
+    @torch.no_grad()
+    def forward(self, X, C=None):
+        """X_rec [n, n_outputs] of the rows [X | C] (cvae.py:89-110), X the latent [n, lat_size]."""
+        return self._decode(X, C, None, None)
+
+    def _decode(self, Z, C, n, seed):
+        if self._pair is None:
+            raise RuntimeError("Decoder.forward runs on the kernels of a fitted CVAE; call CVAE.fit first")
+        desc, flat = self._pair.ready()
+        dev = flat.device
+        Zd = None
+        if Z is not None:
+            Zd = _rows(Z, dev, desc.L, "the latent")
+            n = Zd.shape[0]
+        Cd = None
+        if C is not None:
+            Cd = _rows(C, dev, desc.Cd, "C")
+            n = Cd.shape[0] if n is None else n
+            if Cd.shape[0] != n:
+                raise RuntimeError(f"C must have {n} rows, got {Cd.shape[0]}")
+        if (Cd is None) != (desc.Cd == 0):
+            raise RuntimeError(f"mat1 and mat2 shapes cannot be multiplied: the decoder takes {desc.L + desc.Cd} input "
+                               f"columns, got {desc.L + (0 if Cd is None else Cd.shape[1])}")
+        if seed is None:
+            seed = 0
+        x = torch.empty(n, desc.D, dtype=torch.float32, device=dev)
+        _lib.check(desc.lib.rnvp_cv_decode(desc.h, flat.data_ptr(), None if Zd is None else Zd.data_ptr(),
+                                           None if Cd is None else Cd.data_ptr(), n,
+                                           ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), 0, x.data_ptr(), _stream(dev)),
+                   "rnvp_cv_decode")
+        return x
+
+
+class _NoiseReplay:
+    """The reference's use of the global torch generator during ``fit``, replayed on a helper thread.
+
+    Per epoch the reference's fresh ``DataLoader(shuffle=True)`` draws two int64 (the second seeds the row order), every
+    step's ``sample_z`` draws ``torch.randn(nb, latent)`` and the end-of-epoch ``compute_loss`` draws
+    ``torch.randn(n, latent)``.  The replay runs on a private generator cloned from the global state after init.  With
+    ``values`` the normals are drawn with ``torch.randn`` into one of two pinned buffers (steps in order, then the
+    epoch-end rows), which the fit loop uploads; a buffer is refilled only after the upload of two epochs ago has
+    completed.  Without ``values`` they are skipped in the generator state (``advance``)."""
+
+    def __init__(self, lib, n, bs, L, n_epochs, values):
+        self.lib, self.n, self.L, self.values = lib, n, L, values
+        self.gen = torch.Generator()
+        self.gen.set_state(torch.get_rng_state())
+        self.steps = [nb for _, nb in batch_bounds(n, bs)]
+        self.bufs = [None, None]
+        if values:
+            k = min(n_epochs, 2)
+            pin = torch.cuda.is_available()
+            self.bufs = [torch.empty(2 * n * L, dtype=torch.float32, pin_memory=pin) for _ in range(k)] + [None] * (2 - k)
+        self.seeds, self.released = [], {}
+        self._cv = threading.Condition()
+        self._err, self._closed = None, False
+        self._thread = threading.Thread(target=self._run, args=(n_epochs,), daemon=True)
+        self._thread.start()
+
+    def _run(self, n_epochs):
+        try:
+            L = self.L
+            for e in range(n_epochs):
+                torch.empty((), dtype=torch.int64).random_(generator=self.gen)
+                seed = int(torch.empty((), dtype=torch.int64).random_(generator=self.gen).item())
+                if self.values:
+                    if e >= 2:
+                        with self._cv:
+                            while e - 2 not in self.released and not self._closed:
+                                self._cv.wait()
+                            if self._closed:
+                                return
+                            ev = self.released.pop(e - 2)
+                        ev.synchronize()
+                    buf, off = self.bufs[e & 1], 0
+                    for nb in self.steps + [self.n]:
+                        torch.randn(nb, L, generator=self.gen, out=buf[off:off + nb * L].view(nb, L))
+                        off += nb * L
+                else:
+                    advance(self.lib, self.gen, [nb * L for nb in self.steps] + [self.n * L])
+                with self._cv:
+                    self.seeds.append(seed)
+                    self._cv.notify_all()
+        except Exception as e:                                              # pragma: no cover
+            with self._cv:
+                self._err = e
+                self._cv.notify_all()
+
+    def get(self, epoch):
+        """(sampler seed, pinned noise buffer or None) of ``epoch``, once the helper thread has produced them."""
+        with self._cv:
+            while len(self.seeds) <= epoch and self._err is None:
+                self._cv.wait()
+            if self._err is not None:
+                raise self._err
+            return self.seeds[epoch], self.bufs[epoch & 1]
+
+    def release(self, epoch, event):
+        """The upload of ``epoch``'s buffer completes with ``event``; the buffer may then be refilled."""
+        with self._cv:
+            self.released[epoch] = event
+            self._cv.notify_all()
+
+    def close(self):
+        with self._cv:
+            self._closed = True
+            self._cv.notify_all()
+        self._thread.join()
+
+    def final_state(self):
+        self._thread.join()
+        if self._err is not None:
+            raise self._err
+        return self.gen.get_state()
+
+
+def epoch_plan(lib, n, bs, L, n_epochs, values=True):
+    """Host-only replay of ``fit``'s RNG use from the current global state (a test and inspection aid): returns the
+    per-epoch sampler seeds, epoch 0's noise (every step's ``randn(nb, latent)`` in order, then ``randn(n, latent)``;
+    None without ``values``) and the generator state the reference leaves behind.  The global state is not changed."""
+    rp = _NoiseReplay(lib, n, bs, L, n_epochs, values)
+    eps0 = None
+    try:
+        for e in range(n_epochs):
+            _, buf = rp.get(e)
+            if e == 0 and buf is not None:
+                eps0 = buf.clone()
+            rp.release(e, _Done())
+        state = rp.final_state()
+    finally:
+        rp.close()
+    return list(rp.seeds), eps0, state
+
+
+class _Done:
+    """A completed upload (host-only replays have none to wait for)."""
+
+    @staticmethod
+    def synchronize():
+        pass
+
+
+class CVAE(GenModel):
+    """Conditional VAE model (reference cvae.py:113-292); parameters as upstream:
+
+    latent_dim, hidden, activation ('tanh'; anything else is ReLU), batch_size, n_epochs, lr, weight_decay, KL_weight,
+    verbose (>0: progress bar over epochs).  New: ``noise`` -- 'torch' (default: the reference's latent noise values
+    from the global generator's stream, drawn on the host) or 'device' (Philox in the kernels; the global RNG state
+    after ``fit`` is still the reference's, the trajectory is not).
+    """
+
+    def __init__(self, latent_dim=2, hidden=(10,), activation='tanh', batch_size=32, n_epochs=10, lr=0.0001,
+                 weight_decay=0, KL_weight=0.001, verbose=0, noise='torch'):
+        super().__init__()
+        self.lat_size = latent_dim
+        self.hidden = hidden
+        self.activation = activation
+        self.batch_size = batch_size
+        self.n_epochs = n_epochs
+        self.latent_dim = latent_dim
+        self.lr = lr
+        self.weight_decay = weight_decay
+        self.KL_weight = KL_weight
+        self.verbose = verbose
+        self.noise = noise
+        self.criterion = nn.MSELoss()
+        self.opt = None
+        self._device = None
+        self._perm_host = [None, None]
+
+    def _model_init(self, X, C=None):
+        c_len = 0 if C is None else C.shape[1]
+        self.encoder = Encoder(n_inputs=X.shape[1] + c_len, lat_size=self.lat_size, hidden=self.hidden,
+                               activation=self.activation)
+        self.decoder = Decoder(n_inputs=self.lat_size + c_len, n_outputs=X.shape[1], hidden=self.hidden,
+                               activation=self.activation)
+        self.opt = torch.optim.Adam(list(self.encoder.parameters()) + list(self.decoder.parameters()), lr=self.lr,
+                                    weight_decay=self.weight_decay)
+        if self._device is None:
+            self._device = _default_device()
+        self._attach(X.shape[1], c_len, self._device)
+
+    def _attach(self, D, Cd, dev):
+        pair = _Pair(self.encoder, self.decoder, D, Cd, dev)
+        self.encoder._pair = self.decoder._pair = pair
+
+    def _ready(self):
+        if getattr(self, "encoder", None) is None or not isinstance(self.encoder, Encoder):
+            raise RuntimeError("CVAE: call fit() first")
+        if self.encoder._pair is None:                   # e.g. after unpickling
+            D = self.decoder.n_outputs
+            p = self.encoder.mu.weight
+            self._attach(D, self.encoder.n_inputs - D, p.device if p.device.type == "cuda" else _default_device())
+        return self.encoder._pair.ready()
+
+    def sample_z(self, mu, log_sigma):
+        eps = torch.randn(mu.shape).to(mu.device)
+        return mu + torch.exp(log_sigma / 2) * eps
+
+    def custom_loss(self, x, rec_x, mu, log_sigma):
+        KL = torch.mean(-0.5 * torch.sum(1 + log_sigma - mu ** 2 - log_sigma.exp(), dim=1), dim=0)
+        recon_loss = self.criterion(x, rec_x)
+        return KL * self.KL_weight + recon_loss
+
+    def _batch(self, x_batch, cond_batch):
+        desc, flat = self._ready()
+        dev = flat.device
+        Xd = _rows(x_batch, dev, desc.D, "x_batch")
+        Cd = None
+        if cond_batch is not None:
+            Cd = _rows(cond_batch, dev, desc.Cd, "cond_batch")
+        if (Cd is None) != (desc.Cd == 0) or (Cd is not None and Cd.shape[0] != Xd.shape[0]):
+            raise RuntimeError(f"x_batch must be [n, {desc.D}] and cond_batch [n, {desc.Cd}] (None when 0)")
+        return desc, flat, Xd, Cd
+
+    def compute_loss(self, x_batch, cond_batch):
+        """The reference's loss on one batch (cvae.py:190-199): its eps is ``torch.randn`` from the global generator,
+        as upstream; the encoder, decoder and loss run in the loss kernel (a 0-d device tensor, no autograd graph)."""
+        desc, flat, Xd, Cd = self._batch(x_batch, cond_batch)
+        dev, n = flat.device, Xd.shape[0]
+        eps = torch.randn(n, desc.L).to(dev)
+        ws, nbytes = desc.workspace(0, n, dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        _lib.check(desc.lib.rnvp_cv_loss(desc.h, flat.data_ptr(), Xd.data_ptr(), None if Cd is None else Cd.data_ptr(),
+                                         None, eps.data_ptr(), n, float(self.KL_weight), loss.data_ptr(),
+                                         ws.data_ptr(), nbytes, _stream(dev)), "rnvp_cv_loss")
+        return loss
+
+    def _grad(self, Xd, Cd, eps, idx=None):
+        """(loss, flat gradient) of one batch with the noise ``eps`` [n, latent] through rnvp_cv_grad."""
+        desc, flat = self._ready()
+        dev = flat.device
+        n = idx.numel() if idx is not None else Xd.shape[0]
+        eps = torch.as_tensor(eps, dtype=torch.float32).to(dev).contiguous()
+        ws, nbytes = desc.workspace(n, 0, dev)
+        g = torch.empty(desc.P, dtype=torch.float32, device=dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        _lib.check(desc.lib.rnvp_cv_grad(desc.h, flat.data_ptr(), Xd.data_ptr(), None if Cd is None else Cd.data_ptr(),
+                                         None if idx is None else idx.data_ptr(), eps.data_ptr(), n,
+                                         float(self.KL_weight), g.data_ptr(), loss.data_ptr(), ws.data_ptr(), nbytes,
+                                         _stream(dev)), "rnvp_cv_grad")
+        return loss, g
+
+    def fit(self, X, C=None):
+        """Fit on X [n, var_size], conditions C [n, cond_size] or None (cvae.py:201-261).  Rebuilds the encoder,
+        decoder and Adam on every call, as upstream.  ``loss_history`` gets one 0-d CPU tensor per epoch: the loss
+        over all rows after the epoch's steps.  Returns ``self``."""
+        from ..ingest import upload_resident
+        if self.noise not in ("torch", "device"):
+            raise ValueError(f"noise must be 'torch' or 'device', got {self.noise!r}")
+        if not hasattr(X, "shape"):
+            X = np.asarray(X)
+        if len(tuple(X.shape)) != 2 or X.shape[0] < 1:
+            raise ValueError(f"X must be 2-D [n, var_size] with n >= 1, got shape {tuple(X.shape)}")
+        n = X.shape[0]
+        if C is not None:
+            if not hasattr(C, "shape"):
+                C = np.asarray(C)
+            if len(tuple(C.shape)) != 2 or C.shape[0] != n:
+                raise ValueError(f"C must be 2-D with {n} rows, got shape {tuple(C.shape)}")
+        bs = int(self.batch_size)
+        if bs < 1:
+            raise ValueError("batch_size must be >= 1")
+        if self._device is None:
+            self._device = _default_device()
+        self._model_init(X, C)
+        dev = self._device
+        desc, flat = self._ready()
+        lib, L = desc.lib, desc.L
+        self.encoder.train(True)
+        self.decoder.train(True)
+        self.loss_history = []
+        values = self.noise == "torch"
+        replay = _NoiseReplay(lib, n, bs, L, self.n_epochs, values)
+        try:
+            Xd = upload_resident(lib, X, dev)
+            Cd = upload_resident(lib, C, dev) if desc.Cd else None
+            P = desc.P
+            exp_avg = torch.zeros(P, dtype=torch.float32, device=dev)
+            exp_avg_sq = torch.zeros(P, dtype=torch.float32, device=dev)
+            ws, nbytes = desc.workspace(min(bs, n), n, dev)
+            perm_dev = [torch.empty(n, dtype=torch.int64, device=dev) for _ in range(2)]
+            eps_dev = torch.empty(2 * n * L, dtype=torch.float32, device=dev) if values else None
+            losses = torch.empty(max(self.n_epochs, 1), dtype=torch.float32, device=dev)
+            copied = [None, None]
+            n_steps = len(batch_bounds(n, bs))
+            log = _LossLog(self.loss_history)
+            epochs = range(self.n_epochs)
+            bar = None
+            if self.verbose >= 1:
+                from tqdm.auto import tqdm
+                bar = tqdm(epochs, unit='epoch')
+                epochs = bar
+            stream = _stream(dev)
+            nxt = None
+            if self.n_epochs > 0:
+                nxt = StreamingPermutation(lib, replay.get(0)[0], n, host=self._perm_host[0])
+            for ep in epochs:
+                seed, buf = replay.get(ep)
+                sp = nxt
+                self._perm_host[ep & 1] = sp.host
+                k = ep & 1
+                perm_dev[k].copy_(sp.full(), non_blocking=True)
+                if values:
+                    eps_dev.copy_(buf, non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record(torch.cuda.current_stream(dev))
+                copied[k] = ev
+                if values:
+                    replay.release(ep, ev)
+                _lib.check(lib.rnvp_cv_fit_epoch(desc.h, flat.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
+                                                 Xd.data_ptr(), None if Cd is None else Cd.data_ptr(),
+                                                 perm_dev[k].data_ptr(), n, bs, self.lr, 0.9, 0.999, 1e-8,
+                                                 self.weight_decay, float(self.KL_weight), ep * n_steps,
+                                                 None if eps_dev is None else eps_dev.data_ptr(),
+                                                 ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), losses[ep:].data_ptr(),
+                                                 ws.data_ptr(), nbytes, stream), "rnvp_cv_fit_epoch")
+                if ep + 1 < self.n_epochs:
+                    # the next order is shuffled into the other host buffer while this epoch runs; that buffer's last
+                    # copy (two epochs ago) must have left it
+                    if copied[k ^ 1] is not None:
+                        copied[k ^ 1].synchronize()
+                    nxt = StreamingPermutation(lib, replay.get(ep + 1)[0], n, host=self._perm_host[(ep + 1) & 1])
+                host = log.push(losses[ep:ep + 1])
+                if bar is not None and host is not None:
+                    bar.set_description(f"loss: {float(host[-1]):.4f}")
+            log.flush()
+            final_state = replay.final_state()
+        finally:
+            replay.close()
+        self._publish_state(exp_avg, exp_avg_sq, self.n_epochs * n_steps)
+        torch.set_rng_state(final_state)
+        self.encoder.train(False)
+        self.decoder.train(False)
+        return self
+
+    def _publish_state(self, exp_avg, exp_avg_sq, steps):
+        """``opt.state`` as torch.optim.Adam leaves it: step, exp_avg, exp_avg_sq (views of the device moments)."""
+        self.opt.state.clear()
+        if steps <= 0:
+            return
+        off = 0
+        for p in list(self.encoder.parameters()) + list(self.decoder.parameters()):
+            numel = p.numel()
+            self.opt.state[p] = {"step": torch.tensor(float(steps)),
+                                 "exp_avg": exp_avg[off:off + numel].view(p.shape),
+                                 "exp_avg_sq": exp_avg_sq[off:off + numel].view(p.shape)}
+            off += numel
+
+    def sample(self, C=10, seed=None, z=None):
+        """Rows decoded for the conditions C [n, cond_size], or ``C`` rows without conditions if it is an int
+        (cvae.py:263-292); float32 numpy [n, var_size].  As upstream, an int after a conditional fit and an array after
+        an unconditional one raise RuntimeError.  Latent noise: ``z`` [n, latent_dim] if given (the reference's
+        ``torch.normal`` draw, for parity), else Philox keyed on (seed, row, latent index), ``seed`` drawn as one int64
+        from the global generator when not given (so the values and the RNG state after the call are not the
+        reference's; ``torch.manual_seed`` still makes it reproducible)."""
+        self._ready()
+        if type(C) != type(1):
+            n, Cs = len(C), C
+        else:
+            n, Cs = C, None
+        if z is not None:
+            x = self.decoder(z, Cs)
+        else:
+            if seed is None:
+                seed = int(torch.empty((), dtype=torch.int64).random_().item())
+            x = self.decoder._decode(None, Cs, n, seed)
+        return x.cpu().numpy()
