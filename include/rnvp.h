@@ -322,6 +322,59 @@ int rnvp_cv_fit_epoch(const rnvp_cv_desc* d, float* d_params, float* d_exp_avg, 
                       const float* d_noise, uint64_t seed, float* d_loss, void* d_workspace, int64_t workspace_bytes,
                       void* stream);
 
+/* ConditionalWGAN (rnvp_wgan.cu; probaforms/models/wgan.py).  Generator: model = Linear(latent + Cd, g_h0), act, ...,
+ * act, Linear(g_h_last, D); Discriminator (the critic): model = Linear(D + Cd, d_h0), act, ..., act, Linear(d_h_last, 1)
+ * (wgan.py:12-107).  Parameters cross the boundary as one flat fp32 buffer: generator.parameters() (model.{2k}.weight
+ * [h_k, h_{k-1}], model.{2k}.bias, ..., model.{2 nh}.weight, .bias), then discriminator.parameters() in the same form.
+ * Each net has its own hidden tuple and act (RNVP_ACT_TANH or _RELU: every other activation string is ReLU upstream,
+ * wgan.py:26-31).  Cd may be 0 (the reference's C=None); d_C may then be NULL.  Shapes: D <= 128, Cd <= 256,
+ * latent <= 128, 1 to 4 hidden layers of width <= 512 per net (RNVP_ESHAPE otherwise).  z buffers are [N][latent],
+ * indexed by batch position. */
+typedef struct rnvp_wg_desc rnvp_wg_desc;
+int rnvp_wg_desc_create(int D, int Cd, int latent, int g_hidden_n, const int* g_hidden, int g_act, int d_hidden_n,
+                        const int* d_hidden, int d_act, rnvp_wg_desc** out);
+void rnvp_wg_desc_destroy(rnvp_wg_desc* d);
+/* parameters of the generator (net 0), of the discriminator (net 1) or of both (any other net) */
+int64_t rnvp_wg_param_count(const rnvp_wg_desc* d, int net);
+/* scratch bytes for gradient batches of up to batch_rows rows (per-CTA gradient partials) and loss passes of up to
+ * loss_rows rows (per-CTA score sums) */
+int64_t rnvp_wg_workspace_bytes(const rnvp_wg_desc* d, int64_t batch_rows, int64_t loss_rows);
+/* Generator.forward for inference (wgan.py:38-58): d_x [N][D] of the rows [Z | C]; Z is d_Z [N][latent] when given
+ * (parity mode), else Philox normals keyed on (seed, row_offset + row, j) as in rnvp_sample (replaces the CPU
+ * torch.normal of sample, wgan.py:314-318) */
+int rnvp_wg_generate(const rnvp_wg_desc* d, const float* d_params, const float* d_Z, const float* d_C, int64_t N,
+                     uint64_t seed, int64_t row_offset, float* d_x, void* stream);
+/* Discriminator.forward for inference (wgan.py:86-107): d_score [N] of the rows [X | C] */
+int rnvp_wg_critic(const rnvp_wg_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
+                   float* d_score, void* stream);
+/* One step's loss and gradient on the N rows X[idx[r]], C[idx[r]] (d_idx may be NULL) with the caller's latent z, no
+ * optimizer update: a critic step (generator_step 0: loss_disc = -mean(D([x|c])) + mean(D([G([z|c])|c])), gradient of
+ * the discriminator's parameters) or a generator step (1: loss_gen = -mean(D([G([z|c])|c])), gradient of the
+ * generator's) (wgan.py:225-273).  d_gflat [P] in the flat layout, zero over the other net; *d_loss (may be NULL).
+ * Workspace: rnvp_wg_workspace_bytes(d, N, 0). */
+int rnvp_wg_grad(const rnvp_wg_desc* d, const float* d_params, const float* d_X, const float* d_C,
+                 const int64_t* d_idx, const float* d_z, int64_t N, int generator_step, float* d_gflat, float* d_loss,
+                 void* d_workspace, int64_t workspace_bytes, void* stream);
+/* The epoch losses (wgan.py:280-293) of the N rows: *d_gen_loss = -mean(D([G([z|c])|c])), *d_disc_loss =
+ * mean(D([x|c])) + *d_gen_loss.  Workspace: rnvp_wg_workspace_bytes(d, 0, N). */
+int rnvp_wg_loss(const rnvp_wg_desc* d, const float* d_params, const float* d_X, const float* d_C,
+                 const int64_t* d_idx, const float* d_z, int64_t N, float* d_gen_loss, float* d_disc_loss,
+                 void* d_workspace, int64_t workspace_bytes, void* stream);
+/* One epoch of ConditionalWGAN.fit (wgan.py:222-295) as one call: for every consecutive batch_size slice of d_perm
+ * (last partial batch kept), fit step i = step0, step0 + 1, ... (counted over the whole fit) is a generator step when
+ * i % n_critic == 0 and a critic step otherwise; each runs torch.optim.RMSprop (lr, alpha, eps, weight_decay; momentum
+ * 0, not centred) on its own net with d_square_avg [P] as the state, and a critic step then clamps every discriminator
+ * parameter to [-clip, clip].  Then the epoch losses over all n rows in dataset order into *d_gen_loss, *d_disc_loss.
+ * Noise: d_noise holds every step's [nb][latent] z in step order followed by the [n][latent] z of the epoch losses;
+ * when NULL, Philox keyed on (seed, position in the epoch order, j) for the steps and (seed, n + row, j) for the epoch
+ * losses.  A batch of at most the kernel's tile (64 rows for small nets) is one launch.
+ * Workspace: rnvp_wg_workspace_bytes(d, min(batch_size, n), n). */
+int rnvp_wg_fit_epoch(const rnvp_wg_desc* d, float* d_params, float* d_square_avg, const float* d_X, const float* d_C,
+                      const int64_t* d_perm, int64_t n, int64_t batch_size, int64_t n_critic, int64_t step0, double lr,
+                      double alpha, double eps, double weight_decay, double clip, const float* d_noise, uint64_t seed,
+                      float* d_gen_loss, float* d_disc_loss, void* d_workspace, int64_t workspace_bytes,
+                      void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

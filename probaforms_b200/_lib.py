@@ -98,6 +98,21 @@ SIGNATURES = {
     "rnvp_cv_fit_epoch": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64,
                                     C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
                                     C.c_int64, c_f32_p, C.c_uint64, c_f32_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_wg_desc_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int, C.c_int,
+                                      C.POINTER(C.c_int), C.c_int, C.POINTER(c_desc_p)]),
+    "rnvp_wg_desc_destroy": (None, [c_desc_p]),
+    "rnvp_wg_param_count": (C.c_int64, [c_desc_p, C.c_int]),
+    "rnvp_wg_workspace_bytes": (C.c_int64, [c_desc_p, C.c_int64, C.c_int64]),
+    "rnvp_wg_generate": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, C.c_int64, C.c_uint64, C.c_int64, c_f32_p,
+                                   c_stream]),
+    "rnvp_wg_critic": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, C.c_int64, c_f32_p, c_stream]),
+    "rnvp_wg_grad": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, c_f32_p, C.c_int64, C.c_int, c_f32_p,
+                               c_f32_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_wg_loss": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, c_f32_p, C.c_int64, c_f32_p, c_f32_p,
+                               C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_wg_fit_epoch": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64, C.c_int64,
+                                    C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
+                                    c_f32_p, C.c_uint64, c_f32_p, c_f32_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

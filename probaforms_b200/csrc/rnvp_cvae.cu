@@ -96,23 +96,6 @@ __device__ __forceinline__ float noise_at(const CvNoise& nz, int L, int64_t p, i
   return nz.eps ? nz.eps[p * L + j] : rnvp_rng::normal1(nz.seed, nz.row0 + p, j);
 }
 
-// hidden layers (act) from `in`, then an affine layer or two heads; out2 may be NULL
-__device__ __forceinline__ void mlp_forward(const CvShape& s, const float* __restrict__ params, const float* in, int ldi,
-                                            int ni, float* const* hid, const int* ldh, const int* w, const int* b,
-                                            int w1, int b1, float* out1, int w2, int b2, float* out2, int ldo, int no,
-                                            int nr) {
-#pragma unroll
-  for (int k = 0; k < CV_MAX_HIDDEN; ++k) {           // unrolled: the per-layer arrays are indexed statically
-    if (k >= s.nh) break;
-    dense_rows(in, ldi, ni, params + w[k], params + b[k], hid[k], ldh[k], s.h[k], nr, s.act);
-    __syncthreads();
-    in = hid[k]; ldi = ldh[k]; ni = s.h[k];
-  }
-  dense_rows(in, ldi, ni, params + w1, params + b1, out1, ldo, no, nr, 0);
-  if (out2) dense_rows(in, ldi, ni, params + w2, params + b2, out2, ldo, no, nr, 0);
-  __syncthreads();
-}
-
 // [x|c] rows X[idx[r]], C[idx[r]] into XC (and c into the tail of ZC)
 __device__ __forceinline__ void load_xc(const CvShape& s, const CvTile& t, const float* __restrict__ X,
                                         const float* __restrict__ C, const int64_t* __restrict__ idx, int64_t row0,

@@ -1,6 +1,6 @@
-// Row-tile MLP pieces shared by the FP32 model sweeps (rnvp_cnormal.cu, rnvp_cvae.cu): activations, a dense layer over
-// the rows of a shared-memory tile, its weight and input gradients, a deterministic block sum and torch.optim.Adam's
-// per-step coefficients.  Every helper is a whole-block loop over the calling CTA's threads; the caller synchronises.
+// Row-tile MLP pieces shared by the FP32 model sweeps (rnvp_cnormal.cu, rnvp_cvae.cu, rnvp_wgan.cu): activations, a
+// dense layer over the rows of a shared-memory tile, a whole MLP forward pass, weight and input gradients, a deterministic
+// block sum and torch.optim.Adam's per-step coefficients.  Every helper is a whole-block loop over the calling CTA's threads; the caller synchronises.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -36,20 +36,22 @@ __device__ __forceinline__ void dense_rows(const float* __restrict__ in, int ldi
   }
 }
 
-// gW[i][j] = sum_r dA[r][i] in[r][j], gb[i] = sum_r dA[r][i] (rows in order: the sums are deterministic)
+// gW[i][j] = sum_r dA[r][i] in[r][j], gb[i] = sum_r dA[r][i] (rows in order: the sums are deterministic).  ACC adds the
+// tile's sums to gW / gb instead (each element is read and written by the same thread as in the call it follows).
+template <bool ACC = false>
 __device__ __forceinline__ void wgrad(const float* dA, int lda, int no, const float* in, int ldi, int ni, int nr,
                              float* __restrict__ gW, float* __restrict__ gb) {
   for (int t = threadIdx.x; t < no * ni; t += blockDim.x) {
     const int i = t / ni, j = t - i * ni;
     float acc = 0.0f;
     for (int r = 0; r < nr; ++r) acc = fmaf(dA[r * lda + i], in[r * ldi + j], acc);
-    gW[t] = acc;
+    gW[t] = ACC ? gW[t] + acc : acc;
   }
   if (gb)
     for (int i = threadIdx.x; i < no; i += blockDim.x) {
       float acc = 0.0f;
       for (int r = 0; r < nr; ++r) acc += dA[r * lda + i];
-      gb[i] = acc;
+      gb[i] = ACC ? gb[i] + acc : acc;
     }
 }
 
@@ -63,6 +65,26 @@ __device__ __forceinline__ void back_rows(const float* dA, int lda, int no, cons
     for (int i = 0; i < no; ++i) acc = fmaf(g[i], __ldg(W + (size_t)i * ni + j), acc);
     io[r * ldi + j] = acc * act_d(act, io[r * ldi + j]);
   }
+}
+
+constexpr int MLP_MAX_HIDDEN = 4;
+
+// hidden layers (act) from `in`, then an affine layer or two heads; out2 may be NULL.  Net has nh, h[] and act.
+template <class Net>
+__device__ __forceinline__ void mlp_forward(const Net& s, const float* __restrict__ params, const float* in, int ldi,
+                                            int ni, float* const* hid, const int* ldh, const int* w, const int* b,
+                                            int w1, int b1, float* out1, int w2, int b2, float* out2, int ldo, int no,
+                                            int nr) {
+#pragma unroll
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {          // unrolled: the per-layer arrays are indexed statically
+    if (k >= s.nh) break;
+    dense_rows(in, ldi, ni, params + w[k], params + b[k], hid[k], ldh[k], s.h[k], nr, s.act);
+    __syncthreads();
+    in = hid[k]; ldi = ldh[k]; ni = s.h[k];
+  }
+  dense_rows(in, ldi, ni, params + w1, params + b1, out1, ldo, no, nr, 0);
+  if (out2) dense_rows(in, ldi, ni, params + w2, params + b2, out2, ldo, no, nr, 0);
+  __syncthreads();
 }
 
 // deterministic block sum of one value per thread (fixed tree); result valid in every thread

@@ -77,18 +77,19 @@ class _Desc:
 
 
 class _Pair:
-    """The device side of one encoder-decoder pair: the descriptor and one flat fp32 buffer of which every parameter
-    of both modules is a view (``encoder.parameters()`` then ``decoder.parameters()``, the layout the kernels read)."""
+    """The device side of a pair of modules (encoder-decoder, generator-discriminator): the descriptor ``make_desc()``
+    creates on ``dev`` and one flat fp32 buffer of which every parameter of both modules is a view (the first module's
+    ``parameters()`` then the second's, the layout the kernels read)."""
 
-    def __init__(self, encoder, decoder, D, Cd, dev):
-        self.encoder, self.decoder, self.D, self.Cd = encoder, decoder, D, Cd
+    def __init__(self, first, second, make_desc, dev):
+        self.modules = (first, second)
         with torch.cuda.device(dev):
-            self.desc = _Desc(D, Cd, encoder.lat_size, encoder.hidden, encoder.activation)
+            self.desc = make_desc()
         self.flat = None
         self.pack(dev)
 
     def params(self):
-        return list(self.encoder.parameters()) + list(self.decoder.parameters())
+        return [p for m in self.modules for p in m.parameters()]
 
     def pack(self, dev):
         params = self.params()
@@ -366,7 +367,8 @@ class CVAE(GenModel):
         self._attach(X.shape[1], c_len, self._device)
 
     def _attach(self, D, Cd, dev):
-        pair = _Pair(self.encoder, self.decoder, D, Cd, dev)
+        enc = self.encoder
+        pair = _Pair(enc, self.decoder, lambda: _Desc(D, Cd, enc.lat_size, enc.hidden, enc.activation), dev)
         self.encoder._pair = self.decoder._pair = pair
 
     def _ready(self):
