@@ -208,6 +208,33 @@ int rnvp_mmd_draws(const float* d_X, int64_t n, const float* d_Y, int64_t m, int
                    const uint16_t* d_counts /* [n_draws][n+m] */, int n_draws,
                    double* d_median /* [n_draws] */, double* d_mmd /* [n_draws] */,
                    void* d_workspace, int64_t workspace_bytes, void* stream);
+/* The same computation in stages, so that the pair tiles of one call can be split over n_shards devices (or streams)
+ * and the host can merge the shards between stages (probaforms/metrics/mmd.py:8-21, :55-61; rnvp_mmd_draws is
+ * begin, then hist_pass(p, 0, 1) + select(p) for p = 0, 1, 2, then sum_pass(0, 1) and finish).  Every shard has its own
+ * workspace (rnvp_mmd_workspace_bytes) and all of them get the same leading arguments, as for rnvp_mmd_draws.
+ *   begin      zero the workspace, per-draw count totals, selection state
+ *   hist_pass  radix pass `pass` (0, 1, 2) over the pair tiles of shard `shard` (0 <= shard < n_shards); the shards of
+ *              a call must run on devices with the same SM count
+ *   merge      after each hist_pass: hist of every shard := the sum of the shards' hist (uint64), minval := their
+ *              element-wise minimum (uint32; 0x7fffffff = none, so a signed int32 MIN gives the same result)
+ *   select     pick the buckets of pass `pass`, zero hist; after pass 2, d_median and gamma (every shard, same result)
+ *   sum_pass   the exponential sums of shard `shard`: its per-CTA rows of part, every other row stays +0.0
+ *   merge      part of one workspace := the sum of the shards' part (fp64): exactly the single-shard values
+ *   finish     d_mmd from that workspace
+ * A shard with no pair tiles is valid and contributes zeros.  rnvp_mmd_layout gives the byte offsets and sizes of the
+ * merged blocks within a workspace: offsets = { hist, hist bytes, minval, minval bytes, part, part bytes }. */
+int rnvp_mmd_layout(int64_t n, int64_t m, int n_draws, int64_t* offsets /* [6] */);
+int rnvp_mmd_begin(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+                   void* d_workspace, int64_t workspace_bytes, void* stream);
+int rnvp_mmd_hist_pass(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts,
+                       int n_draws, void* d_workspace, int64_t workspace_bytes, int pass, int shard, int n_shards,
+                       void* stream);
+int rnvp_mmd_select(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+                    void* d_workspace, int64_t workspace_bytes, int pass, double* d_median /* [n_draws] */, void* stream);
+int rnvp_mmd_sum_pass(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts,
+                      int n_draws, void* d_workspace, int64_t workspace_bytes, int shard, int n_shards, void* stream);
+int rnvp_mmd_finish(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+                    void* d_workspace, int64_t workspace_bytes, double* d_mmd /* [n_draws] */, void* stream);
 /* The moments behind X_boot.mean(axis=0) and np.cov(X_boot, rowvar=False) of frechet_distance
  * (probaforms/metrics/fd.py:40-47): d_sum[b] = sum_i c_bi x_i, d_outer[b] = sum_i c_bi x_i x_i^T in fp64
  * (fp32 products, fp64 combination; centre the rows first for an accurate covariance).  d_counts [n_draws][n]. */

@@ -62,6 +62,17 @@ SIGNATURES = {
     "rnvp_mmd_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int, C.c_int]),
     "rnvp_mmd_draws": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_mmd_layout": (C.c_int, [C.c_int64, C.c_int64, C.c_int, C.POINTER(C.c_int64)]),
+    "rnvp_mmd_begin": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                 C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_mmd_hist_pass": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                     C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, c_stream]),
+    "rnvp_mmd_select": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                  C.c_void_p, C.c_int64, C.c_int, C.c_void_p, c_stream]),
+    "rnvp_mmd_sum_pass": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                    C.c_void_p, C.c_int64, C.c_int, C.c_int, c_stream]),
+    "rnvp_mmd_finish": (C.c_int, [c_f32_p, C.c_int64, c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                  C.c_void_p, C.c_int64, C.c_void_p, c_stream]),
     "rnvp_boot_moments": (C.c_int, [c_f32_p, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                     c_stream]),
     "rnvp_rank_workspace_bytes": (C.c_int64, [C.c_int, C.c_int, C.c_int]),

@@ -18,6 +18,11 @@
 // given exactly by the bucket in the last pass).  The sum pass evaluates exp(-gamma d^2) with ex2.approx and keeps fp32
 // partial sums over 64 terms per thread, combined in fp64 in a fixed order (per-warp slots, per-CTA partials summed by
 // the finishing kernel), so a call's result does not depend on the order in which CTAs finish.
+//
+// Sharding (the staged entry points): shard s of N runs the CTAs [s hx, (s+1) hx) of a virtual radix grid N hx wide, and
+// the CTA block [s sx / N, (s+1) sx / N) of every draw group of the sum pass.  Between stages the host adds the shards'
+// histograms (exact integers), takes the minimum of their pending-bucket minima, and finally adds their per-CTA sum
+// partials (each row is written by one shard only, the others hold +0.0), so every shard count gives the single-device bits.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math.h>
@@ -39,6 +44,8 @@ constexpr int HG1 = 16;                    // ... in passes 1 and 2 (one CTA per
 constexpr int SG = 32;                     // draws per CTA in the sum pass
 constexpr int THREADS = 256;               // 16 x 16 threads, 8 x 8 pairs each
 constexpr uint32_t MAX_TILE_COUNT = 46340; // 2 * 46340^2 < 2^32: one doubled tile pair fits a uint32 bucket
+constexpr uint32_t NO_MIN = 0x7fffffffu;   // "no pending minimum": above every d^2 bit pattern (sign bit clear), and
+                                           // still the largest value under a signed int32 MIN reduction
 
 __host__ __device__ constexpr int pass_shift(int p) { return p == 0 ? 20 : (p == 1 ? 9 : 0); }
 __host__ __device__ constexpr int pass_width(int p) { return p == 2 ? 9 : 11; }
@@ -49,7 +56,7 @@ struct MmdState {
   uint32_t lo_prefix;           // bits of d^2 selected so far for rank k
   uint32_t two;                 // (n+m)^2 even: also rank k+1
   uint32_t hi_mode;             // 0: rank k+1 in the same bucket as k; 1: min of bucket hi_prefix pending; 2: hi_bits final
-  uint32_t hi_prefix, hi_shift, hi_bits, minval;
+  uint32_t hi_prefix, hi_shift, hi_bits;
   float ng2;                    // -gamma * log2(e)
 };
 
@@ -57,6 +64,7 @@ struct MmdWs {
   MmdState* st;
   unsigned long long* hist;     // [n_draws][NB]
   double* part;                 // [sum_ctas][n_draws][3]: per-CTA S_XX, S_YY, 2 S_XY of the sum pass
+  uint32_t* minval;             // [n_draws]: smallest d^2 bits of the pending bucket (hi_mode 1), or NO_MIN
   uint32_t* smax;               // largest count sum of one tile over all draws
 };
 
@@ -76,6 +84,7 @@ MmdWs carve(void* ws, int n_draws, int64_t sum_ctas, size_t* bytes) {
   w.st = (MmdState*)(p + o);            o += align256(sizeof(MmdState) * n_draws);
   w.hist = (unsigned long long*)(p + o); o += align256(sizeof(unsigned long long) * NB * (size_t)n_draws);
   w.part = (double*)(p + o);            o += align256(sizeof(double) * 3 * (size_t)n_draws * sum_ctas);
+  w.minval = (uint32_t*)(p + o);        o += align256(sizeof(uint32_t) * (size_t)n_draws);
   w.smax = (uint32_t*)(p + o);          o += align256(sizeof(uint32_t));
   *bytes = o;
   return w;
@@ -192,14 +201,16 @@ __global__ void mmd_init_kernel(MmdWs w, int n_draws) {
   s.two = (W & 1ull) == 0 ? 1u : 0u;
   s.lo_prefix = 0;
   s.hi_mode = 0;
-  s.minval = 0xffffffffu;
+  w.minval[b] = NO_MIN;
 }
 
-// Radix pass PASS (MODE 0) or the exponential-sum pass (MODE 1) for draws [group*blockIdx.y, +group), CTAs striding over
-// pair tiles.  In passes 1 and 2 only pairs inside the bucket ranges still open for some draw of the group (at most a few
-// buckets of the previous pass) reach the per-draw loop.
+// Radix pass PASS (MODE 0) or the exponential-sum pass (MODE 1) for draws [group*blockIdx.y, +group).  CTA blockIdx.x is
+// CTA cta0 + blockIdx.x of a virtual grid `ctas` wide striding over the pair tiles (a shard's part of the grid; cta0 = 0,
+// ctas = gridDim.x on one device).  In passes 1 and 2 only pairs inside the bucket ranges still open for some draw of the
+// group (at most a few buckets of the previous pass) reach the per-draw loop.
 template <int MODE, int PASS>
-__global__ void __launch_bounds__(THREADS, (MODE == 0 && PASS > 0) ? 1 : 2) mmd_pass_kernel(Geo g, MmdWs w, int group) {
+__global__ void __launch_bounds__(THREADS, (MODE == 0 && PASS > 0) ? 1 : 2)
+    mmd_pass_kernel(Geo g, MmdWs w, int group, int64_t cta0, int64_t ctas) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* sA = (float*)smem_raw;
   float* sB = sA + KC * LDS;
@@ -230,7 +241,7 @@ __global__ void __launch_bounds__(THREADS, (MODE == 0 && PASS > 0) ? 1 : 2) mmd_
     s_hmode[tid] = s.hi_mode;
     s_hpfx[tid] = s.hi_prefix;
     s_hshift[tid] = s.hi_shift;
-    s_min[tid] = 0xffffffffu;
+    s_min[tid] = NO_MIN;
     if (MODE == 1) s_ng2[tid] = s.ng2;
   }
   if (tid == 0) {
@@ -258,7 +269,7 @@ __global__ void __launch_bounds__(THREADS, (MODE == 0 && PASS > 0) ? 1 : 2) mmd_
   __syncthreads();
 
   float d2[8][8];
-  for (int64_t q = blockIdx.x; q < ntp; q += gridDim.x) {
+  for (int64_t q = cta0 + blockIdx.x; q < ntp; q += ctas) {
     int64_t ta, tb;
     tile_pair(q, &ta, &tb);
     const float *A, *B;
@@ -387,12 +398,12 @@ __global__ void __launch_bounds__(THREADS, (MODE == 0 && PASS > 0) ? 1 : 2) mmd_
   if (MODE == 0) {
     for (int e = tid; e < nb * NB; e += THREADS)
       if (shist[e]) atomicAdd(&w.hist[(int64_t)b0 * NB + e], (unsigned long long)shist[e]);
-    if (tid < nb && s_hmode[tid] == 1 && s_min[tid] != 0xffffffffu) atomicMin(&w.st[b0 + tid].minval, s_min[tid]);
+    if (tid < nb && s_hmode[tid] == 1 && s_min[tid] != NO_MIN) atomicMin(&w.minval[b0 + tid], s_min[tid]);
   } else {
     for (int e = tid; e < nb * 3; e += THREADS) {
       double t = 0.0;
       for (int wp = 0; wp < THREADS / 32; ++wp) t += ssum[wp * group * 3 + e];
-      w.part[((int64_t)blockIdx.x * g.n_draws + b0) * 3 + e] = t;
+      w.part[((cta0 + blockIdx.x) * g.n_draws + b0) * 3 + e] = t;
     }
   }
 }
@@ -406,7 +417,7 @@ __global__ void mmd_select_kernel(MmdWs w, int pass, double* d_median) {
     MmdState& s = w.st[b];
     const int shift = pass_shift(pass), width = pass_width(pass);
     if (s.hi_mode == 1) {                     // its minimum was taken during this pass
-      s.hi_bits = s.minval;
+      s.hi_bits = w.minval[b];
       s.hi_mode = 2;
     }
     unsigned long long cum = 0;
@@ -427,7 +438,7 @@ __global__ void mmd_select_kernel(MmdWs w, int pass, double* d_median) {
         s.hi_prefix = hp;
         s.hi_shift = shift;
         s.hi_mode = 1;
-        s.minval = 0xffffffffu;
+        w.minval[b] = NO_MIN;
       }
     }
     s.lo_prefix = (s.lo_prefix << width) | (uint32_t)bl;
@@ -541,12 +552,12 @@ size_t pass_smem(int mode, int group) {
 }
 
 template <int MODE, int PASS>
-void launch_pass(const Geo& g, const MmdWs& w, dim3 grid, int group, cudaStream_t st) {
+void launch_pass(const Geo& g, const MmdWs& w, dim3 grid, int group, int64_t cta0, int64_t ctas, cudaStream_t st) {
   const size_t smem = pass_smem(MODE, group);
   // per device, so set on every call (no synchronisation)
   cudaFuncSetAttribute(mmd_pass_kernel<MODE, PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)pass_smem(MODE, MODE == 1 ? SG : (PASS == 0 ? HG : HG1)));
-  mmd_pass_kernel<MODE, PASS><<<grid, THREADS, smem, st>>>(g, w, group);
+  mmd_pass_kernel<MODE, PASS><<<grid, THREADS, smem, st>>>(g, w, group, cta0, ctas);
 }
 
 int launch_fail(const char* what) {
@@ -555,6 +566,85 @@ int launch_fail(const char* what) {
   return rnvp_fail((int)e, what);
 }
 
+// One call's geometry and workspace, shared by the stages of rnvp_mmd_draws and the staged entry points.
+struct MmdCall {
+  Geo g;
+  MmdWs w;
+  int64_t ntp;                  // upper-triangular pair tiles
+  size_t need;                  // workspace bytes
+  int hgroups, hg, h1groups, hg1, sgroups, sg;
+  int64_t sx;                   // sum-pass CTAs per draw group: a function of the problem only
+};
+
+int mmd_setup(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+              void* d_workspace, int64_t workspace_bytes, MmdCall* c) {
+  if (n < 1 || m < 1 || D < 1 || n_draws < 1) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd: bad sizes");
+  if (!d_X || !d_Y || !d_counts || !d_workspace) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd: null buffer");
+  c->g = Geo{d_X, d_Y, n, m, D, (n + TILE - 1) / TILE, (m + TILE - 1) / TILE, d_counts, n_draws};
+  const int64_t T = c->g.tx + c->g.ty;
+  c->ntp = T * (T + 1) / 2;
+  c->sx = sum_ctas_per_group(c->ntp, n_draws);
+  c->w = carve(d_workspace, n_draws, c->sx, &c->need);
+  if (workspace_bytes < (int64_t)c->need)
+    return rnvp_fail(RNVP_EINVAL, "rnvp_mmd: workspace too small (see rnvp_mmd_workspace_bytes)");
+  if (T > 0x7fffffff || n_draws > 65535) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd: too many tiles or draws");
+  // draws split evenly over the fewest groups of at most HG (HG1, SG) draws
+  c->hgroups = (n_draws + HG - 1) / HG;
+  c->hg = (n_draws + c->hgroups - 1) / c->hgroups;
+  c->h1groups = (n_draws + HG1 - 1) / HG1;
+  c->hg1 = (n_draws + c->h1groups - 1) / c->h1groups;
+  c->sgroups = sum_groups(n_draws);
+  c->sg = (n_draws + c->sgroups - 1) / c->sgroups;
+  return 0;
+}
+
+int mmd_begin(const MmdCall& c, void* d_workspace, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(d_workspace, 0, c.need, st);
+  if (e != cudaSuccess) return rnvp_fail((int)e, "rnvp_mmd: workspace memset");
+  const int64_t T = c.g.tx + c.g.ty;
+  mmd_prep_kernel<<<dim3((unsigned)T, (unsigned)c.g.n_draws), TILE, 0, st>>>(c.g, c.w);
+  mmd_init_kernel<<<(c.g.n_draws + 127) / 128, 128, 0, st>>>(c.w, c.g.n_draws);
+  return launch_fail("mmd_prep_kernel");
+}
+
+// Radix pass `pass` of shard `shard` of n_shards: this device's grid (as on one device) at CTA offset shard * grid.
+// Every shard must see the same SM count, so that the shards' grids tile one virtual grid.
+int mmd_hist_pass(const MmdCall& c, int pass, int shard, int n_shards, cudaStream_t st) {
+  const int sms = num_sms();
+  if (pass == 0) {
+    const int64_t hx = std::max<int64_t>(1, std::min<int64_t>(c.ntp, (int64_t)8 * sms / c.hgroups));
+    launch_pass<0, 0>(c.g, c.w, dim3((unsigned)hx, c.hgroups), c.hg, shard * hx, n_shards * hx, st);
+  } else {
+    const int64_t h1x = std::max<int64_t>(1, std::min<int64_t>(c.ntp, (int64_t)4 * sms / c.h1groups));
+    const dim3 grid1((unsigned)h1x, c.h1groups);
+    if (pass == 1) launch_pass<0, 1>(c.g, c.w, grid1, c.hg1, shard * h1x, n_shards * h1x, st);
+    else launch_pass<0, 2>(c.g, c.w, grid1, c.hg1, shard * h1x, n_shards * h1x, st);
+  }
+  return launch_fail("mmd_pass_kernel<hist>");
+}
+
+int mmd_select(const MmdCall& c, int pass, double* d_median, cudaStream_t st) {
+  mmd_select_kernel<<<c.g.n_draws, 256, 0, st>>>(c.w, pass, d_median);
+  return launch_fail("mmd_select_kernel");
+}
+
+// Sum pass of shard `shard`: CTAs [shard sx / n_shards, (shard+1) sx / n_shards) of every draw group (none: no launch).
+int mmd_sum_pass(const MmdCall& c, int shard, int n_shards, cudaStream_t st) {
+  const int64_t c0 = c.sx * shard / n_shards, c1 = c.sx * (shard + 1) / n_shards;
+  if (c1 == c0) return 0;
+  launch_pass<1, 0>(c.g, c.w, dim3((unsigned)(c1 - c0), c.sgroups), c.sg, c0, c.sx, st);
+  return launch_fail("mmd_pass_kernel<sum>");
+}
+
+int mmd_finish(const MmdCall& c, double* d_mmd, cudaStream_t st) {
+  mmd_finish_kernel<<<(c.g.n_draws + 127) / 128, 128, 0, st>>>(c.w, c.g.n_draws, (int)c.sx, d_mmd);
+  return launch_fail("mmd_finish_kernel");
+}
+
+int check_shard(const char* who, int shard, int n_shards) {
+  if (n_shards < 1 || shard < 0 || shard >= n_shards) return rnvp_fail(RNVP_EINVAL, who);
+  return 0;
+}
 
 }  // namespace
 
@@ -570,46 +660,79 @@ int64_t rnvp_mmd_workspace_bytes(int64_t n, int64_t m, int D, int n_draws) {
 
 int rnvp_mmd_draws(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
                    double* d_median, double* d_mmd, void* d_workspace, int64_t workspace_bytes, void* stream) {
-  if (n < 1 || m < 1 || D < 1 || n_draws < 1) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_draws: bad sizes");
-  if (!d_X || !d_Y || !d_counts || !d_median || !d_mmd || !d_workspace)
-    return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_draws: null buffer");
+  if (!d_median || !d_mmd) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_draws: null buffer");
+  MmdCall c;
+  if (int rc = mmd_setup(d_X, n, d_Y, m, D, d_counts, n_draws, d_workspace, workspace_bytes, &c)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  Geo g{d_X, d_Y, n, m, D, (n + TILE - 1) / TILE, (m + TILE - 1) / TILE, d_counts, n_draws};
-  const int64_t T = g.tx + g.ty, ntp = T * (T + 1) / 2;
-  size_t need;
-  MmdWs w = carve(d_workspace, n_draws, sum_ctas_per_group(ntp, n_draws), &need);
-  if (workspace_bytes < (int64_t)need)
-    return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_draws: workspace too small (see rnvp_mmd_workspace_bytes)");
-  if (T > 0x7fffffff || n_draws > 65535) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_draws: too many tiles or draws");
-  cudaError_t e = cudaMemsetAsync(d_workspace, 0, need, st);
-  if (e != cudaSuccess) return rnvp_fail((int)e, "rnvp_mmd_draws: workspace memset");
-
-  mmd_prep_kernel<<<dim3((unsigned)T, (unsigned)n_draws), TILE, 0, st>>>(g, w);
-  mmd_init_kernel<<<(n_draws + 127) / 128, 128, 0, st>>>(w, n_draws);
-  if (int rc = launch_fail("mmd_prep_kernel")) return rc;
-
-  const int sms = num_sms();
-  // draws split evenly over the fewest groups of at most HG (HG1, SG) draws
-  const int hgroups = (n_draws + HG - 1) / HG, hg = (n_draws + hgroups - 1) / hgroups;
-  const int h1groups = (n_draws + HG1 - 1) / HG1, hg1 = (n_draws + h1groups - 1) / h1groups;
-  const int sgroups = sum_groups(n_draws), sg = (n_draws + sgroups - 1) / sgroups;
-  const unsigned hx = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ntp, (int64_t)8 * sms / hgroups));
-  const unsigned h1x = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ntp, (int64_t)4 * sms / h1groups));
-  const unsigned sx = (unsigned)sum_ctas_per_group(ntp, n_draws);   // fixed: the workspace holds one partial per CTA
+  if (int rc = mmd_begin(c, d_workspace, st)) return rc;
   for (int p = 0; p < 3; ++p) {
-    const dim3 grid(hx, hgroups), grid1(h1x, h1groups);
-    if (p == 0) launch_pass<0, 0>(g, w, grid, hg, st);
-    else if (p == 1) launch_pass<0, 1>(g, w, grid1, hg1, st);
-    else launch_pass<0, 2>(g, w, grid1, hg1, st);
-    if (int rc = launch_fail("mmd_pass_kernel<hist>")) return rc;
-    mmd_select_kernel<<<n_draws, 256, 0, st>>>(w, p, d_median);
-    if (int rc = launch_fail("mmd_select_kernel")) return rc;
+    if (int rc = mmd_hist_pass(c, p, 0, 1, st)) return rc;
+    if (int rc = mmd_select(c, p, d_median, st)) return rc;
   }
-  launch_pass<1, 0>(g, w, dim3(sx, sgroups), sg, st);
-  if (int rc = launch_fail("mmd_pass_kernel<sum>")) return rc;
-  mmd_finish_kernel<<<(n_draws + 127) / 128, 128, 0, st>>>(w, n_draws, (int)sx, d_mmd);
-  return launch_fail("mmd_finish_kernel");
+  if (int rc = mmd_sum_pass(c, 0, 1, st)) return rc;
+  return mmd_finish(c, d_mmd, st);
 }
+
+int rnvp_mmd_layout(int64_t n, int64_t m, int n_draws, int64_t* offsets) {
+  if (n < 1 || m < 1 || n_draws < 1 || n_draws > 65535 || !offsets)
+    return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_layout: bad sizes or null buffer");
+  const int64_t T = (n + TILE - 1) / TILE + (m + TILE - 1) / TILE;
+  const int64_t sx = sum_ctas_per_group(T * (T + 1) / 2, n_draws);
+  size_t bytes;
+  const MmdWs w = carve(nullptr, n_draws, sx, &bytes);
+  offsets[0] = (int64_t)(uintptr_t)w.hist;
+  offsets[1] = (int64_t)(sizeof(unsigned long long) * NB * (size_t)n_draws);
+  offsets[2] = (int64_t)(uintptr_t)w.minval;
+  offsets[3] = (int64_t)(sizeof(uint32_t) * (size_t)n_draws);
+  offsets[4] = (int64_t)(uintptr_t)w.part;
+  offsets[5] = (int64_t)(sizeof(double) * 3 * (size_t)n_draws * sx);
+  return 0;
+}
+
+// the common arguments of every stage: validated as rnvp_mmd_draws validates them
+#define MMD_STAGE_SETUP                                                                                           \
+  MmdCall c;                                                                                                      \
+  if (int rc = mmd_setup(d_X, n, d_Y, m, D, d_counts, n_draws, d_workspace, workspace_bytes, &c)) return rc;      \
+  cudaStream_t st = (cudaStream_t)stream;
+
+int rnvp_mmd_begin(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+                   void* d_workspace, int64_t workspace_bytes, void* stream) {
+  MMD_STAGE_SETUP
+  return mmd_begin(c, d_workspace, st);
+}
+
+int rnvp_mmd_hist_pass(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts,
+                       int n_draws, void* d_workspace, int64_t workspace_bytes, int pass, int shard, int n_shards,
+                       void* stream) {
+  if (pass < 0 || pass > 2) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_hist_pass: pass must be 0, 1 or 2");
+  if (int rc = check_shard("rnvp_mmd_hist_pass: need 0 <= shard < n_shards", shard, n_shards)) return rc;
+  MMD_STAGE_SETUP
+  return mmd_hist_pass(c, pass, shard, n_shards, st);
+}
+
+int rnvp_mmd_select(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+                    void* d_workspace, int64_t workspace_bytes, int pass, double* d_median, void* stream) {
+  if (pass < 0 || pass > 2) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_select: pass must be 0, 1 or 2");
+  if (!d_median) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_select: null buffer");
+  MMD_STAGE_SETUP
+  return mmd_select(c, pass, d_median, st);
+}
+
+int rnvp_mmd_sum_pass(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts,
+                      int n_draws, void* d_workspace, int64_t workspace_bytes, int shard, int n_shards, void* stream) {
+  if (int rc = check_shard("rnvp_mmd_sum_pass: need 0 <= shard < n_shards", shard, n_shards)) return rc;
+  MMD_STAGE_SETUP
+  return mmd_sum_pass(c, shard, n_shards, st);
+}
+
+int rnvp_mmd_finish(const float* d_X, int64_t n, const float* d_Y, int64_t m, int D, const uint16_t* d_counts, int n_draws,
+                    void* d_workspace, int64_t workspace_bytes, double* d_mmd, void* stream) {
+  if (!d_mmd) return rnvp_fail(RNVP_EINVAL, "rnvp_mmd_finish: null buffer");
+  MMD_STAGE_SETUP
+  return mmd_finish(c, d_mmd, st);
+}
+
+#undef MMD_STAGE_SETUP
 
 int rnvp_boot_moments(const float* d_X, int64_t n, int D, const uint16_t* d_counts, int n_draws, double* d_sum,
                       double* d_outer, void* stream) {

@@ -3,6 +3,8 @@
     from probaforms_b200.metrics import maximum_mean_discrepancy, frechet_distance
     mu, sd = maximum_mean_discrepancy(X, Y, n_iters=100, standardize=False)
     mu, sd = frechet_distance(X_real, X_fake, n_iters=100, standardize=False)
+    mu, sd = maximum_mean_discrepancy(X, Y, devices=[0, 1, 2, 3])      # pair tiles split over four GPUs
+    mu, sd = maximum_mean_discrepancy(X, Y, shard=True)                # one shard per rank of a process group
 
 Both return ``(mean, std)`` over the bootstrap draws as numpy float64 (``np.std``, ddof 0), like the reference
 (probaforms/metrics/mmd.py:24-64, fd.py:7-61).  The draws are taken on the host from the global ``np.random`` state in
@@ -11,6 +13,10 @@ the reference's order (per iteration ``resample(X)`` then ``resample(Y)``, which
 vector; the kernels of ``rnvp_metrics.cu`` evaluate all draws from the counts without materialising the resampled
 rows or any (n+m)^2 distance matrix.  Inputs are 2-D numpy arrays or torch tensors; a CUDA tensor is used on its device.
 There is no CPU path.
+
+The MMD's cost grows with (n+m)^2, so it can split its pair tiles over several GPUs (``devices=``, in one process) or
+over the ranks of an initialised ``torch.distributed`` group (``shard=True``); the shards' histograms and partial sums are
+merged between the kernel passes, and the result is bit-identical to the one-device call for any number of shards.
 
 The eight per-feature metrics (kolmogorov_smirnov_1d, cramer_von_mises_1d, ...) live in ``onedim.py`` and share the draws
 and input handling above; ``__all__`` holds the ten names of ``probaforms.metrics``.
@@ -143,13 +149,192 @@ def _mmd_draws(X32, Y32, counts):
     return median, mmd
 
 
-def maximum_mean_discrepancy(X, Y, n_iters=100, standardize=False):
+def _process_group():
+    """(rank, world) of the initialised torch.distributed group, or (0, 1) without one."""
+    dist = torch.distributed
+    world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
+    return (dist.get_rank() if world > 1 else 0), world
+
+
+def _shard_ids(rank, world, n_local):
+    """Shard numbers of this process's n_local shards and the total: rank r holds r*n_local .. r*n_local + n_local - 1 of
+    world * n_local, so the shards of all ranks tile the pair tiles once."""
+    return [rank * n_local + i for i in range(n_local)], world * n_local
+
+
+def _cuda_devices(devices):
+    out = []
+    for d in devices:
+        d = torch.device("cuda", d) if isinstance(d, int) else torch.device(d)
+        if d.type != "cuda":
+            raise ValueError(f"devices must name CUDA devices, got {d}")
+        out.append(torch.device("cuda", torch.cuda.current_device() if d.index is None else d.index))
+    return out
+
+
+def _all_reduce(t, op):
+    """torch.distributed.all_reduce of a CUDA tensor: in place with NCCL, staged through the host with gloo."""
+    dist = torch.distributed
+    if dist.get_backend() != "gloo":
+        dist.all_reduce(t, op=op)
+        return t
+    c = t.cpu()
+    dist.all_reduce(c, op=op)
+    return t.copy_(c)
+
+
+def _broadcast(t):
+    """rank 0's contiguous CUDA tensor t on every rank, sent as bytes (neither NCCL nor gloo carries int16); staged
+    through the host with gloo."""
+    dist = torch.distributed
+    b = t.view(torch.uint8)
+    if dist.get_backend() != "gloo":
+        dist.broadcast(b, src=0)
+        return t
+    c = b.cpu()
+    dist.broadcast(c, src=0)
+    b.copy_(c)
+    return t
+
+
+class _MmdShards:
+    """One rnvp_mmd_draws computation split over shards through the staged entry points of rnvp_metrics.cu.
+
+    Every local device in ``devices`` (repeats allowed) holds one shard: its own copy of the fp32 rows and counts and its
+    own workspace.  Under a process group of ``world`` ranks this process runs shards ``_shard_ids(rank, world, k)``.
+    After each radix pass the shards' histograms are summed (exact integers) and their pending-bucket minima MIN-reduced,
+    and the merge is written back to every shard; after the sum pass the per-CTA partials are summed into the first
+    shard, which finishes.  Each partial row is written by exactly one shard and is +0.0 in the others, so the merged
+    values, and therefore the medians and MMD values, are the one-device bits for any number of shards.
+
+    ``run()`` is the whole call; the stage methods are public to tools that time them one by one."""
+
+    def __init__(self, X32, Y32, counts, devices, rank=0, world=1):
+        self.lib = lib = _lib.load()
+        n, D = X32.shape
+        m, nd = Y32.shape[0], counts.shape[0]
+        self.size = (n, m, D, nd)
+        self.devices = list(devices)
+        self.ids, self.n_shards = _shard_ids(rank, world, len(self.devices))
+        self.world = world
+        # a shard's radix grid is sized by its GPU's SM count: the shards' grids tile one virtual grid only if all match
+        sms = [torch.cuda.get_device_properties(d).multi_processor_count for d in set(self.devices)]
+        chk = [min(sms), -max(sms), len(self.devices), -len(self.devices)]
+        if world > 1:
+            t = torch.tensor(chk, dtype=torch.int64, device=self.devices[0])
+            chk = _all_reduce(t, torch.distributed.ReduceOp.MIN).tolist()
+        if chk[0] != -chk[1]:
+            raise ValueError("the shards of one MMD call must run on GPUs with the same SM count")
+        if chk[2] != -chk[3]:
+            raise ValueError("every rank must pass the same number of devices")
+        ws_bytes = int(lib.rnvp_mmd_workspace_bytes(n, m, D, nd))
+        if ws_bytes < 0:
+            _lib.check(ws_bytes, "rnvp_mmd_workspace_bytes")
+        lay = (C.c_int64 * 6)()
+        _lib.check(lib.rnvp_mmd_layout(n, m, nd, lay), "rnvp_mmd_layout")
+        self.layout = [(lay[2 * k], lay[2 * k + 1]) for k in range(3)]     # hist, minval, part: (offset, bytes)
+        inputs, self.shards = {}, []
+        for dev in self.devices:
+            if dev not in inputs:
+                inputs[dev] = tuple(t.to(dev).contiguous() for t in (X32, Y32, counts))
+            with torch.cuda.device(dev):
+                ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+                median = torch.empty(nd, dtype=torch.float64, device=dev)
+            self.shards.append((dev,) + inputs[dev] + (ws, median))
+        self.mmd = torch.empty(nd, dtype=torch.float64, device=self.devices[0])
+
+    def _call(self, name, s, *extra):
+        dev, X, Y, cnt, ws, _ = self.shards[s]
+        n, m, D, nd = self.size
+        with torch.cuda.device(dev):
+            rc = getattr(self.lib, name)(X.data_ptr(), n, Y.data_ptr(), m, D, cnt.data_ptr(), nd, ws.data_ptr(),
+                                         ws.numel(), *extra, _stream(dev))
+        _lib.check(rc, name)
+
+    def _block(self, s, k, dtype):
+        off, nbytes = self.layout[k]
+        return self.shards[s][4][off:off + nbytes].view(dtype)
+
+    def _merged(self, k, dtype, op, reduce_op):
+        """Block k of all shards combined element-wise by op, on the first device, then across the process group."""
+        dev0 = self.devices[0]
+        acc = self._block(0, k, dtype).clone()
+        for s in range(1, len(self.shards)):
+            acc = op(acc, self._block(s, k, dtype).to(dev0))
+        return _all_reduce(acc, reduce_op) if self.world > 1 else acc
+
+    def begin(self):
+        for s in range(len(self.shards)):
+            self._call("rnvp_mmd_begin", s)
+
+    def hist_pass(self, p, s):
+        self._call("rnvp_mmd_hist_pass", s, p, self.ids[s], self.n_shards)
+
+    def merge_hist(self):
+        if self.n_shards == 1:
+            return
+        ReduceOp = torch.distributed.ReduceOp
+        hist = self._merged(0, torch.int64, torch.add, ReduceOp.SUM)          # uint64 counts, far below 2^63
+        minval = self._merged(1, torch.int32, torch.minimum, ReduceOp.MIN)    # d^2 bits and 0x7fffffff: all >= 0
+        for s in range(len(self.shards)):
+            self._block(s, 0, torch.int64).copy_(hist)
+            self._block(s, 1, torch.int32).copy_(minval)
+
+    def select(self, p, s):
+        self._call("rnvp_mmd_select", s, p, self.shards[s][5].data_ptr())
+
+    def sum_pass(self, s):
+        self._call("rnvp_mmd_sum_pass", s, self.ids[s], self.n_shards)
+
+    def merge_part(self):
+        if self.n_shards == 1:
+            return
+        self._block(0, 2, torch.float64).copy_(self._merged(2, torch.float64, torch.add, torch.distributed.ReduceOp.SUM))
+
+    def finish(self):
+        self._call("rnvp_mmd_finish", 0, self.mmd.data_ptr())
+
+    def run(self):
+        """Per-draw (median, MMD) float64 tensors [n_draws] on the first device."""
+        shards = range(len(self.shards))
+        self.begin()
+        for p in range(3):
+            for s in shards:
+                self.hist_pass(p, s)
+            self.merge_hist()
+            for s in shards:
+                self.select(p, s)
+        for s in shards:
+            self.sum_pass(s)
+        self.merge_part()
+        self.finish()
+        return self.shards[0][5], self.mmd
+
+
+def maximum_mean_discrepancy(X, Y, n_iters=100, standardize=False, devices=None, shard=False):
     """Bootstrap Maximum Mean Discrepancy between samples X [n, D] and Y [m, D] (RBF kernel, median heuristic).
 
-    Drop-in for probaforms.metrics.maximum_mean_discrepancy.  Returns (mean, std) over n_iters draws."""
+    Drop-in for probaforms.metrics.maximum_mean_discrepancy.  Returns (mean, std) over n_iters draws.
+
+    Additive, not upstream (the defaults compute on the inputs' device, as upstream computes in one process):
+    ``devices=[d0, d1, ...]`` splits the pair tiles over these GPUs of this process, one shard per entry (an entry may
+    repeat).  The fp32 rows and the draws are copied to each; ``standardize`` is applied once, before.
+    ``shard=True`` under an initialised ``torch.distributed`` group makes rank r run shard r of the world (with
+    ``devices``, one shard per entry on every rank; every rank must list as many).  Every rank consumes ``np.random``
+    as upstream does, but all ranks use rank 0's draws, and every rank returns the same (mean, std).  Without a group
+    it is one shard.  Either way the result is bit-identical to the one-device call."""
     X64, Y64 = _prepare(X, Y, standardize)
-    counts = _counts_to(_bootstrap_counts(X64.shape[0], Y64.shape[0], n_iters), X64.device)
-    _, mmd = _mmd_draws(X64.float().contiguous(), Y64.float().contiguous(), counts)
+    counts = _bootstrap_counts(X64.shape[0], Y64.shape[0], n_iters)
+    X32, Y32 = X64.float().contiguous(), Y64.float().contiguous()
+    rank, world = _process_group() if shard else (0, 1)
+    if not devices and world == 1:
+        _, mmd = _mmd_draws(X32, Y32, _counts_to(counts, X64.device))
+    else:
+        devs = _cuda_devices(devices) if devices else [X64.device]
+        counts = _counts_to(counts, devs[0])
+        if world > 1:
+            _broadcast(counts)                     # every rank evaluates rank 0's draws
+        _, mmd = _MmdShards(X32, Y32, counts, devs, rank, world).run()
     mmds = mmd.cpu().numpy()
     return np.mean(mmds), np.std(mmds)
 
