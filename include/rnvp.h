@@ -170,17 +170,16 @@ int rnvp_perm_create(uint64_t seed, int64_t n, int64_t* out, rnvp_perm** p);
 int64_t rnvp_perm_advance(rnvp_perm* p, int64_t upto);
 void rnvp_perm_destroy(rnvp_perm* p);
 
-/* Host-side ingestion / egress helpers (no device work; HOST pointers).  rnvp_host_gather_rows writes
- * dst[r][0..width) = (float) src[idx ? idx[r] : row0 + r][0..width) for r in [0, n): the rows of one optimisation step,
- * converted from the caller's float64 (src_is_f64 != 0) or float32 array -- torch.tensor(X, dtype=float32) of
- * realnvp.py:226-228 fused with the batch gather of realnvp.py:237 -- into a (pinned) staging buffer, on up to `threads`
- * host threads.  The staging buffer is written with non-temporal stores when it is 16-byte aligned and width % 4 == 0:
- * its next reader is the GPU's DMA engine, and an upload whose source lines are dirty in many cores' caches runs at a
- * quarter of the bus rate.  rnvp_host_copy is a multi-threaded memcpy (the .cpu().numpy() of realnvp.py:281 into a
- * fresh pageable array; RealNVP.sample uses it only beyond the pinned result pool's cap). */
-int rnvp_host_gather_rows(const void* src, int src_is_f64, int64_t width, const int64_t* idx, int64_t row0, int64_t n,
-                          float* dst, int threads);
-/* X and C rows of one step in one pass over idx (src_c may be NULL) */
+/* Host-side ingestion / egress helpers (no device work; HOST pointers).  rnvp_host_gather_xc writes
+ * dst_x[r][0..width_x) = (float) src_x[idx ? idx[r] : row0 + r][0..width_x) for r in [0, n), and the same rows of src_c
+ * into dst_c in the same pass over idx; src_c may be NULL (X rows only: c_is_f64, width_c and dst_c are then ignored).
+ * These are the rows of one optimisation step or one upload chunk, converted from the caller's float64 (x_is_f64 /
+ * c_is_f64 != 0) or float32 arrays -- torch.tensor(X, dtype=float32) of realnvp.py:226-228 fused with the batch gather
+ * of realnvp.py:237 -- into (pinned) staging buffers, on up to `threads` host threads.  A staging buffer is written with
+ * non-temporal stores when it is 16-byte aligned and its width % 4 == 0: its next reader is the GPU's DMA engine, and an
+ * upload whose source lines are dirty in many cores' caches runs at a quarter of the bus rate.  rnvp_host_copy is a
+ * multi-threaded memcpy (the .cpu().numpy() of realnvp.py:281 into a fresh pageable array; RealNVP.sample uses it only
+ * beyond the pinned result pool's cap). */
 int rnvp_host_gather_xc(const void* src_x, int x_is_f64, int64_t width_x, const void* src_c, int c_is_f64, int64_t width_c,
                            const int64_t* idx, int64_t row0, int64_t n, float* dst_x, float* dst_c, int threads);
 int rnvp_host_copy(void* dst, const void* src, int64_t bytes, int threads);

@@ -53,8 +53,6 @@ SIGNATURES = {
     "rnvp_perm_create": (C.c_int, [C.c_uint64, C.c_int64, C.c_void_p, C.POINTER(C.c_void_p)]),
     "rnvp_perm_advance": (C.c_int64, [C.c_void_p, C.c_int64]),
     "rnvp_perm_destroy": (None, [C.c_void_p]),
-    "rnvp_host_gather_rows": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
-                                        C.c_int]),
     "rnvp_host_gather_xc": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_int, C.c_int64, C.c_void_p,
                                          C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]),
     "rnvp_host_copy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int]),

@@ -2,10 +2,11 @@
 // torch.tensor(X, dtype=torch.float32) (realnvp.py:226-228) and .cpu().detach().numpy() (realnvp.py:281) once the
 // kernels are fast enough for those copies to be the wall-clock bound (SURVEY 8f-2).
 //
-// rnvp_host_gather_rows: dst[r][:] = (float) src[idx ? idx[r] : row0 + r][:] -- the rows of one optimisation step (a
-// slice of the epoch permutation), converted from the caller's float64 / float32 numpy array straight into a pinned
-// staging buffer, split over a few host threads.  RealNVP.fit streams these buffers to the GPU one step ahead of
-// the kernels, so every rank uploads only the rows of its own shard.
+// rnvp_host_gather_xc: dst_x[r][:] = (float) src_x[idx ? idx[r] : row0 + r][:], and the same rows of src_c into dst_c
+// unless src_c is NULL -- the rows of one optimisation step (a slice of the epoch permutation) or of one upload chunk,
+// converted from the caller's float64 / float32 numpy arrays straight into pinned staging buffers, split over a few
+// host threads.  RealNVP.fit streams these buffers to the GPU one step ahead of the kernels, so every rank uploads
+// only the rows of its own shard.
 // rnvp_host_copy: multi-threaded memcpy (first-touch of a fresh numpy result array is page-fault bound on one thread).
 #include <stdint.h>
 #include <string.h>
@@ -129,17 +130,6 @@ void run_threads(int64_t n, int64_t min_per_thread, int threads, F f) { Pool::ge
 }  // namespace
 
 extern "C" {
-
-int rnvp_host_gather_rows(const void* src, int src_is_f64, int64_t width, const int64_t* idx, int64_t row0, int64_t n,
-                          float* dst, int threads) {
-  if (!src || !dst || width < 1 || n < 0 || row0 < 0) return RNVP_EINVAL;
-  auto work = [=](int64_t r0, int64_t r1) {
-    if (src_is_f64) gather_range((const double*)src, width, idx, row0, r0, r1, dst);
-    else gather_range((const float*)src, width, idx, row0, r0, r1, dst);
-  };
-  run_threads(n, std::max<int64_t>(1, 65536 / width), threads, work);
-  return 0;
-}
 
 int rnvp_host_gather_xc(const void* src_x, int x_is_f64, int64_t width_x, const void* src_c, int c_is_f64, int64_t width_c,
                            const int64_t* idx, int64_t row0, int64_t n, float* dst_x, float* dst_c, int threads) {

@@ -4,19 +4,22 @@ The reference copies the whole numpy data set through ``torch.tensor(X, dtype=to
 (realnvp.py:226-228) and returns samples through ``.cpu().detach().numpy()`` (realnvp.py:281).  Once a
 fit step takes a millisecond those two copies are the wall-clock bound, so here
 
-* ``upload_resident`` converts (float64 -> float32) and uploads in chunks through two pinned staging
-  buffers: the host conversion of chunk k+1 overlaps the H2D copy of chunk k;
+* ``ChunkUploader`` converts (float64 -> float32) and uploads in chunks through two pinned staging
+  buffers: the host conversion of chunk k+1 overlaps the H2D copy of chunk k, and the consumer may start on the
+  chunks that have arrived.  ``upload_resident`` (a whole row set, as every model's fit needs it) is one
+  ``ChunkUploader`` run to the end, apart from device, pinned and small inputs;
 * ``StepStreamer`` feeds the fit loop with exactly the rows each step needs -- THIS rank's slice of the
-  epoch permutation, gathered and converted by ``rnvp_host_gather_xc`` (a pool of host threads, non-temporal
-  stores) into a ring of pinned buffers and uploaded on a copy stream while the kernels of the previous two
-  steps run.  Under data parallelism every rank therefore uploads 1/world of the rows instead of the whole set;
+  epoch permutation, gathered and converted into a ring of pinned buffers and uploaded on a copy stream while
+  the kernels of the previous two steps run.  Under data parallelism every rank therefore uploads 1/world of the
+  rows instead of the whole set;
 * ``ResultPool`` lends pinned memory to the numpy arrays ``RealNVP.sample`` returns (the D2H copy lands in the
   array itself; the memory is recycled when the caller drops it);
 * ``rows_to_numpy`` brings results back through pinned buffers with a multi-threaded copy into the
   fresh numpy array the API contract returns (first-touch page faults are spread over several cores).
 
 torch is plumbing here (pinned memory, streams, events); the byte moving is the C ABI's
-``rnvp_host_*`` entry points (include/rnvp.h).
+``rnvp_host_*`` entry points (include/rnvp.h).  Every upload path gathers and converts its rows with
+``rnvp_host_gather_xc`` (a pool of host threads, non-temporal stores), called through ``_gather``.
 """
 import collections
 import ctypes as C
@@ -53,17 +56,16 @@ def host_rows(A):
     return np.ascontiguousarray(A)
 
 
-def gather_into(lib, arr, idx, row0, n, dst, threads=None):
-    """dst[:n] = float32(arr[idx[:n]]) (idx: contiguous int64 numpy array / torch tensor, or None for rows row0..)."""
-    if n <= 0:
-        return
-    iptr = None
-    if idx is not None:
-        iptr = C.c_void_p(idx.data_ptr() if isinstance(idx, torch.Tensor) else idx.ctypes.data)
-    rc = lib.rnvp_host_gather_rows(C.c_void_p(arr.ctypes.data), 1 if arr.dtype == np.float64 else 0, arr.shape[1], iptr,
-                                   int(row0), int(n), C.c_void_p(dst.data_ptr()), threads or host_threads())
+def _gather(lib, X, Cn, idx, row0, n, dst_x, dst_c, threads):
+    """dst_x[:n] = float32(X[rows]), and dst_c[:n] = float32(Cn[rows]) unless Cn is None, where rows are idx[:n] (a
+    contiguous int64 numpy array) or, with idx None, row0 .. row0 + n.  X / Cn come from ``host_rows``."""
+    rc = lib.rnvp_host_gather_xc(
+        C.c_void_p(X.ctypes.data), 1 if X.dtype == np.float64 else 0, X.shape[1],
+        C.c_void_p(Cn.ctypes.data) if Cn is not None else None, 1 if (Cn is not None and Cn.dtype == np.float64) else 0,
+        Cn.shape[1] if Cn is not None else 0, C.c_void_p(idx.ctypes.data) if idx is not None else None, int(row0), int(n),
+        C.c_void_p(dst_x.data_ptr()), C.c_void_p(dst_c.data_ptr()) if Cn is not None else None, threads)
     if rc != 0:
-        raise RuntimeError(f"rnvp_host_gather_rows failed (code {rc})")
+        raise RuntimeError(f"rnvp_host_gather_xc failed (code {rc})")
 
 
 _STAGING = {}     # key -> flat pinned float32 buffer, grown on demand and kept for the life of the process
@@ -164,8 +166,8 @@ RESULTS = ResultPool()
 
 def upload_resident(lib, A, dev, chunk_bytes=32 << 20):
     """Whole row set -> contiguous float32 device tensor [n, w].  Pinned float32 torch tensors go up in one asynchronous
-    copy; everything else (numpy float64 / float32, pageable tensors) is converted chunk by chunk into two pinned
-    staging buffers so that the host pass over chunk k+1 runs while chunk k is on the bus."""
+    copy; everything else (numpy float64 / float32, pageable tensors) goes through a ``ChunkUploader``: converted chunk by
+    chunk into two pinned staging buffers so that the host pass over chunk k+1 runs while chunk k is on the bus."""
     if isinstance(A, torch.Tensor):
         if A.device.type != "cpu":
             return A.to(device=dev, dtype=torch.float32).contiguous()
@@ -173,33 +175,18 @@ def upload_resident(lib, A, dev, chunk_bytes=32 << 20):
             return A.to(dev, non_blocking=True)
     arr = host_rows(A)
     n, w = arr.shape
-    out = torch.empty(n, w, dtype=torch.float32, device=dev)
     if n == 0:
-        return out
-    rows = max(1, min(n, chunk_bytes // (4 * w)))
+        return torch.empty(n, w, dtype=torch.float32, device=dev)
     if n * w * 4 <= (1 << 20):                      # small sets: one synchronous hop is cheapest
+        out = torch.empty(n, w, dtype=torch.float32, device=dev)
         stage = torch.empty(n, w, dtype=torch.float32)
-        gather_into(lib, arr, None, 0, n, stage, threads=1)
+        _gather(lib, arr, None, None, 0, n, stage, None, threads=1)
         out.copy_(stage)
         return out
-    stage = [_pinned((rows, w), ("up", 0)), _pinned((rows, w), ("up", 1))]
-    done = [None, None]
-    copy_stream = torch.cuda.Stream(device=dev)
-    for k, r0 in enumerate(range(0, n, rows)):
-        m = min(rows, n - r0)
-        s = k & 1
-        if done[s] is not None:
-            done[s].synchronize()
-        gather_into(lib, arr, None, r0, m, stage[s])
-        with torch.cuda.stream(copy_stream):
-            out[r0:r0 + m].copy_(stage[s][:m], non_blocking=True)
-            done[s] = torch.cuda.Event()
-            done[s].record(copy_stream)
-    torch.cuda.current_stream(dev).wait_stream(copy_stream)
-    for e in done:
-        if e is not None:
-            e.synchronize()                         # the staging buffers die with this call
-    return out
+    # own staging key: an uploader that is still open elsewhere (fit's first epoch, sample's chunk loop) keeps its buffers
+    up = ChunkUploader(lib, arr, None, dev, max(1, min(n, chunk_bytes // (4 * w))), stage_key="up")
+    up.close()
+    return up.X
 
 
 def rows_to_numpy(lib, t, chunk_bytes=32 << 20):
@@ -245,9 +232,10 @@ class ChunkUploader:
     pinned staging buffers, and makes the current stream wait for those copies.  All of it happens on the CALLER's
     thread: the consumer launches its kernels asynchronously, so the conversion of chunk k+1 runs while the GPU is busy
     with chunk k (a helper thread driving the same CUDA context was measured slower, see StepStreamer).
-    ``X`` / ``C`` are the device tensors (valid up to the rows waited for)."""
+    ``X`` / ``C`` are the device tensors (valid up to the rows waited for).  ``stage_key`` names the pinned staging
+    buffers: uploaders that may be open at the same time need different keys."""
 
-    def __init__(self, lib, X, Cn, dev, chunk_rows):
+    def __init__(self, lib, X, Cn, dev, chunk_rows, stage_key="cu"):
         self.lib, self.dev = lib, dev
         self.hX, self.hC = host_rows(X), (host_rows(Cn) if Cn is not None else None)
         n, w = self.hX.shape
@@ -255,7 +243,8 @@ class ChunkUploader:
         self.n, self.chunk = n, max(1, int(chunk_rows))
         self.X = torch.empty(n, w, dtype=torch.float32, device=dev)
         self.C = torch.empty(n, wc, dtype=torch.float32, device=dev) if wc else None
-        self.stage = [(_pinned((self.chunk, w), ("cux", k)), _pinned((self.chunk, wc), ("cuc", k)) if wc else None) for k in range(2)]
+        self.stage = [(_pinned((self.chunk, w), (stage_key + "x", k)),
+                       _pinned((self.chunk, wc), (stage_key + "c", k)) if wc else None) for k in range(2)]
         self.n_chunks = (n + self.chunk - 1) // self.chunk
         self.events = [None] * self.n_chunks
         self._next = 0                      # first chunk not yet enqueued
@@ -269,14 +258,7 @@ class ChunkUploader:
         sx, sc = self.stage[k & 1]
         if k >= 2:
             self.events[k - 2].synchronize()                        # the copy that last used this staging buffer has finished
-        rc = self.lib.rnvp_host_gather_xc(
-            C.c_void_p(self.hX.ctypes.data), 1 if self.hX.dtype == np.float64 else 0, self.hX.shape[1],
-            C.c_void_p(self.hC.ctypes.data) if self.hC is not None else None,
-            1 if (self.hC is not None and self.hC.dtype == np.float64) else 0,
-            self.hC.shape[1] if self.hC is not None else 0, None, r0, m,
-            C.c_void_p(sx.data_ptr()), C.c_void_p(sc.data_ptr()) if sc is not None else None, self.threads)
-        if rc != 0:
-            raise RuntimeError(f"rnvp_host_gather_xc failed (code {rc})")
+        _gather(self.lib, self.hX, self.hC, None, r0, m, sx, sc, self.threads)
         with torch.cuda.stream(self.copy_stream):
             self.X[r0:r0 + m].copy_(sx[:m], non_blocking=True)
             if sc is not None:
@@ -346,15 +328,7 @@ class StepStreamer:
         t1 = time.perf_counter()
         sl = get_idx(hi)[lo:hi]
         t2 = time.perf_counter()
-        rc = self.lib.rnvp_host_gather_xc(
-            C.c_void_p(self.X.ctypes.data), 1 if self.X.dtype == np.float64 else 0, self.X.shape[1],
-            C.c_void_p(self.Cn.ctypes.data) if self.Cn is not None else None,
-            1 if (self.Cn is not None and self.Cn.dtype == np.float64) else 0,
-            self.Cn.shape[1] if self.Cn is not None else 0, C.c_void_p(sl.ctypes.data), 0, m,
-            C.c_void_p(self.hx[s].data_ptr()), C.c_void_p(self.hc[s].data_ptr()) if self.hc is not None else None,
-            self.threads)
-        if rc != 0:
-            raise RuntimeError(f"rnvp_host_gather_xc failed (code {rc})")
+        _gather(self.lib, self.X, self.Cn, sl, 0, m, self.hx[s], self.hc[s] if self.hc is not None else None, self.threads)
         t3 = time.perf_counter()
         with torch.cuda.stream(self.copy_stream):
             if self.trace is not None:

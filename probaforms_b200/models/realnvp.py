@@ -320,10 +320,8 @@ class RealNVP(GenModel):
     def _to_device(self, A, dev):
         """numpy/torch -> contiguous float32 rows on the device (realnvp.py:226-228), chunked through pinned staging
         buffers with the float64 -> float32 conversion fused into the host pass (probaforms_b200/ingest.py)."""
-        if isinstance(A, torch.Tensor) and (A.device.type != "cpu" or A.dim() != 2):
-            return A.to(device=dev, dtype=torch.float32).contiguous()
-        if not isinstance(A, torch.Tensor) and np.asarray(A).ndim != 2:
-            return torch.as_tensor(np.asarray(A), dtype=torch.float32).to(dev)     # let the shape checks speak
+        if np.ndim(A) != 2:                                   # let the shape checks speak
+            return torch.as_tensor(A, dtype=torch.float32, device=dev)
         from ..ingest import upload_resident
         return upload_resident(self.nf._fused(repack=False).lib, A, dev)
 
@@ -603,10 +601,15 @@ class RealNVP(GenModel):
                 seeds = [int(v) for v in t.cpu()]
         else:
             lo, hi = 0, n
-        if devices is not None and len(devices) > 0:
-            out = self._sample_multi_device(C, is_int, lo, hi, seeds, list(devices))
-        else:
+        if devices is None or len(devices) == 0:
             return self._sample_to_host(eng, None if is_int else C[lo:hi], lo, hi, seeds, n_draws is not None)
+
+        def run(eng, dev, b0, b1):
+            Cd = None if is_int else self._to_device(C[b0:b1], dev)
+            return torch.stack([eng.sample(b1 - b0, Cd, seed=sd, row_offset=b0) for sd in seeds])
+
+        out = self._device_blocks(lo, hi, list(devices), run, np.empty((len(seeds), hi - lo, eng.D), dtype=np.float32),
+                                  1, "mdev_x")
         return out if n_draws is not None else out[0]
 
     def _sample_to_host(self, eng, Cs, lo, hi, seeds, stacked, chunk_rows=None):
@@ -662,31 +665,28 @@ class RealNVP(GenModel):
         copy_stream.synchronize()
         return arr
 
-    def _sample_multi_device(self, C, is_int, lo, hi, seeds, devices):
-        """Row blocks of [lo, hi) on several GPUs of this process: replicas of the weights, one launch per (device, draw),
-        results copied back into one host array."""
+    def _device_blocks(self, lo, hi, devices, run, out, axis, key):
+        """Rows [lo, hi) in contiguous blocks over the GPUs ``devices`` of this process: ``run(eng, dev, b0, b1)`` enqueues
+        block [b0, b1) on the device's replica of the weights and returns its device result, which is copied back through
+        pinned buffers ``(key, k)`` into ``out`` (rows along ``axis``).  Rows are independent: no communication."""
         from ..ingest import _pinned
-        n = hi - lo
-        D = self.nf._fused(repack=False).D
-        out = np.empty((len(seeds), n, D), dtype=np.float32)
         pending = []
         for k, d in enumerate(devices):
-            b0, b1 = lo + (n * k) // len(devices), lo + (n * (k + 1)) // len(devices)
+            b0, b1 = lo + ((hi - lo) * k) // len(devices), lo + ((hi - lo) * (k + 1)) // len(devices)
             if b1 <= b0:
                 continue
             dev = torch.device("cuda", d) if not isinstance(d, torch.device) else d
             eng = self.nf._replica(dev)
             with torch.cuda.device(dev):
-                Cd = None if is_int else self._to_device(C[b0:b1], dev)
-                res = torch.stack([eng.sample(b1 - b0, Cd, seed=sd, row_offset=b0) for sd in seeds])
-                host = _pinned(tuple(res.shape), ("mdev_x", k))
+                res = run(eng, dev, b0, b1)
+                host = _pinned(tuple(res.shape), (key, k))
                 host.copy_(res, non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record()
             pending.append((b0 - lo, b1 - lo, host, ev, res))
         for a, b, host, ev, _ in pending:
             ev.synchronize()
-            out[:, a:b] = host.numpy()
+            out[(slice(None),) * axis + (slice(a, b),)] = host.numpy()
         return out
 
     def log_prob_rows(self, X, C=None, devices=None, shard=False):
@@ -697,26 +697,11 @@ class RealNVP(GenModel):
             raise RuntimeError("RealNVP.log_prob_rows: call fit() first")
         n = X.shape[0]
         lo, hi = (self._shard_of(n)[:2] if shard else (0, n))
-        from ..ingest import _pinned
-        devs = list(devices) if devices else [self._device]
-        out = np.empty(hi - lo, dtype=np.float32)
-        pending = []
-        for k, d in enumerate(devs):
-            b0, b1 = lo + ((hi - lo) * k) // len(devs), lo + ((hi - lo) * (k + 1)) // len(devs)
-            if b1 <= b0:
-                continue
-            dev = torch.device("cuda", d) if not isinstance(d, torch.device) else d
-            eng = self.nf._fused() if dev == self._device else self.nf._replica(dev)
-            with torch.cuda.device(dev):
-                Xd = self._to_device(X[b0:b1], dev)
-                Cd = None if C is None else self._to_device(C[b0:b1], dev)
-                lp = eng.forward(Xd, Cd, want_z=False, want_logdet=False)[2]
-                host = _pinned(tuple(lp.shape), ("mdev_lp", k))
-                host.copy_(lp, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record()
-            pending.append((b0 - lo, b1 - lo, host, ev, lp))
-        for a, b, host, ev, _ in pending:
-            ev.synchronize()
-            out[a:b] = host.numpy()
-        return out
+
+        def run(eng, dev, b0, b1):
+            Xd = self._to_device(X[b0:b1], dev)
+            Cd = None if C is None else self._to_device(C[b0:b1], dev)
+            return eng.forward(Xd, Cd, want_z=False, want_logdet=False)[2]
+
+        return self._device_blocks(lo, hi, list(devices) if devices else [self._device], run,
+                                   np.empty(hi - lo, dtype=np.float32), 0, "mdev_lp")

@@ -33,18 +33,27 @@ def test_philox_normal_is_standard_normal_and_shard_invariant():
 
 
 @pytest.mark.parametrize("dtype", [np.float64, np.float32])
-def test_host_gather_rows_matches_numpy(dtype):
+def test_host_gather_xc_matches_numpy(dtype):
     from probaforms_b200 import _lib
-    from probaforms_b200.ingest import gather_into, host_rows
+    from probaforms_b200.ingest import _gather, host_rows
     lib = _lib.load()
     rng = np.random.default_rng(0)
     A = rng.normal(size=(50000, 7)).astype(dtype)
     idx = rng.permutation(50000).astype(np.int64)
     dst = torch.empty(30000, 7, dtype=torch.float32)
-    gather_into(lib, host_rows(A), idx[1000:], 0, 30000, dst, threads=4)
+    _gather(lib, host_rows(A), None, idx[1000:], 0, 30000, dst, None, threads=4)
     assert np.array_equal(dst.numpy(), A[idx[1000:31000]].astype(np.float32))
-    gather_into(lib, host_rows(A), None, 123, 30000, dst, threads=3)
+    _gather(lib, host_rows(A), None, None, 123, 30000, dst, None, threads=3)
     assert np.array_equal(dst.numpy(), A[123:30123].astype(np.float32))
+    # X and C rows in one pass (C of the other dtype, width 8: the streaming-store path)
+    Cn = rng.normal(size=(50000, 8)).astype(np.float32 if dtype == np.float64 else np.float64)
+    dst_c = torch.empty(30000, 8, dtype=torch.float32)
+    _gather(lib, host_rows(A), host_rows(Cn), idx[1000:], 0, 30000, dst, dst_c, threads=4)
+    assert np.array_equal(dst.numpy(), A[idx[1000:31000]].astype(np.float32))
+    assert np.array_equal(dst_c.numpy(), Cn[idx[1000:31000]].astype(np.float32))
+    _gather(lib, host_rows(A), host_rows(Cn), None, 123, 30000, dst, dst_c, threads=3)
+    assert np.array_equal(dst.numpy(), A[123:30123].astype(np.float32))
+    assert np.array_equal(dst_c.numpy(), Cn[123:30123].astype(np.float32))
     out = np.empty(5 << 20, dtype=np.uint8)
     src = rng.integers(0, 255, size=5 << 20, dtype=np.uint8)
     assert lib.rnvp_host_copy(C.c_void_p(out.ctypes.data), C.c_void_p(src.ctypes.data), out.nbytes, 4) == 0
@@ -144,7 +153,7 @@ def test_lent_result_buffers_return_to_the_pool_only_when_every_view_is_gone():
         assert I.RESULTS.lend((1024, 1024)) == (None, None)
 
 
-def test_host_rows_accepts_a_read_only_memmap_without_copying(tmp_path):
+def test_host_gather_xc_reads_a_read_only_memmap_without_copying(tmp_path):
     """Ranks of one node may share one host copy of the data (np.memmap): host_rows must hand the C ABI its pages as is."""
     import probaforms_b200.ingest as I
     from probaforms_b200 import _lib
@@ -160,8 +169,8 @@ def test_host_rows_accepts_a_read_only_memmap_without_copying(tmp_path):
     assert rows.ctypes.data == ro.ctypes.data and rows.dtype == np.float32
     idx = np.random.default_rng(1).permutation(1000)[:300].astype(np.int64)
     dst = torch.empty(300, 8)
-    assert lib.rnvp_host_gather_rows(C.c_void_p(rows.ctypes.data), 0, 8, C.c_void_p(idx.ctypes.data), 0, 300,
-                                     C.c_void_p(dst.data_ptr()), 3) == 0
+    assert lib.rnvp_host_gather_xc(C.c_void_p(rows.ctypes.data), 0, 8, None, 0, 0, C.c_void_p(idx.ctypes.data), 0, 300,
+                                   C.c_void_p(dst.data_ptr()), None, 3) == 0
     assert np.array_equal(dst.numpy(), src[idx])
 
 
