@@ -401,6 +401,21 @@ int rnvp_wg_fit_epoch(const rnvp_wg_desc* d, float* d_params, float* d_square_av
                       float* d_gen_loss, float* d_disc_loss, void* d_workspace, int64_t workspace_bytes,
                       void* stream);
 
+/* Predictive summaries (rnvp_summary.cu; probaforms_b200/predictive.py).  Per cell c < cells of the k draws laid out
+ * d_draws[j * cells + c] (cell = row * D + feature):
+ *   d_mean, d_std (ddof = 0) in fp64 with a fixed summation order; the nq quantiles of numpy's default 'linear' method,
+ *   equal bit for bit to np.quantile(draws, q, axis=0) of the float32 draws (NaN for every quantile of a cell with a
+ *   NaN draw); with d_y [cells]: d_crps = (1/k) sum_j |x_j - y| - (1/(2 k^2)) sum_i sum_j |x_i - x_j| (NaN for a NaN y)
+ *   and d_rank = #{j : x_j < y}.
+ * Output pointers may be NULL (skipped); d_crps / d_rank need d_y.  q is a HOST array of nq <= 32 values in [0, 1].
+ * Quantile plane i is written at d_quant + i * q_stride (q_stride >= cells), so row blocks can write straight into
+ * full-size outputs.  RNVP_EINVAL for k < 1 or k > RNVP_SUMMARY_MAX_DRAWS and the other bad arguments. */
+#define RNVP_SUMMARY_MAX_DRAWS 8192
+#define RNVP_SUMMARY_MAX_QUANTILES 32
+int rnvp_draw_summary(const float* d_draws, int64_t k, int64_t cells, const double* q, int nq, const float* d_y,
+                      double* d_mean, double* d_std, double* d_quant, int64_t q_stride, double* d_crps,
+                      int32_t* d_rank, void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

@@ -122,6 +122,8 @@ SIGNATURES = {
     "rnvp_wg_fit_epoch": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64, C.c_int64,
                                     C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
                                     c_f32_p, C.c_uint64, c_f32_p, c_f32_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_draw_summary": (C.c_int, [c_f32_p, C.c_int64, C.c_int64, C.POINTER(C.c_double), C.c_int, c_f32_p,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

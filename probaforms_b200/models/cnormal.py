@@ -129,11 +129,13 @@ class Net(nn.Module):
         return M
 
     @torch.no_grad()
-    def forward(self, X, C, eps=None, seed=None):
+    def forward(self, X, C, eps=None, seed=None, row_offset=0, out=None):
         """(x_tilde, inv, mu, sigma) as in the reference (cnormal.py:77-91), computed by one inference kernel.
 
-        ``eps`` [n, var_size] supplies the noise (parity mode); otherwise it is Philox keyed on (seed, row, feature),
-        with ``seed`` drawn as one int64 from the global generator when not given.  ``inv`` is None without ``X``."""
+        ``eps`` [n, var_size] supplies the noise (parity mode); otherwise it is Philox keyed on (seed, row_offset + row,
+        feature), with ``seed`` drawn as one int64 from the global generator when not given.  ``inv`` is None without
+        ``X``.  ``out`` (a float32 device tensor [n, var_size]) receives x_tilde; mu and sigma are then not computed and
+        come back None."""
         desc, flat = self._ready()
         dev = flat.device
         Cd = torch.as_tensor(C, dtype=torch.float32).to(dev).contiguous()
@@ -153,12 +155,18 @@ class Net(nn.Module):
             seed = 0
         elif seed is None:
             seed = int(torch.empty((), dtype=torch.int64).random_().item())
-        mu, sigma, xt = (torch.empty(n, D, dtype=torch.float32, device=dev) for _ in range(3))
+        if out is None:
+            mu, sigma, xt = (torch.empty(n, D, dtype=torch.float32, device=dev) for _ in range(3))
+        else:
+            if not (out.device == dev and out.dtype == torch.float32 and tuple(out.shape) == (n, D)
+                    and out.is_contiguous()):
+                raise ValueError(f"out must be a contiguous float32 tensor [{n}, {D}] on {dev}")
+            mu, sigma, xt = None, None, out
         inv = torch.empty(n, D, dtype=torch.float32, device=dev) if Xd is not None else None
         ptr = lambda t: None if t is None else t.data_ptr()   # noqa: E731
         _lib.check(desc.lib.rnvp_cn_forward(desc.h, flat.data_ptr(), ptr(M), ptr(Xd), Cd.data_ptr(), n,
-                                            ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), 0, ptr(eps), mu.data_ptr(),
-                                            sigma.data_ptr(), xt.data_ptr(), ptr(inv), _stream(dev)),
+                                            ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), int(row_offset), ptr(eps), ptr(mu),
+                                            ptr(sigma), xt.data_ptr(), ptr(inv), _stream(dev)),
                    "rnvp_cn_forward")
         return xt, inv, mu, sigma
 
@@ -433,3 +441,17 @@ class ConditionalNormal(GenModel):
             Cs = torch.zeros(C, 1)
         x_tilde, _, _, _ = self.model(None, Cs, eps=eps, seed=seed)
         return x_tilde.cpu().numpy()
+
+    def _draw_hook(self):
+        """(device, var_size, draw) for on-device summaries: ``draw(Cd, seed, r0, m, out)`` writes rows [r0, r0 + m) of
+        ``sample(C, seed=seed)`` for the device-resident conditions Cd (all n rows) into the device buffer out
+        [m, var_size]; one rnvp_cn_forward launch, no host copy."""
+        if getattr(self, "model", None) is None or not isinstance(self.model, Net):
+            raise RuntimeError("ConditionalNormal.sample: call fit() first")
+        net = self.model
+        _, flat = net._ready()
+
+        def draw(Cd, seed, r0, m, out):
+            net(None, Cd[r0:r0 + m], seed=seed, row_offset=r0, out=out)
+
+        return flat.device, net.var_size, draw

@@ -189,7 +189,9 @@ class Decoder(nn.Module):
         """X_rec [n, n_outputs] of the rows [X | C] (cvae.py:89-110), X the latent [n, lat_size]."""
         return self._decode(X, C, None, None)
 
-    def _decode(self, Z, C, n, seed):
+    def _decode(self, Z, C, n, seed, row_offset=0, out=None):
+        """Decoded rows into ``out`` (a float32 device tensor [n, D]) or a new tensor; Philox noise keyed on
+        (seed, row_offset + row, latent index) when Z is None."""
         if self._pair is None:
             raise RuntimeError("Decoder.forward runs on the kernels of a fitted CVAE; call CVAE.fit first")
         desc, flat = self._pair.ready()
@@ -209,10 +211,11 @@ class Decoder(nn.Module):
                                f"columns, got {desc.L + (0 if Cd is None else Cd.shape[1])}")
         if seed is None:
             seed = 0
-        x = torch.empty(n, desc.D, dtype=torch.float32, device=dev)
+        x = torch.empty(n, desc.D, dtype=torch.float32, device=dev) if out is None else out
         _lib.check(desc.lib.rnvp_cv_decode(desc.h, flat.data_ptr(), None if Zd is None else Zd.data_ptr(),
                                            None if Cd is None else Cd.data_ptr(), n,
-                                           ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), 0, x.data_ptr(), _stream(dev)),
+                                           ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), int(row_offset), x.data_ptr(),
+                                           _stream(dev)),
                    "rnvp_cv_decode")
         return x
 
@@ -553,3 +556,15 @@ class CVAE(GenModel):
                 seed = int(torch.empty((), dtype=torch.int64).random_().item())
             x = self.decoder._decode(None, Cs, n, seed)
         return x.cpu().numpy()
+
+    def _draw_hook(self):
+        """(device, var_size, draw) for on-device summaries: ``draw(Cd, seed, r0, m, out)`` writes rows [r0, r0 + m) of
+        ``sample(C, seed=seed)`` for the device-resident conditions Cd (all n rows, or None) into the device buffer out
+        [m, var_size]; one rnvp_cv_decode launch, no host copy."""
+        desc, flat = self._ready()
+        dec = self.decoder
+
+        def draw(Cd, seed, r0, m, out):
+            dec._decode(None, None if Cd is None else Cd[r0:r0 + m], m, seed, row_offset=r0, out=out)
+
+        return flat.device, desc.D, draw

@@ -665,6 +665,19 @@ class RealNVP(GenModel):
         copy_stream.synchronize()
         return arr
 
+    def _draw_hook(self):
+        """(device, var_size, draw) for on-device summaries: ``draw(Cd, seed, r0, m, out)`` writes rows [r0, r0 + m) of
+        ``sample(C, seed=seed)`` for the device-resident conditions Cd (all n rows, or None) into the device buffer out
+        [m, var_size]; one rnvp_sample launch, no host copy."""
+        if self.nf is None:
+            raise RuntimeError("RealNVP.sample: call fit() first")
+        eng = self.nf._fused()
+
+        def draw(Cd, seed, r0, m, out):
+            eng.sample(m, None if Cd is None else Cd[r0:r0 + m], seed=seed, row_offset=r0, out=out)
+
+        return eng.device, eng.D, draw
+
     def _device_blocks(self, lo, hi, devices, run, out, axis, key):
         """Rows [lo, hi) in contiguous blocks over the GPUs ``devices`` of this process: ``run(eng, dev, b0, b1)`` enqueues
         block [b0, b1) on the device's replica of the weights and returns its device result, which is copied back through

@@ -119,7 +119,9 @@ class Generator(_Net):
         """X_gen [n, n_outputs] of the rows [X | C] (wgan.py:38-58), X the latent [n, latent_dim]."""
         return self._generate(X, C, None, None)
 
-    def _generate(self, Z, C, n, seed):
+    def _generate(self, Z, C, n, seed, row_offset=0, out=None):
+        """Generated rows into ``out`` (a float32 device tensor [n, D]) or a new tensor; Philox noise keyed on
+        (seed, row_offset + row, latent index) when Z is None."""
         desc, flat = self._ready()
         dev = flat.device
         Zd = None
@@ -129,11 +131,11 @@ class Generator(_Net):
         if n is None:
             n = len(C)
         Cd = _cond(C, dev, desc, n)
-        x = torch.empty(n, desc.D, dtype=torch.float32, device=dev)
+        x = torch.empty(n, desc.D, dtype=torch.float32, device=dev) if out is None else out
         _lib.check(desc.lib.rnvp_wg_generate(desc.h, flat.data_ptr(), None if Zd is None else Zd.data_ptr(),
                                              None if Cd is None else Cd.data_ptr(), n,
-                                             ct.c_uint64((0 if seed is None else seed) & 0xFFFFFFFFFFFFFFFF), 0,
-                                             x.data_ptr(), _stream(dev)), "rnvp_wg_generate")
+                                             ct.c_uint64((0 if seed is None else seed) & 0xFFFFFFFFFFFFFFFF),
+                                             int(row_offset), x.data_ptr(), _stream(dev)), "rnvp_wg_generate")
         return x
 
 
@@ -382,3 +384,15 @@ class ConditionalWGAN(GenModel):
                 seed = int(torch.empty((), dtype=torch.int64).random_().item())
             x = self.generator._generate(None, Cs, n, seed)
         return x.cpu().numpy()
+
+    def _draw_hook(self):
+        """(device, var_size, draw) for on-device summaries: ``draw(Cd, seed, r0, m, out)`` writes rows [r0, r0 + m) of
+        ``sample(C, seed=seed)`` for the device-resident conditions Cd (all n rows, or None) into the device buffer out
+        [m, var_size]; one rnvp_wg_generate launch, no host copy."""
+        desc, flat = self._ready()
+        gen = self.generator
+
+        def draw(Cd, seed, r0, m, out):
+            gen._generate(None, None if Cd is None else Cd[r0:r0 + m], m, seed, row_offset=r0, out=out)
+
+        return flat.device, desc.D, draw
