@@ -416,6 +416,24 @@ int rnvp_draw_summary(const float* d_draws, int64_t k, int64_t cells, const doub
                       double* d_mean, double* d_std, double* d_quant, int64_t q_stride, double* d_crps,
                       int32_t* d_rank, void* stream);
 
+/* Joint scores of k draws per row (rnvp_summary.cu; probaforms_b200/predictive.py predictive_joint).  The draws of a
+ * block of rows are laid out d_draws[(j * rows + r) * D + d] (draw j, row r, feature d), 1 <= D <= RNVP_JOINT_MAX_D.
+ * Per row r:
+ *   d_mean [rows, D] (required): the fp64 mean of the draws, summed in a fixed order;
+ *   d_cov [rows, D, D] (NULL: skipped): sum_j (x_j - mean)(x_j - mean)^T / k, both triangles;
+ *   with d_y [rows, D]: d_energy [rows] = (1/k) sum_j ||x_j - y|| - (1/(2 k^2)) sum_i sum_j ||x_i - x_j|| (Euclidean)
+ *   and d_variogram [rows] = sum_{d<e} (|y_d - y_e|^p - (1/k) sum_j |x_jd - x_je|^p)^2 (NULL: skipped).
+ * A row with a non-finite draw gives NaN cov, energy and variogram; a NaN in y gives NaN energy and variogram.
+ * d_energy needs a device workspace of rnvp_draw_joint_workspace_bytes(k, rows, D) bytes (rows x tile pairs doubles;
+ * -1 for bad arguments).  Results are bitwise repeatable and do not depend on how rows are split into calls.
+ * RNVP_EINVAL for k outside [1, RNVP_SUMMARY_MAX_DRAWS], D outside [1, RNVP_JOINT_MAX_D], p not finite and > 0, and
+ * the other bad arguments. */
+#define RNVP_JOINT_MAX_D 128
+int64_t rnvp_draw_joint_workspace_bytes(int64_t k, int64_t rows, int D);
+int rnvp_draw_joint(const float* d_draws, int64_t k, int64_t rows, int D, const float* d_y, double p, double* d_mean,
+                    double* d_cov, double* d_energy, double* d_variogram, void* d_workspace, int64_t workspace_bytes,
+                    void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

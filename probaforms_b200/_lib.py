@@ -124,6 +124,9 @@ SIGNATURES = {
                                     c_f32_p, C.c_uint64, c_f32_p, c_f32_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_draw_summary": (C.c_int, [c_f32_p, C.c_int64, C.c_int64, C.POINTER(C.c_double), C.c_int, c_f32_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, c_stream]),
+    "rnvp_draw_joint_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int]),
+    "rnvp_draw_joint": (C.c_int, [c_f32_p, C.c_int64, C.c_int64, C.c_int, c_f32_p, C.c_double, C.c_void_p, C.c_void_p,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

@@ -66,7 +66,7 @@ def device_split(model, C, k, y):
     Cd = upload_resident(lib, C, dev)
     yd = None if y is None else upload_resident(lib, y, dev)
     q = np.asarray(Q, dtype=np.float64)
-    out = P._Outputs(n * D, len(q), y is not None, dev)
+    out = P._Outputs(n, D, k, q, y is not None, dev)
     blocks = P._plan_blocks(n, k, D, P._BLOCK_BYTES)
     buf = torch.empty(k * blocks[0][1] * D, dtype=torch.float32, device=dev)
     result = None
@@ -79,7 +79,7 @@ def device_split(model, C, k, y):
             for j in range(k):
                 draw(Cd, 1000 + j, r0, m, xs[j])
             ev[1].record()
-            out.summarize(lib, xs, k, r0 * D, m * D, q, None if yd is None else yd[r0:r0 + m])
+            out.block(lib, xs, r0, m, None if yd is None else yd[r0:r0 + m])
             ev[2].record()
             marks.append(ev)
         torch.cuda.synchronize()
