@@ -20,8 +20,11 @@
 //   MODE 2 (fit step): the forward sweep additionally stashes (x_T, s) per layer and writes h = act(.) and u = [x_K, c] into
 //   the activation record of (layer, row) (rnvp_wgrad_tc.cu); the same CTA then walks the layers BACKWARDS with the same
 //   thread ownership, streaming the transposed chunk images: delta2 from the stash -> TMEM (hi/lo, 4 DH columns), per chunk
-//   step dh = delta2 W2 (tensor core), delta1 = dh * act'(h) with h read back from the record, du += delta1 W1[:, x_K]
-//   (merged A_hi x [B_hi ; B_lo]); delta2 completes the record, and rnvp_wgrad_tc_kernel contracts the records over rows.
+//   step dh = delta2 W2 (tensor core), delta1 = dh * act'(h), du += delta1 W1[:, x_K] (merged A_hi x [B_hi ; B_lo]); delta2
+//   completes the record, and rnvp_wgrad_tc_kernel contracts the records over rows.  h comes back from the record through
+//   the ring (DH = 16 / 64): each backward stage also carries the tile's h chunk (4 bulk copies of 4 KB, issued up to four
+//   chunk steps ahead), once the tile's forward stores are fenced for the async proxy (WB_RF); DH = 32 has no room for the
+//   larger stages and loads h into registers before it waits for dh.
 // Reference semantics: RealNVPLayer.f / .g (realnvp.py:73-129) looped as in nflow.py:109-115 / 142-143; MODE 2 is the
 // autograd backward of loss = -nf.log_prob(X, C) (realnvp.py:246-250) up to the weight-gradient contraction.
 #include <cuda_runtime.h>
@@ -70,6 +73,20 @@ __device__ __forceinline__ void tmem_ld_w(uint32_t taddr, uint32_t (&r)[W]) {
 
 // barrier indices: ring full / empty first, then the tile hand-offs
 enum { WB_WF = 0, WB_WE = WD_STAGES, WB_UF = 2 * WD_STAGES, WB_D1F0, WB_D1F1, WB_AF0, WB_AF1, WB_D2F, WB_XF, WB_XE, WB_COUNT };
+// one more barrier where h rides in the ring: the tile's forward sweep has written all its activation records (the
+// backward stages copy h out of them).  Appended, so that the layout of the other kernels stays as it is
+constexpr int WB_RF = WB_COUNT;
+
+// h rides in the backward ring stage (fit step): the stage carries the tile's h chunk next to the W2T / W1T images.  Not
+// at DH = 32, whose two CTAs per SM cannot hold four 32 KB stages each; that shape loads h from the record into registers.
+__host__ __device__ constexpr bool wide_hring(int DH, int mode) { return mode == 2 && DH != 32; }
+// floats of one ring stage: forward [W1 chunk | W2 chunk | b2 of a net], backward [W2T chunk | W1T chunk (| h chunk)]
+__host__ __device__ constexpr int wide_stage_floats(int DH, int CDMAX, int mode) {
+  const int CU = 32, K1PMAX = (DH + CDMAX + 1 + 7) & ~7, NTP = (DH + 15) & ~15;
+  const int fwd = 2 * CU * K1PMAX + 2 * NTP * CU + 2 * NTP * 8;
+  const int bwd = 2 * (2 * NTP * CU) + (wide_hring(DH, mode) ? 128 * CU : 0);
+  return ((fwd > bwd ? fwd : bwd) + 31) & ~31;
+}
 
 // DH <= 32: two CTAs per SM (256 TMEM columns each).  DH = 16 keeps the double-buffered D1 / dh chunk ring; DH = 32 only fits
 // with ONE ring buffer (forward 240, backward 256 columns): the GEMM1 of the next chunk step is then issued behind this
@@ -104,11 +121,13 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
   const int nL = a.l1 - a.l0;
   const int w1c = 2 * CU * K1P;                         // floats of one W1 chunk image [hi | lo]
   constexpr int W2C = 2 * NTP * CU, B2C = 2 * NTP * 8;  // W2 chunk image [hi | lo]; b2 image of one net [hi | lo]
-  const int stage_floats = ((2 * CU * K1PMAX + W2C + B2C) + 31) & ~31;      // >= the backward stage: W2T + W1T chunk = 2 * W2C
+  constexpr bool HRING = wide_hring(DH, MODE);
+  constexpr int stage_floats = wide_stage_floats(DH, CDMAX, MODE);
+  constexpr int HCH = 2 * W2C;                          // h chunk of a backward stage: [record block q][8 column groups][32][4]
   const bool do_bwd = MODE == 2 && a.do_bwd;
   const int n_sweeps = do_bwd ? 2 : 1;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sm + WD_STAGES * stage_floats);
-  float* xch = reinterpret_cast<float*>(bars + WB_COUNT);                 // [128][2]: partial (logdet, |z|^2) of the second half-thread
+  float* xch = reinterpret_cast<float*>(bars + WB_COUNT + (HRING ? 1 : 0));   // [128][2]: partial (logdet, |z|^2) of the second half-thread
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(xch + 256);
 
   if (warp == 1) tmem_alloc(tmem_slot, TALLOC);
@@ -119,6 +138,7 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
     mbar_init(&bars[WB_AF0], 256); mbar_init(&bars[WB_AF1], 256);
     mbar_init(&bars[WB_D2F], 1);
     mbar_init(&bars[WB_XF], 128); mbar_init(&bars[WB_XE], 128);       // row-pair exchange of the partial log-dets / norms
+    if (HRING) mbar_init(&bars[WB_RF], 256);
     mbar_fence_init();
   }
   fence_before_sync();
@@ -132,6 +152,17 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
     if (lane == 0) {
       long long step = 0;
       const uint32_t w1c_bytes = (uint32_t)w1c * 4u, w2c_bytes = (uint32_t)W2C * 4u, b2_bytes = (uint32_t)B2C * 4u;
+      constexpr uint32_t h_bytes = HRING ? 128u * CU * 4u : 0u;
+      // h chunk of backward chunk step cc of layer i into ring stage st: columns [col0, col0 + CU) of the tile's four 32-row
+      // record blocks, one contiguous 4 KB range each (rnvp_wgrad_tc.cu layout), kept in the record's slot order
+      auto copy_h = [&](int st, long long tile, int i, int cc) {
+        const int net = cc >= NC ? 1 : 0, col0 = net * H + (cc - net * NC) * CU;
+        const size_t blk = (size_t)(a.rec >> 2) * 128;
+        const float* src = a.records + ((size_t)i * (size_t)(a.Npad >> 5) + (size_t)tile * 4) * blk + (size_t)(col0 >> 2) * 128;
+        float* dst = sm + (size_t)st * stage_floats + HCH;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) bulk_g2s(dst + q * CU * 32, src + q * blk, CU * 32 * 4u, &bars[WB_WF + st]);
+      };
       for (int it = 0; it < my_tiles; ++it)
         for (int sw = 0; sw < n_sweeps; ++sw)
           for (int li = 0; li < nL; ++li) {
@@ -153,9 +184,22 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
                 bulk_g2s(dst + 2 * CU * K1PMAX, W2 + (size_t)(c * 2 + net) * W2C, w2c_bytes, &bars[WB_WF + st]);
                 if (with_b2) bulk_g2s(dst + 2 * CU * K1PMAX + W2C, B2 + (size_t)net * B2C, b2_bytes, &bars[WB_WF + st]);
               } else {
-                mbar_expect_tx(&bars[WB_WF + st], 2 * w2c_bytes);
+                mbar_expect_tx(&bars[WB_WF + st], 2 * w2c_bytes + h_bytes);
                 bulk_g2s(dst, W2T + (size_t)cc * W2C, w2c_bytes, &bars[WB_WF + st]);
                 bulk_g2s(dst + W2C, W1T + (size_t)cc * W2C, w2c_bytes, &bars[WB_WF + st]);
+                if constexpr (HRING) {
+                  // the forward sweep wrote h with generic stores: the async-proxy copies wait for WB_RF.  The first
+                  // stages of the sweep get their images at once (they are armed for the h bytes too) and their h once
+                  // the forward sweep is done, so the turn from forward to backward does not wait for the images
+                  const long long tile = (long long)blockIdx.x + (long long)it * gridDim.x;
+                  const int k = li * NCS + cc, k_first = nL * NCS < WD_STAGES ? nL * NCS : WD_STAGES;
+                  if (k >= k_first) copy_h(st, tile, i, cc);
+                  else if (k + 1 == k_first) {
+                    mbar_wait(&bars[WB_RF], (uint32_t)(it & 1));
+                    for (int k0 = 0; k0 < k_first; ++k0)
+                      copy_h((int)((step - k + k0) % WD_STAGES), tile, a.l1 - 1 - k0 / NCS, k0 % NCS);
+                  }
+                }
               }
             }
           }
@@ -471,6 +515,11 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
         if ((i & 1) == 0) layer(xa, xb, i);              // even layer transforms the even features
         else layer(xb, xa, i);
       }
+      if (HRING && do_bwd) {
+        // this thread's h record stores of the tile, ordered before the producer's async-proxy copies of them
+        asm volatile("fence.proxy.async.global;" ::: "memory");
+        mbar_arrive(&bars[WB_RF]);
+      }
 
       if (valid && a.out_x) {
         if (exact) {
@@ -567,19 +616,40 @@ __global__ void __launch_bounds__(WD_THREADS, DH == 16 ? 2 : (DH == 32 ? RNVP_WI
             fence_before_sync();
             mbar_arrive(&bars[WB_UF]);
             // ---- chunk steps: delta1 = dh * act'(h), dh from the tensor core, h from the record the forward sweep wrote
+            // ring step of chunk step 0, modulo 2^32: only its stage and phase (step % 2 WD_STAGES) are used
+            const uint32_t step0 = ((uint32_t)(2 * it + 1) * (uint32_t)nL + (uint32_t)(a.l1 - 1 - i)) * (uint32_t)NCS;
             for (int cc = 0; cc < NCS; ++cc) {
               const int buf = cc & (NB1 - 1), net = cc >= NC ? 1 : 0;
               const int col0 = net * H + (cc - net * NC) * CU + 16 * half;
               uint32_t hv[16];
+              if constexpr (!HRING) {
 #pragma unroll
-              for (int m = 0; m < 4; ++m) {           // issued before the wait for dh: the L2 / HBM latency hides behind the MMAs
-                const int cg = (col0 >> 2) + m;
-                const float4 v = *reinterpret_cast<const float4*>(rb + cg * 128 + ((lane ^ (cg & 7)) << 2));
-                hv[4 * m] = __float_as_uint(v.x); hv[4 * m + 1] = __float_as_uint(v.y);
-                hv[4 * m + 2] = __float_as_uint(v.z); hv[4 * m + 3] = __float_as_uint(v.w);
+                for (int m = 0; m < 4; ++m) {         // issued before the wait for dh: the L2 / HBM latency hides behind the MMAs
+                  const int cg = (col0 >> 2) + m;
+                  const float4 v = *reinterpret_cast<const float4*>(rb + cg * 128 + ((lane ^ (cg & 7)) << 2));
+                  hv[4 * m] = __float_as_uint(v.x); hv[4 * m + 1] = __float_as_uint(v.y);
+                  hv[4 * m + 2] = __float_as_uint(v.z); hv[4 * m + 3] = __float_as_uint(v.w);
+                }
               }
               mbar_wait(&bars[WB_D1F0 + buf], (ph_d1 >> buf) & 1u); ph_d1 ^= 1u << buf;
               fence_after_sync();
+              if constexpr (HRING) {
+                // h from the ring stage of this chunk step (already full: its gemmA has completed).  The stage is not
+                // refilled under these reads: they complete before this thread's WB_AF arrival below, the issuer commits
+                // the stage's WB_WE only behind the gemmB that waits for that arrival, and the producer refills the stage
+                // only after WB_WE
+                const uint32_t s = step0 + (uint32_t)cc;
+                const int st = (int)(s % WD_STAGES);
+                mbar_wait(&bars[WB_WF + st], (uint32_t)((s / WD_STAGES) & 1));
+                const float* hs = sm + (size_t)st * stage_floats + HCH + quarter * (CU * 32);
+#pragma unroll
+                for (int m = 0; m < 4; ++m) {         // same slot order as the record: conflict-free 512-byte warp reads
+                  const int cg = (col0 >> 2) + m;
+                  const float4 v = *reinterpret_cast<const float4*>(hs + (cg & 7) * 128 + ((lane ^ (cg & 7)) << 2));
+                  hv[4 * m] = __float_as_uint(v.x); hv[4 * m + 1] = __float_as_uint(v.y);
+                  hv[4 * m + 2] = __float_as_uint(v.z); hv[4 * m + 3] = __float_as_uint(v.w);
+                }
+              }
               const uint32_t d1 = trow + DHB + buf * 2 * CU + 16 * half;
               uint32_t dh[16], lo[16];
               tmem_ld_x16(d1, dh);
@@ -646,17 +716,17 @@ cudaError_t launch_wide_shape(int act, int mode, const RnvpWideArgs& a, int grid
 
 }  // namespace
 
-size_t rnvp_wide_smem_bytes(int DH, int CDMAX) {
-  const int K1PMAX = (DH + CDMAX + 1 + 7) & ~7, NTP = (DH + 15) & ~15, CU = 32;
-  const size_t stage = ((size_t)(2 * CU * K1PMAX + 2 * NTP * CU + 2 * NTP * 8) + 31) & ~(size_t)31;
-  return WD_STAGES * stage * 4 + 8 * WB_COUNT + 256 * 4 + 64;
+// the fit step (mode 2) of DH = 16 / 64 has the larger backward stages that carry h; log-prob and sample keep the smaller ones
+size_t rnvp_wide_smem_bytes(int DH, int CDMAX, int mode) {
+  return WD_STAGES * (size_t)wide_stage_floats(DH, CDMAX, mode) * 4 + 8 * (WB_COUNT + (wide_hring(DH, mode) ? 1 : 0)) +
+         256 * 4 + 64;
 }
 
 int rnvp_wide_ctas_per_sm(int DH) { return DH == 16 ? 2 : (DH == 32 ? RNVP_WIDE32_CTAS : 1); }
 
 cudaError_t rnvp_launch_wide(int DH, int act, int mode, const RnvpWideArgs& a, int grid, cudaStream_t st) {
-  if (DH == 64) return launch_wide_shape<64, 32>(act, mode, a, grid, rnvp_wide_smem_bytes(64, 32), st);
-  if (DH == 32) return launch_wide_shape<32, 16>(act, mode, a, grid, rnvp_wide_smem_bytes(32, 16), st);
-  if (DH == 16) return launch_wide_shape<16, 16>(act, mode, a, grid, rnvp_wide_smem_bytes(16, 16), st);
+  if (DH == 64) return launch_wide_shape<64, 32>(act, mode, a, grid, rnvp_wide_smem_bytes(64, 32, mode), st);
+  if (DH == 32) return launch_wide_shape<32, 16>(act, mode, a, grid, rnvp_wide_smem_bytes(32, 16, mode), st);
+  if (DH == 16) return launch_wide_shape<16, 16>(act, mode, a, grid, rnvp_wide_smem_bytes(16, 16, mode), st);
   return cudaErrorInvalidValue;
 }
