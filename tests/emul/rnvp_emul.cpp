@@ -186,7 +186,7 @@ struct Emu {
 extern "C" int rnvp_emulate(int mode, int D, int Cd, int L, int nh, const int* hidden, int act, int TR_force,
                             const float* flat, const float* X, const float* C, const long long* idx, long long N,
                             int l0, int l1, float scale, float* out_x, float* out_logdet, float* out_logp,
-                            float* gflat, double* loss_sum, int* info /* [TR, smem_bytes, n_ops, n_chunks, packed] */) {
+                            float* gflat, double* loss_sum, int* info /* [TR, smem_bytes, n_ops, n_chunks, packed, ops past a layer's first weight-row chunk] */) {
   FlowGeom g;
   g.D = D; g.Cd = Cd; g.L = L; g.nh = nh; g.act = act;
   for (int q = 0; q < nh; ++q) g.hidden[q] = hidden[q];
@@ -198,7 +198,10 @@ extern "C" int rnvp_emulate(int mode, int D, int Cd, int L, int nh, const int* h
   const bool ok = b.plan_best(TR_force);
   if (!ok) return -2;
   b.build();
-  if (info) { info[0] = b.TR; info[1] = b.sm.total_floats * 4; info[2] = (int)b.ops.size(); info[3] = (int)b.chunks.size(); info[4] = (int)g.packed; }
+  if (info) { info[0] = b.TR; info[1] = b.sm.total_floats * 4; info[2] = (int)b.ops.size(); info[3] = (int)b.chunks.size(); info[4] = (int)g.packed;
+    info[5] = 0;
+    for (const RnvpOp& op : b.ops) info[5] += op.n0 > 0;
+  }
   Emu e;
   e.g = &g; e.b = &b; e.mode = mode; e.R = b.R;
   e.X = X; e.C = C; e.idx = idx; e.N = N; e.scale = scale;

@@ -198,18 +198,34 @@ def test_gradients_match_oracle_many_ctas(case, rows):
         assert err <= 2e-5
 
 
-@pytest.mark.parametrize("nb", [32, 50, 100, 4096, 65537])
-def test_critic_output_bias_gradient_is_exactly_zero(nb):
+# the reference fixture's nets (R = 64), and nets whose tiles hold 16, 8 and 4 rows: (D, Cd, latent, g_hidden, d_hidden)
+SMALL_TILE_NETS = {16: (12, 2, 128, (511, 257, 3, 99), (7,)), 8: (128, 256, 128, (512,), (512, 512)),
+                   4: (32, 8, 128, (512, 512, 512, 512), (512, 512, 512, 512))}
+
+
+@pytest.mark.parametrize("nb,R", [(nb, 64) for nb in (32, 50, 100, 4096, 65537)] +
+                         [(nb, R) for R in (16, 8, 4) for nb in (1, R, R + 1, 37 * R + 3)],
+                         ids=[str(nb) for nb in (32, 50, 100, 4096, 65537)] +
+                         [f"R{R}-{nb}" for R in (16, 8, 4) for nb in (1, R, R + 1, 37 * R + 3)])
+def test_critic_output_bias_gradient_is_exactly_zero(nb, R):
     """sum_real(-1/nb) + sum_fake(+1/nb) is exactly 0 in the reference; any rounding noise left here becomes an RMSprop
     step of up to ~lr on a parameter the reference never moves (DESIGN §13)."""
     g = load_golden("wgan_grad_relu")
+    if R != 64:
+        D, Cd, L, gh, dh = SMALL_TILE_NETS[R]
+        torch.manual_seed(R)
+        g = dict(D=D, Cd=Cd, latent=L, g_hidden=np.array(gh), g_act=np.frombuffer(b"relu", np.uint8),
+                 d_hidden=np.array(dh), d_act=np.frombuffer(b"tanh", np.uint8), init=O.init_params(D, Cd, L, gh, dh).numpy())
     m, c = _grad_model(g, g["init"])
+    desc, _ = m._ready()
+    assert max(n for n in range(1, 129) if desc.lib.rnvp_wg_workspace_bytes(desc.h, n, 0) ==
+               desc.lib.rnvp_wg_workspace_bytes(desc.h, 1, 0)) == R
     X, Cc = O.grad_inputs(nb, nb, c["D"], c["Cd"])
     z = O.grad_eps(nb + 1, nb, c["L"])
     _, grad = m._grad(torch.from_numpy(X).cuda(), torch.from_numpy(Cc).cuda(), z, False)
     grad = grad.cpu().numpy()
     assert grad[-1] == 0.0
-    assert np.abs(grad[-129:-1]).max() > 0                         # the output weights do get a gradient
+    assert np.abs(grad[-c["d_hidden"][-1] - 1:-1]).max() > 0      # the output weights do get a gradient
 
 
 def test_losses_and_forward_match_oracle():

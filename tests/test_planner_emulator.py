@@ -43,7 +43,7 @@ def run(lib, mode, D, Cd, L, hidden, act, flat, X, Cn, N, l0=0, l1=None, scale=1
     lp = np.full(N, np.nan, np.float32)
     gflat = np.zeros(flat.size, np.float32)
     loss = C.c_double(0)
-    info = (C.c_int * 5)()
+    info = (C.c_int * 6)()
     rc = lib.rnvp_emulate(mode, D, Cd, L, len(hidden), hid, 1 if act == "tanh" else 2, TR,
                           fptr(flat), fptr(X), fptr(Cn), fptr(idx), C.c_longlong(N), l0, l1, C.c_float(scale),
                           fptr(out_x), fptr(ld), fptr(lp), fptr(gflat), C.byref(loss), info)
@@ -175,3 +175,54 @@ def test_only_tanh_flows_prescale_the_forward_w1_image(emul, D, Cd, L, H):
         w1, w1_scaled, other, other_scaled = list(out)
         assert w1 > 0 and other > 0 and other_scaled == 0
         assert w1_scaled == (w1 if scaled else 0), (act, list(out))
+
+
+# Flows that only the generic tile programs run, at the plans the planner picks for them: (forward / sample TR, fit-step
+# TR, does the fit step split a layer's weight rows over several weight-ring slots).  These plans are what the kernels
+# of tests/test_gpu_fp32_shapes.py run; the assertions keep a planner change from silently moving that coverage.
+FAMILY0_PLANS = [
+    ((16, 4, 3, (256, 256)), "tanh", 4, 4, True),
+    ((200, 10, 2, (64,)), "relu", 8, 4, True),             # D > 128
+    ((130, 5, 2, (100, 37, 300)), "tanh", 4, 2, True),
+    ((64, 0, 2, (1, 513)), "relu", 2, 2, True),            # Cd = 0, widths 1 and 513
+    ((5, 3, 3, (128,) * 8), "tanh", 8, 2, True),           # the 8-hidden-layer maximum
+    ((12, 40, 2, (48,)), "relu", 8, 8, False),             # Cd above the tcgen05 limit, one hidden layer
+    ((9, 2, 3, (32, 24)), "tanh", 8, 8, False),
+]
+
+
+@pytest.mark.parametrize("shape,act,tr_fwd,tr_fit,fit_chunked", FAMILY0_PLANS)
+def test_programs_deep_and_wide_flows(emul, shape, act, tr_fwd, tr_fit, fit_chunked):
+    D, Cd, L, hidden = shape
+    nh, N = len(hidden), 300
+    p = O.init_params(D, Cd, L, hidden, seed=D + L)
+    flat = flat_of(p, L, nh)
+    gen = torch.Generator().manual_seed(D)
+    X, Cn, eps = (torch.randn(N, w, generator=gen) for w in (D, Cd, D))
+    Ct = Cn if Cd else None
+    Ca = Cn.numpy() if Cd else None
+    z, ld, lp, _, _, info = run(emul, 0, D, Cd, L, hidden, act, flat, X.numpy(), Ca, N)
+    assert info[0] == tr_fwd, info
+    zr, ldr, lpr = O.flow_forward_rows(X, Ct, p, L, nh, act)
+    assert rel_err(z, zr) < TOL and rel_err(ld, ldr) < TOL and rel_err(lp, lpr) < TOL
+    x, *_, info1 = run(emul, 1, D, Cd, L, hidden, act, flat, eps.numpy(), Ca, N)
+    assert info1[0] == tr_fwd, info1
+    assert rel_err(x, O.flow_sample_from_noise(eps, Ct, p, L, nh, act)) < TOL
+    _, _, lp2, gflat, loss_sum, info2 = run(emul, 2, D, Cd, L, hidden, act, flat, X.numpy(), Ca, N, scale=-1.0 / N)
+    assert info2[0] == tr_fit and (info2[5] > 0) == fit_chunked, info2
+    loss_ref, grads_ref = O.loss_and_grads(X, Ct, p, L, nh, act)
+    assert rel_err(lp2, lpr) < TOL
+    assert abs(-loss_sum / N - float(loss_ref)) < TOL * abs(float(loss_ref))
+    gref = torch.cat([grads_ref[k].reshape(-1) for k in O.param_order(L, nh)]).numpy()
+    assert rel_err(gflat, gref) < 2e-5
+
+
+@pytest.mark.parametrize("shape,modes", [((33, 40, 2, (512, 512, 512)), (2,)), ((255, 64, 1, (1024,)), (0, 1, 2))])
+def test_unplannable_flows_are_refused(emul, shape, modes):
+    """No tile size fits shared memory: the planner refuses (RNVP_ESHAPE, -2) instead of emitting a program."""
+    D, Cd, L, hidden = shape
+    flat = flat_of(O.init_params(D, Cd, L, hidden, seed=0), L, len(hidden))
+    X, Cn = np.zeros((4, D), np.float32), np.zeros((4, Cd), np.float32)
+    for mode in modes:
+        with pytest.raises(AssertionError, match=r"^-2\b"):
+            run(emul, mode, D, Cd, L, hidden, "tanh", flat, X, Cn, 4, scale=-0.25)
