@@ -284,6 +284,16 @@ int rnvp_cn_inverse(const rnvp_cn_desc* d, const float* d_params, float* d_M, in
 int rnvp_cn_forward(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,
                     int64_t N, uint64_t seed, int64_t row_offset, const float* d_eps, float* d_mu, float* d_sigma,
                     float* d_xtilde, float* d_inv, void* stream);
+/* Exact log-density of the model's draws: d_logp[r] = log p(X[r] | C[r]) in fp64 (ConditionalNormal.log_prob_rows).
+ * mu and log_sigma come from the fp32 net of rnvp_cn_forward (the same bits); then u = (x - out.bias) (W_out^T)^-1 in
+ * full-covariance mode (u = x in independent mode) and
+ *   log p = -1/2 sum_d ((u_d - mu_d) / sigma_d)^2 - sum_d log_sigma_d - (D/2) log 2 pi - log|det W_out|,
+ * summed in fp64, log sigma taken from the head directly.  Full mode first factors W_out^T in fp64 with the partial
+ * pivoting of rnvp_cn_inverse: log|det W_out| = sum of log|pivot|, and the fp64 inverse, into d_workspace (1 + D * D
+ * doubles); an exact-zero pivot sets *d_status = 1 (the caller zeroes it) and leaves d_logp untouched.  Independent
+ * mode needs neither d_workspace nor d_status. */
+int rnvp_cn_log_prob(const rnvp_cn_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
+                     double* d_logp, double* d_workspace, int* d_status, void* stream);
 /* loss (cnormal.py:140-151) and its gradient on the N rows X[idx[r]], C[idx[r]] (d_idx may be NULL): d_gflat [P] in
  * the flat layout (zeros for out.* in independent mode, where the loss does not depend on them), *d_loss */
 int rnvp_cn_grad(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,
@@ -433,6 +443,25 @@ int64_t rnvp_draw_joint_workspace_bytes(int64_t k, int64_t rows, int D);
 int rnvp_draw_joint(const float* d_draws, int64_t k, int64_t rows, int D, const float* d_y, double p, double* d_mean,
                     double* d_cov, double* d_energy, double* d_variogram, void* d_workspace, int64_t workspace_bytes,
                     void* stream);
+
+/* Predictive log scores of k draws per row (rnvp_density.cu; probaforms_b200/predictive.py predictive_density).  The
+ * draws are laid out as for rnvp_draw_joint, 1 <= D <= RNVP_JOINT_MAX_D and D < k <= RNVP_SUMMARY_MAX_DRAWS; d_y
+ * [rows, D] is required.  Per row r, with the draws x_j promoted to fp64, S their covariance (ddof = 1, a centred
+ * two-pass sum) and S = L L^T:
+ *   d_log_score [rows] = -(logsumexp_j(-1/2 ||(f L)^-1 (y - x_j)||^2) - log k - sum_i log(f L_ii) - (D/2) log 2 pi),
+ *     the negative log of the Gaussian KDE with bandwidth matrix f^2 S (scipy's gaussian_kde with factor f), with a
+ *     max-shifted logsumexp;
+ *   d_dss [rows] = 2 sum_i log L_ii + ||L^-1 (y - mean)||^2, the Dawid-Sebastiani score;
+ *   d_marginal [rows, D] (NULL: skipped) = the 1-D KDE log score of each feature, bandwidth factor1 * sigma_d with
+ *     sigma_d^2 = S_dd.
+ * Rules: a row with a non-finite draw or a non-finite y gives NaN log score, DSS and marginals.  A Cholesky pivot
+ * L_ii^2 <= 1e-12 S_ii (this covers a zero-variance feature) makes S degenerate: NaN log score and DSS, while the
+ * marginals stay defined.  A constant feature (S_dd = 0) gives a NaN marginal.  These differ from scipy, which raises
+ * only when LAPACK's factorisation fails.  No workspace.  Results are bitwise repeatable and do not depend on how rows
+ * are split into calls.  RNVP_EINVAL for D outside [1, RNVP_JOINT_MAX_D], k outside (D, RNVP_SUMMARY_MAX_DRAWS], a
+ * factor (or, with d_marginal, factor1) that is not finite and > 0, and the other bad arguments. */
+int rnvp_draw_density(const float* d_draws, int64_t k, int64_t rows, int D, const float* d_y, double factor,
+                      double factor1, double* d_log_score, double* d_dss, double* d_marginal, void* stream);
 
 const char* rnvp_last_error(void);
 int rnvp_version(void);

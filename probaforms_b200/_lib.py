@@ -86,6 +86,8 @@ SIGNATURES = {
     "rnvp_cn_inverse": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, C.c_void_p, c_stream]),
     "rnvp_cn_forward": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, C.c_int64, C.c_uint64, C.c_int64,
                                   c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_stream]),
+    "rnvp_cn_log_prob": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, c_stream]),
     "rnvp_cn_grad": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64, c_f32_p, c_f32_p,
                                C.c_void_p, C.c_int64, c_stream]),
     "rnvp_cn_fit_epoch": (C.c_int, [c_desc_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_f32_p, c_i64_p, C.c_int64,
@@ -127,6 +129,8 @@ SIGNATURES = {
     "rnvp_draw_joint_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int]),
     "rnvp_draw_joint": (C.c_int, [c_f32_p, C.c_int64, C.c_int64, C.c_int, c_f32_p, C.c_double, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_draw_density": (C.c_int, [c_f32_p, C.c_int64, C.c_int64, C.c_int, c_f32_p, C.c_double, C.c_double,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

@@ -376,6 +376,127 @@ __global__ void __launch_bounds__(CN_THREADS) cn_forward_kernel(CnShape s, const
   }
 }
 
+// log|det W_out| and M64 = (W_out^T)^-1 in fp64 for the exact log-density: LU of A = W_out^T in shared memory with the
+// partial pivoting of invert_out (largest |a| in the column, the lowest row on a tie), then column c of A^-1 by thread
+// c, forward and back substitution through ws.  ws[0] = sum_c log|u_cc| in column order, ws[1 + j * D + c] =
+// M64[j][c]; *status = 1 on an exact-zero pivot.
+__global__ void cn_logdet_kernel(CnShape s, const float* __restrict__ params, double* ws, int* status) {
+  extern __shared__ __align__(16) double smd[];
+  __shared__ int piv, perm[CN_MAX_D];
+  __shared__ double pval;
+  const int D = s.D;
+  double* A = smd;
+  for (int e = threadIdx.x; e < D * D; e += blockDim.x) {
+    const int r = e / D, c = e - r * D;
+    A[e] = (double)params[s.out_w + c * D + r];        // W^T
+  }
+  for (int r = threadIdx.x; r < D; r += blockDim.x) perm[r] = r;
+  __syncthreads();
+  for (int c = 0; c < D; ++c) {
+    if (threadIdx.x < 32) {
+      int best = c;
+      double bv = -1.0;
+      for (int r = c + threadIdx.x; r < D; r += 32) {
+        const double a = fabs(A[r * D + c]);
+        if (a > bv) { bv = a; best = r; }
+      }
+      for (int o = 16; o > 0; o >>= 1) {
+        const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int ob = __shfl_xor_sync(0xffffffffu, best, o);
+        if (ov > bv || (ov == bv && ob < best)) { bv = ov; best = ob; }
+      }
+      if (threadIdx.x == 0) { piv = best; pval = A[best * D + c]; }
+    }
+    __syncthreads();
+    if (pval == 0.0) {                                 // uniform: every thread reads the same shared value
+      if (threadIdx.x == 0) *status = 1;
+      return;
+    }
+    const int p = piv;
+    if (p != c) {
+      for (int e = threadIdx.x; e < D; e += blockDim.x) {
+        const double a = A[p * D + e];
+        A[p * D + e] = A[c * D + e];
+        A[c * D + e] = a;
+      }
+      if (threadIdx.x == 0) { const int q = perm[p]; perm[p] = perm[c]; perm[c] = q; }
+    }
+    __syncthreads();
+    for (int r = c + 1 + threadIdx.x; r < D; r += blockDim.x) A[r * D + c] = __ddiv_rn(A[r * D + c], pval);
+    __syncthreads();
+    const int m = D - c - 1;
+    for (int e = threadIdx.x; e < m * m; e += blockDim.x) {
+      const int r = c + 1 + e / m, col = c + 1 + e % m;
+      A[r * D + col] = __fma_rn(-A[r * D + c], A[c * D + col], A[r * D + col]);
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    double ld = 0.0;
+    for (int c = 0; c < D; ++c) ld = __dadd_rn(ld, log(fabs(A[c * D + c])));
+    ws[0] = ld;
+  }
+  const int c = threadIdx.x;
+  if (c < D) {                                         // P A = L U: L U x = P e_c, x = column c of A^-1
+    double* x = ws + 1 + c;
+    for (int i = 0; i < D; ++i) {
+      double v = perm[i] == c ? 1.0 : 0.0;
+      for (int l = 0; l < i; ++l) v = __fma_rn(-A[i * D + l], x[l * D], v);
+      x[i * D] = v;
+    }
+    for (int i = D - 1; i >= 0; --i) {
+      double v = x[i * D];
+      for (int l = i + 1; l < D; ++l) v = __fma_rn(-A[i * D + l], x[l * D], v);
+      x[i * D] = __ddiv_rn(v, A[i * D + i]);
+    }
+  }
+}
+
+// exact log-density of X given C: the fp32 net of cn_forward_kernel (mu and log_sigma with the same bits), then one
+// warp per row in fp64: u = (x - b_out) M64 (u = x in independent mode), sum_d ((u_d - mu_d) / sigma_d)^2 and sum_d
+// log_sigma_d lane-strided and summed by a fixed shuffle tree
+__global__ void __launch_bounds__(CN_THREADS) cn_log_prob_kernel(CnShape s, const float* __restrict__ params,
+    const double* __restrict__ ws, const float* __restrict__ X, const float* __restrict__ C, int64_t N,
+    double* __restrict__ logp, const int* status) {
+  if (status && *status) return;
+  extern __shared__ __align__(16) float smem[];
+  const CnTile t = carve(s, smem);
+  const int64_t row0 = (int64_t)blockIdx.x * s.R;
+  const int nr = (int)(N - row0 < s.R ? N - row0 : s.R);
+  CnShape sx = s;
+  sx.indep = 1;                                        // raw X goes to Z in both modes
+  load_tile(sx, t, params, X, C, nullptr, row0, nr);
+  forward_tile(s, t, params, nullptr, false, nr);
+  const int D = s.D, lane = threadIdx.x & 31;
+  const double* M = ws + 1;
+  for (int r = threadIdx.x >> 5; r < nr; r += CN_THREADS / 32) {
+    const float* x = t.z + r * t.ldd;
+    double q = 0.0, ls = 0.0;
+    for (int c = lane; c < D; c += 32) {
+      double u = x[c];
+      if (!s.indep) {
+        u = 0.0;
+        for (int j = 0; j < D; ++j)
+          u = __fma_rn(__dsub_rn((double)x[j], (double)params[s.out_b + j]), M[j * D + c], u);
+      }
+      const double l = t.ls[r * t.ldd + c];
+      const double z = __dmul_rn(__dsub_rn(u, (double)t.mu[r * t.ldd + c]), exp(-l));
+      q = __fma_rn(z, z, q);
+      ls = __dadd_rn(ls, l);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      q = __dadd_rn(q, __shfl_down_sync(0xffffffffu, q, o));
+      ls = __dadd_rn(ls, __shfl_down_sync(0xffffffffu, ls, o));
+    }
+    if (lane == 0) {
+      double lp = -0.5 * q - ls - 0.5 * D * 1.8378770664093454836;   // log 2 pi
+      if (!s.indep) lp -= ws[0];
+      logp[row0 + r] = lp;
+    }
+  }
+}
+
 int64_t n_tiles(const CnShape& s, int64_t n) { return (n + s.R - 1) / s.R; }
 
 }  // namespace
@@ -457,7 +578,8 @@ int rnvp_cn_desc_create(int D, int Cd, int n_hidden, const int* hidden, int act,
   // maximum less its static shared memory (idempotent), never to this shape's need, which would lower it under a
   // larger model created earlier.
   const void* kernels[] = {(const void*)cn_sweep_kernel, (const void*)cn_tail_kernel, (const void*)cn_step_kernel,
-                           (const void*)cn_inverse_kernel, (const void*)cn_forward_kernel};
+                           (const void*)cn_inverse_kernel, (const void*)cn_forward_kernel,
+                           (const void*)cn_log_prob_kernel};
   for (const void* k : kernels) {
     cudaFuncAttributes fa;
     e = cudaFuncGetAttributes(&fa, k);
@@ -506,6 +628,31 @@ int rnvp_cn_forward(const rnvp_cn_desc* d, const float* d_params, const float* d
       d->s, d_params, d_M, d_X, d_C, N, seed, row_offset, d_eps, d_mu, d_sigma, d_xtilde, d_inv);
   const cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cn_forward_kernel launch");
+}
+
+int rnvp_cn_log_prob(const rnvp_cn_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
+                     double* d_logp, double* d_workspace, int* d_status, void* stream) {
+  if (check_cn(d)) return RNVP_EINVAL;
+  const bool full = !d->s.indep;
+  if (!d_params || !d_X || !d_C || !d_logp || N < 0 || (full && (!d_workspace || !d_status)))
+    return rnvp_fail(RNVP_EINVAL, "rnvp_cn_log_prob: bad argument");
+  const int64_t nt = n_tiles(d->s, N);
+  if (nt > 0x7fffffffLL) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_log_prob: too many rows");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e;
+  if (full) {
+    const int smem = d->s.D * d->s.D * (int)sizeof(double);
+    e = cudaFuncSetAttribute(cn_logdet_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return rnvp_fail((int)e, "rnvp_cn_log_prob: cudaFuncSetAttribute");
+    cn_logdet_kernel<<<1, CN_TAIL_THREADS, smem, st>>>(d->s, d_params, d_workspace, d_status);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return rnvp_fail((int)e, "cn_logdet_kernel launch");
+  }
+  if (N == 0) return 0;
+  cn_log_prob_kernel<<<(unsigned)nt, CN_THREADS, d->s.sweep_smem, st>>>(
+      d->s, d_params, full ? d_workspace : nullptr, d_X, d_C, N, d_logp, full ? d_status : nullptr);
+  e = cudaGetLastError();
+  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cn_log_prob_kernel launch");
 }
 
 int rnvp_cn_grad(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,

@@ -170,6 +170,34 @@ class Net(nn.Module):
                    "rnvp_cn_forward")
         return xt, inv, mu, sigma
 
+    @torch.no_grad()
+    def log_prob(self, X, C):
+        """Exact log p(X | C) per row as a float64 device tensor [n] (rnvp_cn_log_prob): the fp32 net's mu and
+        log_sigma, then the Gaussian density of u = (x - out.bias) (out.weight^T)^-1 (u = x with independent
+        covariance) in fp64, less log|det out.weight|.  Raises torch.linalg.LinAlgError if a pivot of out.weight is
+        exactly zero."""
+        desc, flat = self._ready()
+        dev = flat.device
+        Cd = torch.as_tensor(C, dtype=torch.float32).to(dev).contiguous()
+        if Cd.dim() != 2 or Cd.shape[1] != self.cond_size:
+            raise ValueError(f"C must be [n, {self.cond_size}], got shape {tuple(Cd.shape)}")
+        n, D = Cd.shape[0], self.var_size
+        Xd = torch.as_tensor(X, dtype=torch.float32).to(dev).contiguous()
+        if tuple(Xd.shape) != (n, D):
+            raise ValueError(f"X must be [{n}, {D}], got shape {tuple(Xd.shape)}")
+        logp = torch.empty(n, dtype=torch.float64, device=dev)
+        ws = status = None
+        if not desc.independent:
+            ws = torch.empty(1 + D * D, dtype=torch.float64, device=dev)
+            status = torch.zeros(1, dtype=torch.int32, device=dev)
+        ptr = lambda t: None if t is None else ct.c_void_p(t.data_ptr())   # noqa: E731
+        _lib.check(desc.lib.rnvp_cn_log_prob(desc.h, flat.data_ptr(), Xd.data_ptr(), Cd.data_ptr(), n,
+                                             ptr(logp), ptr(ws), ptr(status), _stream(dev)), "rnvp_cn_log_prob")
+        if status is not None and int(status.item()) != 0:
+            raise torch.linalg.LinAlgError("linalg.inv: The diagonal element 1 is zero, the inversion could not be "
+                                           "completed because the input matrix is singular.")
+        return logp
+
 
 class _RngReplay:
     """The reference's use of the global torch generator during ``fit``, replayed on a helper thread.
@@ -441,6 +469,16 @@ class ConditionalNormal(GenModel):
             Cs = torch.zeros(C, 1)
         x_tilde, _, _, _ = self.model(None, Cs, eps=eps, seed=seed)
         return x_tilde.cpu().numpy()
+
+    def log_prob_rows(self, X, C=None):
+        """Exact per-row log-density log p(X | C) of the fitted Gaussian as a float32 numpy array [n], like
+        ``RealNVP.log_prob_rows``.  ``C=None`` means zero conditions, as in ``fit``.  Summed in fp64 on the fp32 net's
+        mu and sigma (rnvp_cn_log_prob); raises torch.linalg.LinAlgError if ``out.weight`` is singular."""
+        if getattr(self, "model", None) is None or not isinstance(self.model, Net):
+            raise RuntimeError("ConditionalNormal.log_prob_rows: call fit() first")
+        if C is None:
+            C = torch.zeros(len(X), 1)
+        return self.model.log_prob(X, C).float().cpu().numpy()
 
     def _draw_hook(self):
         """(device, var_size, draw) for on-device summaries: ``draw(Cd, seed, r0, m, out)`` writes rows [r0, r0 + m) of

@@ -38,6 +38,25 @@ At D = 1 the energy score is the CRPS above.  A row with a non-finite draw gives
 follows np.mean); a NaN in y gives NaN energy and variogram.  The pair sums run on draws centred at the row mean in
 fp32, so values whose squared centred differences overflow float32 (|x - mean| above about 1e19) are out of range.  At
 most 128 features and 8192 draws; one GPU.
+
+``predictive_density`` / ``summarize_density_draws`` make the same draws and score the observation by the density the
+draws imply (``rnvp_draw_density``, rnvp_density.cu)::
+
+    d = predictive_density(model, C, y, n_draws=1000, bw_method='scott', marginal=False, seed=None)
+    d.log_score          # float64 [n]: -gaussian_kde(draws[:, i].T, bw_method).logpdf(y[i])
+    d.dss                # float64 [n]: log det S + (y - mean)^T S^-1 (y - mean), S the draws' covariance (ddof = 1)
+    d.marginal           # float64 [n, D] with marginal=True: -gaussian_kde(draws[:, i, d]).logpdf(y[i, d]), else None
+    d.factor             # the bandwidth factor of the joint KDE
+
+    d = summarize_density_draws(draws, y, bw_method='scott', marginal=False)
+
+The Gaussian KDE of the draws is the density estimate for every model, CVAE and ConditionalWGAN included, which have no
+tractable density.  ``RealNVP.log_prob_rows`` and ``ConditionalNormal.log_prob_rows`` are the exact log densities of
+those two models.  ``bw_method`` is scipy's: 'scott' k^(-1/(D+4)), 'silverman' (k (D+2)/4)^(-1/(D+4)), or a positive
+float used as the factor; the marginals use the factor at D = 1 (or the same float).  A row with a non-finite draw or
+y gives NaN scores; a degenerate covariance (a Cholesky pivot L_ii^2 <= 1e-12 S_ii) gives NaN log_score and dss, and a
+constant feature a NaN marginal, where scipy raises only when LAPACK fails.  D < k <= 8192, at most 128 features; one
+GPU.
 """
 import ctypes as ct
 from dataclasses import dataclass
@@ -138,10 +157,10 @@ def _check_model(name, model):
 
 
 def _draw_blocks(model, C, k, y, seed, outputs):
-    """The draw loop of ``predictive_summary`` and ``predictive_joint``.  Draws k samples of ``model.sample(C)`` per row
-    on the device, row block by row block, and hands each block to ``out = outputs(n, D, dev, y)``:
-    ``out.block(lib, xs [k, m, D], r0, m, y_block)``, then returns ``out.to_host()``.  ``out.row_bytes`` of per-row
-    device scratch count against the block budget.  ``outputs`` raises its argument errors before allocating."""
+    """The draw loop of ``predictive_summary``, ``predictive_joint`` and ``predictive_density``.  Draws k samples of
+    ``model.sample(C)`` per row on the device, row block by row block, and hands each block to ``out = outputs(n, D,
+    dev, y)``: ``out.block(lib, xs [k, m, D], r0, m, y_block)``, then returns ``out.to_host()``.  ``out.row_bytes`` of
+    per-row device scratch count against the block budget.  ``outputs`` raises its argument errors before allocating."""
     dev, D, draw = model._draw_hook()             # raises what model.sample raises on an unfitted model
     is_int = type(C) == type(1)
     n = C if is_int else len(C)
@@ -319,4 +338,117 @@ def summarize_joint_draws(draws, y=None, p=0.5, cov=False):
         for r0, m in _plan_blocks(n, k, D, _BLOCK_BYTES, out.row_bytes):
             xb = xs if m == n else xs[:, r0:r0 + m].contiguous()
             out.block(lib, xb, r0, m, None if yd is None else yd[r0:r0 + m])
+        return out.to_host()
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Log scores: Gaussian-KDE log score, Dawid-Sebastiani score and per-feature KDE log scores (rnvp_draw_density)
+
+
+@dataclass
+class PredictiveDensity:
+    """Log scores of k draws for n rows of D features."""
+    log_score: np.ndarray                    # float64 [n]: -log of the Gaussian KDE of the draws at y
+    dss: np.ndarray                          # float64 [n]: Dawid-Sebastiani score
+    marginal: Optional[np.ndarray]           # float64 [n, D] with marginal=True: per-feature 1-D KDE log scores
+    factor: float                            # bandwidth factor of the joint KDE
+
+
+def _check_bw(bw_method):
+    if isinstance(bw_method, str):
+        if bw_method not in ("scott", "silverman"):
+            raise ValueError(f"bw_method must be 'scott', 'silverman' or a float > 0, got {bw_method!r}")
+        return bw_method
+    if isinstance(bw_method, bool) or not isinstance(bw_method, (int, float, np.integer, np.floating)) \
+            or not (np.isfinite(bw_method) and bw_method > 0):
+        raise ValueError(f"bw_method must be 'scott', 'silverman' or a finite float > 0, got {bw_method!r}")
+    return float(bw_method)
+
+
+def bandwidth_factor(bw_method, k, D):
+    """scipy.stats.gaussian_kde's factor for k draws of D features: 'scott' k^(-1/(D+4)), 'silverman'
+    (k (D+2)/4)^(-1/(D+4)), a float as given."""
+    if bw_method == "scott":
+        return float(np.power(float(k), -1.0 / (D + 4)))
+    if bw_method == "silverman":
+        return float(np.power(k * (D + 2.0) / 4.0, -1.0 / (D + 4)))
+    return float(bw_method)
+
+
+class _DensityOutputs:
+    """Device outputs of one density request: log score [n], DSS [n] and the marginals [n, D] in one float64 buffer,
+    one copy back at the end.  The kernel needs no scratch."""
+    row_bytes = 0
+
+    def __init__(self, n, D, k, bw_method, marginal, dev):
+        _check_density_shape(k, D)
+        self.n, self.D, self.k, self.marginal, self.dev = n, D, k, marginal, dev
+        self.factor = bandwidth_factor(bw_method, k, D)
+        self.factor1 = bandwidth_factor(bw_method, k, 1)
+        self.f64 = torch.empty(max(n * (2 + (D if marginal else 0)), 1), dtype=torch.float64, device=dev)
+
+    def block(self, lib, draws, r0, m, y):
+        """rnvp_draw_density of rows [r0, r0 + m), whose draws are ``draws`` [k, m, D] (device, float32)."""
+        n, D, base = self.n, self.D, self.f64.data_ptr()
+        _lib.check(lib.rnvp_draw_density(
+            ct.c_void_p(draws.data_ptr()), self.k, m, D, ct.c_void_p(y.data_ptr()), self.factor, self.factor1,
+            ct.c_void_p(base + 8 * r0), ct.c_void_p(base + 8 * (n + r0)),
+            ct.c_void_p(base + 8 * (2 * n + r0 * D)) if self.marginal else None,
+            ct.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)), "rnvp_draw_density")
+
+    def to_host(self):
+        n, D = self.n, self.D
+        f = self.f64.cpu().numpy()
+        return PredictiveDensity(log_score=f[:n].copy(), dss=f[n:2 * n].copy(),
+                                 marginal=f[2 * n:2 * n + n * D].reshape(n, D) if self.marginal else None,
+                                 factor=self.factor)
+
+
+def _check_density_shape(k, D):
+    _check_features(D)
+    if k <= D:
+        raise ValueError(f"the KDE needs more draws than features: n_draws = {k} <= D = {D}")
+
+
+def _check_density_y(y):
+    if y is None:
+        raise ValueError("y [n, D] is required: the log scores are evaluated at the observations")
+
+
+def predictive_density(model, C, y, n_draws=1000, bw_method="scott", marginal=False, seed=None):
+    """Log scores of the observations ``y`` [n, D] under ``n_draws`` draws of ``model.sample(C)`` per row, on the GPU.
+
+    Same models, ``C`` forms and draws as ``predictive_summary`` (``seed`` as there).  Per row: the negative log of the
+    Gaussian KDE of the draws at y (scipy's ``gaussian_kde(draws.T, bw_method).logpdf(y)`` negated), the
+    Dawid-Sebastiani score log det S + (y - mean)^T S^-1 (y - mean) with S the draws' covariance (ddof = 1), and with
+    ``marginal=True`` each feature's 1-D KDE log score.  ``bw_method``: 'scott', 'silverman' or a float > 0.  Needs
+    D < n_draws <= 8192 and D <= 128.  Returns a ``PredictiveDensity``."""
+    _check_model("predictive_density", model)
+    k = _check_draws(n_draws)
+    bw = _check_bw(bw_method)
+    _check_density_y(y)
+    marginal = bool(marginal)
+    return _draw_blocks(model, C, k, y, seed, lambda n, D, dev, y: _DensityOutputs(n, D, k, bw, marginal, dev))
+
+
+def summarize_density_draws(draws, y, bw_method="scott", marginal=False):
+    """The log scores of ``predictive_density`` for given draws [k, n, D]: a CUDA tensor (its device is used) or a
+    numpy array / CPU tensor (scored on the current CUDA device).  The draws are taken as float32."""
+    if len(tuple(draws.shape)) != 3:
+        raise ValueError(f"draws must be 3-D [k, n, D], got shape {tuple(draws.shape)}")
+    k, n, D = (int(v) for v in draws.shape)
+    k = _check_draws(k)
+    bw = _check_bw(bw_method)
+    _check_density_y(y)
+    y = _check_y(y, n, D)
+    _check_density_shape(k, D)
+    dev = _device_of(draws)
+    out = _DensityOutputs(n, D, k, bw, bool(marginal), dev)
+    lib = _lib.load()
+    with torch.cuda.device(dev):
+        xs = upload_resident(lib, draws.reshape(k, n * D), dev).view(k, n, D)
+        yd = upload_resident(lib, y, dev)
+        for r0, m in _plan_blocks(n, k, D, _BLOCK_BYTES, out.row_bytes):
+            xb = xs if m == n else xs[:, r0:r0 + m].contiguous()
+            out.block(lib, xb, r0, m, yd[r0:r0 + m])
         return out.to_host()
