@@ -274,6 +274,24 @@ extern "C" int rnvp_emul_img_scaled(int D, int Cd, int L, int H, int act, long l
   return 0;
 }
 
+// Row-per-thread small-flow layout of a one-hidden-layer flow as rnvp_desc_create builds it.  head[8]: small_ok, sNE, sNC,
+// srec, snet, small_floats, small_off, P.  When small_ok and the buffers are given, s2f[small_floats] receives the flat
+// index held by each slot of the small region (or -1) and f2p2[P] the absolute packed index of each parameter's small-layout
+// copy (or -1).  Call once with null buffers to learn the sizes.
+extern "C" int rnvp_emul_small_layout(int D, int Cd, int L, int H, long long* head, int* s2f, int* f2p2) {
+  FlowGeom g;
+  g.D = D; g.Cd = Cd; g.L = L; g.nh = 1; g.act = 1; g.hidden[0] = H;
+  build_layout(&g);
+  const long long h[8] = {g.small_ok, g.sNE, g.sNC, g.srec, g.snet, g.small_floats, g.small_off, g.P};
+  for (int k = 0; k < 8; ++k) head[k] = h[k];
+  if (!g.small_ok || !s2f || !f2p2) return 0;
+  std::vector<int> p2f(g.packed_gather, -1), f2p2v;
+  build_small_map(&g, p2f, f2p2v);
+  for (int k = 0; k < g.small_floats; ++k) s2f[k] = p2f[g.small_off + k];
+  for (int64_t f = 0; f < g.P; ++f) f2p2[f] = f2p2v[f];
+  return 0;
+}
+
 extern "C" long long rnvp_emul_param_count(int D, int Cd, int L, int nh, const int* hidden) {
   FlowGeom g;
   g.D = D; g.Cd = Cd; g.L = L; g.nh = nh; g.act = 1;

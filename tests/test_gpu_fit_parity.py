@@ -139,14 +139,15 @@ def _fit_check(shape, n, bs, epochs, seed, activation="tanh", **kw):
     D, Cd, L, hidden = shape
     g = torch.Generator().manual_seed(seed + 7)
     X = torch.randn(n, D, generator=g).double().numpy()          # the reference's input contract: numpy float64
-    Cn = torch.randn(n, Cd, generator=g).double().numpy()
+    Cn = torch.randn(n, Cd, generator=g).double().numpy() if Cd else None     # an unconditional flow is fitted with C=None
     torch.manual_seed(seed)
     model = RealNVP(n_layers=L, hidden=hidden, activation=activation, batch_size=bs, n_epochs=epochs, lr=1e-3, **kw)
     model.fit(X, Cn)
     hist = np.array([float(l) for l in model.loss_history])
     torch.manual_seed(seed)
     params = O.init_params(D, Cd, L, hidden)
-    ref_hist, _ = O.fit(X, Cn, params, L, len(hidden), activation, bs, epochs, 1e-3)
+    ref_hist, _ = O.fit(X, Cn, params, L, len(hidden), activation, bs, epochs, 1e-3,
+                        weight_decay=kw.get("weight_decay", 0.0))
     ref_hist = np.array([float(l) for l in ref_hist])
     assert hist.shape == ref_hist.shape
     assert np.allclose(hist, ref_hist, rtol=2e-5, atol=2e-6), np.abs(hist - ref_hist).max()

@@ -11,5 +11,10 @@ for tool in racecheck synccheck memcheck; do
   done
   r=$(timeout 400 compute-sanitizer --tool $tool python tools/c1_steps.py 2>&1 | grep -E "SUMMARY|^ok" | tr '\n' ' ')
   echo "$tool c1_steps (small-flow fit, fused Adam step, sample): $r" >> $out
+  # small-flow fit at the 64 KB layout edge (opt-in shared memory), and over two grid waves (several row blocks per CTA)
+  for args in "8 4 2 255 relu 1000" "2 1 8 10 tanh grid2"; do
+    r=$(timeout 900 compute-sanitizer --tool $tool python tools/c1_steps.py $args 2>&1 | grep -E "SUMMARY|^ok" | tr '\n' ' ')
+    echo "$tool c1_steps $args: $r" >> $out
+  done
 done
 cat $out
