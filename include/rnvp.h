@@ -463,6 +463,35 @@ int rnvp_draw_joint(const float* d_draws, int64_t k, int64_t rows, int D, const 
 int rnvp_draw_density(const float* d_draws, int64_t k, int64_t rows, int D, const float* d_y, double factor,
                       double factor1, double* d_log_score, double* d_dss, double* d_marginal, void* stream);
 
+/* k-nearest-neighbour precision, recall, density and coverage (rnvp_knn.cu; probaforms_b200/metrics/knn.py
+ * precision_recall_density_coverage).  d_R [n][D] real rows, d_F [m][D] fake rows, fp64; 1 <= k <= RNVP_KNN_MAX_K,
+ * k < n, k < m, n, m < 2^31, D >= 1.  The rows must be finite (not checked here).
+ *   d2(a, b)   acc = 0; for c = 0 .. D-1: t = a_c - b_c; acc = acc + t * t  -- every operation rounded on its own (no FMA
+ *              contraction), so a float64 numpy loop over the columns gives the same bits, and d2(a, b) = d2(b, a);
+ *   d_r2[i]    the (k+1)-th smallest d2(R_i, R_j) over j = 0 .. n-1, self and duplicate rows included
+ *              (np.partition(D_RR, k, axis=1)[:, k]); d_s2[j] the same over F;
+ *   d_count[j] #{i : d2(R_i, F_j) < d_r2[i]}  (strict <), uint32 [m];
+ *   d_flags[i] bit 0: some j has d2(R_i, F_j) < d_s2[j] (recall); bit 1: some j has d2(R_i, F_j) < d_r2[i] (coverage);
+ *   d_tallies  uint64 [4] = { #{j : count_j > 0}, sum_j count_j, #{i : bit 0}, #{i : bit 1} }, so that precision =
+ *              t0 / m, density = t1 / (k m), recall = t2 / n, coverage = t3 / n.
+ * Every output is a selected d2 value or an integer: results are bitwise repeatable and independent of the launch
+ * geometry.  No n x n buffer: the workspace (rnvp_knn_workspace_bytes, 0 when the row blocks fill the GPU) holds the
+ * k+1 smallest values per row and candidate slice, at most 1 GiB.  RNVP_EINVAL for sizes outside the ranges above, null
+ * buffers, or a workspace smaller than rnvp_knn_workspace_bytes (which returns RNVP_EINVAL for bad sizes).
+ *   rnvp_knn_radii   one radius pass: d_radius2[i] for the n rows of d_A (workspace: rnvp_knn_workspace_bytes(n, n, D, k))
+ *   rnvp_knn_cross   the cross pass and the tallies, given d_r2 and d_s2 (no workspace)
+ *   rnvp_knn_prdc    both radius passes, then the cross pass: the whole computation */
+#define RNVP_KNN_MAX_K 32
+int64_t rnvp_knn_workspace_bytes(int64_t n, int64_t m, int D, int k);
+int rnvp_knn_radii(const double* d_A, int64_t n, int D, int k, double* d_radius2 /* [n] */, void* d_workspace,
+                   int64_t workspace_bytes, void* stream);
+int rnvp_knn_cross(const double* d_R, int64_t n, const double* d_F, int64_t m, int D, const double* d_r2,
+                   const double* d_s2, uint32_t* d_count /* [m] */, uint32_t* d_flags /* [n] */,
+                   uint64_t* d_tallies /* [4] */, void* stream);
+int rnvp_knn_prdc(const double* d_R, int64_t n, const double* d_F, int64_t m, int D, int k, double* d_r2 /* [n] */,
+                  double* d_s2 /* [m] */, uint32_t* d_count /* [m] */, uint32_t* d_flags /* [n] */,
+                  uint64_t* d_tallies /* [4] */, void* d_workspace, int64_t workspace_bytes, void* stream);
+
 const char* rnvp_last_error(void);
 int rnvp_version(void);
 

@@ -131,6 +131,12 @@ SIGNATURES = {
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_draw_density": (C.c_int, [c_f32_p, C.c_int64, C.c_int64, C.c_int, c_f32_p, C.c_double, C.c_double,
                                     C.c_void_p, C.c_void_p, C.c_void_p, c_stream]),
+    "rnvp_knn_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int, C.c_int]),
+    "rnvp_knn_radii": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "rnvp_knn_cross": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, c_stream]),
+    "rnvp_knn_prdc": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
     "rnvp_last_error": (C.c_char_p, []),
     "rnvp_version": (C.c_int, []),
 }

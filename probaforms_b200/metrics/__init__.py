@@ -397,3 +397,5 @@ def frechet_distance(X_real, X_fake, n_iters=100, standardize=False):
 # the per-feature metrics use the helpers above
 from .onedim import (anderson_darling_1d, cramer_von_mises_1d, jensen_shannon_1d, jensen_shannon_1d_kde,  # noqa: E402
                      kolmogorov_smirnov_1d, kullback_leibler_1d, kullback_leibler_1d_kde, roc_auc_score_1d)
+# additive, not a probaforms.metrics name, so not in __all__
+from .knn import precision_recall_density_coverage  # noqa: E402,F401
