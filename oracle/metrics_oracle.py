@@ -154,6 +154,143 @@ def frechet_distance(X_real, X_fake, n_iters=100, standardize_=False, fp32_rows=
     return frd.mean(), frd.std(), frd
 
 
+# ------------------------------------------------------------------------- bit-exact fp32 emulation of the kernels
+# The kernels of rnvp_metrics.cu build d^2 and the bootstrap moments from fp32 FMA chains (no fast-math), so their fp32
+# results can be reproduced bit for bit on the host.  These functions do that; the float64 functions above are the
+# reference-pinned statement of the mathematics and stay as they are.
+
+_F32_MID = np.uint64(1 << 28)            # float64 mantissa bits below an fp32 ulp: 29; their top bit alone is a midpoint
+_F32_LOW = np.uint64((1 << 29) - 1)
+
+
+def fma32(a, b, c):
+    """Correctly rounded fp32 fma(a, b, c) (round to nearest even) of float32 arrays, as CUDA's fmaf.
+
+    a*b of two fp32 values is exact in float64 and p + c is the float64 rounding of the exact sum, so rounding that to
+    fp32 is correct except where it lands exactly on an fp32 midpoint while the exact sum does not: there the sign of
+    the TwoSum remainder says which neighbour the exact value is nearer to."""
+    a, b, c = np.broadcast_arrays(*(np.asarray(v, dtype=np.float32) for v in (a, b, c)))
+    shape = a.shape
+    p = a.astype(np.float64).reshape(-1) * b.astype(np.float64).reshape(-1)
+    cc = c.astype(np.float64).reshape(-1)
+    s = p + cc
+    with np.errstate(over="ignore"):
+        r = s.astype(np.float32)
+    # candidates: s on an fp32 midpoint of the normal range, or below it (where the fp32 grid is coarser than that test)
+    cand = ((s.view(np.uint64) & _F32_LOW) == _F32_MID) | (np.abs(s) < 2.0 ** -125)
+    idx = np.flatnonzero(cand)
+    if len(idx):
+        ss, pp, cq, rr = s[idx], p[idx], cc[idx], r[idx]
+        bv = ss - pp
+        err = (pp - (ss - bv)) + (cq - bv)                    # TwoSum: p + c = ss + err exactly
+        other = np.nextafter(rr, np.where(ss > rr, np.float32(np.inf), np.float32(-np.inf)).astype(np.float32))
+        mid = 0.5 * (rr.astype(np.float64) + other.astype(np.float64))
+        fix = (ss == mid) & (err != 0) & ((err > 0) == (other > rr))
+        r[idx] = np.where(fix, other, rr)
+    return r.reshape(shape)
+
+
+def pair_d2_fp32(Z, chunk=256):
+    """pair_d2 with the kernel's fp32 arithmetic: for each pair i <= j of the rows Z (rounded to fp32),
+    d2 = 0; d2 = fmaf(d, d, d2) with d = z_i[k] - z_j[k] in fp32, over k = 0, 1, ... in order.  Returns float32 d^2."""
+    Z = np.asarray(Z, dtype=np.float32)
+    N, D = Z.shape
+    idt = np.uint16 if N <= 65535 else np.int32
+    vals, I, J = [], [], []
+    for i0 in range(0, N, chunk):
+        i1 = min(N, i0 + chunk)
+        ii, jj = np.nonzero(np.arange(i0, i1)[:, None] <= np.arange(i0, N)[None, :])
+        A, B = Z[i0 + ii], Z[i0 + jj]
+        d = A[:, 0] - B[:, 0]
+        d2 = d * d                                            # fmaf(d, d, +0) is the rounded square
+        for k in range(1, D):
+            d = A[:, k] - B[:, k]
+            d2 = fma32(d, d, d2)
+        vals.append(d2)
+        I.append((ii + i0).astype(idt))
+        J.append((jj + i0).astype(idt))
+    return np.concatenate(vals), np.concatenate(I), np.concatenate(J)
+
+
+def exact_medians(d2_32, I, J, counts):
+    """Per draw, the median of the kernel: (median float64, d^2 bits of rank k, d^2 bits of rank k+1) as arrays.
+
+    Ranks are 0-based over the W = (sum c)^2 ordered pairs of the drawn rows, pair (i, j) of i <= j weighing c_i c_j,
+    doubled off the diagonal; k = (W - 1) // 2.  When W is odd np.median takes rank k alone and the rank k+1 bits are
+    -1.  median = (sqrt(d2_k) + sqrt(d2_k+1)) / 2 in float64 on the fp32 values, as the select kernel computes it."""
+    u = np.asarray(d2_32, dtype=np.float32).view(np.uint32)
+    # the d^2 of a pair is >= 0, so its bit pattern orders it; (bits << 32 | index) sorts many times faster than argsort
+    key = np.sort((u.astype(np.uint64) << np.uint64(32)) | np.arange(len(u), dtype=np.uint64))
+    bits = (key >> np.uint64(32)).astype(np.int64)
+    order = (key & np.uint64(0xFFFFFFFF)).astype(np.int64)
+    del key
+    Is, Js = np.asarray(I)[order].astype(np.int32), np.asarray(J)[order].astype(np.int32)
+    off = Is != Js
+    counts = np.asarray(counts, dtype=np.int64)
+    meds = np.empty(len(counts))
+    lo_bits = np.empty(len(counts), dtype=np.int64)
+    hi_bits = np.empty(len(counts), dtype=np.int64)
+    for b, c in enumerate(counts):
+        cum = c[Is] * c[Js]
+        cum[off] *= 2
+        np.cumsum(cum, out=cum)
+        W = int(c.sum()) ** 2
+        lo = bits[np.searchsorted(cum, (W - 1) // 2, side="right")]
+        hi = bits[np.searchsorted(cum, W // 2, side="right")]
+        v = np.array([lo, hi], dtype=np.uint32).view(np.float32).astype(np.float64)
+        meds[b] = 0.5 * (np.sqrt(v[0]) + np.sqrt(v[1]))
+        lo_bits[b] = lo
+        hi_bits[b] = hi if W % 2 == 0 else -1
+    return meds, lo_bits, hi_bits
+
+
+# radix passes of the median selection: bits 30..20, 19..9, 8..0 of the fp32 d^2
+_PASS_SHIFTS = (20, 9, 0)
+
+
+def middle_rank_split(lo_bits, hi_bits):
+    """Where ranks k and k+1 of each draw part in a radix selection over bits 30..20, 19..9, 8..0: a list of
+    (split, gap), split one of 'pass0', 'pass1', 'pass2' (the first pass whose digits differ), 'never' (equal d^2) or
+    'odd' (W odd: rank k alone, hi bits -1); gap is True when buckets lie strictly between the two digits at that pass.
+    Ranks k and k+1 are adjacent in the sorted order, so every bucket between them holds no weight."""
+    out = []
+    for lo, hi in zip(np.asarray(lo_bits, dtype=np.int64), np.asarray(hi_bits, dtype=np.int64)):
+        if hi < 0:
+            out.append(("odd", False))
+            continue
+        lo, hi = int(lo), int(hi)
+        if lo == hi:
+            out.append(("never", False))
+            continue
+        for p, sh in enumerate(_PASS_SHIFTS):
+            if (lo >> sh) != (hi >> sh):
+                out.append((f"pass{p}", (hi >> sh) - (lo >> sh) > 1))
+                break
+    return out
+
+
+def boot_moments_fp32(Xc32, counts, chunk=128):
+    """Per-draw sum_i c_i x_i [n_draws, D] and sum_i c_i x_i x_i^T [n_draws, D, D] in float64, bit for bit as
+    rnvp_boot_moments: for every 128-row chunk an fp32 chain p = fmaf(c_r, x_rj * x_rk, p) (s = fmaf(c_r, x_rj, s)) over
+    its rows in order from +0, and the chunk results added to a float64 sum from 0 in chunk order."""
+    X = np.asarray(Xc32, dtype=np.float32)
+    counts = np.asarray(counts).astype(np.float32)           # counts <= 65535 are exact in fp32
+    n, D = X.shape
+    nd = len(counts)
+    s1 = np.zeros((nd, D))
+    s2 = np.zeros((nd, D, D))
+    for c0 in range(0, n, chunk):
+        p1 = np.zeros((nd, D), dtype=np.float32)
+        p2 = np.zeros((nd, D, D), dtype=np.float32)
+        for r in range(c0, min(n, c0 + chunk)):
+            c = counts[:, r]
+            p1 = fma32(c[:, None], X[r][None, :], p1)
+            p2 = fma32(c[:, None, None], (X[r][:, None] * X[r][None, :])[None], p2)
+        s1 += p1.astype(np.float64)
+        s2 += p2.astype(np.float64)
+    return s1, s2
+
+
 def fixture_inputs(g):
     """(X, Y) of a tests/golden/metrics_*.npz fixture: stored, or regenerated from their seed for the larger cases."""
     if "X" in g:
