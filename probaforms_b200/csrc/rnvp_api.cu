@@ -5,7 +5,6 @@
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
-#include <string.h>
 #include <algorithm>
 #include <map>
 #include <mutex>
@@ -68,14 +67,16 @@ struct rnvp_desc : rnvp_planner::FlowGeom {
   int* d_f2m = nullptr;   // [4*P]: positions of each parameter's TF32 hi / lo images (plain, transposed) in the tcgen05 region, or -1
   RnvpWgradLayer* d_wg = nullptr;   // per-layer gradient offsets for the weight-gradient sweep
   int path = 0;           // 0 auto, 1 FP32 tile/small kernels only, 2 tcgen05 where eligible
-  std::map<std::tuple<int, int, int>, Program> programs;
-  std::mutex mu;
+  // FP32 tile programs by (mode, layer range), built on first use: a cache, so entry points that take the descriptor
+  // const may fill it
+  mutable std::map<std::tuple<int, int, int>, Program> programs;
+  mutable std::mutex mu;
 };
 
 namespace {
 using namespace rnvp_planner;
 
-int get_program(rnvp_desc* d, int mode, int l0, int l1, Program** out) {
+int get_program(const rnvp_desc* d, int mode, int l0, int l1, Program** out) {
   std::lock_guard<std::mutex> lock(d->mu);
   auto key = std::make_tuple(mode, l0, l1);
   auto it = d->programs.find(key);
@@ -203,73 +204,100 @@ __global__ void adam_kernel(float* __restrict__ theta, float* __restrict__ packe
 
 int check_desc(const rnvp_desc* d) { return d ? 0 : fail(RNVP_EINVAL, "null descriptor"); }
 
-int run_tile(rnvp_desc* d, int mode, int l0, int l1, RnvpKArgs& a, void* workspace, int64_t workspace_bytes,
-             cudaStream_t stream) {
-  if (l0 < 0 || l1 > d->L || l0 >= l1) return fail(RNVP_EINVAL, "bad layer range");
-  if (a.N <= 0) return 0;
-  Program* p = nullptr;
-  int rc = get_program(d, mode, l0, l1, &p);
-  if (rc) return rc;
-  const int R = 8 * p->TR;
-  const long long n_tiles = (a.N + R - 1) / R;
-  if (n_tiles > 0x7fffffffLL) return fail(RNVP_EINVAL, "too many rows for one launch");
-  int grid = (int)std::min<long long>(n_tiles, (long long)d->num_sms * p->occupancy);
-  if (mode == 2) {
-    const long long per_cta = (long long)p->stash_per_cta * 4;
-    const long long fit = per_cta > 0 ? workspace_bytes / per_cta : grid;
-    if (!workspace || fit < 1) return fail(RNVP_EINVAL, "rnvp_backward: workspace too small (see rnvp_workspace_bytes)");
-    grid = (int)std::min<long long>(grid, fit);
-    a.stash = (float*)workspace;
-    a.stash_per_cta = p->stash_per_cta;
-  }
-  a.ops = p->d_ops;
-  a.chunks = p->d_chunks;
-  a.n_ops = p->n_ops;
-  a.n_chunks = p->n_chunks;
-  a.n_tiles = (int)n_tiles;
-  a.D = d->D;
-  a.Cd = d->Cd;
-  a.sm = p->sm;
-  cudaError_t e = rnvp_launch_tile(mode, p->TR, a, grid, p->smem_bytes, stream);
-  if (e != cudaSuccess) return cuda_fail(e, "tile kernel launch");
+// kernel families, numbered as rnvp_plan_info reports them
+enum Family { FAMILY_TILE = 0, FAMILY_SMALL = 1, FAMILY_MMA = 2 };
+
+// The family that runs mode `mode` (0 forward, 1 inverse, 2 fit step) of a flow: the one place that reads the path and
+// the eligibility flags to choose.  The planner keeps the two eligible sets disjoint (mma_ok needs D > 8, small_ok
+// needs D <= 8: rnvp_planner.h build_layout), so the order of the two tests below decides nothing.
+Family family(const rnvp_desc* d, int mode) {
+  // the tcgen05 fit step (forward + backward sweeps, then the weight-gradient sweep) needs the transposed weight images
+  if (d->mma_ok && d->path != 1 && (mode != 2 || d->m_wt_floats > 0)) return FAMILY_MMA;
+  // the small-flow fit kernel (one launch, no workspace) has a layer limit and three small-layout arrays in shared memory
+  if (d->small_ok && (mode != 2 || (d->L <= rnvp_small_fit_max_layers() && d->small_floats * 12 + 4096 <= d->max_smem)))
+    return FAMILY_SMALL;
+  return FAMILY_TILE;
+}
+
+// One call of the row kernels as an entry point makes it; run_tile, run_small and run_mma fill their kernel's arguments
+// from it.
+struct RowCall {
+  const float *packed = nullptr, *X = nullptr, *C = nullptr;   // X: input rows, or nullptr when an inverse draws them
+  const long long* idx = nullptr;                              // optional row gather
+  long long N = 0;
+  int l0 = 0, l1 = 0;                                          // layer range
+  float *out_x = nullptr, *out_logdet = nullptr, *out_logp = nullptr;
+  unsigned long long seed = 0;                                 // drawn latent rows are keyed on row_offset + row
+  long long row_offset = 0;
+  // fit step (mode 2)
+  float *gpacked = nullptr, *loss_sum = nullptr;
+  float scale = 0.f;
+  void* workspace = nullptr;
+  int64_t workspace_bytes = 0;
+  const RnvpFusedAdam* fused = nullptr;                        // small-flow fit step of one CTA: Adam fused behind it
+};
+
+// Argument rules of the row entry points, reported under the entry point's name: the packed parameters, the input rows
+// unless the call draws them, the output rows of an inverse, the gradient accumulator of a fit step, and C exactly when
+// the flow is conditional.
+int check_rows(const rnvp_desc* d, const char* fn, int mode, const RowCall& c, bool draws) {
+  if (c.N < 0 || c.row_offset < 0 || !c.packed || (mode == 2 && !c.gpacked) ||
+      (c.N > 0 && ((!draws && !c.X) || (mode == 1 && !c.out_x))))
+    return fail(RNVP_EINVAL, std::string(fn) + (draws ? ": bad argument" : ": null buffer"));
+  if (c.N > 0 && (d->Cd > 0) != (c.C != nullptr))
+    return fail(RNVP_EINVAL, std::string(fn) + ": C must be given iff cond_size > 0");
   return 0;
 }
 
-// fit step of small flows on the row-per-thread kernel (one launch, no workspace)
-bool use_small_fit(const rnvp_desc* d) { return d->small_ok && d->L <= rnvp_small_fit_max_layers() && d->small_floats * 12 + 4096 <= d->max_smem; }
+int run_tile(const rnvp_desc* d, int mode, const RowCall& c, cudaStream_t stream) {
+  Program* p = nullptr;
+  int rc = get_program(d, mode, c.l0, c.l1, &p);
+  if (rc) return rc;
+  const int R = 8 * p->TR;
+  const long long n_tiles = (c.N + R - 1) / R;
+  if (n_tiles > 0x7fffffffLL) return fail(RNVP_EINVAL, "too many rows for one launch");
+  int grid = (int)std::min<long long>(n_tiles, (long long)d->num_sms * p->occupancy);
+  RnvpKArgs a{};
+  if (mode == 2) {
+    const long long per_cta = (long long)p->stash_per_cta * 4;
+    const long long fit = per_cta > 0 ? c.workspace_bytes / per_cta : grid;
+    if (!c.workspace || fit < 1) return fail(RNVP_EINVAL, "rnvp_backward: workspace too small (see rnvp_workspace_bytes)");
+    grid = (int)std::min<long long>(grid, fit);
+    a.stash = (float*)c.workspace;
+    a.stash_per_cta = p->stash_per_cta;
+  }
+  a.packed = c.packed; a.X = c.X; a.C = c.C; a.idx = c.idx; a.N = c.N;
+  a.out_x = c.out_x; a.out_logdet = c.out_logdet; a.out_logp = c.out_logp;
+  a.gpacked = c.gpacked; a.loss_sum = c.loss_sum; a.scale = c.scale;
+  a.seed = c.seed; a.row_offset = c.row_offset;
+  a.ops = p->d_ops; a.chunks = p->d_chunks; a.n_ops = p->n_ops; a.n_chunks = p->n_chunks; a.n_tiles = (int)n_tiles;
+  a.D = d->D; a.Cd = d->Cd; a.sm = p->sm;
+  cudaError_t e = rnvp_launch_tile(mode, p->TR, a, grid, p->smem_bytes, stream);
+  return e == cudaSuccess ? 0 : cuda_fail(e, "tile kernel launch");
+}
 
-int run_small(rnvp_desc* d, int mode, int l0, int l1, const float* packed, const float* X, const float* C,
-              const long long* idx, long long N, float* out_x, float* out_logdet, float* out_logp, cudaStream_t stream,
-              float* gpacked = nullptr, float* loss_sum = nullptr, float scale = 0.f, unsigned long long seed = 0,
-              long long row_offset = 0, const RnvpFusedAdam* fused = nullptr) {
-  if (l0 < 0 || l1 > d->L || l0 >= l1) return fail(RNVP_EINVAL, "bad layer range");
-  if (N <= 0) return 0;
-  RnvpSmallArgs a;
-  a.packed_small = packed + d->small_off;
-  a.X = X; a.C = C; a.idx = idx; a.N = N;
-  a.out_x = out_x; a.out_logdet = out_logdet; a.out_logp = out_logp;
+int run_small(const rnvp_desc* d, int mode, const RowCall& c, cudaStream_t stream) {
+  RnvpSmallArgs a{};
+  a.packed_small = c.packed + d->small_off;
+  a.X = c.X; a.C = c.C; a.idx = c.idx; a.N = c.N;
+  a.out_x = c.out_x; a.out_logdet = c.out_logdet; a.out_logp = c.out_logp;
   a.D = d->D; a.Cd = d->Cd; a.H = d->hidden[0]; a.rec = d->srec; a.small_floats = d->small_floats;
-  a.l0 = l0; a.l1 = l1;
-  a.gpacked = gpacked; a.s2g = d->d_s2g; a.loss_sum = loss_sum; a.scale = scale;
-  a.seed = seed; a.row_offset = row_offset;
-  a.fuse_adam = 0;
-  if (fused) {
-    if (mode != 2 || N > rnvp_small_fit_rows_per_block()) return fail(RNVP_EINVAL, "fused Adam needs a single-CTA fit step");
+  a.l0 = c.l0; a.l1 = c.l1;
+  a.gpacked = c.gpacked; a.s2g = d->d_s2g; a.loss_sum = c.loss_sum; a.scale = c.scale;
+  a.seed = c.seed; a.row_offset = c.row_offset;
+  if (c.fused) {
+    if (mode != 2 || c.N > rnvp_small_fit_rows_per_block()) return fail(RNVP_EINVAL, "fused Adam needs a single-CTA fit step");
     a.fuse_adam = 1;
-    a.ad = *fused;
+    a.ad = *c.fused;
   }
   const long long rpb = mode == 2 ? rnvp_small_fit_rows_per_block() : rnvp_small_rows_per_block();
-  const long long blocks = (N + rpb - 1) / rpb;
+  const long long blocks = (c.N + rpb - 1) / rpb;
   const int grid = (int)std::min<long long>(blocks, (long long)d->num_sms * (mode == 2 ? 16 : 8));
   cudaError_t e = rnvp_launch_small(d->sNE, d->sNC, d->act, mode, a, grid, (size_t)d->small_floats * 4, stream);
-  if (e != cudaSuccess) return cuda_fail(e, "small-flow kernel launch");
-  return 0;
+  return e == cudaSuccess ? 0 : cuda_fail(e, "small-flow kernel launch");
 }
 
 long long* g_wg_trace = nullptr;    // development aid: wait accounting of -DRNVP_WG_TRACE builds, see rnvp_debug_set_trace
-bool use_mma(const rnvp_desc* d) { return d->mma_ok && d->path != 1; }
-// fit step entirely on the tensor-core path (tcgen05 forward + backward sweeps, tcgen05 weight-gradient sweep)
-bool use_mma_bwd(const rnvp_desc* d) { return use_mma(d) && d->m_wt_floats > 0; }
 // rows covered by the record / stash arrays of a tensor-core fit step: whole 128-row tiles of the sweep kernel, so that
 // the weight-gradient sweep never reads an unwritten record
 int64_t fit_npad(int64_t N) { return (N + 127) / 128 * 128; }
@@ -279,32 +307,43 @@ int wgrad_rec_floats(const rnvp_desc* d) {
   return 2 * d->hidden[0] + K1P + 2 * d->mDH;               // multiple of 8: an even number of float4 column groups
 }
 
-int run_mma(rnvp_desc* d, int mode, int l0, int l1, const float* packed, const float* X, const float* C,
-            const long long* idx, long long N, float* out_x, float* out_logdet, float* out_logp, cudaStream_t stream,
-            float* stash = nullptr, float* loss_sum = nullptr, float* records = nullptr, float scale = 0.f,
-            unsigned long long seed = 0, long long row_offset = 0) {
-  if (l0 < 0 || l1 > d->L || l0 >= l1) return fail(RNVP_EINVAL, "bad layer range");
-  if (N <= 0) return 0;
-  RnvpWideArgs a;
-  a.wimg = packed + d->mma_off;
-  a.X = X; a.C = C; a.idx = idx; a.N = N;
-  a.out_x = out_x; a.out_logdet = out_logdet; a.out_logp = out_logp;
-  a.Cd = d->Cd; a.H = d->hidden[0]; a.l0 = l0; a.l1 = l1;
+int run_mma(const rnvp_desc* d, int mode, const RowCall& c, cudaStream_t stream) {
+  RnvpWideArgs a{};
+  a.wimg = c.packed + d->mma_off;
+  a.X = c.X; a.C = c.C; a.idx = c.idx; a.N = c.N;
+  a.out_x = c.out_x; a.out_logdet = c.out_logdet; a.out_logp = c.out_logp;
+  a.Cd = d->Cd; a.H = d->hidden[0]; a.l0 = c.l0; a.l1 = c.l1;
   a.layer_floats = d->m_layer_floats; a.w1_floats = d->m_w1_floats; a.w2_floats = d->m_w2_floats;
-  a.stash = stash; a.loss_sum = loss_sum; a.L_total = d->L;
-  a.do_bwd = records != nullptr; a.scale = scale; a.records = records; a.rec = 0; a.Npad = 0;
-  a.wt_floats = records ? d->m_wt_floats : 0;
-  a.seed = seed; a.row_offset = row_offset; a.Dreal = d->D;
+  a.loss_sum = c.loss_sum; a.L_total = d->L; a.scale = c.scale;
+  a.seed = c.seed; a.row_offset = c.row_offset; a.Dreal = d->D;
+  if (mode == 2) {
+    // forward + backward sweeps in one launch (per-layer records to the workspace), then the weight-gradient sweep
+    const int64_t npad = fit_npad(c.N);
+    const int64_t stash_f = npad * d->L * 2 * d->mDH, rec_f = (int64_t)d->L * npad * wgrad_rec_floats(d);   // both blocked by 32 rows
+    if (!c.workspace || c.workspace_bytes < (stash_f + rec_f) * 4)
+      return fail(RNVP_EINVAL, "rnvp_backward: workspace too small (see rnvp_workspace_bytes)");
+    a.stash = (float*)c.workspace; a.records = a.stash + stash_f;
+    a.do_bwd = 1; a.rec = wgrad_rec_floats(d); a.Npad = npad; a.wt_floats = d->m_wt_floats;
+  }
   // one 128-row tile per CTA, two threads per row, weight images streamed per chunk step (rnvp_wide.cu)
-  if (mode == 2 && !records) return fail(RNVP_ESHAPE, "tcgen05 kernels run the fit step with their own backward sweep only");
-  const long long tiles = (N + 127) / 128;
+  const long long tiles = (c.N + 127) / 128;
   if (tiles > 0x7fffffffLL) return fail(RNVP_EINVAL, "too many rows for one launch");
   a.n_tiles = (int)tiles;
-  if (records) { a.rec = wgrad_rec_floats(d); a.Npad = fit_npad(N); }
   const long long ctas = (long long)d->num_sms * rnvp_wide_ctas_per_sm(d->mDH);   // DH <= 32: two CTAs per SM
   cudaError_t e = rnvp_launch_wide(d->mDH, d->act, mode, a, (int)std::min<long long>(tiles, ctas), stream);
   if (e != cudaSuccess) return cuda_fail(e, "tcgen05 streamed kernel launch");
-  return 0;
+  return mode == 2 ? rnvp_wgrad_sweep(d, c.packed, a.Npad, a.records, c.gpacked, stream) : 0;
+}
+
+// a row call on the family that runs it, after the checks all three share
+int run(const rnvp_desc* d, int mode, const RowCall& c, cudaStream_t stream) {
+  if (c.l0 < 0 || c.l1 > d->L || c.l0 >= c.l1) return fail(RNVP_EINVAL, "bad layer range");
+  if (c.N <= 0) return 0;
+  switch (family(d, mode)) {
+    case FAMILY_MMA: return run_mma(d, mode, c, stream);
+    case FAMILY_SMALL: return run_small(d, mode, c, stream);
+    default: return run_tile(d, mode, c, stream);
+  }
 }
 
 }  // namespace
@@ -430,11 +469,11 @@ int64_t rnvp_param_count(const rnvp_desc* d) { return d ? d->P : -1; }
 int64_t rnvp_packed_count(const rnvp_desc* d) { return d ? d->packed : -1; }
 int64_t rnvp_grad_count(const rnvp_desc* d) { return d ? d->packed_tile : -1; }
 
-int64_t rnvp_workspace_bytes(const rnvp_desc* dc, int64_t N) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
+int64_t rnvp_workspace_bytes(const rnvp_desc* d, int64_t N) {
   if (!d) return -1;
-  if (use_small_fit(d)) return 16;                      // the row-per-thread fit kernel keeps its stash in local memory
-  if (use_mma_bwd(d)) {
+  const Family f = family(d, 2);
+  if (f == FAMILY_SMALL) return 16;                     // the row-per-thread fit kernel keeps its stash in local memory
+  if (f == FAMILY_MMA) {
     const int64_t npad = fit_npad(std::max<int64_t>(N, 1));
     return (npad * d->L * 2 * d->mDH + (int64_t)d->L * npad * wgrad_rec_floats(d)) * 4;
   }
@@ -459,8 +498,7 @@ int rnvp_param_tensors(const rnvp_desc* d, int64_t* offsets, int max_tensors) {
   return k;
 }
 
-int rnvp_plan_info(const rnvp_desc* dc, int mode, int* tile_rows, int* smem_bytes, int* n_ops, int* kernel_family) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
+int rnvp_plan_info(const rnvp_desc* d, int mode, int* tile_rows, int* smem_bytes, int* n_ops, int* kernel_family) {
   if (check_desc(d)) return RNVP_EINVAL;
   if (mode < 0 || mode == 3 || mode > 4) return fail(RNVP_EINVAL, "mode must be 0, 1, 2 or 4");
   Program* p = nullptr;
@@ -469,11 +507,8 @@ int rnvp_plan_info(const rnvp_desc* dc, int mode, int* tile_rows, int* smem_byte
   if (tile_rows) *tile_rows = 8 * p->TR;
   if (smem_bytes) *smem_bytes = (int)p->smem_bytes;
   if (n_ops) *n_ops = p->n_ops;
-  if (mode == 4) {          // pseudo-mode: does the whole fit step run on the tensor cores (sweeps + weight gradients)?
-    if (kernel_family) *kernel_family = use_mma_bwd(d) ? 2 : 0;
-    return 0;
-  }
-  if (kernel_family) *kernel_family = (mode == 2 ? use_mma_bwd(d) : use_mma(d)) ? 2 : (((mode < 2 && d->small_ok) || (mode == 2 && use_small_fit(d))) ? 1 : 0);
+  // pseudo-mode 4: does the whole fit step run on the tensor cores (sweeps + weight gradients)?
+  if (kernel_family) *kernel_family = mode == 4 ? (family(d, 2) == FAMILY_MMA ? 2 : 0) : family(d, mode);
   return 0;
 }
 
@@ -500,91 +535,47 @@ int rnvp_unpack_grads(const rnvp_desc* d, const float* d_gpacked, float* d_gflat
   return e == cudaSuccess ? 0 : cuda_fail(e, "unpack_kernel");
 }
 
-int rnvp_forward(const rnvp_desc* dc, const float* d_packed, const float* d_X, const float* d_C,
+int rnvp_forward(const rnvp_desc* d, const float* d_packed, const float* d_X, const float* d_C,
                  const int64_t* d_idx, int64_t N, int layer_begin, int layer_end, float* d_z, float* d_logdet,
                  float* d_logp, void* stream) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
-  if (N < 0 || !d_packed || (N > 0 && !d_X)) return fail(RNVP_EINVAL, "rnvp_forward: null buffer");
-  if ((d->Cd > 0) != (d_C != nullptr) && N > 0) return fail(RNVP_EINVAL, "rnvp_forward: C must be given iff cond_size > 0");
-  if (use_mma(d))
-    return run_mma(d, 0, layer_begin, layer_end, d_packed, d_X, d_C, (const long long*)d_idx, N, d_z, d_logdet, d_logp,
-                   (cudaStream_t)stream);
-  if (d->small_ok)
-    return run_small(d, 0, layer_begin, layer_end, d_packed, d_X, d_C, (const long long*)d_idx, N, d_z, d_logdet,
-                     d_logp, (cudaStream_t)stream);
-  RnvpKArgs a;
-  memset(&a, 0, sizeof(a));
-  a.packed = d_packed; a.X = d_X; a.C = d_C; a.idx = (const long long*)d_idx; a.N = N;
-  a.out_x = d_z; a.out_logdet = d_logdet; a.out_logp = d_logp;
-  return run_tile(d, 0, layer_begin, layer_end, a, nullptr, 0, (cudaStream_t)stream);
+  RowCall c;
+  c.packed = d_packed; c.X = d_X; c.C = d_C; c.idx = (const long long*)d_idx; c.N = N; c.l0 = layer_begin; c.l1 = layer_end;
+  c.out_x = d_z; c.out_logdet = d_logdet; c.out_logp = d_logp;
+  const int rc = check_rows(d, "rnvp_forward", 0, c, false);
+  return rc ? rc : run(d, 0, c, (cudaStream_t)stream);
 }
 
-int rnvp_inverse(const rnvp_desc* dc, const float* d_packed, const float* d_Y, const float* d_C, int64_t N,
+int rnvp_inverse(const rnvp_desc* d, const float* d_packed, const float* d_Y, const float* d_C, int64_t N,
                  int layer_begin, int layer_end, float* d_X, void* stream) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
-  if (N < 0 || !d_packed || (N > 0 && (!d_Y || !d_X))) return fail(RNVP_EINVAL, "rnvp_inverse: null buffer");
-  if ((d->Cd > 0) != (d_C != nullptr) && N > 0) return fail(RNVP_EINVAL, "rnvp_inverse: C must be given iff cond_size > 0");
-  if (use_mma(d))
-    return run_mma(d, 1, layer_begin, layer_end, d_packed, d_Y, d_C, nullptr, N, d_X, nullptr, nullptr, (cudaStream_t)stream);
-  if (d->small_ok)
-    return run_small(d, 1, layer_begin, layer_end, d_packed, d_Y, d_C, nullptr, N, d_X, nullptr, nullptr,
-                     (cudaStream_t)stream);
-  RnvpKArgs a;
-  memset(&a, 0, sizeof(a));
-  a.packed = d_packed; a.X = d_Y; a.C = d_C; a.N = N; a.out_x = d_X;
-  return run_tile(d, 1, layer_begin, layer_end, a, nullptr, 0, (cudaStream_t)stream);
+  RowCall c;
+  c.packed = d_packed; c.X = d_Y; c.C = d_C; c.N = N; c.l0 = layer_begin; c.l1 = layer_end;
+  c.out_x = d_X;
+  const int rc = check_rows(d, "rnvp_inverse", 1, c, false);
+  return rc ? rc : run(d, 1, c, (cudaStream_t)stream);
 }
 
-int rnvp_sample(const rnvp_desc* dc, const float* d_packed, const float* d_C, int64_t N, uint64_t seed, int64_t row_offset,
+int rnvp_sample(const rnvp_desc* d, const float* d_packed, const float* d_C, int64_t N, uint64_t seed, int64_t row_offset,
                 float* d_X, void* stream) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
-  if (N < 0 || row_offset < 0 || !d_packed || (N > 0 && !d_X)) return fail(RNVP_EINVAL, "rnvp_sample: bad argument");
-  if ((d->Cd > 0) != (d_C != nullptr) && N > 0) return fail(RNVP_EINVAL, "rnvp_sample: C must be given iff cond_size > 0");
-  if (use_mma(d))
-    return run_mma(d, 1, 0, d->L, d_packed, nullptr, d_C, nullptr, N, d_X, nullptr, nullptr, (cudaStream_t)stream, nullptr,
-                   nullptr, nullptr, 0.f, seed, row_offset);
-  if (d->small_ok)
-    return run_small(d, 1, 0, d->L, d_packed, nullptr, d_C, nullptr, N, d_X, nullptr, nullptr, (cudaStream_t)stream,
-                     nullptr, nullptr, 0.f, seed, row_offset);
-  RnvpKArgs a;
-  memset(&a, 0, sizeof(a));
-  a.packed = d_packed; a.X = nullptr; a.C = d_C; a.N = N; a.out_x = d_X; a.seed = seed; a.row_offset = row_offset;
-  return run_tile(d, 1, 0, d->L, a, nullptr, 0, (cudaStream_t)stream);
+  RowCall c;
+  c.packed = d_packed; c.C = d_C; c.N = N; c.l1 = d->L;
+  c.out_x = d_X; c.seed = seed; c.row_offset = row_offset;
+  const int rc = check_rows(d, "rnvp_sample", 1, c, true);
+  return rc ? rc : run(d, 1, c, (cudaStream_t)stream);
 }
 
-int rnvp_backward(const rnvp_desc* dc, const float* d_packed, const float* d_X, const float* d_C,
+int rnvp_backward(const rnvp_desc* d, const float* d_packed, const float* d_X, const float* d_C,
                   const int64_t* d_idx, int64_t N, float scale, float* d_gpacked, float* d_logp_sum, float* d_logp,
                   void* d_workspace, int64_t workspace_bytes, void* stream) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
-  if (N < 0 || !d_packed || !d_gpacked || (N > 0 && !d_X)) return fail(RNVP_EINVAL, "rnvp_backward: null buffer");
-  if ((d->Cd > 0) != (d_C != nullptr) && N > 0) return fail(RNVP_EINVAL, "rnvp_backward: C must be given iff cond_size > 0");
-  RnvpKArgs a;
-  memset(&a, 0, sizeof(a));
-  a.packed = d_packed; a.C = d_C; a.idx = (const long long*)d_idx; a.N = N;
-  a.gpacked = d_gpacked; a.scale = scale;
-  if (use_small_fit(d) && N > 0)
-    return run_small(d, 2, 0, d->L, d_packed, d_X, d_C, (const long long*)d_idx, N, nullptr, nullptr, d_logp,
-                     (cudaStream_t)stream, d_gpacked, d_logp_sum, scale);
-  if (use_mma_bwd(d) && N > 0) {
-    // forward + backward sweeps in one tcgen05 launch (per-layer records to the workspace), then the weight-gradient sweep
-    const int64_t npad = fit_npad(N);
-    const int64_t stash_f = npad * d->L * 2 * d->mDH, rec_f = (int64_t)d->L * npad * wgrad_rec_floats(d);   // both blocked by 32 rows
-    if (!d_workspace || workspace_bytes < (stash_f + rec_f) * 4)
-      return fail(RNVP_EINVAL, "rnvp_backward: workspace too small (see rnvp_workspace_bytes)");
-    float* stash = (float*)d_workspace;
-    float* records = stash + stash_f;
-    int rc = run_mma(d, 2, 0, d->L, d_packed, d_X, d_C, (const long long*)d_idx, N, nullptr, nullptr, d_logp,
-                     (cudaStream_t)stream, stash, d_logp_sum, records, scale);
-    if (rc) return rc;
-    return rnvp_wgrad_sweep(d, d_packed, npad, records, d_gpacked, stream);
-  }
-  a.X = d_X;
-  a.out_logp = d_logp; a.loss_sum = d_logp_sum;
-  return run_tile(d, 2, 0, d->L, a, d_workspace, workspace_bytes, (cudaStream_t)stream);
+  RowCall c;
+  c.packed = d_packed; c.X = d_X; c.C = d_C; c.idx = (const long long*)d_idx; c.N = N; c.l1 = d->L;
+  c.out_logp = d_logp; c.gpacked = d_gpacked; c.loss_sum = d_logp_sum; c.scale = scale;
+  c.workspace = d_workspace; c.workspace_bytes = workspace_bytes;
+  const int rc = check_rows(d, "rnvp_backward", 2, c, false);
+  return rc ? rc : run(d, 2, c, (cudaStream_t)stream);
 }
 
 int rnvp_adam_step(const rnvp_desc* d, float* d_flat, float* d_packed, float* d_gpacked, const float* d_gflat_in,
@@ -616,14 +607,15 @@ int rnvp_fit_epoch(const rnvp_desc* d, float* d_flat, float* d_packed, float* d_
                    float* d_losses, void* d_workspace, int64_t workspace_bytes, void* stream) {
   if (check_desc(d)) return RNVP_EINVAL;
   if (n < 0 || batch_size < 1 || step0 < 0 || !d_perm || !d_losses || !d_loss_slot) return fail(RNVP_EINVAL, "rnvp_fit_epoch: bad argument");
+  // A small-flow step of at most one CTA's rows is ONE launch: the fit kernel with the Adam update fused behind it (no
+  // packed-gradient round trip; d_gpacked and the loss slot stay zero, as the two-launch path leaves them).  Arguments it
+  // cannot take go to rnvp_backward and rnvp_adam_step, which report them.
+  const bool fuse = family(d, 2) == FAMILY_SMALL && (d->Cd > 0) == (d_C != nullptr) && d_X && d_flat && d_packed &&
+                    d_exp_avg && d_exp_avg_sq;
   int64_t s = 0;
-  rnvp_desc* dm = const_cast<rnvp_desc*>(d);
   for (int64_t b0 = 0; b0 < n; b0 += batch_size, ++s) {
     const int64_t nb = std::min(batch_size, n - b0);
-    if (use_small_fit(dm) && nb <= rnvp_small_fit_rows_per_block() && (d->Cd > 0) == (d_C != nullptr) && d_X && d_flat && d_packed &&
-        d_exp_avg && d_exp_avg_sq) {
-      // the whole step is ONE single-CTA launch: fit kernel with the Adam update fused behind it (no packed-gradient round
-      // trip; d_gpacked and the loss slot stay zero, as the two-launch path leaves them)
+    if (fuse && nb <= rnvp_small_fit_rows_per_block()) {
       const int64_t step = step0 + s + 1;
       const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
       RnvpFusedAdam ad;
@@ -632,8 +624,10 @@ int rnvp_fit_epoch(const rnvp_desc* d, float* d_flat, float* d_packed, float* d_
       ad.k = RnvpAdamCoef{(float)weight_decay, (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)(lr / bc1),
                           (float)sqrt(bc2), (float)eps};
       ad.loss_dst = d_losses + s; ad.loss_scale = -1.0f / (float)nb;
-      int rc = run_small(dm, 2, 0, d->L, d_packed, d_X, d_C, (const long long*)(d_perm + b0), nb, nullptr, nullptr, nullptr,
-                         (cudaStream_t)stream, d_gpacked, d_loss_slot, -1.0f / (float)nb, 0, 0, &ad);
+      RowCall c;
+      c.packed = d_packed; c.X = d_X; c.C = d_C; c.idx = (const long long*)(d_perm + b0); c.N = nb; c.l1 = d->L;
+      c.gpacked = d_gpacked; c.loss_sum = d_loss_slot; c.scale = -1.0f / (float)nb; c.fused = &ad;
+      int rc = run(d, 2, c, (cudaStream_t)stream);
       if (rc) return rc;
       continue;
     }
@@ -653,9 +647,8 @@ int rnvp_wgrad_record_floats(const rnvp_desc* d) {
   return wgrad_rec_floats(d);
 }
 
-int rnvp_wgrad_sweep(const rnvp_desc* dc, const float* d_packed, int64_t Npad, const float* d_records, float* d_gpacked,
+int rnvp_wgrad_sweep(const rnvp_desc* d, const float* d_packed, int64_t Npad, const float* d_records, float* d_gpacked,
                      void* stream) {
-  rnvp_desc* d = const_cast<rnvp_desc*>(dc);
   if (check_desc(d)) return RNVP_EINVAL;
   if (!d->mma_ok || d->m_wt_floats == 0)
     return fail(RNVP_ESHAPE, "rnvp_wgrad_sweep: needs a flow whose fit step runs on the tensor cores (a tcgen05 flow with D <= 64, "
