@@ -17,49 +17,25 @@ and the global RNG state after ``sample`` are therefore not the reference's.  ``
 autograd).  CUDA only; there is no CPU fallback.
 """
 import ctypes as ct
-import threading
 
-import numpy as np
 import torch
 import torch.nn as nn
 
+from . import _mlp
+from ._mlp import Desc, FlatParams, RngReplay, _stream, advance, check_fit_inputs, publish_state, run_epochs
 from .interfaces import GenModel
-from .realnvp import _LossLog, _default_device
+from .realnvp import _default_device
 from .. import _lib
-from ..batching import StreamingPermutation, batch_bounds
+from ..batching import batch_bounds
 
 ACT = {"tanh": 1, "relu": 2, "sigmoid": 3}         # include/rnvp.h RNVP_ACT_*; every other string is ReLU upstream
 
 
-class _Desc:
-    """Owns one ``rnvp_cn_desc`` (shape, activation, covariance mode) on the current CUDA device."""
-
-    def __init__(self, D, Cd, hidden, activation, independent):
-        self.lib = _lib.load()
-        hid = (ct.c_int * len(hidden))(*hidden)
-        h = ct.c_void_p()
-        rc = self.lib.rnvp_cn_desc_create(D, Cd, len(hidden), hid, ACT.get(activation, 2), int(bool(independent)),
-                                          ct.byref(h))
-        if rc != 0:
-            msg = self.lib.rnvp_last_error().decode()
-            if rc == -2:                                   # RNVP_ESHAPE
-                raise ValueError(msg)
-            raise _lib.RnvpError(f"rnvp_cn_desc_create failed (code {rc}): {msg}")
-        self.h, self.D, self.Cd, self.independent = h, D, Cd, bool(independent)
-        self.P = int(self.lib.rnvp_cn_param_count(h))
-
-    def workspace(self, n, dev):
-        nbytes = int(self.lib.rnvp_cn_workspace_bytes(self.h, max(int(n), 1)))
-        return torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=dev), nbytes
-
-    def __del__(self):
-        if getattr(self, "h", None):
-            self.lib.rnvp_cn_desc_destroy(self.h)
-            self.h = None
-
-
-def _stream(dev):
-    return ct.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+def _desc(D, Cd, hidden, activation, independent):
+    """The ``rnvp_cn_desc`` of a Net (shape, activation, covariance mode) on the current CUDA device; only
+    RNVP_ESHAPE is a ValueError."""
+    return Desc("cn", (D, Cd, len(hidden), (ct.c_int * len(hidden))(*hidden), ACT.get(activation, 2),
+                       int(bool(independent))), (-2,), D=D, Cd=Cd, independent=bool(independent))
 
 
 class Net(nn.Module):
@@ -83,37 +59,29 @@ class Net(nn.Module):
         self.mu = nn.Linear(hidden[-1], var_size)
         self.log_sigma = nn.Linear(hidden[-1], var_size)
         self.out = nn.Linear(var_size, var_size)
-        self._desc, self._flat = None, None
+        self._params = None
 
     def __getstate__(self):
         state = self.__dict__.copy()
-        state["_desc"], state["_flat"] = None, None
+        state["_params"] = None
         return state
 
     def to_device(self, dev):
         """Move the parameters into one flat fp32 buffer on ``dev`` (parameter tensors become views of it)."""
-        if self._desc is None:
-            with torch.cuda.device(dev):
-                self._desc = _Desc(self.var_size, self.cond_size, self.hidden, self.activation,
-                                   self.independent_covariance)
-        params = list(self.parameters())
-        flat = torch.cat([p.detach().reshape(-1).to(torch.float32) for p in params]).to(dev)
-        off = 0
-        for p in params:
-            n = p.numel()
-            p.data = flat[off:off + n].view(p.shape)
-            off += n
-        self._flat = flat
+        if self._params is None:
+            # the child modules (same parameter order), not the Net: a reference back to it would be a cycle, and a
+            # dropped Net would hold its device buffers until the garbage collector runs
+            self._params = FlatParams(self.children(), lambda: _desc(self.var_size, self.cond_size, self.hidden,
+                                                                     self.activation, self.independent_covariance), dev)
+        else:
+            self._params.pack(dev)
         return self
 
     def _ready(self):
-        p = self.mu.weight
-        if self._flat is None or p.data_ptr() != self._flat.data_ptr() + 4 * self.mu_offset() or p.device.type != "cuda":
+        if self._params is None:
+            p = self.mu.weight
             self.to_device(p.device if p.device.type == "cuda" else _default_device())
-        return self._desc, self._flat
-
-    def mu_offset(self):
-        return sum(p.numel() for p in self.model.parameters())
+        return self._params.ready()
 
     def inverse_out(self):
         """M = (out.weight^T)^-1 on the device; raises torch.linalg.LinAlgError if a pivot is exactly zero."""
@@ -199,69 +167,6 @@ class Net(nn.Module):
         return logp
 
 
-class _RngReplay:
-    """The reference's use of the global torch generator during ``fit``, replayed on a helper thread.
-
-    Per epoch the reference's fresh ``DataLoader(shuffle=True)`` draws two int64 (the second seeds the row order) and
-    every step's ``Net.forward`` draws ``torch.randn(nb, D)``.  The replay runs on a private generator cloned from the
-    global state after ``Net`` init: the int64 draws go through torch, the normals are skipped with
-    ``rnvp_cn_rng_advance`` (the words ``torch.randn`` would consume, without computing the values); below 16 elements
-    torch takes a cached double path, so those few draws are made with ``torch.randn`` on the private generator."""
-
-    def __init__(self, lib, n, bs, D, n_epochs):
-        self.lib = lib
-        self.gen = torch.Generator()
-        self.gen.set_state(torch.get_rng_state())
-        self.numels = [nb * D for _, nb in batch_bounds(n, bs)]
-        self.seeds = []
-        self._cv = threading.Condition()
-        self._err = None
-        self._thread = threading.Thread(target=self._run, args=(n_epochs,), daemon=True)
-        self._thread.start()
-
-    def _run(self, n_epochs):
-        try:
-            for _ in range(n_epochs):
-                torch.empty((), dtype=torch.int64).random_(generator=self.gen)
-                seed = int(torch.empty((), dtype=torch.int64).random_(generator=self.gen).item())
-                with self._cv:
-                    self.seeds.append(seed)
-                    self._cv.notify_all()
-                advance(self.lib, self.gen, self.numels)
-        except Exception as e:                                              # pragma: no cover
-            with self._cv:
-                self._err = e
-                self._cv.notify_all()
-
-    def seed(self, epoch):
-        with self._cv:
-            while len(self.seeds) <= epoch and self._err is None:
-                self._cv.wait()
-            if self._err is not None:
-                raise self._err
-            return self.seeds[epoch]
-
-    def final_state(self):
-        self._thread.join()
-        if self._err is not None:
-            raise self._err
-        return self.gen.get_state()
-
-
-def advance(lib, gen, numels):
-    """Advance ``gen`` as ``torch.randn(k)`` (float32) would, for every k in ``numels``, in order."""
-    state = gen.get_state()
-    for k in numels:
-        if k >= 16:
-            _lib.check(lib.rnvp_cn_rng_advance(ct.c_void_p(state.data_ptr()), state.numel(), int(k)),
-                       "rnvp_cn_rng_advance")
-        elif k > 0:
-            gen.set_state(state)
-            torch.randn(int(k), generator=gen)
-            state = gen.get_state()
-    gen.set_state(state)
-
-
 def state_at_step(lib, state, n, bs, D, step):
     """The global generator state the reference leaves when fit step ``step`` (0-based over the whole fit) raises in
     its forward pass: from ``state`` (right after Net init), every epoch's two DataLoader draws and every step's
@@ -283,9 +188,8 @@ def state_at_step(lib, state, n, bs, D, step):
 def epoch_plan(lib, n, bs, D, n_epochs):
     """Host-only replay of ``fit``'s RNG use from the current global state (a test and inspection aid): returns the
     per-epoch sampler seeds and the generator state the reference leaves behind.  The global state is not changed."""
-    rp = _RngReplay(lib, n, bs, D, n_epochs)
-    state = rp.final_state()
-    return list(rp.seeds), state
+    seeds, _, state = _mlp.epoch_plan(lib, n, bs, D, n_epochs, epoch_end=False, values=False)
+    return seeds, state
 
 
 class ConditionalNormal(GenModel):
@@ -356,25 +260,15 @@ class ConditionalNormal(GenModel):
         torch.linalg.LinAlgError when ``out.weight`` becomes singular; ``model`` and ``loss_history`` then hold the
         state before the step that could not run."""
         from ..ingest import upload_resident
-        if not hasattr(X, "shape"):
-            X = np.asarray(X)
-        if len(tuple(X.shape)) != 2:
-            raise ValueError(f"X must be 2-D [n, var_size], got shape {tuple(X.shape)}")
-        n = X.shape[0]
+        X, C, n, bs = check_fit_inputs(X, C, self.batch_size, 0)
         if C is None:
             C = torch.zeros(n, 1)
-        elif not hasattr(C, "shape"):
-            C = np.asarray(C)
-        if len(tuple(C.shape)) != 2 or C.shape[0] != n:
-            raise ValueError(f"C must be 2-D with {n} rows, got shape {tuple(C.shape)}")
         if self._device is None:
             self._device = _default_device()
         self._model_init(X, C)
         dev, net = self._device, self.model
         desc, flat = net._ready()
-        lib, D, bs = desc.lib, net.var_size, int(self.batch_size)
-        if bs < 1:
-            raise ValueError("batch_size must be >= 1")
+        lib, D = desc.lib, net.var_size
         self.model.train(True)
         self.loss_history = []
         init_state = torch.get_rng_state()
@@ -384,77 +278,37 @@ class ConditionalNormal(GenModel):
             if self.n_epochs > 0 and n > 0:      # the reference raises inside step 0, after that step's draws
                 torch.set_rng_state(state_at_step(lib, init_state, n, bs, D, 0))
             raise
-        replay = _RngReplay(lib, n, bs, D, self.n_epochs)
-        Xd = upload_resident(lib, X, dev)
-        Cd = upload_resident(lib, C, dev)
-        P = desc.P
-        exp_avg = torch.zeros(P, dtype=torch.float32, device=dev)
-        exp_avg_sq = torch.zeros(P, dtype=torch.float32, device=dev)
-        status = torch.zeros(1, dtype=torch.int32, device=dev)
-        ws, nbytes = desc.workspace(min(bs, max(n, 1)), dev)
-        perm_dev = [torch.empty(max(n, 1), dtype=torch.int64, device=dev) for _ in range(2)]
-        copied = [None, None]
-        bounds = batch_bounds(n, bs)
-        log = _LossLog(self.loss_history)
-        epochs = range(self.n_epochs)
-        bar = None
-        if self.verbose >= 1:
-            from tqdm.auto import tqdm
-            bar = tqdm(epochs, unit='epoch')
-            epochs = bar
-        stream = _stream(dev)
-        nxt = StreamingPermutation(lib, replay.seed(0), n, host=self._perm_host[0]) if self.n_epochs > 0 else None
-        for ep in epochs:
-            sp = nxt
-            self._perm_host[ep & 1] = sp.host
-            k = ep & 1
-            perm_dev[k][:n].copy_(sp.full(), non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record(torch.cuda.current_stream(dev))
-            copied[k] = ev
-            losses = torch.empty(len(bounds), dtype=torch.float32, device=dev)
-            _lib.check(lib.rnvp_cn_fit_epoch(desc.h, flat.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
-                                             M.data_ptr(), Xd.data_ptr(), Cd.data_ptr(), perm_dev[k].data_ptr(), n, bs,
-                                             self.lr, 0.9, 0.999, 1e-8, self.weight_decay, ep * len(bounds),
-                                             losses.data_ptr(), ct.c_void_p(status.data_ptr()), ws.data_ptr(), nbytes,
-                                             stream), "rnvp_cn_fit_epoch")
-            if ep + 1 < self.n_epochs:
-                # the next order is shuffled into the other host buffer while this epoch runs; that buffer's last copy
-                # (two epochs ago) must have left it
-                if copied[k ^ 1] is not None:
-                    copied[k ^ 1].synchronize()
-                nxt = StreamingPermutation(lib, replay.seed(ep + 1), n, host=self._perm_host[(ep + 1) & 1])
-            host = log.push(losses)
-            if bar is not None and host is not None:
-                bar.set_description(f"loss: {float(host[-1]):.4f}")
-        log.flush()
-        final_state = replay.final_state()
-        self._publish_state(exp_avg, exp_avg_sq, self.n_epochs * len(bounds))
+        n_steps = len(batch_bounds(n, bs))
+        with RngReplay(lib, n, bs, D, self.n_epochs, epoch_end=False, values=False) as replay:
+            Xd = upload_resident(lib, X, dev)
+            Cd = upload_resident(lib, C, dev)
+            exp_avg = torch.zeros(desc.P, dtype=torch.float32, device=dev)
+            exp_avg_sq = torch.zeros(desc.P, dtype=torch.float32, device=dev)
+            status = torch.zeros(1, dtype=torch.int32, device=dev)
+            ws, nbytes = desc.workspace(min(bs, max(n, 1)), dev)
+            stream = _stream(dev)
+
+            def launch(ep, perm, eps, seed):
+                losses = torch.empty(n_steps, dtype=torch.float32, device=dev)
+                _lib.check(lib.rnvp_cn_fit_epoch(desc.h, flat.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
+                                                 M.data_ptr(), Xd.data_ptr(), Cd.data_ptr(), perm.data_ptr(), n, bs,
+                                                 self.lr, 0.9, 0.999, 1e-8, self.weight_decay, ep * n_steps,
+                                                 losses.data_ptr(), ct.c_void_p(status.data_ptr()), ws.data_ptr(),
+                                                 nbytes, stream), "rnvp_cn_fit_epoch")
+                return (losses,)
+            final_state = run_epochs(self, lib, dev, n, replay, launch, [(self.loss_history, "loss")])
+        # Adam state for every tensor that had a gradient: the out tensors get none with independent covariance
+        params = [p for name, p in net.named_parameters()
+                  if not (self.independent_covariance and name.startswith("out."))]
+        publish_state(self.opt, params, self.n_epochs * n_steps, exp_avg=exp_avg, exp_avg_sq=exp_avg_sq)
         failed = int(status.item())
         torch.set_rng_state(final_state if not failed else state_at_step(lib, init_state, n, bs, D, failed - 1))
         if failed:
             del self.loss_history[failed - 1:]
-            self._publish_state(exp_avg, exp_avg_sq, failed - 1)
+            publish_state(self.opt, params, failed - 1, exp_avg=exp_avg, exp_avg_sq=exp_avg_sq)
             raise torch.linalg.LinAlgError(
                 f"ConditionalNormal.fit: out.weight became singular after step {failed - 1} (linalg.inv: the input "
                 "matrix is singular); model and loss_history hold the state before the step that could not run")
-
-    def _publish_state(self, exp_avg, exp_avg_sq, steps):
-        """``opt.state`` as torch.optim.Adam leaves it: step, exp_avg, exp_avg_sq (views of the device moments) for
-        every tensor that had a gradient."""
-        self.opt.state.clear()
-        if steps <= 0:
-            return
-        off = 0
-        params = list(self.model.parameters())
-        n_grad = len(params) - (2 if self.independent_covariance else 0)
-        for i, p in enumerate(params):
-            numel = p.numel()
-            if i < n_grad:
-                self.opt.state[p] = {"step": torch.tensor(float(steps)),
-                                     "exp_avg": exp_avg[off:off + numel].view(p.shape),
-                                     "exp_avg_sq": exp_avg_sq[off:off + numel].view(p.shape)}
-            off += numel
 
     def sample(self, C=100, seed=None, eps=None):
         """Rows drawn for the conditions C [n, cond_size], or ``C`` rows with zero conditions if it is an int

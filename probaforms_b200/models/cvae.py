@@ -25,103 +25,24 @@ supplies the reference's noise for parity.  ``Encoder.forward`` and ``Decoder.fo
 autograd).  CUDA only; there is no CPU fallback.
 """
 import ctypes as ct
-import threading
 
-import numpy as np
 import torch
 import torch.nn as nn
 
+from . import _mlp
+from ._mlp import Desc, FlatParams, RngReplay, _act_code, _layers, _rows, _stream, check_fit_inputs, publish_state, \
+    run_epochs
 from .interfaces import GenModel
-from .realnvp import _LossLog, _default_device
-from .cnormal import _stream, advance
+from .realnvp import _default_device
 from .. import _lib
-from ..batching import StreamingPermutation, batch_bounds
+from ..batching import batch_bounds
 
 
-def _act_code(activation):
-    return 1 if activation == 'tanh' else 2          # include/rnvp.h RNVP_ACT_*: every other string is ReLU upstream
-
-
-def _layers(n_inputs, hidden, activation):
-    layers = []
-    for i in range(len(hidden)):
-        layers.append(nn.Linear(n_inputs if i == 0 else hidden[i - 1], hidden[i]))
-        layers.append(nn.Tanh() if activation == 'tanh' else nn.ReLU())
-    return layers
-
-
-class _Desc:
-    """Owns one ``rnvp_cv_desc`` (shape and activation of an encoder-decoder pair) on the current CUDA device."""
-
-    def __init__(self, D, Cd, latent, hidden, activation):
-        self.lib = _lib.load()
-        hid = (ct.c_int * len(hidden))(*hidden)
-        h = ct.c_void_p()
-        rc = self.lib.rnvp_cv_desc_create(D, Cd, latent, len(hidden), hid, _act_code(activation), ct.byref(h))
-        if rc != 0:
-            msg = self.lib.rnvp_last_error().decode()
-            if rc in (-1, -2):                             # RNVP_EINVAL, RNVP_ESHAPE
-                raise ValueError(msg)
-            raise _lib.RnvpError(f"rnvp_cv_desc_create failed (code {rc}): {msg}")
-        self.h, self.D, self.Cd, self.L = h, D, Cd, latent
-        self.P = int(self.lib.rnvp_cv_param_count(h))
-
-    def workspace(self, batch_rows, loss_rows, dev):
-        nbytes = int(self.lib.rnvp_cv_workspace_bytes(self.h, int(batch_rows), int(loss_rows)))
-        return torch.empty(max(nbytes, 4) // 4, dtype=torch.float32, device=dev), nbytes
-
-    def __del__(self):
-        if getattr(self, "h", None):
-            self.lib.rnvp_cv_desc_destroy(self.h)
-            self.h = None
-
-
-class _Pair:
-    """The device side of a pair of modules (encoder-decoder, generator-discriminator): the descriptor ``make_desc()``
-    creates on ``dev`` and one flat fp32 buffer of which every parameter of both modules is a view (the first module's
-    ``parameters()`` then the second's, the layout the kernels read)."""
-
-    def __init__(self, first, second, make_desc, dev):
-        self.modules = (first, second)
-        with torch.cuda.device(dev):
-            self.desc = make_desc()
-        self.flat = None
-        self.pack(dev)
-
-    def params(self):
-        return [p for m in self.modules for p in m.parameters()]
-
-    def pack(self, dev):
-        params = self.params()
-        flat = torch.cat([p.detach().reshape(-1).to(torch.float32) for p in params]).to(dev)
-        off = 0
-        for p in params:
-            n = p.numel()
-            p.data = flat[off:off + n].view(p.shape)
-            off += n
-        self.flat = flat
-
-    def ready(self):
-        """(desc, flat); re-packs when a parameter is no longer a view of ``flat`` (e.g. after ``Module.to``)."""
-        params = self.params()
-        off, ok = 0, True
-        for p in params:
-            if p.device.type != "cuda" or p.data_ptr() != self.flat.data_ptr() + 4 * off:
-                ok = False
-                break
-            off += p.numel()
-        if not ok:
-            p = params[0]
-            self.pack(p.device if p.device.type == "cuda" else _default_device())
-        return self.desc, self.flat
-
-
-def _rows(A, dev, width, what):
-    """A [n, width] float32 contiguous device tensor; RuntimeError on a width mismatch, as the reference's Linear."""
-    t = torch.as_tensor(A, dtype=torch.float32).to(dev).contiguous()
-    if t.dim() != 2 or t.shape[1] != width:
-        raise RuntimeError(f"{what} must be [n, {width}], got shape {tuple(t.shape)}")
-    return t
+def _desc(D, Cd, latent, hidden, activation):
+    """The ``rnvp_cv_desc`` of an encoder-decoder pair (shapes and activation) on the current CUDA device;
+    RNVP_EINVAL and RNVP_ESHAPE are ValueErrors."""
+    return Desc("cv", (D, Cd, latent, len(hidden), (ct.c_int * len(hidden))(*hidden), _act_code(activation)), (-1, -2),
+                D=D, Cd=Cd, L=latent)
 
 
 class Encoder(nn.Module):
@@ -220,113 +141,12 @@ class Decoder(nn.Module):
         return x
 
 
-class _NoiseReplay:
-    """The reference's use of the global torch generator during ``fit``, replayed on a helper thread.
-
-    Per epoch the reference's fresh ``DataLoader(shuffle=True)`` draws two int64 (the second seeds the row order), every
-    step's ``sample_z`` draws ``torch.randn(nb, latent)`` and the end-of-epoch ``compute_loss`` draws
-    ``torch.randn(n, latent)``.  The replay runs on a private generator cloned from the global state after init.  With
-    ``values`` the normals are drawn with ``torch.randn`` into one of two pinned buffers (steps in order, then the
-    epoch-end rows), which the fit loop uploads; a buffer is refilled only after the upload of two epochs ago has
-    completed.  Without ``values`` they are skipped in the generator state (``advance``)."""
-
-    def __init__(self, lib, n, bs, L, n_epochs, values):
-        self.lib, self.n, self.L, self.values = lib, n, L, values
-        self.gen = torch.Generator()
-        self.gen.set_state(torch.get_rng_state())
-        self.steps = [nb for _, nb in batch_bounds(n, bs)]
-        self.bufs = [None, None]
-        if values:
-            k = min(n_epochs, 2)
-            pin = torch.cuda.is_available()
-            self.bufs = [torch.empty(2 * n * L, dtype=torch.float32, pin_memory=pin) for _ in range(k)] + [None] * (2 - k)
-        self.seeds, self.released = [], {}
-        self._cv = threading.Condition()
-        self._err, self._closed = None, False
-        self._thread = threading.Thread(target=self._run, args=(n_epochs,), daemon=True)
-        self._thread.start()
-
-    def _run(self, n_epochs):
-        try:
-            L = self.L
-            for e in range(n_epochs):
-                torch.empty((), dtype=torch.int64).random_(generator=self.gen)
-                seed = int(torch.empty((), dtype=torch.int64).random_(generator=self.gen).item())
-                if self.values:
-                    if e >= 2:
-                        with self._cv:
-                            while e - 2 not in self.released and not self._closed:
-                                self._cv.wait()
-                            if self._closed:
-                                return
-                            ev = self.released.pop(e - 2)
-                        ev.synchronize()
-                    buf, off = self.bufs[e & 1], 0
-                    for nb in self.steps + [self.n]:
-                        torch.randn(nb, L, generator=self.gen, out=buf[off:off + nb * L].view(nb, L))
-                        off += nb * L
-                else:
-                    advance(self.lib, self.gen, [nb * L for nb in self.steps] + [self.n * L])
-                with self._cv:
-                    self.seeds.append(seed)
-                    self._cv.notify_all()
-        except Exception as e:                                              # pragma: no cover
-            with self._cv:
-                self._err = e
-                self._cv.notify_all()
-
-    def get(self, epoch):
-        """(sampler seed, pinned noise buffer or None) of ``epoch``, once the helper thread has produced them."""
-        with self._cv:
-            while len(self.seeds) <= epoch and self._err is None:
-                self._cv.wait()
-            if self._err is not None:
-                raise self._err
-            return self.seeds[epoch], self.bufs[epoch & 1]
-
-    def release(self, epoch, event):
-        """The upload of ``epoch``'s buffer completes with ``event``; the buffer may then be refilled."""
-        with self._cv:
-            self.released[epoch] = event
-            self._cv.notify_all()
-
-    def close(self):
-        with self._cv:
-            self._closed = True
-            self._cv.notify_all()
-        self._thread.join()
-
-    def final_state(self):
-        self._thread.join()
-        if self._err is not None:
-            raise self._err
-        return self.gen.get_state()
-
-
 def epoch_plan(lib, n, bs, L, n_epochs, values=True):
-    """Host-only replay of ``fit``'s RNG use from the current global state (a test and inspection aid): returns the
-    per-epoch sampler seeds, epoch 0's noise (every step's ``randn(nb, latent)`` in order, then ``randn(n, latent)``;
-    None without ``values``) and the generator state the reference leaves behind.  The global state is not changed."""
-    rp = _NoiseReplay(lib, n, bs, L, n_epochs, values)
-    eps0 = None
-    try:
-        for e in range(n_epochs):
-            _, buf = rp.get(e)
-            if e == 0 and buf is not None:
-                eps0 = buf.clone()
-            rp.release(e, _Done())
-        state = rp.final_state()
-    finally:
-        rp.close()
-    return list(rp.seeds), eps0, state
-
-
-class _Done:
-    """A completed upload (host-only replays have none to wait for)."""
-
-    @staticmethod
-    def synchronize():
-        pass
+    """Host-only replay of ``fit``'s RNG use from the current global state (a test and inspection aid; the WGAN's is
+    the same): returns the per-epoch sampler seeds, epoch 0's noise (every step's ``randn(nb, latent)`` in order, then
+    ``randn(n, latent)``; None without ``values``) and the generator state the reference leaves behind.  The global
+    state is not changed."""
+    return _mlp.epoch_plan(lib, n, bs, L, n_epochs, epoch_end=True, values=values)
 
 
 class CVAE(GenModel):
@@ -371,7 +191,7 @@ class CVAE(GenModel):
 
     def _attach(self, D, Cd, dev):
         enc = self.encoder
-        pair = _Pair(enc, self.decoder, lambda: _Desc(D, Cd, enc.lat_size, enc.hidden, enc.activation), dev)
+        pair = FlatParams([enc, self.decoder], lambda: _desc(D, Cd, enc.lat_size, enc.hidden, enc.activation), dev)
         self.encoder._pair = self.decoder._pair = pair
 
     def _ready(self):
@@ -436,21 +256,7 @@ class CVAE(GenModel):
         decoder and Adam on every call, as upstream.  ``loss_history`` gets one 0-d CPU tensor per epoch: the loss
         over all rows after the epoch's steps.  Returns ``self``."""
         from ..ingest import upload_resident
-        if self.noise not in ("torch", "device"):
-            raise ValueError(f"noise must be 'torch' or 'device', got {self.noise!r}")
-        if not hasattr(X, "shape"):
-            X = np.asarray(X)
-        if len(tuple(X.shape)) != 2 or X.shape[0] < 1:
-            raise ValueError(f"X must be 2-D [n, var_size] with n >= 1, got shape {tuple(X.shape)}")
-        n = X.shape[0]
-        if C is not None:
-            if not hasattr(C, "shape"):
-                C = np.asarray(C)
-            if len(tuple(C.shape)) != 2 or C.shape[0] != n:
-                raise ValueError(f"C must be 2-D with {n} rows, got shape {tuple(C.shape)}")
-        bs = int(self.batch_size)
-        if bs < 1:
-            raise ValueError("batch_size must be >= 1")
+        X, C, n, bs = check_fit_inputs(X, C, self.batch_size, 1, self.noise)
         if self._device is None:
             self._device = _default_device()
         self._model_init(X, C)
@@ -460,82 +266,32 @@ class CVAE(GenModel):
         self.encoder.train(True)
         self.decoder.train(True)
         self.loss_history = []
-        values = self.noise == "torch"
-        replay = _NoiseReplay(lib, n, bs, L, self.n_epochs, values)
-        try:
+        n_steps = len(batch_bounds(n, bs))
+        with RngReplay(lib, n, bs, L, self.n_epochs, epoch_end=True, values=self.noise == "torch") as replay:
             Xd = upload_resident(lib, X, dev)
             Cd = upload_resident(lib, C, dev) if desc.Cd else None
-            P = desc.P
-            exp_avg = torch.zeros(P, dtype=torch.float32, device=dev)
-            exp_avg_sq = torch.zeros(P, dtype=torch.float32, device=dev)
+            exp_avg = torch.zeros(desc.P, dtype=torch.float32, device=dev)
+            exp_avg_sq = torch.zeros(desc.P, dtype=torch.float32, device=dev)
             ws, nbytes = desc.workspace(min(bs, n), n, dev)
-            perm_dev = [torch.empty(n, dtype=torch.int64, device=dev) for _ in range(2)]
-            eps_dev = torch.empty(2 * n * L, dtype=torch.float32, device=dev) if values else None
             losses = torch.empty(max(self.n_epochs, 1), dtype=torch.float32, device=dev)
-            copied = [None, None]
-            n_steps = len(batch_bounds(n, bs))
-            log = _LossLog(self.loss_history)
-            epochs = range(self.n_epochs)
-            bar = None
-            if self.verbose >= 1:
-                from tqdm.auto import tqdm
-                bar = tqdm(epochs, unit='epoch')
-                epochs = bar
             stream = _stream(dev)
-            nxt = None
-            if self.n_epochs > 0:
-                nxt = StreamingPermutation(lib, replay.get(0)[0], n, host=self._perm_host[0])
-            for ep in epochs:
-                seed, buf = replay.get(ep)
-                sp = nxt
-                self._perm_host[ep & 1] = sp.host
-                k = ep & 1
-                perm_dev[k].copy_(sp.full(), non_blocking=True)
-                if values:
-                    eps_dev.copy_(buf, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(torch.cuda.current_stream(dev))
-                copied[k] = ev
-                if values:
-                    replay.release(ep, ev)
+
+            def launch(ep, perm, eps, seed):
                 _lib.check(lib.rnvp_cv_fit_epoch(desc.h, flat.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
-                                                 Xd.data_ptr(), None if Cd is None else Cd.data_ptr(),
-                                                 perm_dev[k].data_ptr(), n, bs, self.lr, 0.9, 0.999, 1e-8,
-                                                 self.weight_decay, float(self.KL_weight), ep * n_steps,
-                                                 None if eps_dev is None else eps_dev.data_ptr(),
+                                                 Xd.data_ptr(), None if Cd is None else Cd.data_ptr(), perm.data_ptr(),
+                                                 n, bs, self.lr, 0.9, 0.999, 1e-8, self.weight_decay,
+                                                 float(self.KL_weight), ep * n_steps,
+                                                 None if eps is None else eps.data_ptr(),
                                                  ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), losses[ep:].data_ptr(),
                                                  ws.data_ptr(), nbytes, stream), "rnvp_cv_fit_epoch")
-                if ep + 1 < self.n_epochs:
-                    # the next order is shuffled into the other host buffer while this epoch runs; that buffer's last
-                    # copy (two epochs ago) must have left it
-                    if copied[k ^ 1] is not None:
-                        copied[k ^ 1].synchronize()
-                    nxt = StreamingPermutation(lib, replay.get(ep + 1)[0], n, host=self._perm_host[(ep + 1) & 1])
-                host = log.push(losses[ep:ep + 1])
-                if bar is not None and host is not None:
-                    bar.set_description(f"loss: {float(host[-1]):.4f}")
-            log.flush()
-            final_state = replay.final_state()
-        finally:
-            replay.close()
-        self._publish_state(exp_avg, exp_avg_sq, self.n_epochs * n_steps)
+                return (losses[ep:ep + 1],)
+            final_state = run_epochs(self, lib, dev, n, replay, launch, [(self.loss_history, "loss")])
+        publish_state(self.opt, list(self.encoder.parameters()) + list(self.decoder.parameters()),
+                      self.n_epochs * n_steps, exp_avg=exp_avg, exp_avg_sq=exp_avg_sq)
         torch.set_rng_state(final_state)
         self.encoder.train(False)
         self.decoder.train(False)
         return self
-
-    def _publish_state(self, exp_avg, exp_avg_sq, steps):
-        """``opt.state`` as torch.optim.Adam leaves it: step, exp_avg, exp_avg_sq (views of the device moments)."""
-        self.opt.state.clear()
-        if steps <= 0:
-            return
-        off = 0
-        for p in list(self.encoder.parameters()) + list(self.decoder.parameters()):
-            numel = p.numel()
-            self.opt.state[p] = {"step": torch.tensor(float(steps)),
-                                 "exp_avg": exp_avg[off:off + numel].view(p.shape),
-                                 "exp_avg_sq": exp_avg_sq[off:off + numel].view(p.shape)}
-            off += numel
 
     def sample(self, C=10, seed=None, z=None):
         """Rows decoded for the conditions C [n, cond_size], or ``C`` rows without conditions if it is an int

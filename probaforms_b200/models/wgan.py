@@ -11,9 +11,9 @@ batches, fit step ``i`` (counted over the whole fit) is a generator step when ``
 otherwise, each net has the reference's RMSprop, the critic is clamped to [-0.01, 0.01] after its steps, and the global
 torch RNG is left exactly where the reference leaves it.  Every step draws ``torch.normal(0, 1, (nb, latent_dim))`` and
 every epoch ends with ``torch.normal(0, 1, (n, latent_dim))``; ``torch.normal(0, 1, size)`` gives the values and
-generator state of ``torch.randn(size)``, so the CVAE's helper-thread replay draws them (``noise='torch'``, the
-default) one epoch ahead of the GPU.  A whole epoch, its two epoch losses included, is one library call; a batch of up
-to 64 rows (the default ``batch_size`` is 32) is one kernel launch.
+generator state of ``torch.randn(size)``, so the CVAE's helper-thread replay (``_mlp.RngReplay``) draws them
+(``noise='torch'``, the default) one epoch ahead of the GPU.  A whole epoch, its two epoch losses included, is one
+library call; a batch of up to 64 rows (the default ``batch_size`` is 32) is one kernel launch.
 
 ``noise='device'`` draws the latent noise from Philox inside the kernels instead, keyed on the epoch's sampler seed
 and the row's position in the epoch; the helper thread then only skips the reference's normals in the generator state.
@@ -26,47 +26,27 @@ autograd).  CUDA only; there is no CPU fallback.
 """
 import ctypes as ct
 
-import numpy as np
 import torch
 import torch.nn as nn
 
+from ._mlp import Desc, FlatParams, RngReplay, _act_code, _layers, _rows, _stream, check_fit_inputs, publish_state, \
+    run_epochs
 from .interfaces import GenModel
-from .realnvp import _LossLog, _default_device
-from .cnormal import _stream
-from .cvae import _NoiseReplay, _Pair, _act_code, _layers, _rows
+from .realnvp import _default_device
 from .. import _lib
-from ..batching import StreamingPermutation, batch_bounds
+from ..batching import batch_bounds
 
 CLIP = 0.01                  # wgan.py:247-248: every critic parameter is clamped to [-0.01, 0.01] after its steps
 
 
-class _Desc:
-    """Owns one ``rnvp_wg_desc`` (shapes and activations of a generator-discriminator pair) on the current device."""
-
-    def __init__(self, D, Cd, latent, g_hidden, g_act, d_hidden, d_act):
-        self.lib = _lib.load()
-        gh = (ct.c_int * len(g_hidden))(*g_hidden)
-        dh = (ct.c_int * len(d_hidden))(*d_hidden)
-        h = ct.c_void_p()
-        rc = self.lib.rnvp_wg_desc_create(D, Cd, latent, len(g_hidden), gh, _act_code(g_act), len(d_hidden), dh,
-                                          _act_code(d_act), ct.byref(h))
-        if rc != 0:
-            msg = self.lib.rnvp_last_error().decode()
-            if rc in (-1, -2):                             # RNVP_EINVAL, RNVP_ESHAPE
-                raise ValueError(msg)
-            raise _lib.RnvpError(f"rnvp_wg_desc_create failed (code {rc}): {msg}")
-        self.h, self.D, self.Cd, self.L = h, D, Cd, latent
-        self.PG = int(self.lib.rnvp_wg_param_count(h, 0))
-        self.P = int(self.lib.rnvp_wg_param_count(h, 2))
-
-    def workspace(self, batch_rows, loss_rows, dev):
-        nbytes = int(self.lib.rnvp_wg_workspace_bytes(self.h, int(batch_rows), int(loss_rows)))
-        return torch.empty(max(nbytes, 4) // 4, dtype=torch.float32, device=dev), nbytes
-
-    def __del__(self):
-        if getattr(self, "h", None):
-            self.lib.rnvp_wg_desc_destroy(self.h)
-            self.h = None
+def _desc(D, Cd, latent, g_hidden, g_act, d_hidden, d_act):
+    """The ``rnvp_wg_desc`` of a generator-discriminator pair (shapes and activations) on the current CUDA device;
+    RNVP_EINVAL and RNVP_ESHAPE are ValueErrors.  ``PG`` counts the generator's parameters, ``P`` both nets'."""
+    desc = Desc("wg", (D, Cd, latent, len(g_hidden), (ct.c_int * len(g_hidden))(*g_hidden), _act_code(g_act),
+                       len(d_hidden), (ct.c_int * len(d_hidden))(*d_hidden), _act_code(d_act)), (-1, -2),
+                count_args=(2,), D=D, Cd=Cd, L=latent)
+    desc.PG = int(desc.lib.rnvp_wg_param_count(desc.h, 0))
+    return desc
 
 
 def _cond(C, dev, desc, n):
@@ -215,8 +195,8 @@ class ConditionalWGAN(GenModel):
 
     def _attach(self, D, Cd, dev):
         G, Dn = self.generator, self.discriminator
-        pair = _Pair(G, Dn, lambda: _Desc(D, Cd, G.n_inputs - Cd, G.hidden, G.activation, Dn.hidden, Dn.activation),
-                     dev)
+        pair = FlatParams([G, Dn], lambda: _desc(D, Cd, G.n_inputs - Cd, G.hidden, G.activation, Dn.hidden,
+                                                 Dn.activation), dev)
         G._pair = Dn._pair = pair
 
     def _ready(self):
@@ -261,21 +241,8 @@ class ConditionalWGAN(GenModel):
         RMSprop optimizers on every call, as upstream.  ``gen_loss_history`` / ``disc_loss_history`` get one 0-d CPU
         tensor per epoch: -mean(D(G(z, C), C)) and mean(D(X, C)) plus that, over all rows after the epoch's steps."""
         from ..ingest import upload_resident
-        if self.noise not in ("torch", "device"):
-            raise ValueError(f"noise must be 'torch' or 'device', got {self.noise!r}")
-        if not hasattr(X, "shape"):
-            X = np.asarray(X)
-        if len(tuple(X.shape)) != 2 or X.shape[0] < 1:
-            raise ValueError(f"X must be 2-D [n, var_size] with n >= 1, got shape {tuple(X.shape)}")
-        n = X.shape[0]
-        if C is not None:
-            if not hasattr(C, "shape"):
-                C = np.asarray(C)
-            if len(tuple(C.shape)) != 2 or C.shape[0] != n:
-                raise ValueError(f"C must be 2-D with {n} rows, got shape {tuple(C.shape)}")
-        bs, nc = int(self.batch_size), int(self.n_critic)
-        if bs < 1:
-            raise ValueError("batch_size must be >= 1")
+        X, C, n, bs = check_fit_inputs(X, C, self.batch_size, 1, self.noise)
+        nc = int(self.n_critic)
         if nc < 1:
             raise ValueError("n_critic must be >= 1")
         if self._device is None:
@@ -288,82 +255,34 @@ class ConditionalWGAN(GenModel):
         self.discriminator.train(True)
         self.disc_loss_history = []
         self.gen_loss_history = []
-        values = self.noise == "torch"
-        replay = _NoiseReplay(lib, n, bs, L, self.n_epochs, values)
-        try:
+        n_steps = len(batch_bounds(n, bs))
+        with RngReplay(lib, n, bs, L, self.n_epochs, epoch_end=True, values=self.noise == "torch") as replay:
             Xd = upload_resident(lib, X, dev)
             Cd = upload_resident(lib, C, dev) if desc.Cd else None
             square_avg = torch.zeros(desc.P, dtype=torch.float32, device=dev)
             ws, nbytes = desc.workspace(min(bs, n), n, dev)
-            perm_dev = [torch.empty(n, dtype=torch.int64, device=dev) for _ in range(2)]
-            eps_dev = torch.empty(2 * n * L, dtype=torch.float32, device=dev) if values else None
             losses = torch.empty(2, max(self.n_epochs, 1), dtype=torch.float32, device=dev)
-            copied = [None, None]
-            n_steps = len(batch_bounds(n, bs))
-            glog, dlog = _LossLog(self.gen_loss_history), _LossLog(self.disc_loss_history)
-            epochs = range(self.n_epochs)
-            bar = None
-            if self.verbose >= 1:
-                from tqdm.auto import tqdm
-                bar = tqdm(epochs, unit='epoch')
-                epochs = bar
             stream = _stream(dev)
-            nxt = None
-            if self.n_epochs > 0:
-                nxt = StreamingPermutation(lib, replay.get(0)[0], n, host=self._perm_host[0])
-            for ep in epochs:
-                seed, buf = replay.get(ep)
-                sp = nxt
-                self._perm_host[ep & 1] = sp.host
-                k = ep & 1
-                perm_dev[k].copy_(sp.full(), non_blocking=True)
-                if values:
-                    eps_dev.copy_(buf, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(torch.cuda.current_stream(dev))
-                copied[k] = ev
-                if values:
-                    replay.release(ep, ev)
+
+            def launch(ep, perm, eps, seed):
                 _lib.check(lib.rnvp_wg_fit_epoch(desc.h, flat.data_ptr(), square_avg.data_ptr(), Xd.data_ptr(),
-                                                 None if Cd is None else Cd.data_ptr(), perm_dev[k].data_ptr(), n, bs,
-                                                 nc, ep * n_steps, self.lr, 0.99, 1e-8, self.weight_decay, CLIP,
-                                                 None if eps_dev is None else eps_dev.data_ptr(),
+                                                 None if Cd is None else Cd.data_ptr(), perm.data_ptr(), n, bs, nc,
+                                                 ep * n_steps, self.lr, 0.99, 1e-8, self.weight_decay, CLIP,
+                                                 None if eps is None else eps.data_ptr(),
                                                  ct.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), losses[0, ep:].data_ptr(),
                                                  losses[1, ep:].data_ptr(), ws.data_ptr(), nbytes, stream),
                            "rnvp_wg_fit_epoch")
-                if ep + 1 < self.n_epochs:
-                    # the next order is shuffled into the other host buffer while this epoch runs; that buffer's last
-                    # copy (two epochs ago) must have left it
-                    if copied[k ^ 1] is not None:
-                        copied[k ^ 1].synchronize()
-                    nxt = StreamingPermutation(lib, replay.get(ep + 1)[0], n, host=self._perm_host[(ep + 1) & 1])
-                gh, dh = glog.push(losses[0, ep:ep + 1]), dlog.push(losses[1, ep:ep + 1])
-                if bar is not None and gh is not None:
-                    bar.set_description(f"G loss: {float(gh[-1]):.4f}, D loss: {float(dh[-1]):.4f}")
-            glog.flush()
-            dlog.flush()
-            final_state = replay.final_state()
-        finally:
-            replay.close()
-        self._publish_state(square_avg, *step_counts(n, bs, nc, self.n_epochs))
+                return losses[0, ep:ep + 1], losses[1, ep:ep + 1]
+            final_state = run_epochs(self, lib, dev, n, replay, launch,
+                                     [(self.gen_loss_history, "G loss"), (self.disc_loss_history, "D loss")])
+        # RMSprop state (step, square_avg) for every parameter of a net that took a step
+        gen_steps, disc_steps = step_counts(n, bs, nc, self.n_epochs)
+        off = publish_state(self.opt_gen, self.generator.parameters(), gen_steps, square_avg=square_avg)
+        publish_state(self.opt_disc, self.discriminator.parameters(), disc_steps, off, square_avg=square_avg)
         torch.set_rng_state(final_state)
         self.generator.train(False)
         self.discriminator.train(False)
         return self
-
-    def _publish_state(self, square_avg, gen_steps, disc_steps):
-        """``opt_gen.state`` / ``opt_disc.state`` as torch.optim.RMSprop leaves them: step and square_avg (views of the
-        device state) for every parameter of a net that took a step."""
-        off = 0
-        for opt, net, steps in ((self.opt_gen, self.generator, gen_steps),
-                                (self.opt_disc, self.discriminator, disc_steps)):
-            opt.state.clear()
-            for p in net.parameters():
-                numel = p.numel()
-                if steps > 0:
-                    opt.state[p] = {"step": torch.tensor(float(steps)),
-                                    "square_avg": square_avg[off:off + numel].view(p.shape)}
-                off += numel
 
     def sample(self, C=10, seed=None, z=None):
         """Rows generated for the conditions C [n, cond_size], or ``C`` rows without conditions if it is an int

@@ -138,6 +138,19 @@ def test_descriptor_rejects_bad_shapes_without_device():
     assert L.rnvp_cn_desc_create(2, 1, 1, (C.c_int * 1)(0), 1, 0, C.byref(h)) == -1
 
 
+def test_descriptor_create_errors_keep_their_types():
+    """A failed create is a ValueError only for a shape limit (RNVP_ESHAPE) in ConditionalNormal, for RNVP_EINVAL too
+    in CVAE; every other code is RnvpError.  No CUDA call is made."""
+    from probaforms_b200._lib import RnvpError
+    from probaforms_b200.models import cnormal, cvae
+    with pytest.raises(ValueError, match="128"):
+        cnormal._desc(129, 1, (10,), "tanh", False)
+    with pytest.raises(RnvpError):
+        cnormal._desc(2, 1, (0,), "tanh", False)                  # a hidden width of 0: RNVP_EINVAL
+    with pytest.raises(ValueError):
+        cvae._desc(2, 1, 2, (0,), "tanh")
+
+
 def test_fit_without_cuda_raises():
     if torch.cuda.is_available():
         pytest.skip("a CUDA device is visible")

@@ -46,7 +46,7 @@ def flops_per_row(D, Cd, hidden, full):
 def rng_advance(out):
     """Host cost of skipping the normals of fit's RNG replay (rnvp_cn_rng_advance) against generating them."""
     from probaforms_b200 import _lib
-    from probaforms_b200.models.cnormal import advance
+    from probaforms_b200.models._mlp import advance
     lib, words, reps = _lib.load(), 65536 * 32, 20
     g = torch.Generator().manual_seed(0)
     t = time.perf_counter()
