@@ -5,8 +5,8 @@
 // A CTA owns a tile of up to R rows of a step's batch and keeps every activation of the tile in shared memory (row-major
 // with an odd row stride, so that both the row-parallel and the column-parallel loops below are free of bank
 // conflicts).  The fit sweep runs forward, loss and backward over its tile and writes per-CTA partial sums of every
-// weight gradient (plus the loss); cn_reduce_kernel adds the partials of all CTAs in CTA order and cn_tail applies what
-// only the whole batch can: dW_out = -M G_M^T M, db_out = -M sum g_z, Adam, the loss hand-off, and in full mode the
+// weight gradient (plus the loss); mlp_reduce_kernel adds the partials of all CTAs in CTA order and cn_tail applies
+// what only the whole batch can: dW_out = -M G_M^T M, db_out = -M sum g_z, Adam, the loss hand-off, and in full mode the
 // Gauss-Jordan inverse for the next step.  A batch of at most R rows is one launch (cn_step_kernel).
 //
 // A zero pivot in the inverse writes the index (+1) of the first step that cannot run to *status; every later kernel
@@ -23,30 +23,21 @@
 #include "rnvp_mlp.cuh"
 #include "rnvp_philox.cuh"
 
-int rnvp_fail(int code, const char* msg);   // rnvp_api.cu: sets rnvp_last_error()
-
 namespace {
-
-constexpr int CN_MAX_D = 128, CN_MAX_CD = 256, CN_MAX_HIDDEN = 4, CN_MAX_WIDTH = 512;
-constexpr int CN_MAX_ROWS = 64;                       // rows per CTA tile
-constexpr int CN_SMEM_BUDGET = 96 * 1024;             // per sweep CTA: two CTAs of 256 threads per SM
-constexpr int CN_THREADS = 256, CN_TAIL_THREADS = 512;
 
 struct CnShape {
   int D, Cd, nh, act, indep, R;
-  int h[CN_MAX_HIDDEN];
-  int w[CN_MAX_HIDDEN], b[CN_MAX_HIDDEN];             // float offsets of model.model.{2k}.weight / .bias
+  int h[MLP_MAX_HIDDEN];
+  int w[MLP_MAX_HIDDEN], b[MLP_MAX_HIDDEN];           // float offsets of model.model.{2k}.weight / .bias
   int mu_w, mu_b, ls_w, ls_b, out_w, out_b, P;
   int stride;                                         // floats of one CTA's partial record (P gradients + loss)
   int sweep_smem, tail_smem;
 };
 
-__host__ __device__ inline int odd_ld(int n) { return n | 1; }
-
 // shared-memory layout of one tile: C | H_0 .. H_{nh-1} | MU | LS | Z | XB, each [R][odd stride]
 struct CnTile {
-  float *c, *h[CN_MAX_HIDDEN], *mu, *ls, *z, *xb;
-  int ldc, ldh[CN_MAX_HIDDEN], ldd;
+  float *c, *h[MLP_MAX_HIDDEN], *mu, *ls, *z, *xb;
+  int ldc, ldh[MLP_MAX_HIDDEN], ldd;
 };
 
 __host__ __device__ inline int tile_floats(const CnShape& s, int R) {
@@ -61,7 +52,7 @@ __device__ __forceinline__ CnTile carve(const CnShape& s, float* sm) {
   t.ldc = odd_ld(s.Cd);
   t.c = sm; sm += R * t.ldc;
 #pragma unroll
-  for (int k = 0; k < CN_MAX_HIDDEN; ++k) {
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {
     t.ldh[k] = k < s.nh ? odd_ld(s.h[k]) : 0;
     t.h[k] = sm;
     sm += R * t.ldh[k];
@@ -99,7 +90,7 @@ __device__ __forceinline__ void forward_tile(const CnShape& s, const CnTile& t, 
   const float* in = t.c;
   int ldi = t.ldc, ni = s.Cd;
 #pragma unroll
-  for (int k = 0; k < CN_MAX_HIDDEN; ++k) {           // unrolled: the per-layer arrays are indexed statically
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {          // unrolled: the per-layer arrays are indexed statically
     if (k >= s.nh) break;
     dense_rows(in, ldi, ni, params + s.w[k], params + s.b[k], t.h[k], t.ldh[k], s.h[k], nr, s.act);
     __syncthreads();
@@ -153,7 +144,7 @@ __device__ __forceinline__ void sweep_tile(const CnShape& s, float* sm, const fl
   int hl = 0, ldl = 0;
   float* Hl = nullptr;
 #pragma unroll
-  for (int k = 0; k < CN_MAX_HIDDEN; ++k)
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k)
     if (k == s.nh - 1) { hl = s.h[k]; Hl = t.h[k]; ldl = t.ldh[k]; }
   wgrad(t.mu, t.ldd, D, Hl, ldl, hl, nr, g + s.mu_w, g + s.mu_b);
   wgrad(t.ls, t.ldd, D, Hl, ldl, hl, nr, g + s.ls_w, g + s.ls_b);
@@ -176,7 +167,7 @@ __device__ __forceinline__ void sweep_tile(const CnShape& s, float* sm, const fl
   }
   __syncthreads();
 #pragma unroll
-  for (int k = CN_MAX_HIDDEN - 1; k >= 0; --k) {
+  for (int k = MLP_MAX_HIDDEN - 1; k >= 0; --k) {
     if (k >= s.nh) continue;
     const float* in = k ? t.h[k - 1] : t.c;
     const int ldi = k ? t.ldh[k - 1] : t.ldc, ni = k ? s.h[k - 1] : s.Cd;
@@ -292,7 +283,7 @@ __device__ __forceinline__ void cn_tail(const CnShape& s, float* sm, float* __re
   if (!invert_out(s, params, M, sm) && threadIdx.x == 0) *status = (int)(st.step + 2);   // step+1 cannot run
 }
 
-__global__ void __launch_bounds__(CN_THREADS) cn_sweep_kernel(CnShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) cn_sweep_kernel(CnShape s, const float* __restrict__ params,
     const float* __restrict__ M, const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx,
     int64_t nb, float inv_bd, float* __restrict__ partials, const int* status) {
   if (status && *status) return;
@@ -302,28 +293,18 @@ __global__ void __launch_bounds__(CN_THREADS) cn_sweep_kernel(CnShape s, const f
   sweep_tile(s, smem, params, M, X, C, idx, row0, nr, inv_bd, partials + (size_t)blockIdx.x * s.stride);
 }
 
-__global__ void cn_reduce_kernel(const float* __restrict__ partials, int n_ctas, int stride, int P, int indep_from,
-                                 float* __restrict__ g, const int* status) {
-  if (status && *status) return;
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c > P || (c >= indep_from && c < P)) return;
-  float acc = 0.0f;
-  for (int b = 0; b < n_ctas; ++b) acc += partials[(size_t)b * stride + c];
-  g[c] = acc;
-}
-
-__global__ void __launch_bounds__(CN_TAIL_THREADS) cn_tail_kernel(CnShape s, float* params, float* m, float* v, float* M,
-                                                                 float* g, float* gflat, float* loss_dst, int* status,
-                                                                 CnStep st) {
+__global__ void __launch_bounds__(MLP_TAIL_THREADS) cn_tail_kernel(CnShape s, float* params, float* m, float* v,
+                                                                  float* M, float* g, float* gflat, float* loss_dst,
+                                                                  int* status, CnStep st) {
   if (status && *status) return;
   extern __shared__ __align__(16) float smem[];
   cn_tail(s, smem, params, m, v, M, g, gflat, loss_dst, status, st);
 }
 
 // a whole step of a batch that fits one tile
-__global__ void __launch_bounds__(CN_TAIL_THREADS) cn_step_kernel(CnShape s, float* params, float* m, float* v, float* M,
-    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int nb, float* g,
-    float* gflat, float* loss_dst, int* status, CnStep st) {
+__global__ void __launch_bounds__(MLP_TAIL_THREADS) cn_step_kernel(CnShape s, float* params, float* m, float* v,
+    float* M, const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int nb,
+    float* g, float* gflat, float* loss_dst, int* status, CnStep st) {
   if (status && *status) return;
   extern __shared__ __align__(16) float smem[];
   sweep_tile(s, smem, params, M, X, C, idx, 0, nb, st.inv_bd, g);
@@ -338,7 +319,7 @@ __global__ void cn_inverse_kernel(CnShape s, const float* params, float* M, int*
 
 // Net.forward for inference: mu, sigma, x_tilde (noise from Philox keyed on (seed, row_offset + row, j), or eps),
 // inv = (X - b_out) M; every output may be NULL
-__global__ void __launch_bounds__(CN_THREADS) cn_forward_kernel(CnShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) cn_forward_kernel(CnShape s, const float* __restrict__ params,
     const float* __restrict__ M, const float* __restrict__ X, const float* __restrict__ C, int64_t N,
     unsigned long long seed, long long row_offset, const float* __restrict__ eps, float* mu_o, float* sigma_o,
     float* xt_o, float* inv_o) {
@@ -382,7 +363,7 @@ __global__ void __launch_bounds__(CN_THREADS) cn_forward_kernel(CnShape s, const
 // M64[j][c]; *status = 1 on an exact-zero pivot.
 __global__ void cn_logdet_kernel(CnShape s, const float* __restrict__ params, double* ws, int* status) {
   extern __shared__ __align__(16) double smd[];
-  __shared__ int piv, perm[CN_MAX_D];
+  __shared__ int piv, perm[MLP_MAX_D];
   __shared__ double pval;
   const int D = s.D;
   double* A = smd;
@@ -455,7 +436,7 @@ __global__ void cn_logdet_kernel(CnShape s, const float* __restrict__ params, do
 // exact log-density of X given C: the fp32 net of cn_forward_kernel (mu and log_sigma with the same bits), then one
 // warp per row in fp64: u = (x - b_out) M64 (u = x in independent mode), sum_d ((u_d - mu_d) / sigma_d)^2 and sum_d
 // log_sigma_d lane-strided and summed by a fixed shuffle tree
-__global__ void __launch_bounds__(CN_THREADS) cn_log_prob_kernel(CnShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) cn_log_prob_kernel(CnShape s, const float* __restrict__ params,
     const double* __restrict__ ws, const float* __restrict__ X, const float* __restrict__ C, int64_t N,
     double* __restrict__ logp, const int* status) {
   if (status && *status) return;
@@ -469,7 +450,7 @@ __global__ void __launch_bounds__(CN_THREADS) cn_log_prob_kernel(CnShape s, cons
   forward_tile(s, t, params, nullptr, false, nr);
   const int D = s.D, lane = threadIdx.x & 31;
   const double* M = ws + 1;
-  for (int r = threadIdx.x >> 5; r < nr; r += CN_THREADS / 32) {
+  for (int r = threadIdx.x >> 5; r < nr; r += MLP_THREADS / 32) {
     const float* x = t.z + r * t.ldd;
     double q = 0.0, ls = 0.0;
     for (int c = lane; c < D; c += 32) {
@@ -497,37 +478,33 @@ __global__ void __launch_bounds__(CN_THREADS) cn_log_prob_kernel(CnShape s, cons
   }
 }
 
-int64_t n_tiles(const CnShape& s, int64_t n) { return (n + s.R - 1) / s.R; }
-
 }  // namespace
 
 struct rnvp_cn_desc {
   CnShape s;
-  int max_smem;
 };
 
 namespace {
 
 int check_cn(const rnvp_cn_desc* d) { return d ? 0 : rnvp_fail(RNVP_EINVAL, "null ConditionalNormal descriptor"); }
 
-cudaError_t launch_step(const rnvp_cn_desc* d, float* params, float* m, float* v, float* M, const float* X,
-                        const float* C, const int64_t* idx, int64_t nb, float* gflat, float* loss_dst, int* status,
-                        const CnStep& st, float* ws, cudaStream_t stream) {
+void launch_step(const rnvp_cn_desc* d, float* params, float* m, float* v, float* M, const float* X,
+                 const float* C, const int64_t* idx, int64_t nb, float* gflat, float* loss_dst, int* status,
+                 const CnStep& st, float* ws, cudaStream_t stream) {
   const CnShape& s = d->s;
-  const int64_t nt = n_tiles(s, nb);
+  const int64_t nt = n_tiles(s.R, nb);
   float* g = ws;                                       // reduced gradient + loss (stride floats), then the partials
   if (nt == 1) {
-    cn_step_kernel<<<1, CN_TAIL_THREADS, std::max(s.sweep_smem, s.tail_smem), stream>>>(
+    cn_step_kernel<<<1, MLP_TAIL_THREADS, std::max(s.sweep_smem, s.tail_smem), stream>>>(
         s, params, m, v, M, X, C, idx, (int)nb, g, gflat, loss_dst, status, st);
-    return cudaGetLastError();
+    return;
   }
   float* partials = ws + s.stride;
-  cn_sweep_kernel<<<(unsigned)nt, CN_THREADS, s.sweep_smem, stream>>>(s, params, M, X, C, idx, nb, st.inv_bd, partials,
-                                                                     status);
-  const int indep_from = s.indep ? s.out_w : s.P;
-  cn_reduce_kernel<<<(s.P + 1 + 255) / 256, 256, 0, stream>>>(partials, (int)nt, s.stride, s.P, indep_from, g, status);
-  cn_tail_kernel<<<1, CN_TAIL_THREADS, s.tail_smem, stream>>>(s, params, m, v, M, g, gflat, loss_dst, status, st);
-  return cudaGetLastError();
+  cn_sweep_kernel<<<(unsigned)nt, MLP_THREADS, s.sweep_smem, stream>>>(s, params, M, X, C, idx, nb, st.inv_bd,
+                                                                      partials, status);
+  // the gradients and the loss; in independent mode the out slots (last) have no gradient
+  launch_reduce(partials, (int)nt, s.stride, s.P, 0, s.indep ? s.out_w : s.P, 1, g, status, stream);
+  cn_tail_kernel<<<1, MLP_TAIL_THREADS, s.tail_smem, stream>>>(s, params, m, v, M, g, gflat, loss_dst, status, st);
 }
 
 }  // namespace
@@ -540,60 +517,29 @@ int rnvp_cn_desc_create(int D, int Cd, int n_hidden, const int* hidden, int act,
   if (!hidden || D < 1 || Cd < 1 || n_hidden < 1) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_desc_create: bad shape");
   if (act != RNVP_ACT_TANH && act != RNVP_ACT_RELU && act != RNVP_ACT_SIGMOID)
     return rnvp_fail(RNVP_EINVAL, "rnvp_cn_desc_create: act must be RNVP_ACT_TANH, _RELU or _SIGMOID");
-  if (D > CN_MAX_D) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: var_size D must be <= 128");
-  if (Cd > CN_MAX_CD) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: cond_size must be <= 256");
-  if (n_hidden > CN_MAX_HIDDEN) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: at most 4 hidden layers");
+  if (D > MLP_MAX_D) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: var_size D must be <= 128");
+  if (Cd > MLP_MAX_CD) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: cond_size must be <= 256");
+  if (n_hidden > MLP_MAX_HIDDEN) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: at most 4 hidden layers");
   CnShape s{};
   s.D = D; s.Cd = Cd; s.nh = n_hidden; s.act = act; s.indep = independent ? 1 : 0;
   int64_t off = 0;
-  int prev = Cd;
-  for (int k = 0; k < n_hidden; ++k) {
-    if (hidden[k] < 1) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_desc_create: hidden widths must be >= 1");
-    if (hidden[k] > CN_MAX_WIDTH) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: hidden widths must be <= 512");
-    s.h[k] = hidden[k];
-    s.w[k] = (int)off; off += (int64_t)hidden[k] * prev;
-    s.b[k] = (int)off; off += hidden[k];
-    prev = hidden[k];
-  }
-  s.mu_w = (int)off; off += (int64_t)D * prev;
-  s.mu_b = (int)off; off += D;
-  s.ls_w = (int)off; off += (int64_t)D * prev;
-  s.ls_b = (int)off; off += D;
-  s.out_w = (int)off; off += (int64_t)D * D;
-  s.out_b = (int)off; off += D;
+  if (int rc = hidden_layout(n_hidden, hidden, Cd, s.h, s.w, s.b, off, "ConditionalNormal", "rnvp_cn_desc_create"))
+    return rc;
+  const int hl = hidden[n_hidden - 1];
+  linear_layout(s.mu_w, s.mu_b, hl, D, off);
+  linear_layout(s.ls_w, s.ls_b, hl, D, off);
+  linear_layout(s.out_w, s.out_b, D, D, off);
   s.P = (int)off;
   s.stride = (s.P + 1 + 3) & ~3;
-  int R = CN_MAX_ROWS;
-  while (R > 1 && tile_floats(s, R) * 4 > CN_SMEM_BUDGET) R >>= 1;
-  s.R = R;
-  s.sweep_smem = tile_floats(s, R) * 4;
+  s.R = rows_per_tile(s);
+  s.sweep_smem = tile_floats(s, s.R) * 4;
   s.tail_smem = (2 * D * D + D) * 4;
-  int dev = 0, max_optin = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  if (e != cudaSuccess) return rnvp_fail(RNVP_ENODEVICE, "rnvp_cn_desc_create: no CUDA device");
-  const int need = std::max(s.sweep_smem, s.tail_smem);
-  if (need > max_optin) return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: shape exceeds the shared memory of one CTA");
-  // The limit is a property of the kernel on this device, shared by every descriptor: set it to the device's opt-in
-  // maximum less its static shared memory (idempotent), never to this shape's need, which would lower it under a
-  // larger model created earlier.
-  const void* kernels[] = {(const void*)cn_sweep_kernel, (const void*)cn_tail_kernel, (const void*)cn_step_kernel,
-                           (const void*)cn_inverse_kernel, (const void*)cn_forward_kernel,
-                           (const void*)cn_log_prob_kernel};
-  for (const void* k : kernels) {
-    cudaFuncAttributes fa;
-    e = cudaFuncGetAttributes(&fa, k);
-    const int dyn_max = max_optin - (int)fa.sharedSizeBytes;          // opt-in limit less the static shared memory
-    if (e == cudaSuccess && need > dyn_max)
-      return rnvp_fail(RNVP_ESHAPE, "ConditionalNormal: shape exceeds the shared memory of one CTA");
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_max);
-    if (e != cudaSuccess) {
-      cudaGetLastError();                                             // do not leave the error for the caller's next call
-      return rnvp_fail((int)e, "rnvp_cn_desc_create: cudaFuncSetAttribute");
-    }
-  }
-  rnvp_cn_desc* d = new rnvp_cn_desc{s, need};
-  *out = d;
+  if (int rc = opt_in_smem({(const void*)cn_sweep_kernel, (const void*)cn_tail_kernel, (const void*)cn_step_kernel,
+                            (const void*)cn_inverse_kernel, (const void*)cn_forward_kernel,
+                            (const void*)cn_log_prob_kernel},
+                           std::max(s.sweep_smem, s.tail_smem), "ConditionalNormal", "rnvp_cn_desc_create"))
+    return rc;
+  *out = new rnvp_cn_desc{s};
   return 0;
 }
 
@@ -603,16 +549,15 @@ int64_t rnvp_cn_param_count(const rnvp_cn_desc* d) { return d ? d->s.P : -1; }
 
 int64_t rnvp_cn_workspace_bytes(const rnvp_cn_desc* d, int64_t N) {
   if (!d || N < 0) return -1;
-  const int64_t nt = n_tiles(d->s, N);
+  const int64_t nt = n_tiles(d->s.R, N);
   return 4 * (int64_t)d->s.stride * (1 + (nt > 1 ? nt : 0));
 }
 
 int rnvp_cn_inverse(const rnvp_cn_desc* d, const float* d_params, float* d_M, int* d_status, void* stream) {
   if (check_cn(d)) return RNVP_EINVAL;
   if (!d_params || !d_M || !d_status) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_inverse: null buffer");
-  cn_inverse_kernel<<<1, CN_TAIL_THREADS, d->s.tail_smem, (cudaStream_t)stream>>>(d->s, d_params, d_M, d_status);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cn_inverse_kernel launch");
+  cn_inverse_kernel<<<1, MLP_TAIL_THREADS, d->s.tail_smem, (cudaStream_t)stream>>>(d->s, d_params, d_M, d_status);
+  return launched("cn_inverse_kernel launch");
 }
 
 int rnvp_cn_forward(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,
@@ -622,12 +567,10 @@ int rnvp_cn_forward(const rnvp_cn_desc* d, const float* d_params, const float* d
   if (!d_params || !d_C || N < 0 || (d_inv && (!d_X || !d_M)))
     return rnvp_fail(RNVP_EINVAL, "rnvp_cn_forward: bad argument");
   if (N == 0) return 0;
-  const int64_t nt = n_tiles(d->s, N);
-  if (nt > 0x7fffffffLL) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_forward: too many rows");
-  cn_forward_kernel<<<(unsigned)nt, CN_THREADS, d->s.sweep_smem, (cudaStream_t)stream>>>(
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_forward: too many rows");
+  cn_forward_kernel<<<(unsigned)n_tiles(d->s.R, N), MLP_THREADS, d->s.sweep_smem, (cudaStream_t)stream>>>(
       d->s, d_params, d_M, d_X, d_C, N, seed, row_offset, d_eps, d_mu, d_sigma, d_xtilde, d_inv);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cn_forward_kernel launch");
+  return launched("cn_forward_kernel launch");
 }
 
 int rnvp_cn_log_prob(const rnvp_cn_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
@@ -636,23 +579,19 @@ int rnvp_cn_log_prob(const rnvp_cn_desc* d, const float* d_params, const float* 
   const bool full = !d->s.indep;
   if (!d_params || !d_X || !d_C || !d_logp || N < 0 || (full && (!d_workspace || !d_status)))
     return rnvp_fail(RNVP_EINVAL, "rnvp_cn_log_prob: bad argument");
-  const int64_t nt = n_tiles(d->s, N);
-  if (nt > 0x7fffffffLL) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_log_prob: too many rows");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_log_prob: too many rows");
   cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t e;
   if (full) {
     const int smem = d->s.D * d->s.D * (int)sizeof(double);
-    e = cudaFuncSetAttribute(cn_logdet_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    const cudaError_t e = cudaFuncSetAttribute(cn_logdet_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return rnvp_fail((int)e, "rnvp_cn_log_prob: cudaFuncSetAttribute");
-    cn_logdet_kernel<<<1, CN_TAIL_THREADS, smem, st>>>(d->s, d_params, d_workspace, d_status);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return rnvp_fail((int)e, "cn_logdet_kernel launch");
+    cn_logdet_kernel<<<1, MLP_TAIL_THREADS, smem, st>>>(d->s, d_params, d_workspace, d_status);
+    if (int rc = launched("cn_logdet_kernel launch")) return rc;
   }
   if (N == 0) return 0;
-  cn_log_prob_kernel<<<(unsigned)nt, CN_THREADS, d->s.sweep_smem, st>>>(
+  cn_log_prob_kernel<<<(unsigned)n_tiles(d->s.R, N), MLP_THREADS, d->s.sweep_smem, st>>>(
       d->s, d_params, full ? d_workspace : nullptr, d_X, d_C, N, d_logp, full ? d_status : nullptr);
-  e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cn_log_prob_kernel launch");
+  return launched("cn_log_prob_kernel launch");
 }
 
 int rnvp_cn_grad(const rnvp_cn_desc* d, const float* d_params, const float* d_M, const float* d_X, const float* d_C,
@@ -663,13 +602,13 @@ int rnvp_cn_grad(const rnvp_cn_desc* d, const float* d_params, const float* d_M,
     return rnvp_fail(RNVP_EINVAL, "rnvp_cn_grad: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_cn_workspace_bytes(d, N))
     return rnvp_fail(RNVP_EINVAL, "rnvp_cn_grad: workspace smaller than rnvp_cn_workspace_bytes(N)");
-  if (n_tiles(d->s, N) > 0x7fffffffLL) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_grad: too many rows");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cn_grad: too many rows");
   CnStep st{};
   st.inv_bd = (float)(1.0 / ((double)N * d->s.D));
   st.adam = 0;
-  const cudaError_t e = launch_step(d, const_cast<float*>(d_params), nullptr, nullptr, const_cast<float*>(d_M), d_X, d_C,
-                                    d_idx, N, d_gflat, d_loss, nullptr, st, (float*)d_workspace, (cudaStream_t)stream);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "ConditionalNormal gradient launch");
+  launch_step(d, const_cast<float*>(d_params), nullptr, nullptr, const_cast<float*>(d_M), d_X, d_C, d_idx, N, d_gflat,
+              d_loss, nullptr, st, (float*)d_workspace, (cudaStream_t)stream);
+  return launched("ConditionalNormal gradient launch");
 }
 
 int rnvp_cn_fit_epoch(const rnvp_cn_desc* d, float* d_params, float* d_exp_avg, float* d_exp_avg_sq, float* d_M,
@@ -690,9 +629,9 @@ int rnvp_cn_fit_epoch(const rnvp_cn_desc* d, float* d_params, float* d_exp_avg, 
     st.inv_bd = (float)(1.0 / ((double)nb * d->s.D));
     st.adam = 1;
     st.step = step0 + s;
-    const cudaError_t e = launch_step(d, d_params, d_exp_avg, d_exp_avg_sq, d_M, d_X, d_C, d_perm + b0, nb, nullptr,
-                                      d_losses + s, d_status, st, (float*)d_workspace, (cudaStream_t)stream);
-    if (e != cudaSuccess) return rnvp_fail((int)e, "ConditionalNormal fit step launch");
+    launch_step(d, d_params, d_exp_avg, d_exp_avg_sq, d_M, d_X, d_C, d_perm + b0, nb, nullptr, d_losses + s, d_status,
+                st, (float*)d_workspace, (cudaStream_t)stream);
+    if (int rc = launched("ConditionalNormal fit step launch")) return rc;
   }
   return 0;
 }

@@ -7,7 +7,7 @@
 // [z|c], the decoder's hidden layers and x_rec.  The fit sweep runs the encoder, the reparameterisation, the decoder,
 // the loss, the decoder's backward pass down to dz (no gradient for the c columns, no activation derivative on the
 // linear input), dmu / dls, and the encoder's backward pass, and writes per-CTA partial sums of every weight gradient
-// plus the loss.  cv_reduce_kernel adds the partials in CTA order and cv_tail_kernel runs Adam, so repeated fits are
+// plus the loss.  mlp_reduce_kernel adds the partials in CTA order and cv_tail_kernel runs Adam, so repeated fits are
 // bitwise identical.  A batch of at most R rows is one launch (cv_step_kernel).  The same sweep without the backward
 // pass gives the loss alone (per-CTA partials, then cv_loss_reduce_kernel in a fixed order).
 //
@@ -21,35 +21,25 @@
 #include "../../include/rnvp.h"
 #include "rnvp_adam.cuh"
 #include "rnvp_mlp.cuh"
-#include "rnvp_philox.cuh"
-
-int rnvp_fail(int code, const char* msg);   // rnvp_api.cu: sets rnvp_last_error()
 
 namespace {
 
-constexpr int CV_MAX_D = 128, CV_MAX_CD = 256, CV_MAX_LAT = 128, CV_MAX_HIDDEN = 4, CV_MAX_WIDTH = 512;
-constexpr int CV_MAX_ROWS = 64;                       // rows per CTA tile
-constexpr int CV_SMEM_BUDGET = 96 * 1024;             // per sweep CTA: two CTAs of 256 threads per SM
-constexpr int CV_THREADS = 256, CV_TAIL_THREADS = 512;
-
 struct CvShape {
   int D, Cd, L, nh, act, R;
-  int h[CV_MAX_HIDDEN];
-  int ew[CV_MAX_HIDDEN], eb[CV_MAX_HIDDEN];           // float offsets of encoder.model.{2k}.weight / .bias
+  int h[MLP_MAX_HIDDEN];
+  int ew[MLP_MAX_HIDDEN], eb[MLP_MAX_HIDDEN];         // float offsets of encoder.model.{2k}.weight / .bias
   int mu_w, mu_b, ls_w, ls_b;                         // encoder.mu, encoder.log_sigma
-  int dw[CV_MAX_HIDDEN], db[CV_MAX_HIDDEN];           // decoder.model.{2k}.weight / .bias
+  int dw[MLP_MAX_HIDDEN], db[MLP_MAX_HIDDEN];         // decoder.model.{2k}.weight / .bias
   int out_w, out_b, P;                                // decoder.model.{2 nh}
   int stride;                                         // floats of one CTA's partial record (P gradients + loss)
   int smem;
 };
 
-__host__ __device__ inline int odd_ld(int n) { return n | 1; }
-
 // shared-memory layout of one tile: XC | EH_0 .. EH_{nh-1} | MU | LS | EP | ZC | DH_0 .. DH_{nh-1} | XR, each
 // [R][odd stride]; EP holds exp(ls / 2) eps once the latent is drawn
 struct CvTile {
-  float *xc, *eh[CV_MAX_HIDDEN], *mu, *ls, *ep, *zc, *dh[CV_MAX_HIDDEN], *xr;
-  int ldxc, ldh[CV_MAX_HIDDEN], ldl, ldz, ldx;
+  float *xc, *eh[MLP_MAX_HIDDEN], *mu, *ls, *ep, *zc, *dh[MLP_MAX_HIDDEN], *xr;
+  int ldxc, ldh[MLP_MAX_HIDDEN], ldl, ldz, ldx;
 };
 
 __host__ __device__ inline int tile_floats(const CvShape& s, int R) {
@@ -64,7 +54,7 @@ __device__ __forceinline__ CvTile carve(const CvShape& s, float* sm) {
   t.ldxc = odd_ld(s.D + s.Cd);
   t.xc = sm; sm += R * t.ldxc;
 #pragma unroll
-  for (int k = 0; k < CV_MAX_HIDDEN; ++k) {
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {
     t.ldh[k] = k < s.nh ? odd_ld(s.h[k]) : 0;
     t.eh[k] = sm;
     sm += R * t.ldh[k];
@@ -76,24 +66,13 @@ __device__ __forceinline__ CvTile carve(const CvShape& s, float* sm) {
   t.ldz = odd_ld(s.L + s.Cd);
   t.zc = sm; sm += R * t.ldz;
 #pragma unroll
-  for (int k = 0; k < CV_MAX_HIDDEN; ++k) {
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {
     t.dh[k] = sm;
     sm += R * t.ldh[k];
   }
   t.ldx = odd_ld(s.D);
   t.xr = sm;
   return t;
-}
-
-// eps of batch position p, latent j: eps[p * L + j] if given, else Philox(seed, row0 + p, j)
-struct CvNoise {
-  const float* eps;
-  unsigned long long seed;
-  long long row0;
-};
-
-__device__ __forceinline__ float noise_at(const CvNoise& nz, int L, int64_t p, int j) {
-  return nz.eps ? nz.eps[p * L + j] : rnvp_rng::normal1(nz.seed, nz.row0 + p, j);
 }
 
 // [x|c] rows X[idx[r]], C[idx[r]] into XC (and c into the tail of ZC)
@@ -119,7 +98,7 @@ __device__ __forceinline__ void load_xc(const CvShape& s, const CvTile& t, const
 // *loss_dst and, with g, its gradient partials to g[0..P)
 __device__ __forceinline__ void sweep_tile(const CvShape& s, float* sm, const float* __restrict__ params,
                                            const float* __restrict__ X, const float* __restrict__ C,
-                                           const int64_t* __restrict__ idx, int64_t row0, int nr, const CvNoise& nz,
+                                           const int64_t* __restrict__ idx, int64_t row0, int nr, const MlpNoise& nz,
                                            float inv_bd, float kl_b, float* __restrict__ g, float* loss_dst) {
   const CvTile t = carve(s, sm);
   float* scratch = t.xr + s.R * t.ldx;                 // the 64 floats after the tile (tile_floats)
@@ -161,14 +140,14 @@ __device__ __forceinline__ void sweep_tile(const CvShape& s, float* sm, const fl
   int hl = 0, ldl = 0;
   float *DHl = nullptr, *EHl = nullptr;
 #pragma unroll
-  for (int k = 0; k < CV_MAX_HIDDEN; ++k)
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k)
     if (k == s.nh - 1) { hl = s.h[k]; DHl = t.dh[k]; EHl = t.eh[k]; ldl = t.ldh[k]; }
   wgrad(t.xr, t.ldx, D, DHl, ldl, hl, nr, g + s.out_w, g + s.out_b);
   __syncthreads();
   back_rows(t.xr, t.ldx, D, params + s.out_w, DHl, ldl, hl, nr, s.act);
   __syncthreads();
 #pragma unroll
-  for (int k = CV_MAX_HIDDEN - 1; k >= 0; --k) {
+  for (int k = MLP_MAX_HIDDEN - 1; k >= 0; --k) {
     if (k >= s.nh) continue;
     const float* in = k ? t.dh[k - 1] : t.zc;
     const int ldi = k ? t.ldh[k - 1] : t.ldz, ni = k ? s.h[k - 1] : L + Cd;
@@ -209,7 +188,7 @@ __device__ __forceinline__ void sweep_tile(const CvShape& s, float* sm, const fl
   }
   __syncthreads();
 #pragma unroll
-  for (int k = CV_MAX_HIDDEN - 1; k >= 0; --k) {
+  for (int k = MLP_MAX_HIDDEN - 1; k >= 0; --k) {
     if (k >= s.nh) continue;
     const float* in = k ? t.eh[k - 1] : t.xc;
     const int ldi = k ? t.ldh[k - 1] : t.ldxc, ni = k ? s.h[k - 1] : D + Cd;
@@ -245,8 +224,8 @@ __device__ __forceinline__ void cv_tail(const CvShape& s, float* __restrict__ pa
 }
 
 // with bwd: gradient partials + loss per CTA at partials + b * stride; without: the loss sum alone at partials[b]
-__global__ void __launch_bounds__(CV_THREADS) cv_sweep_kernel(CvShape s, const float* __restrict__ params,
-    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int64_t nb, CvNoise nz,
+__global__ void __launch_bounds__(MLP_THREADS) cv_sweep_kernel(CvShape s, const float* __restrict__ params,
+    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int64_t nb, MlpNoise nz,
     float inv_bd, float kl_b, float* __restrict__ partials, int bwd) {
   extern __shared__ __align__(16) float smem[];
   const int64_t row0 = (int64_t)blockIdx.x * s.R;
@@ -255,34 +234,24 @@ __global__ void __launch_bounds__(CV_THREADS) cv_sweep_kernel(CvShape s, const f
   sweep_tile(s, smem, params, X, C, idx, row0, nr, nz, inv_bd, kl_b, g, bwd ? g + s.P : partials + blockIdx.x);
 }
 
-__global__ void cv_reduce_kernel(const float* __restrict__ partials, int n_ctas, int stride, int P,
-                                 float* __restrict__ g) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c > P) return;
-  float acc = 0.0f;
-  for (int b = 0; b < n_ctas; ++b) acc += partials[(size_t)b * stride + c];
-  g[c] = acc;
-}
-
 // *dst = sum of n loss partials: strided per-thread sums in order, then the fixed block tree
-__global__ void __launch_bounds__(CV_THREADS) cv_loss_reduce_kernel(const float* __restrict__ partials, int64_t n,
+__global__ void __launch_bounds__(MLP_THREADS) cv_loss_reduce_kernel(const float* __restrict__ partials, int64_t n,
                                                                     float* dst) {
   __shared__ float scratch[32];
-  float acc = 0.0f;
-  for (int64_t i = threadIdx.x; i < n; i += blockDim.x) acc += partials[i];
-  const float tot = block_sum(acc, scratch);
+  float tot;
+  block_sums_strided<1>(partials, n, scratch, &tot);
   if (threadIdx.x == 0) *dst = tot;
 }
 
-__global__ void __launch_bounds__(CV_TAIL_THREADS) cv_tail_kernel(CvShape s, float* params, float* m, float* v,
+__global__ void __launch_bounds__(MLP_TAIL_THREADS) cv_tail_kernel(CvShape s, float* params, float* m, float* v,
                                                                  const float* g, float* gflat, float* loss_dst,
                                                                  CvStep st) {
   cv_tail(s, params, m, v, g, gflat, loss_dst, st);
 }
 
 // a whole step of a batch that fits one tile
-__global__ void __launch_bounds__(CV_TAIL_THREADS) cv_step_kernel(CvShape s, float* params, float* m, float* v,
-    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int nb, CvNoise nz,
+__global__ void __launch_bounds__(MLP_TAIL_THREADS) cv_step_kernel(CvShape s, float* params, float* m, float* v,
+    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int nb, MlpNoise nz,
     float* g, float* gflat, float* loss_dst, CvStep st) {
   extern __shared__ __align__(16) float smem[];
   sweep_tile(s, smem, params, X, C, idx, 0, nb, nz, st.inv_bd, st.kl_b, g, g + s.P);
@@ -291,7 +260,7 @@ __global__ void __launch_bounds__(CV_TAIL_THREADS) cv_step_kernel(CvShape s, flo
 }
 
 // Encoder.forward for inference: mu, log_sigma of rows [X|C]
-__global__ void __launch_bounds__(CV_THREADS) cv_encode_kernel(CvShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) cv_encode_kernel(CvShape s, const float* __restrict__ params,
     const float* __restrict__ X, const float* __restrict__ C, int64_t N, float* mu_o, float* ls_o) {
   extern __shared__ __align__(16) float smem[];
   const CvTile t = carve(s, smem);
@@ -310,7 +279,7 @@ __global__ void __launch_bounds__(CV_THREADS) cv_encode_kernel(CvShape s, const 
 }
 
 // Decoder.forward for inference: x of rows [z|C], z from Z or from Philox keyed on (seed, row_offset + row, j)
-__global__ void __launch_bounds__(CV_THREADS) cv_decode_kernel(CvShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) cv_decode_kernel(CvShape s, const float* __restrict__ params,
     const float* __restrict__ Z, const float* __restrict__ C, int64_t N, unsigned long long seed, long long row_offset,
     float* x_o) {
   extern __shared__ __align__(16) float smem[];
@@ -318,7 +287,7 @@ __global__ void __launch_bounds__(CV_THREADS) cv_decode_kernel(CvShape s, const 
   const int64_t row0 = (int64_t)blockIdx.x * s.R;
   const int nr = (int)(N - row0 < s.R ? N - row0 : s.R);
   const int L = s.L, Cd = s.Cd, W = L + Cd;
-  const CvNoise nz{Z, seed, row_offset};
+  const MlpNoise nz{Z, seed, row_offset};
   for (int e = threadIdx.x; e < nr * W; e += blockDim.x) {
     const int r = e / W, j = e - r * W;
     const int64_t row = row0 + r;
@@ -334,8 +303,6 @@ __global__ void __launch_bounds__(CV_THREADS) cv_decode_kernel(CvShape s, const 
   }
 }
 
-int64_t n_tiles(const CvShape& s, int64_t n) { return (n + s.R - 1) / s.R; }
-
 }  // namespace
 
 struct rnvp_cv_desc {
@@ -347,37 +314,32 @@ namespace {
 int check_cv(const rnvp_cv_desc* d) { return d ? 0 : rnvp_fail(RNVP_EINVAL, "null CVAE descriptor"); }
 
 // the gradient (gflat, with m == NULL) or the Adam step of one batch of nb positions of idx
-cudaError_t launch_step(const CvShape& s, float* params, float* m, float* v, const float* X, const float* C,
-                        const int64_t* idx, int64_t nb, const CvNoise& nz, float* gflat, float* loss_dst,
-                        const CvStep& st, float* ws, cudaStream_t stream) {
-  const int64_t nt = n_tiles(s, nb);
+void launch_step(const CvShape& s, float* params, float* m, float* v, const float* X, const float* C,
+                 const int64_t* idx, int64_t nb, const MlpNoise& nz, float* gflat, float* loss_dst, const CvStep& st,
+                 float* ws, cudaStream_t stream) {
+  const int64_t nt = n_tiles(s.R, nb);
   float* g = ws;                                       // reduced gradient + loss (stride floats), then the partials
   if (nt == 1) {
-    cv_step_kernel<<<1, CV_TAIL_THREADS, s.smem, stream>>>(s, params, m, v, X, C, idx, (int)nb, nz, g, gflat, loss_dst,
+    cv_step_kernel<<<1, MLP_TAIL_THREADS, s.smem, stream>>>(s, params, m, v, X, C, idx, (int)nb, nz, g, gflat, loss_dst,
                                                            st);
-    return cudaGetLastError();
+    return;
   }
   float* partials = ws + s.stride;
-  cv_sweep_kernel<<<(unsigned)nt, CV_THREADS, s.smem, stream>>>(s, params, X, C, idx, nb, nz, st.inv_bd, st.kl_b,
+  cv_sweep_kernel<<<(unsigned)nt, MLP_THREADS, s.smem, stream>>>(s, params, X, C, idx, nb, nz, st.inv_bd, st.kl_b,
                                                                 partials, 1);
-  cv_reduce_kernel<<<(s.P + 1 + 255) / 256, 256, 0, stream>>>(partials, (int)nt, s.stride, s.P, g);
-  cv_tail_kernel<<<1, CV_TAIL_THREADS, 0, stream>>>(s, params, m, v, g, gflat, loss_dst, st);
-  return cudaGetLastError();
+  launch_reduce(partials, (int)nt, s.stride, s.P, 0, s.P, 1, g, nullptr, stream);
+  cv_tail_kernel<<<1, MLP_TAIL_THREADS, 0, stream>>>(s, params, m, v, g, gflat, loss_dst, st);
 }
 
 // the loss alone over N positions of idx into *loss_dst
-cudaError_t launch_loss(const CvShape& s, const float* params, const float* X, const float* C, const int64_t* idx,
-                        int64_t N, const CvNoise& nz, float kl_weight, float* loss_dst, float* ws,
-                        cudaStream_t stream) {
-  const int64_t nt = n_tiles(s, N);
+void launch_loss(const CvShape& s, const float* params, const float* X, const float* C, const int64_t* idx, int64_t N,
+                 const MlpNoise& nz, float kl_weight, float* loss_dst, float* ws, cudaStream_t stream) {
+  const int64_t nt = n_tiles(s.R, N);
   const float inv_bd = (float)(1.0 / ((double)N * s.D)), kl_b = (float)((double)kl_weight / (double)N);
-  cv_sweep_kernel<<<(unsigned)nt, CV_THREADS, s.smem, stream>>>(s, params, X, C, idx, N, nz, inv_bd, kl_b,
+  cv_sweep_kernel<<<(unsigned)nt, MLP_THREADS, s.smem, stream>>>(s, params, X, C, idx, N, nz, inv_bd, kl_b,
                                                                 nt == 1 ? loss_dst : ws, 0);
-  if (nt > 1) cv_loss_reduce_kernel<<<1, CV_THREADS, 0, stream>>>(ws, nt, loss_dst);
-  return cudaGetLastError();
+  if (nt > 1) cv_loss_reduce_kernel<<<1, MLP_THREADS, 0, stream>>>(ws, nt, loss_dst);
 }
-
-bool bad_rows(const CvShape& s, int64_t N) { return n_tiles(s, N) > 0x7fffffffLL; }
 
 }  // namespace
 
@@ -390,64 +352,28 @@ int rnvp_cv_desc_create(int D, int Cd, int latent, int n_hidden, const int* hidd
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_desc_create: bad shape");
   if (act != RNVP_ACT_TANH && act != RNVP_ACT_RELU)
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_desc_create: act must be RNVP_ACT_TANH or _RELU");
-  if (D > CV_MAX_D) return rnvp_fail(RNVP_ESHAPE, "CVAE: var_size D must be <= 128");
-  if (Cd > CV_MAX_CD) return rnvp_fail(RNVP_ESHAPE, "CVAE: cond_size must be <= 256");
-  if (latent > CV_MAX_LAT) return rnvp_fail(RNVP_ESHAPE, "CVAE: latent_dim must be <= 128");
-  if (n_hidden > CV_MAX_HIDDEN) return rnvp_fail(RNVP_ESHAPE, "CVAE: at most 4 hidden layers");
+  if (D > MLP_MAX_D) return rnvp_fail(RNVP_ESHAPE, "CVAE: var_size D must be <= 128");
+  if (Cd > MLP_MAX_CD) return rnvp_fail(RNVP_ESHAPE, "CVAE: cond_size must be <= 256");
+  if (latent > MLP_MAX_LAT) return rnvp_fail(RNVP_ESHAPE, "CVAE: latent_dim must be <= 128");
+  if (n_hidden > MLP_MAX_HIDDEN) return rnvp_fail(RNVP_ESHAPE, "CVAE: at most 4 hidden layers");
   CvShape s{};
   s.D = D; s.Cd = Cd; s.L = latent; s.nh = n_hidden; s.act = act;
-  for (int k = 0; k < n_hidden; ++k) {
-    if (hidden[k] < 1) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_desc_create: hidden widths must be >= 1");
-    if (hidden[k] > CV_MAX_WIDTH) return rnvp_fail(RNVP_ESHAPE, "CVAE: hidden widths must be <= 512");
-    s.h[k] = hidden[k];
-  }
   int64_t off = 0;
-  int prev = D + Cd;
-  for (int k = 0; k < n_hidden; ++k) {                // encoder.parameters()
-    s.ew[k] = (int)off; off += (int64_t)hidden[k] * prev;
-    s.eb[k] = (int)off; off += hidden[k];
-    prev = hidden[k];
-  }
-  s.mu_w = (int)off; off += (int64_t)latent * prev;
-  s.mu_b = (int)off; off += latent;
-  s.ls_w = (int)off; off += (int64_t)latent * prev;
-  s.ls_b = (int)off; off += latent;
-  prev = latent + Cd;
-  for (int k = 0; k < n_hidden; ++k) {                // decoder.parameters()
-    s.dw[k] = (int)off; off += (int64_t)hidden[k] * prev;
-    s.db[k] = (int)off; off += hidden[k];
-    prev = hidden[k];
-  }
-  s.out_w = (int)off; off += (int64_t)D * prev;
-  s.out_b = (int)off; off += D;
+  const int hl = hidden[n_hidden - 1];
+  // encoder.parameters(), then decoder.parameters()
+  if (int rc = hidden_layout(n_hidden, hidden, D + Cd, s.h, s.ew, s.eb, off, "CVAE", "rnvp_cv_desc_create")) return rc;
+  linear_layout(s.mu_w, s.mu_b, hl, latent, off);
+  linear_layout(s.ls_w, s.ls_b, hl, latent, off);
+  hidden_layout(n_hidden, hidden, latent + Cd, s.h, s.dw, s.db, off, "CVAE", "rnvp_cv_desc_create");   // checked above
+  linear_layout(s.out_w, s.out_b, hl, D, off);
   s.P = (int)off;
   s.stride = (s.P + 1 + 3) & ~3;
-  int R = CV_MAX_ROWS;
-  while (R > 1 && tile_floats(s, R) * 4 > CV_SMEM_BUDGET) R >>= 1;
-  s.R = R;
-  s.smem = tile_floats(s, R) * 4;
-  int dev = 0, max_optin = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  if (e != cudaSuccess) return rnvp_fail(RNVP_ENODEVICE, "rnvp_cv_desc_create: no CUDA device");
-  if (s.smem > max_optin) return rnvp_fail(RNVP_ESHAPE, "CVAE: shape exceeds the shared memory of one CTA");
-  // The limit is a property of the kernel on this device, shared by every descriptor: set it to the device's opt-in
-  // maximum less its static shared memory (idempotent), never to this shape's need, which would lower it under a
-  // larger model created earlier.
-  const void* kernels[] = {(const void*)cv_sweep_kernel, (const void*)cv_step_kernel, (const void*)cv_encode_kernel,
-                           (const void*)cv_decode_kernel};
-  for (const void* k : kernels) {
-    cudaFuncAttributes fa;
-    e = cudaFuncGetAttributes(&fa, k);
-    const int dyn_max = max_optin - (int)fa.sharedSizeBytes;          // opt-in limit less the static shared memory
-    if (e == cudaSuccess && s.smem > dyn_max)
-      return rnvp_fail(RNVP_ESHAPE, "CVAE: shape exceeds the shared memory of one CTA");
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_max);
-    if (e != cudaSuccess) {
-      cudaGetLastError();                                             // do not leave the error for the caller's next call
-      return rnvp_fail((int)e, "rnvp_cv_desc_create: cudaFuncSetAttribute");
-    }
-  }
+  s.R = rows_per_tile(s);
+  s.smem = tile_floats(s, s.R) * 4;
+  if (int rc = opt_in_smem({(const void*)cv_sweep_kernel, (const void*)cv_step_kernel, (const void*)cv_encode_kernel,
+                            (const void*)cv_decode_kernel},
+                           s.smem, "CVAE", "rnvp_cv_desc_create"))
+    return rc;
   *out = new rnvp_cv_desc{s};
   return 0;
 }
@@ -458,8 +384,8 @@ int64_t rnvp_cv_param_count(const rnvp_cv_desc* d) { return d ? d->s.P : -1; }
 
 int64_t rnvp_cv_workspace_bytes(const rnvp_cv_desc* d, int64_t batch_rows, int64_t loss_rows) {
   if (!d || batch_rows < 0 || loss_rows < 0) return -1;
-  const int64_t nt = n_tiles(d->s, batch_rows);
-  return 4 * std::max((int64_t)d->s.stride * (1 + (nt > 1 ? nt : 0)), n_tiles(d->s, loss_rows));
+  const int64_t nt = n_tiles(d->s.R, batch_rows);
+  return 4 * std::max((int64_t)d->s.stride * (1 + (nt > 1 ? nt : 0)), n_tiles(d->s.R, loss_rows));
 }
 
 int rnvp_cv_encode(const rnvp_cv_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
@@ -468,12 +394,10 @@ int rnvp_cv_encode(const rnvp_cv_desc* d, const float* d_params, const float* d_
   if (!d_params || !d_X || (d->s.Cd && !d_C) || !d_mu || !d_log_sigma || N < 0)
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_encode: bad argument");
   if (N == 0) return 0;
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_encode: too many rows");
-  cv_encode_kernel<<<(unsigned)n_tiles(d->s, N), CV_THREADS, d->s.smem, (cudaStream_t)stream>>>(d->s, d_params, d_X,
-                                                                                                 d_C, N, d_mu,
-                                                                                                 d_log_sigma);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cv_encode_kernel launch");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_encode: too many rows");
+  cv_encode_kernel<<<(unsigned)n_tiles(d->s.R, N), MLP_THREADS, d->s.smem, (cudaStream_t)stream>>>(
+      d->s, d_params, d_X, d_C, N, d_mu, d_log_sigma);
+  return launched("cv_encode_kernel launch");
 }
 
 int rnvp_cv_decode(const rnvp_cv_desc* d, const float* d_params, const float* d_Z, const float* d_C, int64_t N,
@@ -481,11 +405,10 @@ int rnvp_cv_decode(const rnvp_cv_desc* d, const float* d_params, const float* d_
   if (check_cv(d)) return RNVP_EINVAL;
   if (!d_params || (d->s.Cd && !d_C) || !d_x || N < 0) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_decode: bad argument");
   if (N == 0) return 0;
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_decode: too many rows");
-  cv_decode_kernel<<<(unsigned)n_tiles(d->s, N), CV_THREADS, d->s.smem, (cudaStream_t)stream>>>(
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_decode: too many rows");
+  cv_decode_kernel<<<(unsigned)n_tiles(d->s.R, N), MLP_THREADS, d->s.smem, (cudaStream_t)stream>>>(
       d->s, d_params, d_Z, d_C, N, seed, row_offset, d_x);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "cv_decode_kernel launch");
+  return launched("cv_decode_kernel launch");
 }
 
 int rnvp_cv_grad(const rnvp_cv_desc* d, const float* d_params, const float* d_X, const float* d_C,
@@ -496,15 +419,14 @@ int rnvp_cv_grad(const rnvp_cv_desc* d, const float* d_params, const float* d_X,
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_grad: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_cv_workspace_bytes(d, N, 0))
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_grad: workspace smaller than rnvp_cv_workspace_bytes(N, 0)");
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_grad: too many rows");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_grad: too many rows");
   CvStep st{};
   st.inv_bd = (float)(1.0 / ((double)N * d->s.D));
   st.kl_b = (float)(kl_weight / (double)N);
   st.adam = 0;
-  const cudaError_t e = launch_step(d->s, const_cast<float*>(d_params), nullptr, nullptr, d_X, d_C, d_idx, N,
-                                    CvNoise{d_eps, 0, 0}, d_gflat, d_loss, st, (float*)d_workspace,
-                                    (cudaStream_t)stream);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "CVAE gradient launch");
+  launch_step(d->s, const_cast<float*>(d_params), nullptr, nullptr, d_X, d_C, d_idx, N, MlpNoise{d_eps, 0, 0}, d_gflat,
+              d_loss, st, (float*)d_workspace, (cudaStream_t)stream);
+  return launched("CVAE gradient launch");
 }
 
 int rnvp_cv_loss(const rnvp_cv_desc* d, const float* d_params, const float* d_X, const float* d_C,
@@ -515,10 +437,10 @@ int rnvp_cv_loss(const rnvp_cv_desc* d, const float* d_params, const float* d_X,
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_loss: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_cv_workspace_bytes(d, 0, N))
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_loss: workspace smaller than rnvp_cv_workspace_bytes(0, N)");
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_loss: too many rows");
-  const cudaError_t e = launch_loss(d->s, d_params, d_X, d_C, d_idx, N, CvNoise{d_eps, 0, 0}, (float)kl_weight, d_loss,
-                                    (float*)d_workspace, (cudaStream_t)stream);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "CVAE loss launch");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_loss: too many rows");
+  launch_loss(d->s, d_params, d_X, d_C, d_idx, N, MlpNoise{d_eps, 0, 0}, (float)kl_weight, d_loss, (float*)d_workspace,
+              (cudaStream_t)stream);
+  return launched("CVAE loss launch");
 }
 
 int rnvp_cv_fit_epoch(const rnvp_cv_desc* d, float* d_params, float* d_exp_avg, float* d_exp_avg_sq, const float* d_X,
@@ -532,7 +454,7 @@ int rnvp_cv_fit_epoch(const rnvp_cv_desc* d, float* d_params, float* d_exp_avg, 
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_fit_epoch: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_cv_workspace_bytes(d, std::min(n, batch_size), n))
     return rnvp_fail(RNVP_EINVAL, "rnvp_cv_fit_epoch: workspace smaller than rnvp_cv_workspace_bytes(batch_size, n)");
-  if (bad_rows(d->s, n)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_fit_epoch: too many rows");
+  if (bad_rows(d->s.R, n)) return rnvp_fail(RNVP_EINVAL, "rnvp_cv_fit_epoch: too many rows");
   const CvShape& s = d->s;
   const cudaStream_t st_ = (cudaStream_t)stream;
   int64_t k = 0;
@@ -543,16 +465,15 @@ int rnvp_cv_fit_epoch(const rnvp_cv_desc* d, float* d_params, float* d_exp_avg, 
     st.inv_bd = (float)(1.0 / ((double)nb * s.D));
     st.kl_b = (float)(kl_weight / (double)nb);
     st.adam = 1;
-    const CvNoise nz{d_noise ? d_noise + b0 * s.L : nullptr, seed, (long long)b0};
-    const cudaError_t e = launch_step(s, d_params, d_exp_avg, d_exp_avg_sq, d_X, d_C, d_perm + b0, nb, nz, nullptr,
-                                      nullptr, st, (float*)d_workspace, st_);
-    if (e != cudaSuccess) return rnvp_fail((int)e, "CVAE fit step launch");
+    const MlpNoise nz{d_noise ? d_noise + b0 * s.L : nullptr, seed, (long long)b0};
+    launch_step(s, d_params, d_exp_avg, d_exp_avg_sq, d_X, d_C, d_perm + b0, nb, nz, nullptr, nullptr, st,
+                (float*)d_workspace, st_);
+    if (int rc = launched("CVAE fit step launch")) return rc;
   }
   // compute_loss(X_real, C): every row in dataset order, with its own noise (rows n .. 2n - 1 of the Philox stream)
-  const CvNoise nz{d_noise ? d_noise + n * s.L : nullptr, seed, (long long)n};
-  const cudaError_t e = launch_loss(s, d_params, d_X, d_C, nullptr, n, nz, (float)kl_weight, d_loss,
-                                    (float*)d_workspace, st_);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "CVAE epoch loss launch");
+  const MlpNoise nz{d_noise ? d_noise + n * s.L : nullptr, seed, (long long)n};
+  launch_loss(s, d_params, d_X, d_C, nullptr, n, nz, (float)kl_weight, d_loss, (float*)d_workspace, st_);
+  return launched("CVAE epoch loss launch");
 }
 
 }  // extern "C"

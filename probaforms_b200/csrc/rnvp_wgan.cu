@@ -12,9 +12,9 @@
 // interleaved sum would leave rounding noise there that RMSprop turns into steps of up to ~lr.  A generator step runs
 // the critic backward down to the x columns of the fake rows (no weight gradients, nothing into c) and then the
 // generator backward.  Per-CTA partial records hold the stepped net's gradient and the tile's two score sums;
-// wg_reduce_kernel adds them in CTA order and wg_tail_kernel runs RMSprop (and the clamp), so repeated fits are bitwise
-// identical.  A batch of at most R rows is one launch (wg_step_kernel).  The loss pass (the epoch losses) runs both
-// forward passes and writes per-CTA score sums, added by wg_loss_reduce_kernel in a fixed order.
+// mlp_reduce_kernel adds them in CTA order and wg_tail_kernel runs RMSprop (and the clamp), so repeated fits are
+// bitwise identical.  A batch of at most R rows is one launch (wg_step_kernel).  The loss pass (the epoch losses) runs
+// both forward passes and writes per-CTA score sums, added by wg_loss_reduce_kernel in a fixed order.
 //
 // z is either a caller buffer indexed by batch position, or Philox keyed on (seed, row base + batch position, j).
 #include <cuda_runtime.h>
@@ -25,23 +25,15 @@
 
 #include "../../include/rnvp.h"
 #include "rnvp_mlp.cuh"
-#include "rnvp_philox.cuh"
 #include "rnvp_rmsprop.cuh"
 
-int rnvp_fail(int code, const char* msg);   // rnvp_api.cu: sets rnvp_last_error()
-
 namespace {
-
-constexpr int WG_MAX_D = 128, WG_MAX_CD = 256, WG_MAX_LAT = 128, WG_MAX_HIDDEN = MLP_MAX_HIDDEN, WG_MAX_WIDTH = 512;
-constexpr int WG_MAX_ROWS = 64;                       // rows per CTA tile
-constexpr int WG_SMEM_BUDGET = 96 * 1024;             // per sweep CTA: two CTAs of 256 threads per SM
-constexpr int WG_THREADS = 256, WG_TAIL_THREADS = 512;
 
 // one MLP: hidden layers (act), then a linear output layer of nout columns
 struct WgNet {
   int nh, act, nin, nout;
-  int h[WG_MAX_HIDDEN];
-  int w[WG_MAX_HIDDEN], b[WG_MAX_HIDDEN];             // float offsets of model.{2k}.weight / .bias in the flat buffer
+  int h[MLP_MAX_HIDDEN];
+  int w[MLP_MAX_HIDDEN], b[MLP_MAX_HIDDEN];           // float offsets of model.{2k}.weight / .bias in the flat buffer
   int ow, ob;                                         // model.{2 nh}
 };
 
@@ -53,12 +45,10 @@ struct WgShape {
   int smem;
 };
 
-__host__ __device__ inline int odd_ld(int n) { return n | 1; }
-
 // shared-memory layout of one tile: ZC | GH_0 .. | XF | XR | DH_0 .. | O, each [R][odd stride] (O: [R])
 struct WgTile {
-  float *zc, *gh[WG_MAX_HIDDEN], *xf, *xr, *dh[WG_MAX_HIDDEN], *o;
-  int ldz, ldg[WG_MAX_HIDDEN], ldx, ldd[WG_MAX_HIDDEN];
+  float *zc, *gh[MLP_MAX_HIDDEN], *xf, *xr, *dh[MLP_MAX_HIDDEN], *o;
+  int ldz, ldg[MLP_MAX_HIDDEN], ldx, ldd[MLP_MAX_HIDDEN];
 };
 
 __host__ __device__ inline int tile_floats(const WgShape& s, int R) {
@@ -74,7 +64,7 @@ __device__ __forceinline__ WgTile carve(const WgShape& s, float* sm) {
   t.ldz = odd_ld(s.L + s.Cd);
   t.zc = sm; sm += R * t.ldz;
 #pragma unroll
-  for (int k = 0; k < WG_MAX_HIDDEN; ++k) {
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {
     t.ldg[k] = k < s.g.nh ? odd_ld(s.g.h[k]) : 0;
     t.gh[k] = sm;
     sm += R * t.ldg[k];
@@ -83,7 +73,7 @@ __device__ __forceinline__ WgTile carve(const WgShape& s, float* sm) {
   t.xf = sm; sm += R * t.ldx;
   t.xr = sm; sm += R * t.ldx;
 #pragma unroll
-  for (int k = 0; k < WG_MAX_HIDDEN; ++k) {
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k) {
     t.ldd[k] = k < s.d.nh ? odd_ld(s.d.h[k]) : 0;
     t.dh[k] = sm;
     sm += R * t.ldd[k];
@@ -92,21 +82,10 @@ __device__ __forceinline__ WgTile carve(const WgShape& s, float* sm) {
   return t;
 }
 
-// z of batch position p, latent j: z[p * L + j] if given, else Philox(seed, row0 + p, j)
-struct WgNoise {
-  const float* z;
-  unsigned long long seed;
-  long long row0;
-};
-
-__device__ __forceinline__ float noise_at(const WgNoise& nz, int L, int64_t p, int j) {
-  return nz.z ? nz.z[p * L + j] : rnvp_rng::normal1(nz.seed, nz.row0 + p, j);
-}
-
 // ZC = [z|c] of the tile's rows; with real, XR = [x|c]; the c columns of XF too
 __device__ __forceinline__ void load_tile(const WgShape& s, const WgTile& t, const float* __restrict__ X,
                                           const float* __restrict__ C, const int64_t* __restrict__ idx, int64_t row0,
-                                          int nr, const WgNoise& nz, bool real) {
+                                          int nr, const MlpNoise& nz, bool real) {
   const int D = s.D, Cd = s.Cd, L = s.L;
   for (int e = threadIdx.x; e < nr * L; e += blockDim.x) {
     const int r = e / L, j = e - r * L;
@@ -155,7 +134,7 @@ __device__ __forceinline__ void critic_backward(const WgShape& s, const WgTile& 
   int hl = 0, ldl = 0;
   float* Hl = nullptr;
 #pragma unroll
-  for (int k = 0; k < WG_MAX_HIDDEN; ++k)
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k)
     if (k == n.nh - 1) { hl = n.h[k]; Hl = t.dh[k]; ldl = t.ldd[k]; }
   if (g) {
     wgrad<ACC>(t.o, 1, 1, Hl, ldl, hl, nr, g + n.ow, g + n.ob);
@@ -164,7 +143,7 @@ __device__ __forceinline__ void critic_backward(const WgShape& s, const WgTile& 
   back_rows(t.o, 1, 1, params + n.ow, Hl, ldl, hl, nr, n.act);
   __syncthreads();
 #pragma unroll
-  for (int k = WG_MAX_HIDDEN - 1; k >= 0; --k) {
+  for (int k = MLP_MAX_HIDDEN - 1; k >= 0; --k) {
     if (k >= n.nh) continue;
     const float* x = k ? t.dh[k - 1] : in;
     const int ldi = k ? t.ldd[k - 1] : t.ldx, ni = k ? n.h[k - 1] : s.D + s.Cd;
@@ -185,7 +164,7 @@ enum { WG_LOSS = 0, WG_CRITIC = 1, WG_GENERATOR = 2 };
 // g[0..P) (the other net's entries are not written); the tile's fake and real score sums go to sums[0], sums[1]
 __device__ __forceinline__ void sweep_tile(const WgShape& s, float* sm, const float* __restrict__ params,
                                            const float* __restrict__ X, const float* __restrict__ C,
-                                           const int64_t* __restrict__ idx, int64_t row0, int nr, const WgNoise& nz,
+                                           const int64_t* __restrict__ idx, int64_t row0, int nr, const MlpNoise& nz,
                                            float inv_nb, int kind, float* __restrict__ g, float* sums) {
   const WgTile t = carve(s, sm);
   float* scratch = t.o + s.R;                          // the 64 floats after the tile (tile_floats)
@@ -220,14 +199,14 @@ __device__ __forceinline__ void sweep_tile(const WgShape& s, float* sm, const fl
   int hl = 0, ldl = 0;
   float* Hl = nullptr;
 #pragma unroll
-  for (int k = 0; k < WG_MAX_HIDDEN; ++k)
+  for (int k = 0; k < MLP_MAX_HIDDEN; ++k)
     if (k == n.nh - 1) { hl = n.h[k]; Hl = t.gh[k]; ldl = t.ldg[k]; }
   wgrad(t.xf, t.ldx, s.D, Hl, ldl, hl, nr, g + n.ow, g + n.ob);
   __syncthreads();
   back_rows(t.xf, t.ldx, s.D, params + n.ow, Hl, ldl, hl, nr, n.act);
   __syncthreads();
 #pragma unroll
-  for (int k = WG_MAX_HIDDEN - 1; k >= 0; --k) {
+  for (int k = MLP_MAX_HIDDEN - 1; k >= 0; --k) {
     if (k >= n.nh) continue;
     const float* x = k ? t.gh[k - 1] : t.zc;
     const int ldi = k ? t.ldg[k - 1] : t.ldz, ni = k ? n.h[k - 1] : s.L + s.Cd;
@@ -270,8 +249,8 @@ __device__ __forceinline__ void wg_tail(const WgShape& s, float* __restrict__ pa
 
 // gradient partials + score sums per CTA at partials + b * stride (steps), or the score sums alone at partials[b],
 // partials[n_ctas + b] (loss)
-__global__ void __launch_bounds__(WG_THREADS) wg_sweep_kernel(WgShape s, const float* __restrict__ params,
-    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int64_t nb, WgNoise nz,
+__global__ void __launch_bounds__(MLP_THREADS) wg_sweep_kernel(WgShape s, const float* __restrict__ params,
+    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int64_t nb, MlpNoise nz,
     float inv_nb, int kind, float* __restrict__ partials) {
   extern __shared__ __align__(16) float smem[];
   const int64_t row0 = (int64_t)blockIdx.x * s.R;
@@ -289,42 +268,27 @@ __global__ void __launch_bounds__(WG_THREADS) wg_sweep_kernel(WgShape s, const f
   sweep_tile(s, smem, params, X, C, idx, row0, nr, nz, inv_nb, kind, g, g + s.P);
 }
 
-// g[c] = sum over CTAs in order, for c in lo .. hi and the two score sums P, P + 1
-__global__ void wg_reduce_kernel(const float* __restrict__ partials, int n_ctas, int stride, int P, int lo, int hi,
-                                 float* __restrict__ g) {
-  const int t = blockIdx.x * blockDim.x + threadIdx.x, m = hi - lo;
-  if (t >= m + 2) return;
-  const int c = t < m ? lo + t : P + (t - m);
-  float acc = 0.0f;
-  for (int b = 0; b < n_ctas; ++b) acc += partials[(size_t)b * stride + c];
-  g[c] = acc;
-}
-
 // the epoch losses from n_ctas per-CTA fake and real score sums: gen = -mean(D(fake)), disc = mean(D(real)) + gen
-__global__ void __launch_bounds__(WG_THREADS) wg_loss_reduce_kernel(const float* __restrict__ partials, int64_t n_ctas,
+__global__ void __launch_bounds__(MLP_THREADS) wg_loss_reduce_kernel(const float* __restrict__ partials, int64_t n_ctas,
                                                                     int64_t N, float* gen_dst, float* disc_dst) {
   __shared__ float scratch[32];
-  float af = 0.0f, ar = 0.0f;
-  for (int64_t i = threadIdx.x; i < n_ctas; i += blockDim.x) {
-    af += partials[i];
-    ar += partials[n_ctas + i];
-  }
-  const float sf = block_sum(af, scratch), sr = block_sum(ar, scratch);
+  float s[2];                                         // fake, real
+  block_sums_strided<2>(partials, n_ctas, scratch, s);
   if (threadIdx.x == 0) {
-    const float gen = -(sf / (float)N);
+    const float gen = -(s[0] / (float)N);
     *gen_dst = gen;
-    *disc_dst = sr / (float)N + gen;
+    *disc_dst = s[1] / (float)N + gen;
   }
 }
 
-__global__ void __launch_bounds__(WG_TAIL_THREADS) wg_tail_kernel(WgShape s, float* params, float* sq, const float* g,
+__global__ void __launch_bounds__(MLP_TAIL_THREADS) wg_tail_kernel(WgShape s, float* params, float* sq, const float* g,
                                                                  float* gflat, float* loss_dst, WgStep st) {
   wg_tail(s, params, sq, g, gflat, loss_dst, st);
 }
 
 // a whole step of a batch that fits one tile
-__global__ void __launch_bounds__(WG_TAIL_THREADS) wg_step_kernel(WgShape s, float* params, float* sq,
-    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int nb, WgNoise nz,
+__global__ void __launch_bounds__(MLP_TAIL_THREADS) wg_step_kernel(WgShape s, float* params, float* sq,
+    const float* __restrict__ X, const float* __restrict__ C, const int64_t* __restrict__ idx, int nb, MlpNoise nz,
     float* g, float* gflat, float* loss_dst, WgStep st) {
   extern __shared__ __align__(16) float smem[];
   sweep_tile(s, smem, params, X, C, idx, 0, nb, nz, st.inv_nb, st.kind, g, g + s.P);
@@ -333,14 +297,14 @@ __global__ void __launch_bounds__(WG_TAIL_THREADS) wg_step_kernel(WgShape s, flo
 }
 
 // Generator.forward for inference: x of rows [z|C], z from Z or from Philox keyed on (seed, row_offset + row, j)
-__global__ void __launch_bounds__(WG_THREADS) wg_generate_kernel(WgShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) wg_generate_kernel(WgShape s, const float* __restrict__ params,
     const float* __restrict__ Z, const float* __restrict__ C, int64_t N, unsigned long long seed, long long row_offset,
     float* x_o) {
   extern __shared__ __align__(16) float smem[];
   const WgTile t = carve(s, smem);
   const int64_t row0 = (int64_t)blockIdx.x * s.R;
   const int nr = (int)(N - row0 < s.R ? N - row0 : s.R);
-  load_tile(s, t, nullptr, C, nullptr, row0, nr, WgNoise{Z, seed, row_offset}, false);
+  load_tile(s, t, nullptr, C, nullptr, row0, nr, MlpNoise{Z, seed, row_offset}, false);
   __syncthreads();
   gen_forward(s, t, params, nr);
   const int D = s.D;
@@ -351,7 +315,7 @@ __global__ void __launch_bounds__(WG_THREADS) wg_generate_kernel(WgShape s, cons
 }
 
 // Discriminator.forward for inference: the scores [N] of rows [X|C]
-__global__ void __launch_bounds__(WG_THREADS) wg_critic_kernel(WgShape s, const float* __restrict__ params,
+__global__ void __launch_bounds__(MLP_THREADS) wg_critic_kernel(WgShape s, const float* __restrict__ params,
     const float* __restrict__ X, const float* __restrict__ C, int64_t N, float* score_o) {
   extern __shared__ __align__(16) float smem[];
   const WgTile t = carve(s, smem);
@@ -368,8 +332,6 @@ __global__ void __launch_bounds__(WG_THREADS) wg_critic_kernel(WgShape s, const 
   for (int r = threadIdx.x; r < nr; r += blockDim.x) score_o[row0 + r] = t.o[r];
 }
 
-int64_t n_tiles(const WgShape& s, int64_t n) { return (n + s.R - 1) / s.R; }
-
 }  // namespace
 
 struct rnvp_wg_desc {
@@ -381,35 +343,30 @@ namespace {
 int check_wg(const rnvp_wg_desc* d) { return d ? 0 : rnvp_fail(RNVP_EINVAL, "null ConditionalWGAN descriptor"); }
 
 // the gradient (gflat, update 0) or the RMSprop step of one batch of nb positions of idx
-cudaError_t launch_step(const WgShape& s, float* params, float* sq, const float* X, const float* C, const int64_t* idx,
-                        int64_t nb, const WgNoise& nz, float* gflat, float* loss_dst, const WgStep& st, float* ws,
-                        cudaStream_t stream) {
-  const int64_t nt = n_tiles(s, nb);
+void launch_step(const WgShape& s, float* params, float* sq, const float* X, const float* C, const int64_t* idx,
+                 int64_t nb, const MlpNoise& nz, float* gflat, float* loss_dst, const WgStep& st, float* ws,
+                 cudaStream_t stream) {
+  const int64_t nt = n_tiles(s.R, nb);
   float* g = ws;                                       // reduced record (stride floats), then the partials
   if (nt == 1) {
-    wg_step_kernel<<<1, WG_TAIL_THREADS, s.smem, stream>>>(s, params, sq, X, C, idx, (int)nb, nz, g, gflat, loss_dst,
+    wg_step_kernel<<<1, MLP_TAIL_THREADS, s.smem, stream>>>(s, params, sq, X, C, idx, (int)nb, nz, g, gflat, loss_dst,
                                                            st);
-    return cudaGetLastError();
+    return;
   }
   float* partials = ws + s.stride;
-  wg_sweep_kernel<<<(unsigned)nt, WG_THREADS, s.smem, stream>>>(s, params, X, C, idx, nb, nz, st.inv_nb, st.kind,
+  wg_sweep_kernel<<<(unsigned)nt, MLP_THREADS, s.smem, stream>>>(s, params, X, C, idx, nb, nz, st.inv_nb, st.kind,
                                                                 partials);
-  const int m = st.hi - st.lo + 2;
-  wg_reduce_kernel<<<(m + 255) / 256, 256, 0, stream>>>(partials, (int)nt, s.stride, s.P, st.lo, st.hi, g);
-  wg_tail_kernel<<<1, WG_TAIL_THREADS, 0, stream>>>(s, params, sq, g, gflat, loss_dst, st);
-  return cudaGetLastError();
+  launch_reduce(partials, (int)nt, s.stride, s.P, st.lo, st.hi, 2, g, nullptr, stream);   // + fake and real score sums
+  wg_tail_kernel<<<1, MLP_TAIL_THREADS, 0, stream>>>(s, params, sq, g, gflat, loss_dst, st);
 }
 
 // the epoch losses over N positions of idx into *gen_dst, *disc_dst
-cudaError_t launch_loss(const WgShape& s, const float* params, const float* X, const float* C, const int64_t* idx,
-                        int64_t N, const WgNoise& nz, float* gen_dst, float* disc_dst, float* ws, cudaStream_t stream) {
-  const int64_t nt = n_tiles(s, N);
-  wg_sweep_kernel<<<(unsigned)nt, WG_THREADS, s.smem, stream>>>(s, params, X, C, idx, N, nz, 0.0f, WG_LOSS, ws);
-  wg_loss_reduce_kernel<<<1, WG_THREADS, 0, stream>>>(ws, nt, N, gen_dst, disc_dst);
-  return cudaGetLastError();
+void launch_loss(const WgShape& s, const float* params, const float* X, const float* C, const int64_t* idx, int64_t N,
+                 const MlpNoise& nz, float* gen_dst, float* disc_dst, float* ws, cudaStream_t stream) {
+  const int64_t nt = n_tiles(s.R, N);
+  wg_sweep_kernel<<<(unsigned)nt, MLP_THREADS, s.smem, stream>>>(s, params, X, C, idx, N, nz, 0.0f, WG_LOSS, ws);
+  wg_loss_reduce_kernel<<<1, MLP_THREADS, 0, stream>>>(ws, nt, N, gen_dst, disc_dst);
 }
-
-bool bad_rows(const WgShape& s, int64_t N) { return n_tiles(s, N) > 0x7fffffffLL; }
 
 WgStep make_step(const WgShape& s, int generator, int64_t nb, int update) {
   WgStep st{};
@@ -420,22 +377,6 @@ WgStep make_step(const WgShape& s, int generator, int64_t nb, int update) {
   st.inv_nb = (float)(1.0 / (double)nb);
   st.update = update;
   return st;
-}
-
-int net_layout(WgNet& n, int nin, int nout, int nh, const int* hidden, int act, int64_t& off, const char* which) {
-  n.nh = nh; n.act = act; n.nin = nin; n.nout = nout;
-  int prev = nin;
-  for (int k = 0; k < nh; ++k) {
-    if (hidden[k] < 1) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_desc_create: hidden widths must be >= 1");
-    if (hidden[k] > WG_MAX_WIDTH) return rnvp_fail(RNVP_ESHAPE, which);
-    n.h[k] = hidden[k];
-    n.w[k] = (int)off; off += (int64_t)hidden[k] * prev;
-    n.b[k] = (int)off; off += hidden[k];
-    prev = hidden[k];
-  }
-  n.ow = (int)off; off += (int64_t)nout * prev;
-  n.ob = (int)off; off += nout;
-  return 0;
 }
 
 }  // namespace
@@ -451,46 +392,30 @@ int rnvp_wg_desc_create(int D, int Cd, int latent, int g_hidden_n, const int* g_
   for (int a : {g_act, d_act})
     if (a != RNVP_ACT_TANH && a != RNVP_ACT_RELU)
       return rnvp_fail(RNVP_EINVAL, "rnvp_wg_desc_create: act must be RNVP_ACT_TANH or _RELU");
-  if (D > WG_MAX_D) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: var_size D must be <= 128");
-  if (Cd > WG_MAX_CD) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: cond_size must be <= 256");
-  if (latent > WG_MAX_LAT) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: latent_dim must be <= 128");
-  if (g_hidden_n > WG_MAX_HIDDEN || d_hidden_n > WG_MAX_HIDDEN)
+  if (D > MLP_MAX_D) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: var_size D must be <= 128");
+  if (Cd > MLP_MAX_CD) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: cond_size must be <= 256");
+  if (latent > MLP_MAX_LAT) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: latent_dim must be <= 128");
+  if (g_hidden_n > MLP_MAX_HIDDEN || d_hidden_n > MLP_MAX_HIDDEN)
     return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: at most 4 hidden layers per net");
   WgShape s{};
   s.D = D; s.Cd = Cd; s.L = latent;
+  s.g = WgNet{g_hidden_n, g_act, latent + Cd, D};
+  s.d = WgNet{d_hidden_n, d_act, D + Cd, 1};
+  const char *model = "ConditionalWGAN", *fn = "rnvp_wg_desc_create";
   int64_t off = 0;
-  const char* wide = "ConditionalWGAN: hidden widths must be <= 512";
-  if (int rc = net_layout(s.g, latent + Cd, D, g_hidden_n, g_hidden, g_act, off, wide)) return rc;   // generator
+  if (int rc = hidden_layout(g_hidden_n, g_hidden, latent + Cd, s.g.h, s.g.w, s.g.b, off, model, fn)) return rc;
+  linear_layout(s.g.ow, s.g.ob, g_hidden[g_hidden_n - 1], D, off);
   s.PG = (int)off;
-  if (int rc = net_layout(s.d, D + Cd, 1, d_hidden_n, d_hidden, d_act, off, wide)) return rc;        // critic
+  if (int rc = hidden_layout(d_hidden_n, d_hidden, D + Cd, s.d.h, s.d.w, s.d.b, off, model, fn)) return rc;
+  linear_layout(s.d.ow, s.d.ob, d_hidden[d_hidden_n - 1], 1, off);
   s.P = (int)off;
   s.stride = (s.P + 2 + 3) & ~3;
-  int R = WG_MAX_ROWS;
-  while (R > 1 && tile_floats(s, R) * 4 > WG_SMEM_BUDGET) R >>= 1;
-  s.R = R;
-  s.smem = tile_floats(s, R) * 4;
-  int dev = 0, max_optin = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  if (e != cudaSuccess) return rnvp_fail(RNVP_ENODEVICE, "rnvp_wg_desc_create: no CUDA device");
-  if (s.smem > max_optin) return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: shape exceeds the shared memory of one CTA");
-  // The limit is a property of the kernel on this device, shared by every descriptor: set it to the device's opt-in
-  // maximum less its static shared memory (idempotent), never to this shape's need, which would lower it under a
-  // larger model created earlier.
-  const void* kernels[] = {(const void*)wg_sweep_kernel, (const void*)wg_step_kernel, (const void*)wg_generate_kernel,
-                           (const void*)wg_critic_kernel};
-  for (const void* k : kernels) {
-    cudaFuncAttributes fa;
-    e = cudaFuncGetAttributes(&fa, k);
-    const int dyn_max = max_optin - (int)fa.sharedSizeBytes;          // opt-in limit less the static shared memory
-    if (e == cudaSuccess && s.smem > dyn_max)
-      return rnvp_fail(RNVP_ESHAPE, "ConditionalWGAN: shape exceeds the shared memory of one CTA");
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_max);
-    if (e != cudaSuccess) {
-      cudaGetLastError();                                             // do not leave the error for the caller's next call
-      return rnvp_fail((int)e, "rnvp_wg_desc_create: cudaFuncSetAttribute");
-    }
-  }
+  s.R = rows_per_tile(s);
+  s.smem = tile_floats(s, s.R) * 4;
+  if (int rc = opt_in_smem({(const void*)wg_sweep_kernel, (const void*)wg_step_kernel, (const void*)wg_generate_kernel,
+                            (const void*)wg_critic_kernel},
+                           s.smem, model, fn))
+    return rc;
   *out = new rnvp_wg_desc{s};
   return 0;
 }
@@ -506,8 +431,8 @@ int64_t rnvp_wg_param_count(const rnvp_wg_desc* d, int net) {
 
 int64_t rnvp_wg_workspace_bytes(const rnvp_wg_desc* d, int64_t batch_rows, int64_t loss_rows) {
   if (!d || batch_rows < 0 || loss_rows < 0) return -1;
-  const int64_t nt = n_tiles(d->s, batch_rows);
-  return 4 * std::max((int64_t)d->s.stride * (1 + (nt > 1 ? nt : 0)), 2 * n_tiles(d->s, loss_rows));
+  const int64_t nt = n_tiles(d->s.R, batch_rows);
+  return 4 * std::max((int64_t)d->s.stride * (1 + (nt > 1 ? nt : 0)), 2 * n_tiles(d->s.R, loss_rows));
 }
 
 int rnvp_wg_generate(const rnvp_wg_desc* d, const float* d_params, const float* d_Z, const float* d_C, int64_t N,
@@ -515,11 +440,10 @@ int rnvp_wg_generate(const rnvp_wg_desc* d, const float* d_params, const float* 
   if (check_wg(d)) return RNVP_EINVAL;
   if (!d_params || (d->s.Cd && !d_C) || !d_x || N < 0) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_generate: bad argument");
   if (N == 0) return 0;
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_generate: too many rows");
-  wg_generate_kernel<<<(unsigned)n_tiles(d->s, N), WG_THREADS, d->s.smem, (cudaStream_t)stream>>>(
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_generate: too many rows");
+  wg_generate_kernel<<<(unsigned)n_tiles(d->s.R, N), MLP_THREADS, d->s.smem, (cudaStream_t)stream>>>(
       d->s, d_params, d_Z, d_C, N, seed, row_offset, d_x);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "wg_generate_kernel launch");
+  return launched("wg_generate_kernel launch");
 }
 
 int rnvp_wg_critic(const rnvp_wg_desc* d, const float* d_params, const float* d_X, const float* d_C, int64_t N,
@@ -528,11 +452,10 @@ int rnvp_wg_critic(const rnvp_wg_desc* d, const float* d_params, const float* d_
   if (!d_params || !d_X || (d->s.Cd && !d_C) || !d_score || N < 0)
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_critic: bad argument");
   if (N == 0) return 0;
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_critic: too many rows");
-  wg_critic_kernel<<<(unsigned)n_tiles(d->s, N), WG_THREADS, d->s.smem, (cudaStream_t)stream>>>(d->s, d_params, d_X,
-                                                                                                 d_C, N, d_score);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "wg_critic_kernel launch");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_critic: too many rows");
+  wg_critic_kernel<<<(unsigned)n_tiles(d->s.R, N), MLP_THREADS, d->s.smem, (cudaStream_t)stream>>>(
+      d->s, d_params, d_X, d_C, N, d_score);
+  return launched("wg_critic_kernel launch");
 }
 
 int rnvp_wg_grad(const rnvp_wg_desc* d, const float* d_params, const float* d_X, const float* d_C,
@@ -543,11 +466,11 @@ int rnvp_wg_grad(const rnvp_wg_desc* d, const float* d_params, const float* d_X,
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_grad: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_wg_workspace_bytes(d, N, 0))
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_grad: workspace smaller than rnvp_wg_workspace_bytes(N, 0)");
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_grad: too many rows");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_grad: too many rows");
   const WgStep st = make_step(d->s, generator_step, N, 0);
-  const cudaError_t e = launch_step(d->s, const_cast<float*>(d_params), nullptr, d_X, d_C, d_idx, N,
-                                    WgNoise{d_z, 0, 0}, d_gflat, d_loss, st, (float*)d_workspace, (cudaStream_t)stream);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "ConditionalWGAN gradient launch");
+  launch_step(d->s, const_cast<float*>(d_params), nullptr, d_X, d_C, d_idx, N, MlpNoise{d_z, 0, 0}, d_gflat, d_loss, st,
+              (float*)d_workspace, (cudaStream_t)stream);
+  return launched("ConditionalWGAN gradient launch");
 }
 
 int rnvp_wg_loss(const rnvp_wg_desc* d, const float* d_params, const float* d_X, const float* d_C,
@@ -558,10 +481,10 @@ int rnvp_wg_loss(const rnvp_wg_desc* d, const float* d_params, const float* d_X,
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_loss: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_wg_workspace_bytes(d, 0, N))
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_loss: workspace smaller than rnvp_wg_workspace_bytes(0, N)");
-  if (bad_rows(d->s, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_loss: too many rows");
-  const cudaError_t e = launch_loss(d->s, d_params, d_X, d_C, d_idx, N, WgNoise{d_z, 0, 0}, d_gen_loss, d_disc_loss,
-                                    (float*)d_workspace, (cudaStream_t)stream);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "ConditionalWGAN loss launch");
+  if (bad_rows(d->s.R, N)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_loss: too many rows");
+  launch_loss(d->s, d_params, d_X, d_C, d_idx, N, MlpNoise{d_z, 0, 0}, d_gen_loss, d_disc_loss, (float*)d_workspace,
+              (cudaStream_t)stream);
+  return launched("ConditionalWGAN loss launch");
 }
 
 int rnvp_wg_fit_epoch(const rnvp_wg_desc* d, float* d_params, float* d_square_avg, const float* d_X, const float* d_C,
@@ -575,7 +498,7 @@ int rnvp_wg_fit_epoch(const rnvp_wg_desc* d, float* d_params, float* d_square_av
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_fit_epoch: bad argument");
   if (!d_workspace || workspace_bytes < rnvp_wg_workspace_bytes(d, std::min(n, batch_size), n))
     return rnvp_fail(RNVP_EINVAL, "rnvp_wg_fit_epoch: workspace smaller than rnvp_wg_workspace_bytes(batch_size, n)");
-  if (bad_rows(d->s, n)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_fit_epoch: too many rows");
+  if (bad_rows(d->s.R, n)) return rnvp_fail(RNVP_EINVAL, "rnvp_wg_fit_epoch: too many rows");
   const WgShape& s = d->s;
   const cudaStream_t st_ = (cudaStream_t)stream;
   const RnvpRmspropCoef k{(float)lr, (float)alpha, (float)(1.0 - alpha), (float)eps, (float)weight_decay};
@@ -586,16 +509,15 @@ int rnvp_wg_fit_epoch(const rnvp_wg_desc* d, float* d_params, float* d_square_av
     WgStep st = make_step(s, generator, nb, 1);
     st.k = k;
     st.clip = generator ? 0.0f : (float)clip;
-    const WgNoise nz{d_noise ? d_noise + b0 * s.L : nullptr, seed, (long long)b0};
-    const cudaError_t e = launch_step(s, d_params, d_square_avg, d_X, d_C, d_perm + b0, nb, nz, nullptr, nullptr, st,
-                                      (float*)d_workspace, st_);
-    if (e != cudaSuccess) return rnvp_fail((int)e, "ConditionalWGAN fit step launch");
+    const MlpNoise nz{d_noise ? d_noise + b0 * s.L : nullptr, seed, (long long)b0};
+    launch_step(s, d_params, d_square_avg, d_X, d_C, d_perm + b0, nb, nz, nullptr, nullptr, st, (float*)d_workspace,
+                st_);
+    if (int rc = launched("ConditionalWGAN fit step launch")) return rc;
   }
   // the epoch losses: every row in dataset order, with its own noise (rows n .. 2n - 1 of the Philox stream)
-  const WgNoise nz{d_noise ? d_noise + n * s.L : nullptr, seed, (long long)n};
-  const cudaError_t e = launch_loss(s, d_params, d_X, d_C, nullptr, n, nz, d_gen_loss, d_disc_loss,
-                                    (float*)d_workspace, st_);
-  return e == cudaSuccess ? 0 : rnvp_fail((int)e, "ConditionalWGAN epoch loss launch");
+  const MlpNoise nz{d_noise ? d_noise + n * s.L : nullptr, seed, (long long)n};
+  launch_loss(s, d_params, d_X, d_C, nullptr, n, nz, d_gen_loss, d_disc_loss, (float*)d_workspace, st_);
+  return launched("ConditionalWGAN epoch loss launch");
 }
 
 }  // extern "C"

@@ -128,14 +128,25 @@ def test_descriptor_rejects_bad_shapes_without_device():
     L = lib()
     h = C.c_void_p()
     hid = (C.c_int * 1)(10)
-    assert L.rnvp_cn_desc_create(2, 1, 1, hid, 1, 0, None) == -1
+
+    def err():
+        return L.rnvp_last_error().decode()
+    assert L.rnvp_cn_desc_create(2, 1, 1, hid, 1, 0, None) == -1 and err() == "rnvp_cn_desc_create: out is null"
     assert L.rnvp_cn_desc_create(129, 1, 1, hid, 1, 0, C.byref(h)) == -2
-    assert b"128" in L.rnvp_last_error()
+    assert err() == "ConditionalNormal: var_size D must be <= 128"
     assert L.rnvp_cn_desc_create(2, 257, 1, hid, 1, 0, C.byref(h)) == -2
+    assert err() == "ConditionalNormal: cond_size must be <= 256"
     assert L.rnvp_cn_desc_create(2, 1, 5, (C.c_int * 5)(1, 1, 1, 1, 1), 1, 0, C.byref(h)) == -2
+    assert err() == "ConditionalNormal: at most 4 hidden layers"
     assert L.rnvp_cn_desc_create(2, 1, 1, (C.c_int * 1)(513), 1, 0, C.byref(h)) == -2
+    assert err() == "ConditionalNormal: hidden widths must be <= 512"
     assert L.rnvp_cn_desc_create(2, 1, 1, hid, 9, 0, C.byref(h)) == -1
+    assert err() == "rnvp_cn_desc_create: act must be RNVP_ACT_TANH, _RELU or _SIGMOID"
     assert L.rnvp_cn_desc_create(2, 1, 1, (C.c_int * 1)(0), 1, 0, C.byref(h)) == -1
+    assert err() == "rnvp_cn_desc_create: hidden widths must be >= 1"
+    assert L.rnvp_cn_desc_create(2, 1, 2, (C.c_int * 2)(0, 513), 1, 0, C.byref(h)) == -1     # widths in layer order
+    assert err() == "rnvp_cn_desc_create: hidden widths must be >= 1"
+    assert L.rnvp_cn_desc_create(0, 1, 1, hid, 1, 0, C.byref(h)) == -1 and err() == "rnvp_cn_desc_create: bad shape"
 
 
 def test_descriptor_create_errors_keep_their_types():

@@ -114,17 +114,26 @@ def test_descriptor_rejects_bad_shapes_without_device():
     L = lib()
     h = C.c_void_p()
     hid = (C.c_int * 1)(10)
-    assert L.rnvp_cv_desc_create(2, 1, 2, 1, hid, 1, None) == -1
+
+    def err():
+        return L.rnvp_last_error().decode()
+    assert L.rnvp_cv_desc_create(2, 1, 2, 1, hid, 1, None) == -1 and err() == "rnvp_cv_desc_create: out is null"
     assert L.rnvp_cv_desc_create(129, 1, 2, 1, hid, 1, C.byref(h)) == -2
-    assert b"128" in L.rnvp_last_error()
-    assert L.rnvp_cv_desc_create(2, 257, 2, 1, hid, 1, C.byref(h)) == -2
-    assert L.rnvp_cv_desc_create(2, 1, 129, 1, hid, 1, C.byref(h)) == -2
+    assert err() == "CVAE: var_size D must be <= 128"
+    assert L.rnvp_cv_desc_create(2, 257, 2, 1, hid, 1, C.byref(h)) == -2 and err() == "CVAE: cond_size must be <= 256"
+    assert L.rnvp_cv_desc_create(2, 1, 129, 1, hid, 1, C.byref(h)) == -2 and err() == "CVAE: latent_dim must be <= 128"
     assert L.rnvp_cv_desc_create(2, 1, 2, 5, (C.c_int * 5)(1, 1, 1, 1, 1), 1, C.byref(h)) == -2
+    assert err() == "CVAE: at most 4 hidden layers"
     assert L.rnvp_cv_desc_create(2, 1, 2, 1, (C.c_int * 1)(513), 1, C.byref(h)) == -2
+    assert err() == "CVAE: hidden widths must be <= 512"
     assert L.rnvp_cv_desc_create(2, 1, 2, 1, hid, 3, C.byref(h)) == -1       # sigmoid is not a CVAE activation
+    assert err() == "rnvp_cv_desc_create: act must be RNVP_ACT_TANH or _RELU"
     assert L.rnvp_cv_desc_create(2, 1, 2, 1, (C.c_int * 1)(0), 1, C.byref(h)) == -1
-    assert L.rnvp_cv_desc_create(2, -1, 2, 1, hid, 1, C.byref(h)) == -1
-    assert L.rnvp_cv_desc_create(2, 1, 0, 1, hid, 1, C.byref(h)) == -1
+    assert err() == "rnvp_cv_desc_create: hidden widths must be >= 1"
+    assert L.rnvp_cv_desc_create(2, 1, 2, 2, (C.c_int * 2)(513, 0), 1, C.byref(h)) == -2     # widths in layer order
+    assert err() == "CVAE: hidden widths must be <= 512"
+    assert L.rnvp_cv_desc_create(2, -1, 2, 1, hid, 1, C.byref(h)) == -1 and err() == "rnvp_cv_desc_create: bad shape"
+    assert L.rnvp_cv_desc_create(2, 1, 0, 1, hid, 1, C.byref(h)) == -1 and err() == "rnvp_cv_desc_create: bad shape"
     assert L.rnvp_cv_workspace_bytes(None, 1, 1) == -1
 
 

@@ -162,17 +162,25 @@ def test_descriptor_rejects_bad_shapes_without_device():
 
     def create(D=2, Cd=1, lat=2, gh=h1, ng=1, ga=2, dh=h1, nd=1, da=2, out=True):
         return L.rnvp_wg_desc_create(D, Cd, lat, ng, gh, ga, nd, dh, da, C.byref(h) if out else None)
-    assert create(out=False) == -1
-    assert create(D=129) == -2 and b"128" in L.rnvp_last_error()
-    assert create(Cd=257) == -2 and b"256" in L.rnvp_last_error()
-    assert create(lat=129) == -2 and b"128" in L.rnvp_last_error()
-    assert create(gh=(C.c_int * 5)(1, 1, 1, 1, 1), ng=5) == -2 and b"4" in L.rnvp_last_error()
-    assert create(dh=(C.c_int * 5)(1, 1, 1, 1, 1), nd=5) == -2
-    assert create(gh=(C.c_int * 1)(513)) == -2 and b"512" in L.rnvp_last_error()
-    assert create(dh=(C.c_int * 1)(513)) == -2
-    assert create(ga=3) == -1 and create(da=3) == -1                 # sigmoid is not a WGAN activation code
-    assert create(dh=(C.c_int * 1)(0)) == -1
-    assert create(Cd=-1) == -1 and create(lat=0) == -1 and create(D=0) == -1
+
+    def err():
+        return L.rnvp_last_error().decode()
+    assert create(out=False) == -1 and err() == "rnvp_wg_desc_create: out is null"
+    assert create(D=129) == -2 and err() == "ConditionalWGAN: var_size D must be <= 128"
+    assert create(Cd=257) == -2 and err() == "ConditionalWGAN: cond_size must be <= 256"
+    assert create(lat=129) == -2 and err() == "ConditionalWGAN: latent_dim must be <= 128"
+    five = "ConditionalWGAN: at most 4 hidden layers per net"
+    assert create(gh=(C.c_int * 5)(1, 1, 1, 1, 1), ng=5) == -2 and err() == five
+    assert create(dh=(C.c_int * 5)(1, 1, 1, 1, 1), nd=5) == -2 and err() == five
+    wide = "ConditionalWGAN: hidden widths must be <= 512"
+    assert create(gh=(C.c_int * 1)(513)) == -2 and err() == wide
+    assert create(dh=(C.c_int * 1)(513)) == -2 and err() == wide
+    act = "rnvp_wg_desc_create: act must be RNVP_ACT_TANH or _RELU"
+    assert create(ga=3) == -1 and err() == act and create(da=3) == -1 and err() == act   # sigmoid is not a WGAN code
+    assert create(dh=(C.c_int * 1)(0)) == -1 and err() == "rnvp_wg_desc_create: hidden widths must be >= 1"
+    assert create(gh=(C.c_int * 1)(513), dh=(C.c_int * 1)(0)) == -2 and err() == wide     # the generator is checked first
+    for kw in (dict(Cd=-1), dict(lat=0), dict(D=0)):
+        assert create(**kw) == -1 and err() == "rnvp_wg_desc_create: bad shape"
     assert L.rnvp_wg_workspace_bytes(None, 1, 1) == -1
     assert L.rnvp_wg_param_count(None, 0) == -1
 

@@ -138,7 +138,7 @@ def run_gpu(out, reps):
             torch.cuda.synchronize()
         per = {}
         for ev in prof.key_averages():
-            for k in ("cn_sweep_kernel", "cn_reduce_kernel", "cn_tail_kernel"):
+            for k in ("cn_sweep_kernel", "mlp_reduce_kernel", "cn_tail_kernel"):
                 if k in ev.key:
                     per[k] = per.get(k, 0.0) + ev.device_time_total / steps      # us per step
         rec["kernel_us_per_step"] = per

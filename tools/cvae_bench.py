@@ -126,7 +126,7 @@ def run_gpu(out, reps):
             torch.cuda.synchronize()
         per = {}
         for ev in prof.key_averages():
-            for k in ("cv_sweep_kernel", "cv_reduce_kernel", "cv_tail_kernel", "cv_loss_reduce_kernel"):
+            for k in ("cv_sweep_kernel", "mlp_reduce_kernel", "cv_tail_kernel", "cv_loss_reduce_kernel"):
                 if k in ev.key:
                     per[k] = per.get(k, 0.0) + ev.device_time_total
         rec["kernel_us_per_epoch_call"] = per

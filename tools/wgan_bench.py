@@ -149,7 +149,7 @@ def run_gpu(out, reps):
                 torch.cuda.synchronize()
             per = {}
             for ev in prof.key_averages():
-                for k in ("wg_sweep_kernel", "wg_reduce_kernel", "wg_tail_kernel", "wg_loss_reduce_kernel"):
+                for k in ("wg_sweep_kernel", "mlp_reduce_kernel", "wg_tail_kernel", "wg_loss_reduce_kernel"):
                     if k in ev.key:
                         per[k] = per.get(k, 0.0) + ev.device_time_total
             rec["kernel_us_per_epoch_call"] = per
