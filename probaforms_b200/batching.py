@@ -6,6 +6,13 @@ Kept separate from the CUDA plumbing so that the data-parallel arithmetic can be
 import torch
 
 
+def process_group():
+    """(rank, world) of the initialised torch.distributed group, or (0, 1) without one."""
+    dist = torch.distributed
+    world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
+    return (dist.get_rank() if world > 1 else 0), world
+
+
 def epoch_seed(group=None, device=None):
     """The sampler seed of one epoch, consuming the global torch RNG exactly as the reference's fresh
     ``DataLoader(dataset, batch_size, shuffle=True)`` does (realnvp.py:237): one int64 draw for the
@@ -15,8 +22,7 @@ def epoch_seed(group=None, device=None):
     RNG states).  Must be called on the thread that owns the training loop, once per epoch, in order."""
     torch.empty((), dtype=torch.int64).random_()
     seed = torch.empty((), dtype=torch.int64).random_()
-    if group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()
-                             and torch.distributed.get_world_size() > 1):
+    if group is not None or process_group()[1] > 1:
         s = seed.reshape(1).to(device) if device is not None else seed.reshape(1)
         torch.distributed.broadcast(s, src=0, group=group)
         seed = s.cpu().reshape(())

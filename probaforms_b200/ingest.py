@@ -280,11 +280,13 @@ class ChunkUploader:
             self._waited += 1
 
     def close(self):
-        """Upload whatever has not been asked for yet and wait for the staging buffers (shared by later calls)."""
+        """Upload whatever has not been asked for yet and wait for the staging buffers (shared by later calls); returns the
+        number of bytes uploaded."""
         self.wait_rows(self.n)
         for ev in self.events[-2:]:
             if ev is not None:
                 ev.synchronize()
+        return 4 * (self.X.numel() + (self.C.numel() if self.C is not None else 0))
 
 
 class StepStreamer:
@@ -354,6 +356,8 @@ class StepStreamer:
         self.free.append((slot, ev))
 
     def close(self):
+        """Waits for the steps that used the pinned slots (shared by later fits of the process); returns ``bytes_h2d``."""
         for _, ev in self.free:
             if ev is not None:
-                ev.synchronize()                    # the pinned slots are shared by later fits of the process
+                ev.synchronize()
+        return self.bytes_h2d

@@ -27,6 +27,7 @@ import numpy as np
 import torch
 
 from .. import _lib
+from ..batching import process_group
 
 __all__ = [
     "frechet_distance",
@@ -147,13 +148,6 @@ def _mmd_draws(X32, Y32, counts):
                                 mmd.data_ptr(), ws.data_ptr(), ws_bytes, _stream(dev))
     _lib.check(rc, "rnvp_mmd_draws")
     return median, mmd
-
-
-def _process_group():
-    """(rank, world) of the initialised torch.distributed group, or (0, 1) without one."""
-    dist = torch.distributed
-    world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
-    return (dist.get_rank() if world > 1 else 0), world
 
 
 def _shard_ids(rank, world, n_local):
@@ -326,7 +320,7 @@ def maximum_mean_discrepancy(X, Y, n_iters=100, standardize=False, devices=None,
     X64, Y64 = _prepare(X, Y, standardize)
     counts = _bootstrap_counts(X64.shape[0], Y64.shape[0], n_iters)
     X32, Y32 = X64.float().contiguous(), Y64.float().contiguous()
-    rank, world = _process_group() if shard else (0, 1)
+    rank, world = process_group() if shard else (0, 1)
     if not devices and world == 1:
         _, mmd = _mmd_draws(X32, Y32, _counts_to(counts, X64.device))
     else:

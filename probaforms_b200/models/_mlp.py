@@ -13,7 +13,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from .realnvp import _LossLog, _default_device
+from ._common import _LossLog, _default_device, progress
 from .. import _lib
 from ..batching import StreamingPermutation, batch_bounds
 
@@ -288,12 +288,7 @@ def run_epochs(owner, lib, dev, n, replay, launch, logs):
     eps_dev = torch.empty(replay.numel, dtype=torch.float32, device=dev) if replay.values else None
     copied = [None, None]
     loss_logs = [_LossLog(history) for history, _ in logs]
-    epochs = range(n_epochs)
-    bar = None
-    if owner.verbose >= 1:
-        from tqdm.auto import tqdm
-        bar = tqdm(epochs, unit='epoch')
-        epochs = bar
+    epochs, bar = progress(n_epochs, owner.verbose)
     nxt = StreamingPermutation(lib, replay.get(0)[0], n, host=owner._perm_host[0]) if n_epochs > 0 else None
     for ep in epochs:
         seed, buf = replay.get(ep)

@@ -29,11 +29,11 @@ import ctypes as ct
 import torch
 import torch.nn as nn
 
+from ._common import _default_device
 from . import _mlp
 from ._mlp import Desc, FlatParams, RngReplay, _act_code, _layers, _rows, _stream, check_fit_inputs, publish_state, \
     run_epochs
 from .interfaces import GenModel
-from .realnvp import _default_device
 from .. import _lib
 from ..batching import batch_bounds
 

@@ -11,31 +11,17 @@ Device: CUDA only.  ``cuda:{LOCAL_RANK}`` under torchrun, else the current CUDA
 device; the reference's env var ``device`` (realnvp.py:12-15) is honoured when
 it names a CUDA device and rejected otherwise -- there is no CPU fallback.
 """
-import os
 import weakref
 
 import numpy as np
 import torch
 import torch.nn as nn
 
+from ._common import _LossLog, _default_device, progress
 from .interfaces import GenModel
 from .nflow import InvertibleLayer, NormalizingFlow
 from ..engine import FlowEngine
-from ..batching import PermutationPrefetcher, batch_bounds, epoch_seed, shard_bounds
-
-
-def _default_device():
-    env = os.environ.get("device")
-    if env:
-        dev = torch.device(env)
-        if dev.type != "cuda":
-            raise RuntimeError(f"probaforms_b200 is CUDA-only (sm_100a); env var device={env!r} is not supported")
-        return dev
-    if not torch.cuda.is_available():
-        raise RuntimeError("probaforms_b200 needs a CUDA device (sm_100a); none is visible and there is no CPU fallback")
-    if "LOCAL_RANK" in os.environ:
-        return torch.device("cuda", int(os.environ["LOCAL_RANK"]))
-    return torch.device("cuda", torch.cuda.current_device())
+from ..batching import PermutationPrefetcher, batch_bounds, epoch_seed, process_group, shard_bounds
 
 
 def gen_network(n_inputs, n_outputs, hidden=(10,), activation='tanh'):
@@ -216,40 +202,62 @@ class FusedAdam(torch.optim.Adam):
         return loss
 
 
-class _LossLog:
-    """Per-step losses of ``fit`` -> ``loss_history`` (one 0-d CPU tensor per step, as upstream) without a device
-    synchronisation at the end of every epoch: an epoch's losses are copied to pinned memory asynchronously and collected
-    one epoch later, so the host prepares epoch e+1 (row order, uploads) while the GPU still runs epoch e."""
+def _on_host(A):
+    return not (isinstance(A, torch.Tensor) and A.device.type != "cpu")
 
-    def __init__(self, history):
-        self.history, self.pending = history, None
-        self._stage, self._flip = [None, None], 0          # two pinned staging buffers alternate (allocating one per epoch
-                                                           # would cost more than the synchronisation it replaces)
 
-    def push(self, losses_dev):
-        """Call after the epoch's steps were enqueued; returns the PREVIOUS epoch's losses (CPU tensor) or None."""
-        k, n = self._flip, losses_dev.numel()
-        self._flip ^= 1
-        if self._stage[k] is None or self._stage[k].numel() < n:
-            self._stage[k] = torch.empty(max(n, 1), dtype=torch.float32, pin_memory=True)
-        host = self._stage[k][:n]
-        host.copy_(losses_dev, non_blocking=True)
-        ev = torch.cuda.Event()
-        ev.record(torch.cuda.current_stream(losses_dev.device))
-        prev, self.pending = self.pending, (host, ev, losses_dev)
-        return self._collect(prev)
+def _device_order(n, dev, salt=0, chunk_rows=None):
+    """One epoch's row order with ``shuffle='device'``: ``torch.randperm(n)`` on the GPU, seeded with ``epoch_seed()`` +
+    ``salt``; with ``chunk_rows``, the concatenation of independent permutations of consecutive chunks of that many rows."""
+    gen = torch.Generator(device=dev)
+    gen.manual_seed((epoch_seed(device=dev) + salt) & 0x7FFFFFFFFFFFFFFF)
+    if chunk_rows is None:
+        return torch.randperm(n, device=dev, generator=gen)
+    return torch.cat([torch.randperm(min(chunk_rows, n - c0), device=dev, generator=gen) + c0
+                      for c0 in range(0, n, chunk_rows)])
 
-    def _collect(self, p):
-        if p is None:
-            return None
-        p[1].synchronize()
-        vals = p[0].clone()                     # off the pinned staging block
-        self.history.extend(vals.unbind(0))
-        return vals
 
-    def flush(self):
-        self._collect(self.pending)
-        self.pending = None
+class _EpochOrder:
+    """The row order of every epoch of one fit, the same on every rank: ``next_epoch()`` moves on to the next epoch,
+    then ``host(hi)`` / ``device(hi)`` is a host / device int64 tensor whose first ``hi`` entries are final.
+    ``shuffle='device'``: ``_device_order``.  Else the reference's order (``PermutationPrefetcher``, seeds drawn on this
+    thread) is shuffled one epoch ahead by a helper thread into two alternating host buffers that later fits reuse,
+    ``model._perm_host`` (pinned) when it is copied to the device, else ``model._perm_host_pageable``."""
+
+    def __init__(self, model, n, lib, to_device):
+        self.n, self.dev, self.to_device, self.perms = n, model._device, to_device, None
+        if getattr(model, "shuffle", "reference") != "device":
+            bufs = model._perm_host if to_device else model.__dict__.setdefault("_perm_host_pageable", [None, None])
+            self.perms = PermutationPrefetcher(n, model.n_epochs, device=self.dev, lib=lib, host_buffers=bufs, pin=to_device)
+            self.perm = torch.empty(max(n, 1), dtype=torch.int64, device=self.dev) if to_device else None
+        self.sp, self.whole, self.copied, self.copied_ev = None, None, 0, None
+
+    def next_epoch(self):
+        if self.perms is None:
+            self.perm, self.copied = _device_order(self.n, self.dev), self.n
+            self.whole = None if self.to_device else self.perm.cpu()
+            return
+        if self.perms.streaming:
+            if self.copied_ev is not None:
+                # next_stream() starts shuffling the epoch after this one into the host buffer the previous epoch's order
+                # was copied from: the last (asynchronous) copy from it must have run
+                self.copied_ev.synchronize()
+            self.sp = self.perms.next_stream()
+        else:                                       # very large n: torch.randperm's 64-bit scheme, whole tensor
+            self.whole = self.perms.next()
+        self.copied = 0
+
+    def host(self, hi):
+        return self.sp.wait(hi) if self.sp is not None else self.whole
+
+    def device(self, hi):
+        if self.copied < hi:                        # enqueue the upload of whatever is final by now, at least [0, hi)
+            upto = max(hi, min(self.n, self.sp.available())) if self.sp is not None else self.n
+            self.perm[self.copied:upto].copy_(self.host(upto)[self.copied:upto], non_blocking=True)
+            self.copied = upto
+            if self.sp is not None:                 # after every copy: a rank's copies may stop short of n
+                self.copied_ev = torch.cuda.current_stream(self.dev).record_event()
+        return self.perm
 
 
 class RealNVP(GenModel):
@@ -361,7 +369,8 @@ class RealNVP(GenModel):
         Ingestion (``ingest=`` constructor option): ``'resident'`` uploads the whole set once (chunked, conversion
         fused) and gathers batches on the device; ``'stream'`` uploads, two steps ahead of the kernels, only the rows
         THIS rank needs for each step (host gather + conversion into pinned buffers by a pool of host threads);
-        ``'auto'`` streams when that moves fewer bytes (host data, n_epochs <= world size, large batches).
+        ``'auto'`` streams when that moves fewer bytes (host data, n_epochs <= world size, large batches), or keeps a
+        shard per rank (``_shards``).  ``h2d_bytes_last_fit``: the row bytes uploaded.
         """
         if not hasattr(X, "shape") or (C is not None and not hasattr(C, "shape")):
             X = np.asarray(X)
@@ -369,10 +378,7 @@ class RealNVP(GenModel):
         if len(tuple(X.shape)) != 2:
             raise ValueError(f"X must be 2-D [n, var_size], got shape {tuple(X.shape)}")
         self._model_init(X, C)
-        dev = self._device
-        dist = torch.distributed
-        world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
-        rank = dist.get_rank() if world > 1 else 0
+        rank, world = process_group()
         n = X.shape[0]
         bs = int(self.batch_size)
         eng = self.nf._fused()
@@ -380,96 +386,84 @@ class RealNVP(GenModel):
         if getattr(eng, "_adam_owner", None) is not self.opt:       # rebuilt engine / loaded checkpoint: resume Adam
             self.opt._import_state(eng)
             eng._adam_owner = self.opt
-        device_shuffle = getattr(self, "shuffle", "reference") == "device"
-        on_host = not (isinstance(X, torch.Tensor) and X.device.type != "cpu")
-        mode = getattr(self, "ingest", "auto")
-        stream_rows = mode == "stream" or (mode == "auto" and on_host and self.n_epochs <= world
-                                           and min(bs, n) // world >= 8192)
-        stream_rows = stream_rows and on_host and n > 0
-        if device_shuffle and on_host and mode == "auto" and n >= world and min(bs, n) // world >= 4096:
-            # shuffle='device' from host data: every rank keeps and shuffles its OWN contiguous shard of the rows, and the
-            # first epoch trains while the shard is still being uploaded
-            return self._fit_local_shards(X, C, eng, rank, world)
-        # identical row order on every rank (the sampler seed of rank 0 is broadcast); computed one epoch ahead on a
-        # helper thread, the first one while the rows are uploaded
-        perms = None if device_shuffle else PermutationPrefetcher(
-            n, self.n_epochs, device=dev if world > 1 else None, lib=eng.lib,
-            host_buffers=(self.__dict__.setdefault("_perm_host_pageable", [None, None]) if stream_rows else self._perm_host),
-            pin=not stream_rows)
-        streamed_perm = perms is not None and perms.streaming
-        bounds = batch_bounds(n, bs)
-        if stream_rows:
-            return self._fit_streamed(X, C, eng, perms, bounds, rank, world, device_shuffle)
-        Xd = self._to_device(X, dev)
-        Cd = self._to_device(C, dev) if C is not None else None
-        Xd = eng._check_rows(Xd, eng.D, "X")
-        Cd = eng._check_cond(Cd, n)
-        perm_dev = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
-
-        epochs = range(self.n_epochs)
-        bar = None
-        if self.verbose >= 1:
-            from tqdm.auto import tqdm
-            bar = tqdm(epochs, unit='epoch')
-            epochs = bar
+        steps, run_epoch, finish = getattr(self, "_" + self._ingest_mode(X, n, bs, world))(X, C, eng, n, bs, rank, world)
         eng.zero_grads()
         log = _LossLog(self.loss_history)
-        order_copied = [None, None]                         # per host order buffer: its last H2D copy
+        epochs, bar = progress(self.n_epochs, self.verbose)
         for ep in epochs:
-            # the epoch's row order streams in from a helper thread (rnvp_perm_*, same order as the reference's
-            # DataLoader): a step only waits for its own batch, the tail of the shuffle overlaps the GPU work
-            losses = torch.empty(len(bounds), dtype=torch.float32, device=dev)
-            loss_ptr = losses.data_ptr()
-            if device_shuffle:
-                gen = torch.Generator(device=dev)
-                gen.manual_seed(epoch_seed(device=dev if world > 1 else None) & 0x7FFFFFFFFFFFFFFF)
-                perm_dev = torch.randperm(n, device=dev, generator=gen)
-                stream, copied = None, n
-            elif streamed_perm:
-                # next_stream() starts shuffling the epoch after this one into the host buffer the PREVIOUS epoch was copied
-                # from: its (asynchronous) copies must have run -- the loss read-back no longer synchronises every epoch
-                if order_copied[(ep + 1) & 1] is not None:
-                    order_copied[(ep + 1) & 1].synchronize()
-                stream, copied = perms.next_stream(), 0
-            else:                                           # very large n: torch.randperm's 64-bit scheme, whole tensor
-                perm_dev.copy_(perms.next(), non_blocking=True)
-                stream, copied = None, n
-            perm_ptr = perm_dev.data_ptr()
-            if world == 1 and bs <= 4096 and len(bounds) > 1:
-                # small batches: the host side of a step (Python + ctypes, ~50 us) costs more than its two kernels (~15 us), so
-                # the whole epoch goes down in one library call (rnvp_fit_epoch: same kernels, same order, same arithmetic)
-                if copied < n:
-                    host = stream.wait(n)
-                    perm_dev[copied:n].copy_(host[copied:n], non_blocking=True)
-                    copied = n
-                eng.fit_epoch(Xd, Cd, perm_dev, n, bs, self.lr, self.weight_decay, losses)
-                bounds_iter = ()
-            else:
-                bounds_iter = bounds
-            for s, (b0, nb) in enumerate(bounds_iter):      # last partial batch is kept (drop_last=False)
-                if copied < b0 + nb:                        # upload whatever is final by now, at least this batch
-                    upto = max(b0 + nb, min(n, stream.available()))
-                    host = stream.wait(upto)
-                    perm_dev[copied:upto].copy_(host[copied:upto], non_blocking=True)
-                    copied = upto
-                lo, hi = shard_bounds(b0, nb, rank, world)
-                # raw device addresses instead of tensor slices: the host side of a 32-row step is the bottleneck
-                eng.fit_step(Xd, Cd, perm_ptr + 8 * lo, hi - lo, nb, self.lr, self.weight_decay,
-                             loss_ptr + 4 * s, world=world)
-            if streamed_perm and not device_shuffle:
-                order_copied[ep & 1] = torch.cuda.Event()            # epoch ep read host buffer ep & 1
-                order_copied[ep & 1].record(torch.cuda.current_stream(dev))
+            losses = torch.empty(len(steps), dtype=torch.float32, device=self._device)
+            run_epoch(ep, losses)                           # enqueues the epoch's steps
             host = log.push(losses)                         # collects the previous epoch's losses: no sync on this one
             if bar is not None and host is not None:
                 bar.set_description(f"loss: {float(host[-1]):.4f}")
         log.flush()
+        self.h2d_bytes_last_fit = finish()
         self.opt._publish_state(eng)
 
-    def _fit_local_shards(self, X, C, eng, rank, world):
-        """Fit with ``shuffle='device'`` from host arrays: rank r uploads only rows [n*r/world, n*(r+1)/world) of the
-        (identical) host arrays -- sequentially, in chunks, conversion fused (ingest.ChunkUploader) -- and shuffles that
-        shard on the device.  A global batch is the union of the ranks' local batches of batch_size/world rows; the
-        gradient all-reduce and the loss are scaled by the true global row count of the step.
+    def _ingest_mode(self, X, n, bs, world):
+        """'shards', 'stream' or 'resident' (see ``fit``)."""
+        on_host, mode, rows = _on_host(X), getattr(self, "ingest", "auto"), min(bs, n) // world     # rows: local batch
+        if getattr(self, "shuffle", "reference") == "device" and on_host and mode == "auto" and n >= world and rows >= 4096:
+            return "shards"
+        if on_host and n > 0 and (mode == "stream" or (mode == "auto" and self.n_epochs <= world and rows >= 8192)):
+            return "stream"
+        return "resident"
+
+    # The method of each ingestion mode returns the epoch's steps (this rank's rows [lo, hi) of the epoch order, rows of
+    # the global batch), run_epoch(ep, losses), which enqueues them, and finish(), which ends the uploads and returns
+    # their bytes.
+    def _resident(self, X, C, eng, n, bs, rank, world):
+        order = _EpochOrder(self, n, eng.lib, True)
+        Xd, Cd = self._to_device(X, self._device), (self._to_device(C, self._device) if C is not None else None)
+        Xd, Cd = eng._check_rows(Xd, eng.D, "X"), eng._check_cond(Cd, n)
+        steps = [(*shard_bounds(b0, nb, rank, world), nb) for b0, nb in batch_bounds(n, bs)]
+        # small batches: the host side of a step (Python + ctypes, ~50 us) costs more than its two kernels (~15 us), so
+        # the whole epoch goes down in one library call (rnvp_fit_epoch: same kernels, same order, same arithmetic)
+        fused = world == 1 and bs <= 4096 and len(steps) > 1
+
+        def run_epoch(ep, losses):
+            order.next_epoch()
+            if fused:
+                eng.fit_epoch(Xd, Cd, order.device(n), n, bs, self.lr, self.weight_decay, losses)
+            else:
+                self._fit_steps(eng, Xd, Cd, order.device(0), losses, steps, world, None if order.perms is None else order.device)
+
+        return steps, run_epoch, lambda: 4 * n * ((eng.D if _on_host(X) else 0) + (eng.Cd if _on_host(C) else 0))
+
+    def _stream(self, X, C, eng, n, bs, rank, world):
+        """The rows of every step are streamed from the host (ingest.StepStreamer): the batches are the same slices of
+        the same epoch orders as in resident mode, so the trajectory is identical."""
+        from ..ingest import StepStreamer
+        order = _EpochOrder(self, n, eng.lib, False)
+        steps = [(*shard_bounds(b0, nb, rank, world), nb) for b0, nb in batch_bounds(n, bs)]
+
+        get = lambda hi: order.host(hi).numpy()            # noqa: E731
+
+        # The streamer gathers on THIS thread, so the plan generator below runs here too: seeds are drawn in epoch order exactly
+        # as in resident mode, and epoch e+1's order is requested only after the last gather of epoch e -- the prefetcher then
+        # starts shuffling epoch e+2 into the host buffer epoch e has just finished with (two buffers alternate).
+        def plan():
+            for _ in range(self.n_epochs):
+                order.next_epoch()
+                for lo, hi, _ in steps:
+                    yield get, lo, hi
+
+        streamer = StepStreamer(eng.lib, X, C, self._device, max(max(hi - lo for lo, hi, _ in steps), 1), plan())
+
+        def run_epoch(ep, losses):
+            loss_ptr = losses.data_ptr()
+            for s, (_, _, nb) in enumerate(steps):
+                Xs, Cs, m, slot = streamer.next()
+                eng.fit_step(Xs, Cs, None, m, nb, self.lr, self.weight_decay, loss_ptr + 4 * s, world=world)
+                streamer.release(slot)
+
+        return steps, run_epoch, streamer.close
+
+    def _shards(self, X, C, eng, n, bs, rank, world):
+        """``shuffle='device'`` from host arrays: rank r uploads only rows [n*r/world, n*(r+1)/world) of the (identical)
+        host arrays -- sequentially, in chunks, conversion fused (ingest.ChunkUploader) -- and shuffles that shard on the
+        device.  A global batch is the union of the ranks' local batches of batch_size/world rows; the gradient all-reduce
+        and the loss are scaled by the true global row count of the step.
 
         The FIRST epoch of the call starts training while the shard is still arriving: its row order is the
         concatenation of independent device permutations of consecutive chunks (a block-wise shuffle, as streaming data
@@ -478,94 +472,36 @@ class RealNVP(GenModel):
         as ``shuffle='device'`` on one GPU; not the reference's batch composition, like every ``'device'`` run.  The
         global torch RNG is consumed exactly as by the reference's loop (two int64 draws per epoch)."""
         from ..ingest import ChunkUploader
-        dev, n = self._device, X.shape[0]
-        lo_r, hi_r = (n * rank) // world, (n * (rank + 1)) // world
-        n_r = hi_r - lo_r
         sizes = [(n * (r + 1)) // world - (n * r) // world for r in range(world)]
-        bs_r = max(1, int(self.batch_size) // world)
-        steps = (max(sizes) + bs_r - 1) // bs_r
+        lo_r, n_r = (n * rank) // world, sizes[rank]
+        bs_r = max(1, bs // world)
+        steps = [(b0, max(b0, min(b0 + bs_r, n_r)), sum(max(0, min(bs_r, sz - b0)) for sz in sizes))
+                 for b0 in range(0, max(sizes), bs_r)]
         chunk_rows = bs_r * max(1, min(8, (4 << 20) // max(bs_r * (eng.D + eng.Cd), 1) + 1))   # whole local batches per chunk
-        up = ChunkUploader(eng.lib, X[lo_r:hi_r], None if C is None else C[lo_r:hi_r], dev, chunk_rows)
-        Xd, Cd = up.X, up.C
-        eng.zero_grads()
-        log = _LossLog(self.loss_history)
-        for ep in range(self.n_epochs):
-            seed = epoch_seed(device=dev if world > 1 else None)   # same draws on every rank; rank 0's value is broadcast
-            gen = torch.Generator(device=dev)
-            gen.manual_seed((seed + 0x9E3779B97F4A7C15 * (rank + 1)) & 0x7FFFFFFFFFFFFFFF)
-            if ep == 0:
-                perm = torch.empty(max(n_r, 1), dtype=torch.int64, device=dev)
-                for c0 in range(0, n_r, chunk_rows):
-                    m = min(chunk_rows, n_r - c0)
-                    perm[c0:c0 + m] = torch.randperm(m, device=dev, generator=gen) + c0
-            else:
-                perm = torch.randperm(n_r, device=dev, generator=gen)
-            perm_ptr = perm.data_ptr()
-            losses = torch.empty(steps, dtype=torch.float32, device=dev)
-            loss_ptr = losses.data_ptr()
-            for s in range(steps):
-                b0 = s * bs_r
-                m = max(0, min(bs_r, n_r - b0))
-                if ep == 0 and m > 0:
-                    up.wait_rows(b0 + m)                            # the current stream waits for the chunk(s) holding these rows
-                n_glob = sum(max(0, min(bs_r, sz - b0)) for sz in sizes)
-                eng.fit_step(Xd, Cd, perm_ptr + 8 * b0, m, n_glob, self.lr, self.weight_decay, loss_ptr + 4 * s, world=world)
-            log.push(losses)
-        log.flush()
-        up.close()
-        self.h2d_bytes_last_fit = 4 * n_r * (eng.D + eng.Cd)
-        self.opt._publish_state(eng)
+        up = ChunkUploader(eng.lib, X[lo_r:lo_r + n_r], None if C is None else C[lo_r:lo_r + n_r], self._device, chunk_rows)
 
-    def _fit_streamed(self, X, C, eng, perms, bounds, rank, world, device_shuffle):
-        """The fit loop with the rows of every step streamed from the host (see ``fit`` and ingest.StepStreamer): the
-        batches are the same slices of the same epoch permutations as in resident mode, so the trajectory is identical."""
-        from ..ingest import StepStreamer
-        dev, n = self._device, X.shape[0]
-        def order_provider():
-            if device_shuffle:
-                gen = torch.Generator(device=dev)
-                gen.manual_seed(epoch_seed(device=dev if world > 1 else None) & 0x7FFFFFFFFFFFFFFF)
-                host = torch.randperm(n, device=dev, generator=gen).cpu().numpy()
-                return lambda hi: host
-            if perms.streaming:
-                sp = perms.next_stream()
-                return lambda hi: sp.wait(hi).numpy()
-            host = perms.next().numpy()
-            return lambda hi: host
+        def run_epoch(ep, losses):
+            perm = _device_order(n_r, self._device, 0x9E3779B97F4A7C15 * (rank + 1), chunk_rows if ep == 0 else None)
+            # the first epoch's steps make the current stream wait for the chunk(s) holding their rows
+            self._fit_steps(eng, up.X, up.C, perm, losses, steps, world, up.wait_rows if ep == 0 else None)
 
-        # The streamer gathers on THIS thread, so the plan generator below runs here too: seeds are drawn in epoch order exactly
-        # as in resident mode, and epoch e+1's order is requested only after the last gather of epoch e -- the prefetcher then
-        # starts shuffling epoch e+2 into the host buffer epoch e has just finished with (two buffers alternate).
-        def plan():
-            for e in range(self.n_epochs):
-                get = order_provider()
-                for (b0, nb) in bounds:
-                    lo, hi = shard_bounds(b0, nb, rank, world)
-                    yield get, lo, hi
+        return steps, run_epoch, up.close
 
-        max_rows = max(shard_bounds(b0, nb, rank, world)[1] - shard_bounds(b0, nb, rank, world)[0] for b0, nb in bounds)
-        streamer = StepStreamer(eng.lib, X, C, dev, max(max_rows, 1), plan())
-        eng.zero_grads()
-        log = _LossLog(self.loss_history)
-        for e in range(self.n_epochs):
-            losses = torch.empty(len(bounds), dtype=torch.float32, device=dev)
-            loss_ptr = losses.data_ptr()
-            for s, (b0, nb) in enumerate(bounds):
-                Xs, Cs, m, slot = streamer.next()
-                eng.fit_step(Xs, Cs, None, m, nb, self.lr, self.weight_decay, loss_ptr + 4 * s, world=world)
-                streamer.release(slot)
-            log.push(losses)
-        log.flush()
-        streamer.close()
-        self.h2d_bytes_last_fit = streamer.bytes_h2d
-        self.opt._publish_state(eng)
+    def _fit_steps(self, eng, Xd, Cd, perm, losses, steps, world, wait=None):
+        """The per-step path: step s trains on the rows perm[lo:hi] of (Xd, Cd) in a global batch of n_glob rows, for
+        (lo, hi, n_glob) in ``steps``, after ``wait(hi)`` if given."""
+        perm_ptr, loss_ptr = perm.data_ptr(), losses.data_ptr()
+        for s, (lo, hi, n_glob) in enumerate(steps):
+            if wait is not None:
+                wait(hi)
+            # raw device addresses instead of tensor slices: the host side of a 32-row step is the bottleneck
+            eng.fit_step(Xd, Cd, perm_ptr + 8 * lo, hi - lo, n_glob, self.lr, self.weight_decay, loss_ptr + 4 * s,
+                         world=world)
 
     # ------------------------------------------------------------------ sample
     def _shard_of(self, n):
         """This rank's contiguous block [lo, hi) of an n-row request under an initialised process group."""
-        dist = torch.distributed
-        world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
-        rank = dist.get_rank() if world > 1 else 0
+        rank, world = process_group()
         return (n * rank) // world, (n * (rank + 1)) // world, world
 
     def sample(self, C=100, n_draws=None, seed=None, devices=None, shard=False):

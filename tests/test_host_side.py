@@ -87,6 +87,31 @@ def test_fit_rejects_bad_shapes_before_touching_the_device():
         m.fit(np.zeros(5))                          # 1-D X
 
 
+def test_no_model_module_imports_another():
+    """The models (the modules of probaforms_b200/models that define a GenModel) share code only through the private
+    modules beside them: none imports another, at module level or inside a function."""
+    import ast
+    import pathlib
+    import probaforms_b200.models as M
+    trees = {p.stem: ast.parse(p.read_text()) for p in pathlib.Path(M.__file__).parent.glob("*.py")}
+    models = {name for name, tree in trees.items() for node in ast.walk(tree)
+              if isinstance(node, ast.ClassDef) and any(getattr(b, "id", None) == "GenModel" for b in node.bases)}
+    assert {"realnvp", "cnormal", "cvae", "wgan"} <= models
+    for name in models:
+        for node in ast.walk(trees[name]):
+            if isinstance(node, ast.ImportFrom):
+                mod = node.module or ""
+                local = node.level == 1 or mod.startswith("probaforms_b200.models")
+                targets = {mod.split(".")[-1]} | ({a.name for a in node.names} if mod in ("", "probaforms_b200.models")
+                                                  else set())
+            elif isinstance(node, ast.Import):
+                local = True
+                targets = {a.name.split(".")[-1] for a in node.names if a.name.startswith("probaforms_b200.models.")}
+            else:
+                continue
+            assert not (local and targets & (models - {name})), f"models/{name}.py imports {targets & models}"
+
+
 def test_permutation_prefetcher_falls_back_to_whole_tensor_for_huge_n():
     from probaforms_b200.batching import PermutationPrefetcher
     from probaforms_b200 import _lib
